@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--hidden H]
                     [--condition rope|sorted|shuffled|rankpe|distpe] [--obs-vehicles N] [--d-embed D]
+                    [--dump-outputs DIR]
 
 BASELINE.json configs (the default is configs[1]):
     configs[2]: --condition rankpe --d-embed 16 --obs-vehicles 30 --envs 16384      (also distpe, d 4 / 8 / 16)
@@ -68,7 +69,15 @@ def parse():
     p.add_argument("--e2e-eager", action="store_true", help="host-buffer loop without CUDA graphs")
     p.add_argument("--e2e-copy-engine", action="store_true",
                    help="observation H2D by cudaMemcpyAsync instead of the fetch kernel (hrp_fetch_host)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step returned (policy outputs, observation, reward, flags of rank 0) "
+                        "as DIR/<name>.npy, to compare two builds output for output")
+    args = p.parse_args()
+    if args.impl == "ours" and args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs records the GPU path (--impl ours)")
+    return args
 
 
 def condition_of(args):
@@ -173,6 +182,27 @@ def algorithmic_bytes_per_env_step(V=51, N=15, Fout=4):
     the same minus the two per-episode constants (target_speed, delta) = 40 B; per env: action 8, time 8+8,
     episode/draw counters 16, obs 4 N Fout, reward 4, flags 2."""
     return 88 * V + 4 * N * Fout + 46
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write every array (leading axis: env) as float32 `path/<name>.npy`.  When they hold more than DUMP_LIMIT_BYTES
+    in all, the same fixed, seeded sample of env rows is kept from each, and its row indices go to env_index.npy."""
+    import numpy as np
+
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    rows = next(iter(arrays.values())).shape[0]
+    per_row = sum(a.nbytes for a in arrays.values()) // rows
+    if per_row * rows > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 128 * (len(arrays) + 1)) // (per_row + 8)   # 128: .npy header; 8: float64 index
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -404,11 +434,15 @@ def run_ours(args):
         flush.zero_()                       # evict the (L2-sized) working set between timed iterations
         ev[k][0].record()
         agent.act(obs, out=out)             # no event between the two: the env kernel is launched programmatically
-        env.step(out["action"])             # dependent on the policy's last kernel and overlaps its tail
+        stepped = env.step(out["action"])   # dependent on the policy's last kernel and overlaps its tail
         ev[k][1].record()
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:   # before the passes below step the same env and agent again
+        dump_outputs(args.dump_outputs, {**{k: v.cpu() for k, v in out.items()},
+                                         **{k: v.cpu() for k, v in zip(("obs", "reward", "terminated", "truncated"),
+                                                                       stepped)}})
     # kernels of this library launched inside the timed region: counted calls x kernels per call (a policy call is
     # 3 tcgen05 GEMM launches + heads_act, an env step is one fused kernel; profiles/r02_launches_bench.csv)
     gpu_launches = (agent.launches - calls0[0]) * KERNELS_PER_ACT + (env.launches - calls0[1]) * KERNELS_PER_ENV_STEP

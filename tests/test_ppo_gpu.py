@@ -283,7 +283,7 @@ def test_sharded_sampling_equals_single_process_sampling():
     assert whole.actor_critic.workspace_generation == g0 + 1
 
 
-def test_loads_a_checkpoint_written_by_the_reference_agent():
+def test_loads_a_checkpoint_written_by_the_reference_agent(tmp_path):
     """tests/golden/checkpoint_ref_s12_h16.pth was written by the reference's PPOAgent.save (agent.py:310-318) after
     one update; dims are inferred the way visualize.py:53-58 does.  Outputs must match the reference network's, the
     Adam state must land in the flat moment buffers."""
@@ -311,7 +311,7 @@ def test_loads_a_checkpoint_written_by_the_reference_agent():
     w1 = opt.exp_avg[n0:n0 + hidden_dim * state_dim].cpu().numpy().reshape(hidden_dim, state_dim)
     np.testing.assert_array_equal(w1, g["exp_avg_w1"])
     # and the round trip: what this agent saves, torch loads back with the reference's key names and shapes
-    out = os.path.join(os.environ.get("TMPDIR", "/tmp"), "hrp_ckpt_roundtrip.pth")
+    out = str(tmp_path / "ckpt_roundtrip.pth")
     agent.save(out)
     back = torch.load(out, map_location="cpu")
     assert list(back["model"]) == list(sd)
