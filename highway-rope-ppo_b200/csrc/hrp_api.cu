@@ -192,6 +192,11 @@ int hrp_env_create_ex(const hrp_cfg *cfg, const float *embed_table_host, int64_t
     P.normalize_reward = cfg->normalize_reward; P.offroad_terminal = cfg->offroad_terminal;
     P.real64 = (flags & HRP_ENV_REAL64) ? 1 : 0;
     P.dt64 = 1.0 / cfg->simulation_frequency;
+    // collide_pair's pre-check radius is sqrt(5^2 + 2^2) + v dt.  Above 40 m/s the speed only decays (the clip of
+    // Vehicle.clip_actions), so |v| <= 40 + 10 dt (10 m/s^2: the largest acceleration, the ego's continuous action);
+    // 1e-2 m covers the fp32 working copies of x.  8.8 m is the window of 15 Hz and above.  The bound holds for the
+    // speeds a simulation reaches; a state injected with |speed| > 40 + 10 dt (hrp_env_set_state) can miss a pair.
+    P.coll_window = fmax(8.8, sqrt(29.0) + (40.0 + 10.0 * P.dt64) * P.dt64 + 1e-2);
     P.dtime = 1.0 / cfg->policy_frequency; P.duration = cfg->duration;
     P.collision_reward = cfg->collision_reward; P.right_lane_reward = cfg->right_lane_reward;
     P.high_speed_reward = cfg->high_speed_reward;

@@ -286,9 +286,10 @@ template <typename R> __device__ void rank_full(WarpS<R> &S, int V, int lane)
 }
 template <typename R> __device__ void rank_repair(WarpS<R> &S, int V, int lane)
 {
-    // pre-check on the ego-relative working copies: an inversion (true gap <= 0) shows up as a working-copy gap
-    // below the margin (fp32, |xr| < 4096 m: two roundings <= 5e-4 m), so "every gap >= 4e-3" proves the order
-    // without fp64 loads
+    // pre-check on the ego-relative working copies: xr = (R)(x - xref) is recomputed from the fp64 x every frame, and
+    // the subtraction of a common xref and the rounding to R are both monotone, so an inversion (true gap <= 0) shows
+    // up as a working-copy gap <= 0 at any distance from the ego: "every gap >= 4e-3" proves the order without fp64
+    // loads
     {
         bool sus = false;
 #pragma unroll
@@ -640,6 +641,7 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
 {
     const int V = P.V;
     const R dt = (R)P.dt64;
+    const R window = (R)P.coll_window;
     const bool ego_ctrl = P.ego_mode == 1;
     const R kPi = R(kPiD);
 
@@ -822,7 +824,7 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
             b[q] = 0;
             if (cand[q]) {
                 b[q] = S.order[s2];
-                cand[q] = S.rec[b[q]].xr - xa[q] <= R(8.8);  // >= sqrt(29) + max speed * dt
+                cand[q] = S.rec[b[q]].xr - xa[q] <= window;  // >= sqrt(29) + max speed * dt
             }
         }
         if (!__any_sync(HRP_FULL, cand[0] || cand[1])) break;

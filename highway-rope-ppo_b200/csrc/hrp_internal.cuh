@@ -20,6 +20,7 @@ struct EnvDev {
     int ego_mode, autoreset, normalize_reward, offroad_terminal;
     int real64;      // 0: product arithmetic (fp32 + fp64 x / timer); 1: fp64 validation instantiation (fp64 state arrays)
     double dt64;     // 1/simulation_frequency (IDM timer is advanced in fp64, SURVEY A.6)
+    double coll_window;  // rank-order x gap beyond which no pair can pass collide_pair's pre-check (hrp_env_create_ex)
     double dtime;    // 1/policy_frequency
     double duration;
     double collision_reward, right_lane_reward, high_speed_reward, rs_lo, rs_hi;

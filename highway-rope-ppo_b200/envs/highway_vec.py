@@ -176,6 +176,10 @@ class HighwayVecEnv:
         # handed to a new one, a counter cannot
         HighwayVecEnv._next_uid += 1
         self.uid = HighwayVecEnv._next_uid
+        # a launch passes the handle's parameters (seed, per-env seeds, step mask, trace) by value, so a captured launch
+        # keeps the ones of its capture: every change of them bumps this version, and caches of captured launches
+        # compare it
+        self.param_version = 0
 
     # ------------------------------------------------------------------ lifetime
     def close(self) -> None:
@@ -201,7 +205,7 @@ class HighwayVecEnv:
               out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """``env.reset(seed=...)`` for every env (or those with a non-zero ``mask`` byte)."""
         if seed is not None:
-            self.seed = int(seed)
+            self._set_seed(seed)
         obs = self.obs if out is None else out
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
@@ -286,16 +290,22 @@ class HighwayVecEnv:
         self.launches += 1
 
     def reset_host(self, seed: int, obs: np.ndarray) -> None:
-        self.seed = int(seed)
+        self._set_seed(seed)
         _lib.check(self._lib.hrp_env_reset_host(self._h, self.seed & 0xFFFFFFFFFFFFFFFF, obs.ctypes.data),
                    "hrp_env_reset_host")
         self.launches += 1
+
+    def _set_seed(self, seed: int) -> None:
+        if int(seed) != self.seed:
+            self.seed = int(seed)
+            self.param_version += 1
 
     # ------------------------------------------------------------------ multiplexed experiments
     def set_env_seeds(self, seeds: Optional[torch.Tensor]) -> None:
         """Per-env seeds (int64 / uint64 CUDA tensor [E], kept alive by this object): env e then behaves exactly like
         the single-env handle of an experiment that called ``reset(seed=seeds[e])``.  ``None`` switches back to
         (handle seed, global env id)."""
+        self.param_version += 1
         if seeds is None:
             _lib.check(self._lib.hrp_env_set_seeds(self._h, None), "hrp_env_set_seeds")
             self._seeds = None
@@ -308,6 +318,7 @@ class HighwayVecEnv:
     def set_step_mask(self, mask: Optional[torch.Tensor]) -> None:
         """uint8 CUDA tensor [E] (kept alive by this object; rewrite its contents between steps): ``step`` leaves env e
         untouched unless ``mask[e]``.  ``None``: every env steps."""
+        self.param_version += 1
         if mask is None:
             _lib.check(self._lib.hrp_env_set_step_mask(self._h, None), "hrp_env_set_step_mask")
             self._step_mask = None
@@ -321,6 +332,7 @@ class HighwayVecEnv:
     def enable_trace(self, on: bool = True) -> Optional[torch.Tensor]:
         """Record every vehicle's state at the end of every simulation frame of the following steps (parity tests):
         returns the float64 tensor [E, frames, V, 7] the kernel writes (x, y, speed, heading, impact_x, impact_y, flags)."""
+        self.param_version += 1
         if not on:
             _lib.check(self._lib.hrp_env_set_trace(self._h, None), "hrp_env_set_trace")
             self._trace = None

@@ -47,7 +47,7 @@ class HostBufferPipeline:
                  "out": {"action": torch.empty((Eg, A), device=dev), "pre_tanh": torch.empty((Eg, A), device=dev),
                          "log_prob": torch.empty(Eg, device=dev), "value": torch.empty(Eg, device=dev)},
                  "draw": agent.actor_critic.new_draw_counter(), "draw0": agent.actor_critic._draw, "steps": 0,
-                 "graph": None, "lane": 1 + gi * self.chunks,
+                 "graph": None, "version": None, "lane": 1 + gi * self.chunks,
                  # chunked only when the chunks are whole and 16-byte aligned (hrp_fetch_host)
                  "C": self.chunks if Eg % self.chunks == 0 and (Eg // self.chunks * S * 4) % 16 == 0 else 1,
                  "draws": [agent.actor_critic.new_draw_counter() for _ in range(self.chunks)],
@@ -121,13 +121,14 @@ class HostBufferPipeline:
         try:
             if not self.use_graphs:
                 self._enqueue(g)
-            elif g["graph"] is None:
+            elif g["graph"] is None or g["version"] != g["env"].param_version:
+                # a captured env step keeps the seed / masks of its capture: capture again after they changed
                 self._enqueue(g)          # eager first: warms every kernel variant and the workspace lane
                 g["stream"].synchronize()
                 graph = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(graph, stream=g["stream"]):
                     self._enqueue(g)
-                g["graph"] = graph
+                g["graph"], g["version"] = graph, g["env"].param_version
             else:
                 g["graph"].replay()
             g["done"].record(g["stream"])

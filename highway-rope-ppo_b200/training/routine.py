@@ -215,7 +215,8 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
         # (a single env acts through the matrix-vector kernel, which keeps its draw counter on the host)
         use_graph = noise is None and E > 1 and getattr(agent, "use_cuda_graphs", True)
     cache = getattr(agent, "_rollout_graph", None)
-    key = (getattr(vec_env, "uid", id(vec_env)), T, E, S, A, ac.workspace_generation, ac.row_base)
+    key = (getattr(vec_env, "uid", id(vec_env)), getattr(vec_env, "param_version", 0), T, E, S, A,
+           ac.workspace_generation, ac.row_base)
     if use_graph and cache is not None and cache["key"] == key and agent.memory.rollout is None:
         agent.memory.rollout = cache["r"]     # the buffers the captured launches write (PPOAgent.update dropped them)
     r = agent.memory.begin_rollout(T, E, S, A)

@@ -151,6 +151,78 @@ def test_sweep_expansion():
     assert {(h.lr, h.hidden_dim) for h in out} == {(a, b) for a in (1e-4, 3e-4) for b in (256, 384, 512)}
 
 
+_F8 = ["presence", "x", "y", "vx", "vy", "heading", "cos_h", "sin_h"]
+# (case, config overrides, embedding (kind, d, use_euclidean, ego_idx) or None, accepted, what the error names)
+_CFG_EDGES = [
+    ("vehicles 63", dict(vehicles_count=63), None, True, None),
+    ("vehicles 64", dict(vehicles_count=64), None, False, "vehicles_count"),
+    ("lanes 1", dict(lanes_count=1), None, True, None),
+    ("lanes 0", dict(lanes_count=0), None, False, "lanes_count"),
+    ("lanes 8", dict(lanes_count=8), None, True, None),
+    ("lanes 9", dict(lanes_count=9), None, False, "lanes_count"),
+    ("rows 64", dict(observation=dict(vehicles_count=64)), None, True, None),
+    ("rows 65", dict(observation=dict(vehicles_count=65)), None, False, "observation vehicles_count"),
+    ("features 8", dict(observation=dict(features=_F8)), None, True, None),
+    ("features 9", dict(observation=dict(features=_F8)), None, False, "feature count"),   # obs_nfeat forced to 9
+    ("sim = policy", dict(simulation_frequency=3, policy_frequency=3), None, True, None),
+    ("sim < policy", dict(simulation_frequency=2, policy_frequency=3), None, False, "frequency"),
+    ("rope d = F", {}, ("rope", 4, True, 0), True, None),
+    ("rope d = F + 2", {}, ("rope", 6, True, 0), False, "rotate_dim"),
+    ("rope d odd", {}, ("rope", 3, True, 0), False, "rotate_dim"),
+    ("rope F = 1", dict(observation=dict(features=["presence"])), ("rope", 0, True, 0), False, "RoPE needs"),
+    ("dist d 64", {}, ("dist", 64, True, 0), True, None),
+    ("dist d 66", {}, ("dist", 66, True, 0), False, "DistPE d_embed"),
+    ("dist d odd", {}, ("dist", 7, True, 0), False, "DistPE d_embed"),
+    ("dist F = 1 |dx|", dict(observation=dict(features=["x"])), ("dist", 4, False, 0), True, None),
+    ("dist F = 1 euclid", dict(observation=dict(features=["x"])), ("dist", 4, True, 0), False, "DistPE needs"),
+    ("rank d 1", {}, ("rank", 1, True, 0), True, None),
+    ("rank d 64", {}, ("rank", 64, True, 0), True, None),
+    ("rank d 65", {}, ("rank", 65, True, 0), False, "RankPE d_embed"),
+    ("ego_idx N-1", {}, ("rope", 4, True, 14), True, None),
+    ("ego_idx N", {}, ("rope", 4, True, 15), False, "ego_idx"),
+]
+
+
+@pytest.mark.parametrize("case,over,emb,accepted,field", _CFG_EDGES, ids=[c[0] for c in _CFG_EDGES])
+def test_env_config_limits(highway_config, case, over, emb, accepted, field):
+    """Both sides of every limit hrp_env_create_ex checks.  The configuration is validated before the device is looked
+    at: without a GPU an accepted configuration gets -3 (no CUDA device), a rejected one -1 and a message naming the
+    field; with a GPU an accepted configuration creates a handle."""
+    from highway_rope_ppo_b200 import _lib
+    from highway_rope_ppo_b200.envs.highway_vec import EmbedSpec, build_cfg
+
+    lib = _lib.load()
+    cfg = copy.deepcopy(highway_config)
+    for k, v in over.items():
+        if isinstance(v, dict):
+            cfg[k].update(v)
+        else:
+            cfg[k] = v
+    spec = None
+    if emb is not None:
+        kind, d, eu, ego = emb
+        kind = {"rope": _lib.EMBED_ROPE, "dist": _lib.EMBED_DIST, "rank": _lib.EMBED_RANK}[kind]
+        spec = EmbedSpec(kind, d, use_euclidean=eu, ego_idx=ego)
+    c = build_cfg(cfg, spec)
+    if case == "features 9":
+        with pytest.raises(ValueError):
+            build_cfg(dict(cfg, observation=dict(cfg["observation"], features=_F8 + ["x"])))
+        c.obs_nfeat = 9
+    n = 0
+    if emb is not None:   # the table length each kind expects, so that only the field under test can be wrong
+        n = c.obs_vehicles * d if emb[0] == "rank" else d // 2
+    table = np.zeros(max(n, 1), dtype=np.float32)
+    h = C.c_void_p()
+    rc = lib.hrp_env_create_ex(C.byref(c), table.ctypes.data if emb is not None else None, n, 4, 0, 0, 0, C.byref(h))
+    if accepted:
+        has_device = lib.hrp_device_count() > 0
+        assert rc == (0 if has_device else -3), (rc, _lib.last_error())
+        if rc == 0:
+            assert lib.hrp_env_destroy(h) == 0
+    else:
+        assert rc == -1 and field in _lib.last_error(), (rc, _lib.last_error())
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-device behaviour")
 def test_no_cpu_fallback(highway_config):
     from highway_rope_ppo_b200 import _lib

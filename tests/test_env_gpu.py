@@ -96,11 +96,14 @@ def test_reset_matches_oracle(highway_config, seed, base, real64):
     env.close()
 
 
-def _injected_parity(cfg, E, steps, seed, action_fn, sorted_obs=True, obs_tol=2e-5, real64=False):
+def _injected_parity(cfg, E, steps, seed, action_fn, sorted_obs=True, obs_tol=2e-5, real64=False, embed=None):
     """State-injection parity.  Returns a dict: agree / flipped / neither env-step counts, the kinds of the decisions
-    that had to be flipped, the worst continuous errors of the agreeing steps and the first few failures."""
+    that had to be flipped, the worst continuous errors of the agreeing steps and the first few failures.  With an
+    EmbedSpec `embed`, a second handle with that fused embedding is injected and stepped alongside: "embedded" lists
+    (plain observation, fused observation) per step."""
     N = cfg["observation"]["vehicles_count"]
     env = _vec(cfg, E, autoreset=False, real64=real64)
+    fused = None if embed is None else _vec(cfg, E, autoreset=False, real64=real64, embed=embed)
     ktrace = env.enable_trace()   # per-frame snapshots, for the frame-by-frame search
     oracles = [oh.OracleEnv(cfg) for _ in range(E)]
     for e, o in enumerate(oracles):
@@ -109,7 +112,8 @@ def _injected_parity(cfg, E, steps, seed, action_fn, sorted_obs=True, obs_tol=2e
     rows = torch.zeros((E, N), dtype=torch.int32, device="cuda:0")
     tol, rew_tol = (TOL64, 1e-6) if real64 else (TOL, 2e-5)
     obs_tol = 1e-6 if real64 else obs_tol
-    stats = {"agree": 0, "flipped": 0, "neither": 0, "kinds": Counter(), "worst": {}, "failures": [], "by_frames": 0}
+    stats = {"agree": 0, "flipped": 0, "neither": 0, "kinds": Counter(), "worst": {}, "failures": [], "by_frames": 0,
+             "embedded": []}
     for t in range(steps):
         sts = [o.get_state() for o in oracles]
         st = {k: np.stack([s[k] for s in sts]) for k in oh.STATE_F64 + oh.STATE_I32}
@@ -124,6 +128,10 @@ def _injected_parity(cfg, E, steps, seed, action_fn, sorted_obs=True, obs_tol=2e
                                          row_vehicle=rows)
         state = env.get_state()
         obs, rew, term, trunc, rv = (x.cpu().numpy() for x in (obs, rew, term, trunc, rows))
+        if fused is not None:
+            fused.set_state(st)
+            fo = fused.step(torch.from_numpy(actions).cuda(), perm=None if perm is None else torch.from_numpy(perm).cuda())[0]
+            stats["embedded"].append((obs, fo.cpu().numpy()))
         trace_host = None
         for e, o in enumerate(oracles):
             got = _Got(state, e, obs, rew, term, trunc, rv)
@@ -155,6 +163,8 @@ def _injected_parity(cfg, E, steps, seed, action_fn, sorted_obs=True, obs_tol=2e
             if te or tr:  # reference loop: reset right after done
                 o.reset(seed, env_id=e, episode=1 + t)
     env.close()
+    if fused is not None:
+        fused.close()
     return stats
 
 
