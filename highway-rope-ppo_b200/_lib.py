@@ -21,6 +21,7 @@ HRP_MAX_EMBED = 64
 
 FEATURE_CODES = {"presence": 0, "x": 1, "y": 2, "vx": 3, "vy": 4, "heading": 5, "cos_h": 6, "sin_h": 7}
 EMBED_NONE, EMBED_ROPE, EMBED_DIST, EMBED_RANK = 0, 1, 2, 3
+PPO_CATEGORICAL = 1   # HRP_PPO_CATEGORICAL
 
 
 class HrpError(RuntimeError):
@@ -96,10 +97,12 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_philox4x32_10": (C.c_int, [_vp, _vp, _vp]),
     "hrp_embed_apply": (C.c_int, [_i32, _i32, _i32, _i32, _f32, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp]),
     "hrp_ppo_param_count": (_i64, [_i32, _i32, _i32]),
+    "hrp_ppo_param_count_ex": (_i64, [_i32, _i32, _i32, C.c_uint32]),
     "hrp_ppo_set_math": (C.c_int, [_i32]),
     "hrp_ppo_get_math": (C.c_int, []),
     "hrp_gemm_strided": (C.c_int, [_i32, _i32, _i32, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _i32, _vp, _i32, _i32, _vp]),
     "hrp_ppo_create": (C.c_int, [_i32, _i32, _i32, _i64, _i32, C.POINTER(_vp)]),
+    "hrp_ppo_create_ex": (C.c_int, [_i32, _i32, _i32, _i64, _i32, C.c_uint32, C.POINTER(_vp)]),
     "hrp_ppo_destroy": (C.c_int, [_vp]),
     "hrp_ppo_hold_weights": (C.c_int, [_vp, _i32]),
     "hrp_ppo_forward": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp]),

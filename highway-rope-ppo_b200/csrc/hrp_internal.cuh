@@ -109,8 +109,8 @@ inline cudaError_t hrp_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 bloc
 struct TcDots {
     const float *wa;   // actor head weights [A][H]   (columns [0, H) of the output)
     const float *wc;   // critic head weights [H]     (columns [H, 2 H))
-    int H, A;
-    float *out;        // [N / BN tiles][M][4] partial sums
+    int H, A;          // A: head rows, 1..8
+    float *out;        // [N / BN tiles][M][A <= 4 ? 4 : 8] partial sums
     int skip_store;    // do not write the activation itself
 };
 

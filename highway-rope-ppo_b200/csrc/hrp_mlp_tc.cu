@@ -293,10 +293,11 @@ __host__ __device__ constexpr int tc_stages()
 // Optional fused consumer (TcDots, hrp_ppo.cu's act path): the output is [a1 | c1], the hidden activations of the two
 // heads, and all the policy needs of it are A + 1 dot products per row -- mean_a = a1 . Wa2[a], value = c1 . Wc2.  A tile
 // lies entirely in a1 or in c1 (H % BN == 0, checked by the host); every thread multiplies its four columns of a row
-// by the head weights it keeps in registers, the CQ threads of the row add up by shuffles, and the tile leaves four
-// partial sums per row in out[tile][row][4]; a tiny kernel adds the tiles (heads_finish_kernel).  With skip_store the
-// activation itself is never written.
-template <int BN, bool DUAL>
+// by the head weights it keeps in registers, the CQ threads of the row add up by shuffles, and the tile leaves NP
+// partial sums per row in out[tile][row][NP]; a tiny kernel adds the tiles (heads_finish_kernel, NP = 4 for the
+// Gaussian head; heads_finish_cat_kernel, NP = 4 or 8 for the categorical one).  With skip_store the activation itself
+// is never written.
+template <int BN, bool DUAL, int NP>
 __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p, uint32_t tmem_d, int nkb, int M, int N,
                                             int m0, int n0, int bn0, float *__restrict__ C, int ldc,
                                             const float *__restrict__ biasp, int relu, const float *__restrict__ mask,
@@ -365,12 +366,12 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
         float *crow = Cz + (size_t)(m0 + tid / CQ) * ldc + gn;
         const float *mrow = mask ? mask + (size_t)(m0 + tid / CQ) * ldm + gn : nullptr;
         const float *srow = stage_c + (tid / CQ) * LDS + 4 * cq;
-        float4 hwv[4];
+        float4 hwv[NP];
         if (dots.out) {
             const bool actor = n0 < dots.H;
             const int nd = actor ? dots.A : 1;
 #pragma unroll
-            for (int a = 0; a < 4; ++a) {
+            for (int a = 0; a < NP; ++a) {
                 const float *w = actor ? dots.wa + (size_t)a * dots.H + gn : dots.wc + (gn - dots.H);
                 hwv[a] = a < nd ? make_float4(w[0], w[1], w[2], w[3]) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
@@ -392,15 +393,18 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
                 x.x = mk[j].x > 0.f ? x.x : 0.f; x.y = mk[j].y > 0.f ? x.y : 0.f;
                 x.z = mk[j].z > 0.f ? x.z : 0.f; x.w = mk[j].w > 0.f ? x.w : 0.f;
                 if (dots.out) {
-                    float d[4];
+                    float d[NP];
 #pragma unroll
-                    for (int a = 0; a < 4; ++a) {
+                    for (int a = 0; a < NP; ++a) {
                         d[a] = fmaf(x.w, hwv[a].w, fmaf(x.z, hwv[a].z, fmaf(x.y, hwv[a].y, x.x * hwv[a].x)));
 #pragma unroll
                         for (int off = CQ / 2; off > 0; off >>= 1) d[a] += __shfl_xor_sync(0xffffffffu, d[a], off);
                     }
-                    if (cq == 0 && m0 + rb + j * RSTEP < M)
-                        *(float4 *)(dots.out + ((size_t)blockIdx.x * M + (m0 + rb + j * RSTEP)) * 4) = make_float4(d[0], d[1], d[2], d[3]);
+                    if (cq == 0 && m0 + rb + j * RSTEP < M) {
+                        float *o = dots.out + ((size_t)blockIdx.x * M + (m0 + rb + j * RSTEP)) * NP;
+#pragma unroll
+                        for (int q = 0; q < NP; q += 4) *(float4 *)(o + q) = make_float4(d[q], d[q + 1], d[q + 2], d[q + 3]);
+                    }
                 }
                 if (m0 + rb + j * RSTEP < M && !dots.skip_store) {
                     *(float4 *)(crow + (size_t)j * RSTEP * ldc) = x;
@@ -452,7 +456,7 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
     if (tid == 0) TC_PHASE(7);   // tile written
 }
 
-template <int AMODE, int BMODE, int NSPLIT, int BN, bool ASYNC>
+template <int AMODE, int BMODE, int NSPLIT, int BN, bool ASYNC, int NP>
 __global__ void __launch_bounds__(TC_LAUNCH_THREADS)
 tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, long long sak,
                const float *__restrict__ B, long long sbn, long long sbk, float *__restrict__ C, int ldc,
@@ -660,7 +664,7 @@ tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, 
         }
     }
 
-    tc_epilogue<BN, NSPLIT == 3>(smem, &bar_done, tmem_d, nkb, M, N, m0, n0, bn0, C, ldc, biasp, relu, mask, ldm, accumulate, C_lo, dots);
+    tc_epilogue<BN, NSPLIT == 3, NP>(smem, &bar_done, tmem_d, nkb, M, N, m0, n0, bn0, C, ldc, biasp, relu, mask, ldm, accumulate, C_lo, dots);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0)
@@ -676,7 +680,8 @@ tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, 
 // tensor pipe (~88 cycles per 128 x 64 x 8 instruction) while a stash takes ~580 and the stage hand-over ~430, i.e.
 // the main loop is paced by the UMMA stream itself, whichever memory the A operand comes from.
 
-template <int AMODE, int BMODE, int NSPLIT, int BN, bool ASYNC = false>
+// NP: partial sums per row of the fused row-dot epilogue (TcDots): 4, or 8 for a categorical head of more than four logits
+template <int AMODE, int BMODE, int NSPLIT, int BN, bool ASYNC = false, int NP = 4>
 int launch(dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam, long long sak,
            const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias, int relu,
            const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2, const float *bias2, float *C_lo,
@@ -689,7 +694,7 @@ int launch(dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long 
     constexpr int SMEM = (OPERANDS > EPILOGUE ? OPERANDS : EPILOGUE) + 1024;
     // the attribute is per device (a process may drive several GPUs)
     static bool configured[HRP_MAX_DEVICES] = {false};
-    auto kern = tc_gemm_kernel<AMODE, BMODE, NSPLIT, BN, ASYNC>;
+    auto kern = tc_gemm_kernel<AMODE, BMODE, NSPLIT, BN, ASYNC, NP>;
     int dev = 0;
     HRP_CUDA_OK(cudaGetDevice(&dev));
     if (dev < 0 || dev >= HRP_MAX_DEVICES) { hrp_set_error("device index %d not supported", dev); return -1; }
@@ -702,20 +707,23 @@ int launch(dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long 
     return 0;
 }
 
-template <int AMODE, int BMODE>
+template <int AMODE, int BMODE, int NP = 4>
 int dispatch(int bn, int nsplit, dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam,
              long long sak, const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias,
              int relu, const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2,
              const float *bias2, float *C_lo, const TcDots &dots)
 {
 #define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots
-    if (bn == 32 && nsplit == 3) return launch<AMODE, BMODE, 3, 32>(HRP_TC_ARGS);
-    if (bn <= 64) return nsplit == 3 ? launch<AMODE, BMODE, 3, 64>(HRP_TC_ARGS) : launch<AMODE, BMODE, 1, 64>(HRP_TC_ARGS);
-    return nsplit == 3 ? launch<AMODE, BMODE, 3, 128>(HRP_TC_ARGS) : launch<AMODE, BMODE, 1, 128>(HRP_TC_ARGS);
+    if constexpr (NP == 4)   // (never with the fused epilogue, the only user of NP = 8)
+        if (bn == 32 && nsplit == 3) return launch<AMODE, BMODE, 3, 32>(HRP_TC_ARGS);
+    if (bn <= 64)
+        return nsplit == 3 ? launch<AMODE, BMODE, 3, 64, false, NP>(HRP_TC_ARGS) : launch<AMODE, BMODE, 1, 64, false, NP>(HRP_TC_ARGS);
+    return nsplit == 3 ? launch<AMODE, BMODE, 3, 128, false, NP>(HRP_TC_ARGS) : launch<AMODE, BMODE, 1, 128, false, NP>(HRP_TC_ARGS);
 #undef HRP_TC_ARGS
 }
 
 // forward-pass operands (activations x weights, both K-contiguous and aligned): cp.async staging
+template <int NP = 4>
 int dispatch_async(int bn, int nsplit, dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam,
                    long long sak, const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias,
                    int relu, const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2,
@@ -723,8 +731,8 @@ int dispatch_async(int bn, int nsplit, dim3 grid, cudaStream_t s, int M, int N, 
 {
 #define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots
     if (bn == 64)
-        return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 64, true>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 64, true>(HRP_TC_ARGS);
-    return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 128, true>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 128, true>(HRP_TC_ARGS);
+        return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 64, true, NP>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 64, true, NP>(HRP_TC_ARGS);
+    return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 128, true, NP>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 128, true, NP>(HRP_TC_ARGS);
 #undef HRP_TC_ARGS
 }
 
@@ -770,8 +778,10 @@ int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sa
     if (narrow && bn32 && bn == 64 && nsplit == 3 && N % 32 == 0 && N >= 64 && mt * ((N + 63) / 64) * splits <= 148 && !dots.out)
         bn = 32;
     dim3 grid((N + bn - 1) / bn, mt, splits);
-    if (dots.out && (splits != 1 || dots.H % bn != 0 || N % bn != 0 || ldc % 4 != 0 || !aligned(C, 16) || mask || C_lo)) {
-        hrp_set_error("hrp_tc_gemm: the fused row-dot epilogue needs whole, aligned tiles that do not straddle H");
+    if (dots.out && (splits != 1 || dots.H % bn != 0 || N % bn != 0 || ldc % 4 != 0 || !aligned(C, 16) || mask || C_lo ||
+                     dots.A < 1 || dots.A > 8)) {
+        hrp_set_error("hrp_tc_gemm: the fused row-dot epilogue needs whole, aligned tiles that do not straddle H, and 1..8 "
+                      "head rows");
         return -1;
     }
     const bool akc = sak == 1, bkc = sbk == 1;
@@ -781,6 +791,24 @@ int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sa
     const bool b_k4 = bkc && K % 4 == 0 && sbn % 4 == 0 && aligned(B, 16) && (nseg == 0 || aligned(B2, 16));
 #define HRP_TC_GO(am, bm) dispatch<am, bm>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots)
     int rc;
+    if (dots.out && dots.A > 4) {
+        // a categorical head of more than four logits: eight partial sums per row.  Only the operand layouts of the act
+        // path are instantiated (K-contiguous activations and weights), chosen by the rule below; the alignment of
+        // critic.0 in the flat buffer follows n (offset = n mod 4 floats past a 16-byte boundary)
+#define HRP_TC_GO8(am, bm) dispatch<am, bm, 8>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots)
+        if (a_k4 && b_k2 && nsplit == 1)
+            rc = dispatch_async<8>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate,
+                                   k_chunk, nseg, B2, bias2, C_lo, dots);
+        else if (a_k4 && b_k4) rc = HRP_TC_GO8(ST_K4, ST_K4);
+        else if (a_k4 && b_k2) rc = HRP_TC_GO8(ST_K4, ST_K2);
+        else if (akc && bkc) rc = HRP_TC_GO8(ST_K1, ST_K1);
+        else {
+            hrp_set_error("hrp_tc_gemm: the eight-wide fused row-dot epilogue needs K-contiguous operands");
+            return -1;
+        }
+#undef HRP_TC_GO8
+        return rc < 0 ? rc : splits;
+    }
     // cp.async staging pays off for the single-pass mode only (measured: 3xTF32 hidden forward 12.6 us register-staged
     // vs 14.5 us cp.async -- the lo tiles need a second pass through shared memory; TF32 H=512 19.6 -> 16.6 us)
     if (a_k4 && b_k2 && nsplit == 1) rc = dispatch_async(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots);

@@ -11,7 +11,8 @@
 // shared.2.{weight[H,H],bias[H]}, actor_mean.0.{weight[H,H],bias[H]},
 // actor_mean.2.{weight[A,H],bias[A]}, critic.0.{weight[H,H],bias[H]}, critic.2.{weight[1,H],bias[1]}.
 // Gradients, Adam moments use the same layout, so the optimizer (and the multi-GPU
-// all-reduce) touch one contiguous range.
+// all-reduce) touch one contiguous range.  The categorical policy (HRP_PPO_CATEGORICAL) has the same layout without
+// log_std, A = n logits in actor_mean.2.
 #include <cooperative_groups.h>
 #include <math.h>
 #include <stdlib.h>
@@ -24,12 +25,12 @@ struct Layout {
     int S, A, H;
     long long log_std, w1, b1, w2, b2, wa1, ba1, wa2, ba2, wc1, bc1, wc2, bc2, total;
 };
-__host__ __device__ inline Layout make_layout(int S, int A, int H)
+__host__ __device__ inline Layout make_layout(int S, int A, int H, bool categorical = false)
 {
     Layout L;
     L.S = S; L.A = A; L.H = H;
     long long o = 0;
-    L.log_std = o; o += A;
+    L.log_std = o; o += categorical ? 0 : A;
     L.w1 = o; o += (long long)H * S; L.b1 = o; o += H;
     L.w2 = o; o += (long long)H * H; L.b2 = o; o += H;
     L.wa1 = o; o += (long long)H * H; L.ba1 = o; o += H;
@@ -214,17 +215,18 @@ colsum_partial_kernel(const float *__restrict__ G, int ldg, long long B, int N, 
 
 // head weight/bias gradients, stage 1 (agent.py actor_mean.2 / critic.2): for a chunk of rows,
 //   dWa2[a,h] = sum_b dmean[b,a] a1[b,h], dba2[a] = sum_b dmean[b,a], dWc2[h] = sum_b dvalue[b] c1[b,h], dbc2 = sum_b dvalue[b]
-// part[y] holds [A*H | A | H | 1] floats.
+// part[y] holds [A*H | A | H | 1] floats.  A <= MAXA: 4 (the Gaussian head), or 8 (categorical heads of up to 8 logits).
+template <int MAXA>
 __global__ void __launch_bounds__(256)
 heads_wgrad_partial_kernel(const float *__restrict__ dmean, const float *__restrict__ dvalue,
                            const float *__restrict__ a1, const float *__restrict__ c1, int ld, long long B, int H, int A,
                            int rows_per, float *__restrict__ part)
 {
-    __shared__ float red[8][6][33];
+    __shared__ float red[8][MAXA + 2][33];
     const int l = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int h = blockIdx.x * 32 + l;
     const long long r0 = (long long)blockIdx.y * rows_per, r1 = min(B, r0 + rows_per);
-    float acc[4] = {0.f, 0.f, 0.f, 0.f}, accc = 0.f, accb = 0.f;
+    float acc[MAXA] = {}, accc = 0.f, accb = 0.f;
     for (long long b = r0 + w; b < r1; b += 8) {
         float dv = dvalue[b];
         if (h < H) {
@@ -234,24 +236,24 @@ heads_wgrad_partial_kernel(const float *__restrict__ dmean, const float *__restr
         }
         if (blockIdx.x == 0 && l <= A) accb += l < A ? dmean[b * A + l] : dv;
     }
-    for (int a = 0; a < 4; ++a) red[w][a][l] = acc[a];
-    red[w][4][l] = accc;
-    red[w][5][l] = accb;
+    for (int a = 0; a < MAXA; ++a) red[w][a][l] = acc[a];
+    red[w][MAXA][l] = accc;
+    red[w][MAXA + 1][l] = accb;
     __syncthreads();
     if (w == 0) {
         float *out = part + (size_t)blockIdx.y * ((size_t)A * H + A + H + 1);
-        float t[6];
-        for (int q = 0; q < 6; ++q) {
+        float t[MAXA + 2];
+        for (int q = 0; q < MAXA + 2; ++q) {
             t[q] = 0.f;
             for (int i = 0; i < 8; ++i) t[q] += red[i][q][l];
         }
         if (h < H) {
             for (int a = 0; a < A; ++a) out[(size_t)a * H + h] = t[a];
-            out[(size_t)A * H + A + h] = t[4];
+            out[(size_t)A * H + A + h] = t[MAXA];
         }
         if (blockIdx.x == 0 && l <= A) {
-            if (l < A) out[(size_t)A * H + l] = t[5];
-            else out[(size_t)A * H + A + H] = t[5];
+            if (l < A) out[(size_t)A * H + l] = t[MAXA + 1];
+            else out[(size_t)A * H + A + H] = t[MAXA + 1];
         }
     }
 }
@@ -647,6 +649,384 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// Categorical policy (HRP_PPO_CATEGORICAL): softmax over the n <= CAT_MAX logits of actor_mean.2, same trunk, critic and
+// loss formula as the Gaussian head.  The sample conditions the loss through pre_tanh[b] = id.
+constexpr int CAT_MAX = 8;
+
+// Softmax, draw and log-prob of one row from its n logits (biases added).  One uniform per row: Philox4x32-10 with the
+// Gaussian path's counter (row_base + b, draw) and key, u = ((r0 >> 8) + 0.5) / 2^24 (or noise[b] for mode 1); the id
+// is the first j with u < sum_{i <= j} p_i, the sum formed in index order in fp32, and n - 1 if there is none.
+// Deterministic mode takes the first maximum (torch.argmax) and reports log-prob 0, as the Gaussian path does.
+__device__ __forceinline__ void cat_sample_row(const float (&lg)[CAT_MAX], int n, int mode, const float *__restrict__ noise,
+                                               unsigned long long seed, unsigned long long draw, unsigned long long row_base,
+                                               long long b, int &id, float &lp)
+{
+    float m = lg[0];
+    int amax = 0;
+#pragma unroll
+    for (int j = 1; j < CAT_MAX; ++j)
+        if (j < n && lg[j] > m) { m = lg[j]; amax = j; }
+    float e[CAT_MAX], s = 0.f;
+#pragma unroll
+    for (int j = 0; j < CAT_MAX; ++j) {
+        e[j] = j < n ? expf(lg[j] - m) : 0.f;
+        s += e[j];
+    }
+    if (mode == 0) {
+        id = amax;
+        lp = 0.f;
+        return;
+    }
+    float u;
+    if (mode == 2) {
+        uint32_t r[4];
+        const unsigned long long gb = row_base + (unsigned long long)b;
+        hrp_philox((uint32_t)gb, (uint32_t)(gb >> 32), (uint32_t)draw, (uint32_t)(draw >> 32),
+                   (uint32_t)seed, (uint32_t)(seed >> 32) ^ 0x5A5A5A5Au, r);
+        u = ((float)(r[0] >> 8) + 0.5f) * (1.0f / 16777216.0f);
+    } else {
+        u = noise[b];
+    }
+    id = n - 1;
+    float cum = 0.f, lsel = lg[n - 1];
+    bool found = false;
+#pragma unroll
+    for (int j = 0; j < CAT_MAX; ++j) {
+        if (j < n && !found) {
+            cum += e[j] / s;
+            if (u < cum) { id = j; lsel = lg[j]; found = true; }
+        }
+    }
+    lp = (lsel - m) - logf(s);
+}
+
+// device-resident draw counter of the capturable sampling path (heads_act_kernel has the same protocol)
+__device__ __forceinline__ unsigned long long cat_take_draw(unsigned long long *draw_ctr, unsigned long long draw)
+{
+    __shared__ unsigned long long sdraw;
+    if (draw_ctr) {
+        if (threadIdx.x == 0) {
+            sdraw = *(volatile unsigned long long *)draw_ctr + 1ull;
+            __threadfence();
+            if (atomicAdd(draw_ctr + 1, 1ull) == (unsigned long long)gridDim.x - 1ull) {
+                draw_ctr[1] = 0ull;
+                draw_ctr[0] = sdraw;
+            }
+        }
+    }
+    __syncthreads();
+    return draw_ctr ? sdraw : draw;
+}
+
+// heads + categorical get_action for the rollout (the categorical heads_act_kernel): a warp per HA_ROWS rows forms the
+// n logits and the value (n + 1 dot products with the head weights held in shared memory, all loads of the rows in
+// flight together, shuffle reductions), then draws as cat_sample_row says.  action[b] = (id, 0) is what hrp_env_step
+// reads for the meta-action ego; pre_tanh[b] = id.
+__global__ void __launch_bounds__(256)
+heads_act_cat_kernel(const float *__restrict__ a1, const float *__restrict__ c1, const float *__restrict__ wa2,
+                     const float *__restrict__ ba2, const float *__restrict__ wc2, const float *__restrict__ bc2,
+                     const float *__restrict__ noise, int mode /*0 det, 1 noise[], 2 philox*/, unsigned long long seed,
+                     unsigned long long draw, unsigned long long row_base, int ld, long long B, int H, int n,
+                     float *__restrict__ action, float *__restrict__ pre_tanh, float *__restrict__ log_prob,
+                     float *__restrict__ value, unsigned long long *draw_ctr, int vec)
+{
+    extern __shared__ __align__(16) float hw[];   // [n + 1][H]
+    hrp_pdl_release();
+    hrp_pdl_wait();
+    for (int i = threadIdx.x; i < (n + 1) * H; i += 256) hw[i] = i < n * H ? wa2[i] : wc2[i - n * H];
+    draw = cat_take_draw(draw_ctr, draw);
+    const int lane = threadIdx.x & 31;
+    const long long b0 = ((long long)blockIdx.x * 8 + (threadIdx.x >> 5)) * HA_ROWS;
+    if (b0 >= B) return;
+    float accs[HA_ROWS][CAT_MAX + 1] = {};
+    if (vec) {   // H % 128 == 0, 16-byte aligned rows: lane owns 4 consecutive k per 128
+        for (int k = 4 * lane; k < H; k += 128) {
+            float4 xa[HA_ROWS], xc[HA_ROWS];
+#pragma unroll
+            for (int r = 0; r < HA_ROWS; ++r) {
+                const long long b = min(b0 + r, B - 1);
+                xa[r] = *reinterpret_cast<const float4 *>(a1 + (size_t)b * ld + k);
+                xc[r] = *reinterpret_cast<const float4 *>(c1 + (size_t)b * ld + k);
+            }
+            const float4 wc = *reinterpret_cast<const float4 *>(hw + n * H + k);
+#pragma unroll
+            for (int a = 0; a < CAT_MAX; ++a)
+                if (a < n) {
+                    const float4 w = *reinterpret_cast<const float4 *>(hw + a * H + k);
+#pragma unroll
+                    for (int r = 0; r < HA_ROWS; ++r)
+                        accs[r][a] = fmaf(xa[r].w, w.w, fmaf(xa[r].z, w.z, fmaf(xa[r].y, w.y, fmaf(xa[r].x, w.x, accs[r][a]))));
+                }
+#pragma unroll
+            for (int r = 0; r < HA_ROWS; ++r)
+                accs[r][CAT_MAX] = fmaf(xc[r].w, wc.w, fmaf(xc[r].z, wc.z, fmaf(xc[r].y, wc.y, fmaf(xc[r].x, wc.x, accs[r][CAT_MAX]))));
+        }
+    } else {
+        for (int k = lane; k < H; k += 32) {
+#pragma unroll
+            for (int r = 0; r < HA_ROWS; ++r) {
+                const long long b = min(b0 + r, B - 1);
+                const float xa = a1[(size_t)b * ld + k], xc = c1[(size_t)b * ld + k];
+#pragma unroll
+                for (int a = 0; a < CAT_MAX; ++a)
+                    if (a < n) accs[r][a] = fmaf(xa, hw[a * H + k], accs[r][a]);
+                accs[r][CAT_MAX] = fmaf(xc, hw[n * H + k], accs[r][CAT_MAX]);
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < HA_ROWS; ++r)
+#pragma unroll
+        for (int a = 0; a <= CAT_MAX; ++a)
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) accs[r][a] += __shfl_xor_sync(HRP_FULL, accs[r][a], d);
+    // every lane holds every sum now; lane r writes row b0 + r
+#pragma unroll
+    for (int r = 0; r < HA_ROWS; ++r) {
+        const long long b = b0 + r;
+        if (lane != r || b >= B) continue;
+        float lg[CAT_MAX];
+#pragma unroll
+        for (int j = 0; j < CAT_MAX; ++j) lg[j] = j < n ? accs[r][j] + ba2[j] : 0.f;
+        int id;
+        float lp;
+        cat_sample_row(lg, n, mode, noise, seed, draw, row_base, b, id, lp);
+        action[2 * b] = (float)id;
+        action[2 * b + 1] = 0.f;
+        pre_tanh[b] = (float)id;
+        if (log_prob) log_prob[b] = lp;
+        value[b] = accs[r][CAT_MAX] + bc2[0];
+    }
+}
+
+// The categorical act path with the heads fused into the [a1 | c1] GEMM (TcDots, NP partial sums per tile and row): a
+// thread per row adds the tiles in tile order, adds the biases and draws exactly as heads_act_cat_kernel does.
+template <int NP>
+__global__ void __launch_bounds__(128)
+heads_finish_cat_kernel(const float *__restrict__ part, int tiles_a, int tiles, const float *__restrict__ ba2,
+                        const float *__restrict__ bc2, const float *__restrict__ noise, int mode, unsigned long long seed,
+                        unsigned long long draw, unsigned long long row_base, long long B, int n,
+                        float *__restrict__ action, float *__restrict__ pre_tanh, float *__restrict__ log_prob,
+                        float *__restrict__ value, unsigned long long *draw_ctr)
+{
+    hrp_pdl_release();
+    hrp_pdl_wait();
+    draw = cat_take_draw(draw_ctr, draw);
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    float lg[CAT_MAX] = {}, val = 0.f;
+    for (int t = 0; t < tiles; ++t) {
+        const float *p = part + ((size_t)t * B + b) * NP;
+        if (t < tiles_a) {
+#pragma unroll
+            for (int q = 0; q < NP; q += 4) {
+                const float4 v = *reinterpret_cast<const float4 *>(p + q);
+                lg[q] += v.x; lg[q + 1] += v.y; lg[q + 2] += v.z; lg[q + 3] += v.w;
+            }
+        } else {
+            val += p[0];
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < CAT_MAX; ++j) lg[j] = j < n ? lg[j] + ba2[j] : 0.f;
+    int id;
+    float lp;
+    cat_sample_row(lg, n, mode, noise, seed, draw, row_base, b, id, lp);
+    action[2 * b] = (float)id;
+    action[2 * b + 1] = 0.f;
+    pre_tanh[b] = (float)id;
+    if (log_prob) log_prob[b] = lp;
+    value[b] = val + bc2[0];
+}
+
+// heads + categorical PPO loss + the gradient of the hidden head layers in one launch, heads_loss_backward_kernel's
+// structure for the softmax head.  Phase 0: a warp per row forms the n logits and the value.  Phase 1: a thread per row
+// takes id = pre_tanh[b], log p = log_softmax(logits), the entropy H = -sum p log p, the ratio and the clipped surrogate
+// (same tie rule), and writes
+//   d(logit_j) = scale [-g ratio (delta_{id,j} - p_j) + c_ent p_j (log p_j + H)]   (g = d min(surr1, surr2) / d ratio)
+// and d(value).  Phase 2: d(a1) | d(c1) under the ReLU masks.  Partial sums per CTA: policy loss, value error, clip
+// count, approx-KL, entropy; the last CTA adds them in block order and writes the metrics.  No log_std gradient.
+__global__ void __launch_bounds__(256)
+heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__restrict__ c1, int ld, int H,
+                               const float *__restrict__ wa2, const float *__restrict__ ba2,
+                               const float *__restrict__ wc2, const float *__restrict__ bc2,
+                               const float *__restrict__ ids, const float *__restrict__ old_lp,
+                               const float *__restrict__ adv, const float *__restrict__ ret, long long B, int n,
+                               float eps_clip, float value_coef, float entropy_coef, float scale,
+                               float *__restrict__ dlogit, float *__restrict__ dvalue, float *__restrict__ da1,
+                               float *__restrict__ dc1, float *__restrict__ d_lo /* nullable */,
+                               float *__restrict__ metrics, float *__restrict__ part, unsigned *__restrict__ counter)
+{
+    __shared__ float out_s[HLB_ROWS][CAT_MAX + 1], dl_s[HLB_ROWS][CAT_MAX], dvalue_s[HLB_ROWS];
+    __shared__ float red[8][8];
+    __shared__ bool last;
+    hrp_pdl_release();
+    hrp_pdl_wait();
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const long long row0 = (long long)blockIdx.x * HLB_ROWS;
+    const int rows = (int)min((long long)HLB_ROWS, B - row0);
+    // ---- phase 0: logits and value
+    for (int r = w; r < rows; r += 8) {
+        const float *ra = a1 + (size_t)(row0 + r) * ld, *rc = c1 + (size_t)(row0 + r) * ld;
+        float acc[CAT_MAX + 1] = {};
+        for (int k = lane; k < H; k += 32) {
+            const float xa = ra[k], xc = rc[k];
+#pragma unroll
+            for (int a = 0; a < CAT_MAX; ++a)
+                if (a < n) acc[a] = fmaf(xa, wa2[(size_t)a * H + k], acc[a]);
+            acc[CAT_MAX] = fmaf(xc, wc2[k], acc[CAT_MAX]);
+        }
+#pragma unroll
+        for (int a = 0; a <= CAT_MAX; ++a)
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) acc[a] += __shfl_xor_sync(HRP_FULL, acc[a], d);
+        if (lane == 0) {
+#pragma unroll
+            for (int a = 0; a < CAT_MAX; ++a)
+                if (a < n) out_s[r][a] = acc[a] + ba2[a];
+            out_s[r][CAT_MAX] = acc[CAT_MAX] + bc2[0];
+        }
+    }
+    __syncthreads();
+    // ---- phase 1: loss terms, one thread per row (warps 0 and 1)
+    float vals[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // pol, val, clip, kl, entropy
+    if (threadIdx.x < rows) {
+        const int r = threadIdx.x;
+        const long long b = row0 + r;
+        float m = out_s[r][0];
+#pragma unroll
+        for (int j = 1; j < CAT_MAX; ++j)
+            if (j < n) m = fmaxf(m, out_s[r][j]);
+        float e[CAT_MAX], s = 0.f;
+#pragma unroll
+        for (int j = 0; j < CAT_MAX; ++j) {
+            e[j] = j < n ? expf(out_s[r][j] - m) : 0.f;
+            s += e[j];
+        }
+        const float lse = logf(s);
+        const int id = min(max((int)ids[b], 0), n - 1);
+        float logp[CAT_MAX], p[CAT_MAX], ent = 0.f, lp = 0.f;
+#pragma unroll
+        for (int j = 0; j < CAT_MAX; ++j) {
+            logp[j] = j < n ? (out_s[r][j] - m) - lse : 0.f;
+            p[j] = e[j] / s;
+            ent -= p[j] * logp[j];
+            lp = j == id ? logp[j] : lp;
+        }
+        float lr = lp - old_lp[b];
+        float ratio = expf(lr);
+        float ad = adv[b];
+        float surr1 = ratio * ad;
+        float rc2 = fminf(fmaxf(ratio, 1.f - eps_clip), 1.f + eps_clip);
+        float surr2 = rc2 * ad;
+        bool inr = ratio >= 1.f - eps_clip && ratio <= 1.f + eps_clip;
+        // d min(surr1, surr2) / d ratio with torch's tie rule (half each on equality)
+        float g;
+        if (surr1 < surr2) g = ad;
+        else if (surr1 == surr2) g = 0.5f * ad + (inr ? 0.5f * ad : 0.f);
+        else g = inr ? ad : 0.f;
+        const float dlp = -g * ratio * scale, ce = entropy_coef * scale;
+#pragma unroll
+        for (int j = 0; j < CAT_MAX; ++j) {
+            const float dl = dlp * ((j == id ? 1.f : 0.f) - p[j]) + ce * p[j] * (logp[j] + ent);
+            dl_s[r][j] = j < n ? dl : 0.f;
+            if (j < n) dlogit[b * n + j] = dl;
+        }
+        float dv = out_s[r][CAT_MAX] - ret[b];
+        float dvv = value_coef * 2.f * dv * scale;
+        dvalue[b] = dvv;
+        dvalue_s[r] = dvv;
+        vals[0] = -fminf(surr1, surr2);
+        vals[1] = dv * dv;
+        vals[2] = fabsf(ratio - 1.f) > eps_clip ? 1.f : 0.f;
+        vals[3] = (ratio - 1.f) - lr;
+        vals[4] = ent;
+    }
+    if (w < 2) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            float x = vals[i];
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) x += __shfl_xor_sync(HRP_FULL, x, d);
+            if (lane == 0) red[w][i] = x;
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 8) {
+        part[blockIdx.x * 8 + threadIdx.x] = red[0][threadIdx.x] + red[1][threadIdx.x];
+        __threadfence();
+    }
+    // ---- phase 2: d(a1) | d(c1) for the CTA's rows
+    for (int k = threadIdx.x; k < H; k += 256) {
+        float wk[CAT_MAX];
+#pragma unroll
+        for (int a = 0; a < CAT_MAX; ++a) wk[a] = a < n ? wa2[(size_t)a * H + k] : 0.f;
+        const float wck = wc2[k];
+        float ma[HLB_ROWS], mc[HLB_ROWS];
+#pragma unroll
+        for (int r = 0; r < HLB_ROWS; ++r) {
+            const size_t o = (size_t)(row0 + r) * ld + k;
+            ma[r] = r < rows ? a1[o] : 0.f;
+            mc[r] = r < rows ? c1[o] : 0.f;
+        }
+#pragma unroll
+        for (int r = 0; r < HLB_ROWS; ++r) {
+            if (r >= rows) break;
+            const size_t o = (size_t)(row0 + r) * ld + k;
+            float sacc = 0.f;
+#pragma unroll
+            for (int a = 0; a < CAT_MAX; ++a) sacc = fmaf(dl_s[r][a], wk[a], sacc);
+            const float ga = ma[r] > 0.f ? sacc : 0.f, gc = mc[r] > 0.f ? dvalue_s[r] * wck : 0.f;
+            da1[o] = ga;
+            dc1[o] = gc;
+            if (d_lo) {   // the TMA GEMMs' pre-split operand: x - trunc_tf32(x), same [B, 2H] layout
+                d_lo[o] = ga - __uint_as_float(__float_as_uint(ga) & 0xFFFFE000u);
+                d_lo[o + (dc1 - da1)] = gc - __uint_as_float(__float_as_uint(gc) & 0xFFFFE000u);
+            }
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned prev = atomicAdd(counter, 1u);
+        last = prev == gridDim.x - 1;
+        if (last) *counter = 0u;
+    }
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    // thread t adds the sums of CTAs t, t + 256, ... in order; then warps, then the 8 warps, always in index order
+    float v8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    for (unsigned c = threadIdx.x; c < gridDim.x; c += 256)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) v8[j] += __ldcg(part + c * 8 + j);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        float x = v8[j];
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) x += __shfl_xor_sync(HRP_FULL, x, d);
+        v8[j] = x;
+    }
+    if (lane == 0)
+        for (int j = 0; j < 8; ++j) red[w][j] = v8[j];
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float tot[8];
+        for (int j = 0; j < 8; ++j) {
+            float x = 0.f;
+            for (int i = 0; i < 8; ++i) x += red[i][j];
+            tot[j] = x;
+        }
+        float pol = tot[0] * scale, val = tot[1] * scale, ent = tot[4] * scale;   // ent: this shard's share of the mean
+        float frac = (float)B * scale;
+        float loss = pol + value_coef * val - entropy_coef * ent;
+        if (metrics) {
+            metrics[0] += loss; metrics[1] += pol; metrics[2] += val; metrics[3] += ent;
+            metrics[4] += tot[2] * scale; metrics[5] += tot[3] * scale; metrics[6] += frac;
+        }
+    }
+}
+
 // PPOMemory.compute_advantages (agent.py:126-138): fp64 arithmetic, float32 store of every A_t
 __global__ void gae_kernel(const float *__restrict__ reward, const float *__restrict__ value,
                            const uint8_t *__restrict__ done, const float *__restrict__ last_value, long long T,
@@ -771,13 +1151,14 @@ clip_adam_kernel(float *__restrict__ p, const float *__restrict__ g, float *__re
 // ---------------------------------------------------------------------------------------
 struct hrp_ppo {
     Layout L;
+    bool cat;                                // HRP_PPO_CATEGORICAL: L.A = n logits, no log_std
     long long max_batch;
     int device;
     float *ws;  // one arena
     float *x, *z, *olp, *adv, *ret;          // gathered minibatch
     float *h1, *h2;                          // trunk activations [B,H]
     float *ac;                               // actor | critic hidden activations, one [B, 2H] matrix
-    float *mean, *value, *dmean, *dvalue;    // heads and their gradients
+    float *mean, *value, *dmean, *dvalue;    // heads and their gradients (mean / dmean: logits when categorical)
     float *d12;                              // d(actor hidden) | d(critic hidden), [B, 2H]
     float *dh2, *dh1;                        // trunk activation gradients [B,H]
     float *wt_ac, *wt_2;                     // transposed weights: [H, 2H] (actor_mean.0 | critic.0) and [H, H] (shared.2)
@@ -1138,11 +1519,18 @@ static int act_impl(hrp_ppo *h, const float *params, const float *states, const 
         if (fuse_on && g_math_mode != 0 && !(use_tma(h) && Bi >= 32) && H % 64 == 0 && Bi >= 32 && H % bn == 0) {
             if (gemm(false, true, Bi, H, L.S, states, L.S, params + L.w1, L.S, h->h1, H, params + L.b1, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
             if (gemm(false, true, Bi, H, H, h->h1, H, params + L.w2, H, h->h2, H, params + L.b2, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
-            // partial sums in the (idle) backward scratch d12: [2 H / bn tiles][B][4] <= [B][2 H] floats
+            // partial sums in the (idle) backward scratch d12: [2 H / bn tiles][B][4 or 8] <= [B][2 H] floats
             const TcDots dots{params + L.wa2, params + L.wc2, H, L.A, h->d12, 1};
             if (hrp_tc_gemm(Bi, 2 * H, H, h->h2, H, 1, params + L.wa1, H, 1, h->ac, 2 * H, params + L.ba1, 1, nullptr, 0, 0, 1,
                             g_math_mode == 1 ? 1 : 3, s, H, params + L.wc1, params + L.bc1, nullptr, &dots, 1) < 0)
                 return -2;
+            if (h->cat) {
+                auto kern = L.A <= 4 ? heads_finish_cat_kernel<4> : heads_finish_cat_kernel<8>;
+                HRP_CUDA_OK(hrp_launch_pdl(kern, dim3((unsigned)((batch + 127) / 128)), dim3(128), 0, s, (const float *)h->d12,
+                                           H / bn, 2 * H / bn, params + L.ba2, params + L.bc2, noise, mode, seed, draw,
+                                           row_base, (long long)batch, L.A, action, pre_tanh, log_prob, value, draw_ctr));
+                return 0;
+            }
             HRP_CUDA_OK(hrp_launch_pdl(heads_finish_kernel, dim3((unsigned)((batch + 127) / 128)), dim3(128), 0, s,
                                        (const float *)h->d12, H / bn, 2 * H / bn, params + L.ba2, params + L.bc2,
                                        params + L.log_std, noise, mode, seed, draw, row_base, (long long)batch, L.A, action,
@@ -1154,6 +1542,13 @@ static int act_impl(hrp_ppo *h, const float *params, const float *states, const 
     const float *pa = h->ac, *pc = h->ac + L.H;
     const int vec = L.H % 128 == 0 && (((uintptr_t)pa | (uintptr_t)pc) & 15) == 0 ? 1 : 0;   // row pitch 2 H: a multiple of 4 with H
     const size_t smem = (size_t)(L.A + 1) * L.H * sizeof(float);
+    if (h->cat) {
+        HRP_CUDA_OK(hrp_launch_pdl(heads_act_cat_kernel, dim3((unsigned)((batch + 8 * HA_ROWS - 1) / (8 * HA_ROWS))), dim3(256),
+                                   smem, s, pa, pc, params + L.wa2, params + L.ba2, params + L.wc2, params + L.bc2, noise, mode,
+                                   seed, draw, row_base, 2 * L.H, (long long)batch, L.H, L.A, action, pre_tanh, log_prob, value,
+                                   draw_ctr, vec));
+        return 0;
+    }
     HRP_CUDA_OK(hrp_launch_pdl(heads_act_kernel, dim3((unsigned)((batch + 8 * HA_ROWS - 1) / (8 * HA_ROWS))), dim3(256), smem, s,
                                pa, pc, params + L.wa2, params + L.ba2, params + L.wc2, params + L.bc2,
                                params + L.log_std, noise, mode, seed, draw, row_base, 2 * L.H, (long long)batch, L.H, L.A,
@@ -1200,6 +1595,14 @@ int64_t hrp_ppo_param_count(int32_t state_dim, int32_t action_dim, int32_t hidde
     return make_layout(state_dim, action_dim, hidden_dim).total;
 }
 
+int64_t hrp_ppo_param_count_ex(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, uint32_t flags)
+{
+    return make_layout(state_dim, action_dim, hidden_dim, (flags & HRP_PPO_CATEGORICAL) != 0).total;
+}
+
+static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch, int32_t device,
+                      bool cat, hrp_ppo **out);
+
 int hrp_ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch, int32_t device,
                    hrp_ppo **out)
 {
@@ -1207,12 +1610,42 @@ int hrp_ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, in
         hrp_set_error("hrp_ppo_create: bad arguments (action_dim must be 1..4)");
         return -1;
     }
+    return ppo_create(state_dim, action_dim, hidden_dim, max_batch, device, false, out);
+}
+
+int hrp_ppo_create_ex(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch, int32_t device,
+                      uint32_t flags, hrp_ppo **out)
+{
+    if (flags & ~HRP_PPO_CATEGORICAL) { hrp_set_error("hrp_ppo_create_ex: flags 0x%x has unknown bits", (unsigned)flags); return -1; }
+    if (!(flags & HRP_PPO_CATEGORICAL)) return hrp_ppo_create(state_dim, action_dim, hidden_dim, max_batch, device, out);
+    if (!out) { hrp_set_error("hrp_ppo_create_ex: out is NULL"); return -1; }
+    if (state_dim < 1) { hrp_set_error("hrp_ppo_create_ex: state_dim %d must be >= 1", (int)state_dim); return -1; }
+    if (hidden_dim < 1) { hrp_set_error("hrp_ppo_create_ex: hidden_dim %d must be >= 1", (int)hidden_dim); return -1; }
+    if (max_batch < 1) { hrp_set_error("hrp_ppo_create_ex: max_batch %lld must be >= 1", (long long)max_batch); return -1; }
+    if (action_dim < 2 || action_dim > CAT_MAX) {
+        hrp_set_error("hrp_ppo_create_ex: action_dim %d (the number of discrete actions) must be in [2, %d]",
+                      (int)action_dim, CAT_MAX);
+        return -1;
+    }
+    return ppo_create(state_dim, action_dim, hidden_dim, max_batch, device, true, out);
+}
+
+static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch, int32_t device,
+                      bool cat, hrp_ppo **out)
+{
     int ndev = hrp_device_count();
     if (ndev <= 0) { hrp_set_error("no CUDA device: this library has no CPU path"); return -3; }
     if (device < 0 || device >= ndev) { hrp_set_error("device %d not in [0, %d)", device, ndev); return -1; }
     HRP_CUDA_OK(cudaSetDevice(device));
+    if (cat) {
+        // the categorical act kernel keeps its n + 1 head rows in shared memory
+        const size_t smem = (size_t)(action_dim + 1) * hidden_dim * sizeof(float);
+        if (smem > 48 * 1024)
+            HRP_CUDA_OK(cudaFuncSetAttribute(heads_act_cat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    }
     hrp_ppo *h = new hrp_ppo();
-    h->L = make_layout(state_dim, action_dim, hidden_dim);
+    h->L = make_layout(state_dim, action_dim, hidden_dim, cat);
+    h->cat = cat;
     h->max_batch = max_batch; h->device = device;
     h->splits_cap = 32;
     size_t B = (size_t)max_batch, H = hidden_dim, S = state_dim, A = action_dim;
@@ -1390,6 +1823,16 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         cudaError_t ce = cudaEventRecord(h->ev[e], from);
         return ce != cudaSuccess ? ce : cudaStreamWaitEvent(to, h->ev[e], 0);
     };
+    const int Az = h->cat ? 1 : A;   // floats per row of pre_tanh: the sampled id of a categorical policy
+    // the categorical head's loss kernel (the Gaussian one is launched in place below)
+    auto heads_loss_cat = [&](const float *z_, const float *olp_, const float *ad_, const float *rt_, float *d_lo) {
+        return hrp_launch_pdl(heads_loss_backward_cat_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
+                              (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
+                              params + L.wc2, params + L.bc2, z_, olp_, ad_, rt_, B, A, eps_clip, value_coef, entropy_coef,
+                              loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, d_lo, metrics, h->loss_part,
+                              h->loss_counter);
+    };
+    auto heads_wgrad = h->cat && A > 4 ? heads_wgrad_partial_kernel<8> : heads_wgrad_partial_kernel<4>;
     h->hold_prepared = false;   // the caller is about to change the parameters (optimizer step)
     if (use_tma(h) && Bi >= 32) {
         // ---- TMA path: every GEMM operand has a "lo" twin written by its producer; the weight-gradient GEMMs read
@@ -1401,9 +1844,9 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         const float *x_lo = h->x_lo;
         if (idx) {
             const long long *ix = (const long long *)idx;
-            long long tot = B * (S + A + 3);
+            long long tot = B * (S + Az + 3);
             gather_batch_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix,
-                                                                             B, S, A, h->x, h->x_lo, h->z, h->olp, h->adv,
+                                                                             B, S, Az, h->x, h->x_lo, h->z, h->olp, h->adv,
                                                                              h->ret);
             HRP_CUDA_OK(cudaGetLastError());
             x = h->x; z = h->z; olp = h->olp; ad = h->adv; rt = h->ret;
@@ -1412,7 +1855,8 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         }
         HRP_CUDA_OK(cudaStreamWaitEvent(s, h->ev[3], 0));
         if (int rc = forward_tma(h, params, x, x_lo, B, s)) return rc;
-        HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
+        if (h->cat) HRP_CUDA_OK(heads_loss_cat(z, olp, ad, rt, h->d12_lo));
+        else HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
                                    (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
                                    params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip,
                                    value_coef, entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, h->d12_lo,
@@ -1441,8 +1885,7 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
             if (chunks > 64) chunks = 64;
             int rows_per = (int)((B + chunks - 1) / chunks);
             dim3 grid((H + 31) / 32, chunks);
-            heads_wgrad_partial_kernel<<<grid, 256, 0, s0>>>(h->dmean, h->dvalue, h->ac, h->ac + H, H2, B, H, A, rows_per,
-                                                             h->part_h);
+            heads_wgrad<<<grid, 256, 0, s0>>>(h->dmean, h->dvalue, h->ac, h->ac + H, H2, B, H, A, rows_per, h->part_h);
             HRP_CUDA_OK(cudaGetLastError());
             plan_add(plan, h->part_h, (long long)A * H + A + H + 1, chunks, grad + L.wa2, (long long)A * H + A, grad + L.wc2);
         }
@@ -1480,14 +1923,15 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
     }
     if (idx) {
         const long long *ix = (const long long *)idx;
-        long long tot = B * (S + A + 3);
+        long long tot = B * (S + Az + 3);
         gather_batch_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix, B,
-                                                                         S, A, h->x, h->x_lo, h->z, h->olp, h->adv, h->ret);
+                                                                         S, Az, h->x, h->x_lo, h->z, h->olp, h->adv, h->ret);
         HRP_CUDA_OK(cudaGetLastError());
         x = h->x; z = h->z; olp = h->olp; ad = h->adv; rt = h->ret;
     }
     if (int rc = forward_impl(h, params, x, B, nullptr, nullptr, s)) return rc;   // trunk + hidden head layers
-    HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
+    if (h->cat) HRP_CUDA_OK(heads_loss_cat(z, olp, ad, rt, (float *)nullptr));
+    else HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
                                (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
                                params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip, value_coef,
                                entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, (float *)nullptr,
@@ -1504,7 +1948,7 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         if (chunks > 64) chunks = 64;
         int rows_per = (int)((B + chunks - 1) / chunks);
         dim3 grid((H + 31) / 32, chunks);
-        heads_wgrad_partial_kernel<<<grid, 256, 0, s0>>>(h->dmean, h->dvalue, a1, c1, H2, B, H, A, rows_per, h->part_h);
+        heads_wgrad<<<grid, 256, 0, s0>>>(h->dmean, h->dvalue, a1, c1, H2, B, H, A, rows_per, h->part_h);
         HRP_CUDA_OK(cudaGetLastError());
         plan_add(plan, h->part_h, (long long)A * H + A + H + 1, chunks, grad + L.wa2, (long long)A * H + A, grad + L.wc2);
     }

@@ -8,6 +8,9 @@ format as the reference; the arithmetic runs in ``libhrp_b200.so``:
   ``actor_mean.0.*``, ``actor_mean.2.*``, ``critic.0.*``, ``critic.2.*``); the per-layer tensors
   of ``state_dict()`` are views into it, so gradients, Adam moments and the multi-GPU all-reduce
   all touch one contiguous range.
+* ``discrete=True`` (keyword-only, beside the reference's signature) selects the categorical policy for the
+  ``DiscreteMetaAction`` ego: a softmax over ``action_dim`` = n logits on the same trunk and critic, the same layout
+  without ``log_std`` (``hrp_ppo_create_ex`` with ``HRP_PPO_CATEGORICAL``).
 * ``PPOMemory`` keeps the list-based ``store`` API of the reference loop and adds a device-resident
   [T, E] rollout for the vectorised loop.
 * ``PPOAgent.update`` = GAE kernel -> advantage normalisation -> for every epoch and minibatch:
@@ -37,9 +40,8 @@ _PARAM_ORDER = ("log_std", "shared.0.weight", "shared.0.bias", "shared.2.weight"
                 "critic.0.weight", "critic.0.bias", "critic.2.weight", "critic.2.bias")
 
 
-def _param_shapes(S: int, A: int, H: int) -> "OrderedDict[str, tuple]":
-    return OrderedDict([
-        ("log_std", (A,)),
+def _param_shapes(S: int, A: int, H: int, discrete: bool = False) -> "OrderedDict[str, tuple]":
+    return OrderedDict(([] if discrete else [("log_std", (A,))]) + [
         ("shared.0.weight", (H, S)), ("shared.0.bias", (H,)),
         ("shared.2.weight", (H, H)), ("shared.2.bias", (H,)),
         ("actor_mean.0.weight", (H, H)), ("actor_mean.0.bias", (H,)),
@@ -62,14 +64,19 @@ class ActorCritic:
 
     Weight initialisation builds the reference's ``nn.Linear`` stack on the CPU in the reference's
     construction order (``agent.py:22-42``), so a seeded run starts from the same parameters.
+
+    ``discrete=True``: a categorical policy over ``action_dim`` actions (2..8).  ``actor_mean.2`` gives the logits,
+    there is no ``log_std``; ``forward`` returns ``(logits, None, value)``.
     """
 
     def __init__(self, state_dim: int, action_dim: int, hidden_dim: int = 128,
-                 device: Any = "cuda", max_batch: int = 4096):
+                 device: Any = "cuda", max_batch: int = 4096, *, discrete: bool = False):
         self._lib = _lib.load()
         _lib.require_device()
         self.device = _cuda_device(device)
         self.state_dim, self.action_dim, self.hidden_dim = int(state_dim), int(action_dim), int(hidden_dim)
+        self.discrete = bool(discrete)
+        self._flags = _lib.PPO_CATEGORICAL if self.discrete else 0
         S, A, H = self.state_dim, self.action_dim, self.hidden_dim
         shared = nn.Sequential(nn.Linear(S, H), nn.ReLU(), nn.Linear(H, H), nn.ReLU())
         actor_mean = nn.Sequential(nn.Linear(H, H), nn.ReLU(), nn.Linear(H, A))
@@ -79,8 +86,8 @@ class ActorCritic:
         for prefix, seq in (("shared", shared), ("actor_mean", actor_mean), ("critic", critic)):
             for k, v in seq.state_dict().items():
                 init[f"{prefix}.{k}"] = v
-        self.shapes = _param_shapes(S, A, H)
-        self.num_params = int(self._lib.hrp_ppo_param_count(S, A, H))
+        self.shapes = _param_shapes(S, A, H, self.discrete)
+        self.num_params = int(self._lib.hrp_ppo_param_count_ex(S, A, H, self._flags))
         assert self.num_params == sum(int(np.prod(s)) for s in self.shapes.values())
         self.flat = torch.empty(self.num_params, dtype=torch.float32, device=self.device)
         self._views: "OrderedDict[str, torch.Tensor]" = OrderedDict()
@@ -114,8 +121,8 @@ class ActorCritic:
             torch.cuda.synchronize(self.device)
             self._lib.hrp_ppo_destroy(self._h)
             self._h = C.c_void_p()
-        _lib.check(self._lib.hrp_ppo_create(self.state_dim, self.action_dim, self.hidden_dim, int(batch),
-                                            self.device.index, C.byref(self._h)), "hrp_ppo_create")
+        _lib.check(self._lib.hrp_ppo_create_ex(self.state_dim, self.action_dim, self.hidden_dim, int(batch),
+                                               self.device.index, self._flags, C.byref(self._h)), "hrp_ppo_create_ex")
         self.max_batch = int(batch)
         self.workspace_generation += 1
 
@@ -200,7 +207,7 @@ class ActorCritic:
         self._sync_weight_copies()
         _lib.check(self._lib.hrp_ppo_forward(self._h, self.flat.data_ptr(), xb.data_ptr(), B, mean.data_ptr(),
                                              value.data_ptr(), self._stream()), "hrp_ppo_forward")
-        std = self.log_std.exp()
+        std = None if self.discrete else self.log_std.exp()
         if single:
             return mean[0], std, value[0]
         return mean, std, value
@@ -221,20 +228,19 @@ class ActorCritic:
         later steps of a captured rollout).
 
         ``lane`` > 0 selects a separate native workspace (same parameters) so that calls on different CUDA streams
-        may overlap: the two env groups of the pipelined host-buffer loop (bench.py e2e) act concurrently."""
+        may overlap: the two env groups of the pipelined host-buffer loop (bench.py e2e) act concurrently.
+
+        Categorical policy: action [B, 2] = (id, 0) -- what the meta-action env step reads --, pre_tanh [B, 1] = id;
+        ``noise`` holds one uniform in (0, 1) per row; B = 1 goes through the batched kernels."""
         states = self._as_states(states)
         B = states.shape[0]
-        if B == 1 and noise is None and not lane and draw_counter is None:
+        if B == 1 and noise is None and not lane and draw_counter is None and not self.discrete:
             return self._act_one(states, deterministic, out, stream)
         if lane:
             return self._act_lane(states, B, out, lane, deterministic, noise, draw_counter)
         self._ensure_workspace(B)
-        A = self.action_dim
         if out is None:
-            out = {"action": torch.empty((B, A), dtype=torch.float32, device=self.device),
-                   "pre_tanh": torch.empty((B, A), dtype=torch.float32, device=self.device),
-                   "log_prob": torch.empty(B, dtype=torch.float32, device=self.device),
-                   "value": torch.empty(B, dtype=torch.float32, device=self.device)}
+            out = self._new_act_out(B)
         if draw_counter is not None:
             self._lib.hrp_ppo_hold_weights(self._h, 1 if reuse_weight_copies else 0)
             self._held_key = None
@@ -265,10 +271,23 @@ class ActorCritic:
                    "hrp_ppo_act")
         return out
 
+    def act_widths(self):
+        """Floats per row of ``act``'s action and pre_tanh outputs."""
+        return (2, 1) if self.discrete else (self.action_dim, self.action_dim)
+
+    def _new_act_out(self, B: int) -> Dict[str, torch.Tensor]:
+        wa, wz = self.act_widths()
+        return {"action": torch.empty((B, wa), dtype=torch.float32, device=self.device),
+                "pre_tanh": torch.empty((B, wz), dtype=torch.float32, device=self.device),
+                "log_prob": torch.empty(B, dtype=torch.float32, device=self.device),
+                "value": torch.empty(B, dtype=torch.float32, device=self.device)}
+
     # -- one state: the matrix-vector kernel (what the reference's single-env loop calls once per env step) -------
     def act_item(self, state: torch.Tensor, out_row: torch.Tensor, deterministic: bool) -> "_lib.HrpActItem":
         """The ``hrp_act_item`` of one ``get_action`` call of this policy (advances the draw counter when sampling):
-        ``hrp_ppo_act_multi`` serves many such items, of different policies, in one launch."""
+        ``hrp_ppo_act_multi`` serves many such items, of different policies, in one launch.  Gaussian policies only."""
+        if self.discrete:
+            raise ValueError("hrp_ppo_act_multi serves Gaussian policies only")
         if not deterministic:
             self._draw += 1
         it = _lib.HrpActItem()
@@ -313,15 +332,11 @@ class ActorCritic:
                 torch.cuda.synchronize(self.device)
                 self._lib.hrp_ppo_destroy(h[0])
             hp = C.c_void_p()
-            _lib.check(self._lib.hrp_ppo_create(self.state_dim, self.action_dim, self.hidden_dim, int(B), self.device.index,
-                                                C.byref(hp)), "hrp_ppo_create")
+            _lib.check(self._lib.hrp_ppo_create_ex(self.state_dim, self.action_dim, self.hidden_dim, int(B),
+                                                   self.device.index, self._flags, C.byref(hp)), "hrp_ppo_create_ex")
             h = lanes[lane] = (hp, int(B))
-        A = self.action_dim
         if out is None:
-            out = {"action": torch.empty((B, A), dtype=torch.float32, device=self.device),
-                   "pre_tanh": torch.empty((B, A), dtype=torch.float32, device=self.device),
-                   "log_prob": torch.empty(B, dtype=torch.float32, device=self.device),
-                   "value": torch.empty(B, dtype=torch.float32, device=self.device)}
+            out = self._new_act_out(B)
         if draw_counter is not None:
             self._lib.hrp_ppo_hold_weights(h[0], 0)
             _lib.check(self._lib.hrp_ppo_act_sample_ctr(h[0], self.flat.data_ptr(), states.data_ptr(), self._noise_seed,
@@ -339,7 +354,16 @@ class ActorCritic:
 
     # -- ActorCritic.get_action (agent.py:56-74): one state, numpy results -----------------------
     def get_action(self, state, deterministic: bool = False):
+        """Gaussian: (action, pre_tanh, log_prob | None, value).  Categorical: (int id, float32 array([id]),
+        log_prob | None, value)."""
         x = self._as_states(state).view(1, -1)
+        if self.discrete:
+            buf = torch.empty(5, dtype=torch.float32, device=self.device)
+            out = {"action": buf[0:2], "pre_tanh": buf[2:3], "log_prob": buf[3:4], "value": buf[4:5]}
+            self.act(x, deterministic=deterministic, out=out)
+            host = buf.cpu().numpy()
+            log_prob = None if deterministic else float(host[3])
+            return int(host[0]), host[2:3].copy(), log_prob, np.float32(host[4])
         A = self.action_dim
         buf = torch.empty(2 * A + 2, dtype=torch.float32, device=self.device)
         out = {"action": buf[0:A], "pre_tanh": buf[A:2 * A], "log_prob": buf[2 * A:2 * A + 1],
@@ -354,6 +378,11 @@ class ActorCritic:
     def evaluate(self, states, actions, pre_tanh_actions):
         mean, std, value = self.forward(states)
         z = self._as_states(pre_tanh_actions)
+        if self.discrete:   # pre_tanh holds the sampled ids
+            logp_all = torch.log_softmax(mean, dim=-1)
+            ids = z.reshape(-1).long().view(-1, 1)
+            entropy = -(logp_all.exp() * logp_all).sum(-1)
+            return logp_all.gather(-1, ids).view(-1), value, entropy
         var = std * std
         logp = -((z - mean) ** 2) / (2 * var) - self.log_std - 0.5 * float(np.log(2 * np.pi))
         logp = logp - torch.log1p(-torch.tanh(z).pow(2) + 1e-6)
@@ -399,15 +428,19 @@ class PPOMemory:
         return len(self.states)
 
     # -- device-resident [T, E] rollout -----------------------------------------------------------
-    def begin_rollout(self, T: int, E: int, state_dim: int, action_dim: int) -> Dict[str, torch.Tensor]:
+    def begin_rollout(self, T: int, E: int, state_dim: int, action_dim: int,
+                      pre_dim: Optional[int] = None) -> Dict[str, torch.Tensor]:
         """Allocate (or reuse) time-major buffers: states [T+1,E,S] (slot T holds the bootstrap
-        observation), pre_tanh/action [T,E,A], log_prob/value/reward [T,E], done [T,E] uint8."""
+        observation), action [T,E,A], pre_tanh [T,E,pre_dim] (default A), log_prob/value/reward [T,E],
+        done [T,E] uint8."""
+        pre_dim = action_dim if pre_dim is None else pre_dim
         r = self.rollout
-        if r is None or r["reward"].shape != (T, E) or r["states"].shape[2] != state_dim:
+        if (r is None or r["reward"].shape != (T, E) or r["states"].shape[2] != state_dim
+                or r["action"].shape[2] != action_dim or r["pre_tanh"].shape[2] != pre_dim):
             d = self.device
             r = {"states": torch.empty((T + 1, E, state_dim), dtype=torch.float32, device=d),
                  "action": torch.empty((T, E, action_dim), dtype=torch.float32, device=d),
-                 "pre_tanh": torch.empty((T, E, action_dim), dtype=torch.float32, device=d),
+                 "pre_tanh": torch.empty((T, E, pre_dim), dtype=torch.float32, device=d),
                  "log_prob": torch.empty((T, E), dtype=torch.float32, device=d),
                  "value": torch.empty((T, E), dtype=torch.float32, device=d),
                  "reward": torch.empty((T, E), dtype=torch.float32, device=d),
@@ -452,9 +485,9 @@ class PPOMemory:
 
     def get_tensors(self):
         r = self.as_rollout()
-        S, A = r["states"].shape[-1], r["action"].shape[-1]
+        S, A, Z = r["states"].shape[-1], r["action"].shape[-1], r["pre_tanh"].shape[-1]
         n = r["reward"].numel()
-        return (r["states"].reshape(-1, S)[:n], r["action"].reshape(-1, A), r["pre_tanh"].reshape(-1, A),
+        return (r["states"].reshape(-1, S)[:n], r["action"].reshape(-1, A), r["pre_tanh"].reshape(-1, Z),
                 r["log_prob"].reshape(-1))
 
 
@@ -530,11 +563,12 @@ class PPOAgent:
     def __init__(self, state_dim: int, action_dim: int, lr: float = 1e-4, gamma: float = 0.99, lam: float = 0.95,
                  eps_clip: float = 0.2, value_coef: float = 0.5, entropy_coef: float = 0.005,
                  max_grad_norm: float = 0.5, epochs: int = 6, batch_size: int = 64, hidden_dim: int = 128,
-                 logger: Optional[logging.Logger] = None, device: Any = "cuda"):
+                 logger: Optional[logging.Logger] = None, device: Any = "cuda", *, discrete: bool = False):
         self._lib = _lib.load()
         self.device = _cuda_device(device)
+        self.discrete = bool(discrete)
         self.actor_critic = ActorCritic(state_dim, action_dim, hidden_dim, device=self.device,
-                                        max_batch=max(int(batch_size), 1))
+                                        max_batch=max(int(batch_size), 1), discrete=self.discrete)
         self.optimizer = _AdamState(self.actor_critic, lr)
         self.gamma, self.lam, self.eps_clip = gamma, lam, eps_clip
         self.value_coef, self.entropy_coef, self.max_grad_norm = value_coef, entropy_coef, max_grad_norm
@@ -761,7 +795,7 @@ class PPOAgent:
         r = mem.as_rollout()
         T, E = r["reward"].shape
         n = T * E
-        S, A = ac.state_dim, ac.action_dim
+        S = ac.state_dim
         world = self._world()
         stream = ac._stream()
         adv, ret = gae(r["reward"], r["value"], r["done"], last_value, self.gamma, self.lam)
@@ -773,7 +807,8 @@ class PPOAgent:
         _lib.check(self._lib.hrp_adv_normalize(adv_n.data_ptr(), n, self._stats.data_ptr(), stream),
                    "hrp_adv_normalize")
         self.launches += 3
-        flat = {"states": r["states"].reshape(-1, S)[:n].contiguous(), "pre_tanh": r["pre_tanh"].reshape(n, A),
+        flat = {"states": r["states"].reshape(-1, S)[:n].contiguous(),
+                "pre_tanh": r["pre_tanh"].reshape(n, ac.act_widths()[1]),
                 "log_prob": r["log_prob"].reshape(n), "adv": adv_n.view(n), "ret": ret.view(n)}
         # one permutation per update, reused by every epoch (agent.py:140-147,205)
         perm = np.arange(n, dtype=np.int64)

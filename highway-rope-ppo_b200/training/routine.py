@@ -193,6 +193,23 @@ def training_coroutine(memory, max_episodes: int = 500, target_reward: float = 0
 
 # --------------------------------------------------------------------------------------------
 # batched loops
+META_ACTIONS = 5   # DiscreteMetaAction: LANE_LEFT, IDLE, LANE_RIGHT, FASTER, SLOWER
+
+
+def _act_widths(vec_env, agent):
+    """(action, pre_tanh) floats per env of the agent's rollout on this env; ValueError when they do not fit."""
+    ac = agent.actor_critic
+    meta = getattr(getattr(vec_env, "cfg", None), "ego_mode", 0) == 1
+    if getattr(ac, "discrete", False):
+        if not meta:
+            raise ValueError("a discrete (categorical) agent needs a DiscreteMetaAction env; this env takes "
+                             "ContinuousAction")
+        if ac.action_dim != META_ACTIONS:
+            raise ValueError(f"the discrete agent has {ac.action_dim} actions; the DiscreteMetaAction env has "
+                             f"{META_ACTIONS}")
+    return ac.act_widths()
+
+
 def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
                     noise: Optional[torch.Tensor] = None, use_graph: Optional[bool] = None) -> Dict[str, torch.Tensor]:
     """T lock-step policy steps of every env into ``agent.memory``'s device rollout.
@@ -206,8 +223,12 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     With in-kernel sampling (``noise is None``) the whole rollout -- 5 T launches -- is captured ONCE as a CUDA graph
     (the sampling kernel's draw counter lives on the device) and replayed by later calls with the same env, agent and
     shape: the host-side cost of a rollout is one graph launch.  ``use_graph=False`` issues the launches one by one.
+
+    A discrete agent on a ``DiscreteMetaAction`` env writes action [T, E, 2] = (id, 0), which the env step reads as it
+    is, and pre_tanh [T, E, 1] = id.
     """
-    E, S, A = vec_env.num_envs, vec_env.N * vec_env.F_out, agent.actor_critic.action_dim
+    A, Z = _act_widths(vec_env, agent)
+    E, S = vec_env.num_envs, vec_env.N * vec_env.F_out
     ac = agent.actor_critic
     # exploration noise is keyed by the GLOBAL env id: a shard's rows start at its first global env
     ac.row_base = int(getattr(vec_env, "env_id_base", 0))
@@ -215,11 +236,11 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
         # (a single env acts through the matrix-vector kernel, which keeps its draw counter on the host)
         use_graph = noise is None and E > 1 and getattr(agent, "use_cuda_graphs", True)
     cache = getattr(agent, "_rollout_graph", None)
-    key = (getattr(vec_env, "uid", id(vec_env)), getattr(vec_env, "param_version", 0), T, E, S, A,
+    key = (getattr(vec_env, "uid", id(vec_env)), getattr(vec_env, "param_version", 0), T, E, S, A, Z,
            ac.workspace_generation, ac.row_base)
     if use_graph and cache is not None and cache["key"] == key and agent.memory.rollout is None:
         agent.memory.rollout = cache["r"]     # the buffers the captured launches write (PPOAgent.update dropped them)
-    r = agent.memory.begin_rollout(T, E, S, A)
+    r = agent.memory.begin_rollout(T, E, S, A, Z)
     states = r["states"]
     if obs is None:
         vec_env.observe(out=states[0].view(E, vec_env.N, vec_env.F_out))
@@ -286,6 +307,7 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
     """``iterations`` PPO iterations on E lock-step envs; returns the list of update metrics with
     mean step reward and samples/s added."""
     logger = logger or logging.getLogger(__name__)
+    _act_widths(vec_env, agent)
     obs = vec_env.reset(seed=seed)
     history = []
     for it in range(iterations):

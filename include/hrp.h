@@ -199,6 +199,14 @@ int hrp_embed_apply(int32_t kind, int32_t embed_dim, int32_t use_euclidean, int3
  *      actor_mean.2.*, critic.0.*, critic.2.*; nn.Linear weights row-major [out,in].
  *      hrp_ppo_param_count gives P. */
 int64_t hrp_ppo_param_count(int32_t state_dim, int32_t action_dim, int32_t hidden_dim);
+/* Categorical policy (flag HRP_PPO_CATEGORICAL): a softmax over action_dim = n discrete actions, 2 <= n <= 8 (n = 5 for
+ * the DiscreteMetaAction ego, hrp_cfg.ego_mode = 1), on the same trunk and critic with the same loss formula: log-prob
+ * log_softmax(logits)[a], state-dependent entropy -sum p log p, clipped surrogate, value MSE, entropy bonus.  Its flat
+ * buffer is the layout above WITHOUT log_std: shared.0.*, shared.2.*, actor_mean.0.*, actor_mean.2.{weight[n,H],
+ * bias[n]} (the logits), critic.0.*, critic.2.*.  hrp_ppo_param_count_ex(S, n, H, flags) gives its P; flags 0 is
+ * hrp_ppo_param_count. */
+#define HRP_PPO_CATEGORICAL 1u
+int64_t hrp_ppo_param_count_ex(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, uint32_t flags);
 /* arithmetic of the hidden-layer GEMMs (process-wide): 3 = tcgen05 tensor cores, 3xTF32 split (fp32-grade
  * accuracy; default), 1 = tcgen05 single-pass TF32, 0 = fp32 CUDA-core GEMM.  torch's nn.Linear in the
  * reference is fp32 (ppo/agent.py:22-42). */
@@ -214,6 +222,23 @@ typedef struct hrp_ppo hrp_ppo;
 /* workspace for batches up to max_batch rows */
 int hrp_ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch,
                    int32_t device, hrp_ppo **out);
+/* the same with flags: HRP_PPO_CATEGORICAL makes a categorical handle (action_dim = n in [2, 8]); flags 0 is exactly
+ * hrp_ppo_create.  The arguments are validated before any device query (-1, with a message naming the field).
+ * A categorical handle goes through the entry points below unchanged:
+ *   hrp_ppo_forward          mean_dev[B, n] receives the logits;
+ *   hrp_ppo_act, _act_sample, _act_sample_ctr
+ *                            action_dev[B, 2] = (id, 0.0f) -- what hrp_env_step reads for ego_mode = 1 --,
+ *                            pre_tanh_dev[B] = id as float (the sample the loss conditions on), log_prob, value.
+ *                            Deterministic: the argmax, first maximum on ties, log-prob 0.  noise_dev (nullable) holds
+ *                            ONE uniform in (0, 1) per row.  Sampling draws one uniform per row from Philox4x32-10 with
+ *                            the Gaussian path's counter (row_base + row, draw) and key, u = ((r0 >> 8) + 0.5) / 2^24,
+ *                            and takes the first id j with u < sum_{i <= j} p_i (summed in index order in fp32), n - 1
+ *                            if there is none;
+ *   hrp_ppo_loss_grad        reads the ids from pre_tanh_dev[B]; same metrics layout, with the state-dependent
+ *                            entropy; there is no log_std gradient.
+ * hrp_ppo_act_multi is Gaussian-only. */
+int hrp_ppo_create_ex(int32_t state_dim, int32_t action_dim, int32_t hidden_dim, int64_t max_batch,
+                      int32_t device, uint32_t flags, hrp_ppo **out);
 int hrp_ppo_destroy(hrp_ppo *h);
 
 /* The tensor-core path multiplies 16-byte aligned copies of the weight matrices (plus their 3xTF32 "lo" parts), which
