@@ -104,7 +104,6 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_ppo_create": (C.c_int, [_i32, _i32, _i32, _i64, _i32, C.POINTER(_vp)]),
     "hrp_ppo_create_ex": (C.c_int, [_i32, _i32, _i32, _i64, _i32, C.c_uint32, C.POINTER(_vp)]),
     "hrp_ppo_destroy": (C.c_int, [_vp]),
-    "hrp_ppo_hold_weights": (C.c_int, [_vp, _i32]),
     "hrp_ppo_forward": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "hrp_ppo_act": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "hrp_ppo_act_sample": (C.c_int, [_vp, _vp, _vp, _u64, _u64, _u64, _i64, _vp, _vp, _vp, _vp, _vp]),

@@ -301,7 +301,7 @@ template <int BN, bool DUAL, int NP>
 __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p, uint32_t tmem_d, int nkb, int M, int N,
                                             int m0, int n0, int bn0, float *__restrict__ C, int ldc,
                                             const float *__restrict__ biasp, int relu, const float *__restrict__ mask,
-                                            int ldm, int accumulate, float *__restrict__ C_lo, const TcDots &dots)
+                                            int ldm, int accumulate, const TcDots &dots)
 {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // ---- epilogue: TMEM -> registers -> shared (row-major, padded) -> coalesced global rows.
@@ -352,9 +352,7 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
     __syncthreads();
     if (tid == 0) TC_PHASE(6);   // tile staged in shared memory
     float *Cz = C + (size_t)blockIdx.z * M * ldc;
-    // optional "lo" twin of the output, x - trunc_tf32(x): the pre-split operand of the TMA-fed kernel (hrp_gemm_tma.cu)
-    float *Clz = C_lo ? C_lo + (size_t)blockIdx.z * M * ldc : nullptr;
-    const bool vec = n0 + BN <= N && ldc % 4 == 0 && ((uintptr_t)Cz & 15) == 0 && (!Clz || ((uintptr_t)Clz & 15) == 0) &&
+    const bool vec = n0 + BN <= N && ldc % 4 == 0 && ((uintptr_t)Cz & 15) == 0 &&
                      (mask == nullptr || (ldm % 4 == 0 && ((uintptr_t)mask & 15) == 0));
     if (vec && tid < TC_THREADS) {
         // whole tile inside the matrix and 16-byte aligned rows: a warp writes 512 contiguous bytes per instruction.
@@ -406,17 +404,7 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
                         for (int q = 0; q < NP; q += 4) *(float4 *)(o + q) = make_float4(d[q], d[q + 1], d[q + 2], d[q + 3]);
                     }
                 }
-                if (m0 + rb + j * RSTEP < M && !dots.skip_store) {
-                    *(float4 *)(crow + (size_t)j * RSTEP * ldc) = x;
-                    if (Clz) {
-                        float4 l;
-                        l.x = x.x - __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u);
-                        l.y = x.y - __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u);
-                        l.z = x.z - __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u);
-                        l.w = x.w - __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
-                        *(float4 *)(Clz + (crow - Cz) + (size_t)j * RSTEP * ldc) = l;
-                    }
-                }
+                if (m0 + rb + j * RSTEP < M && !dots.skip_store) *(float4 *)(crow + (size_t)j * RSTEP * ldc) = x;
             }
             crow += (size_t)RSTEP * GROUP * ldc;
             if (mask) mrow += (size_t)RSTEP * GROUP * ldm;
@@ -445,10 +433,7 @@ __device__ __forceinline__ void tc_epilogue(uint8_t *smem, uint64_t *bar_done_p,
                     float x = stage_c[r * LDS + c] + bv + prev[j];
                     if (relu) x = fmaxf(x, 0.f);
                     x = mk[j] > 0.f ? x : 0.f;
-                    if (gm < M) {
-                        Cz[(size_t)gm * ldc + gn] = x;
-                        if (Clz) Clz[(size_t)gm * ldc + gn] = x - __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-                    }
+                    if (gm < M) Cz[(size_t)gm * ldc + gn] = x;
                 }
             }
         }
@@ -461,8 +446,7 @@ __global__ void __launch_bounds__(TC_LAUNCH_THREADS)
 tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, long long sak,
                const float *__restrict__ B, long long sbn, long long sbk, float *__restrict__ C, int ldc,
                const float *__restrict__ bias, int relu, const float *__restrict__ mask, int ldm, int accumulate,
-               int k_chunk, int nseg, const float *__restrict__ B2, const float *__restrict__ bias2, float *__restrict__ C_lo,
-               const TcDots dots)
+               int k_chunk, int nseg, const float *__restrict__ B2, const float *__restrict__ bias2, const TcDots dots)
 {
     constexpr int PARTS = NSPLIT == 3 ? 2 : 1;                  // hi (+ lo) copy of every operand tile
     constexpr int B_TILE_BYTES = BN * BK * 4;
@@ -664,7 +648,7 @@ tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, 
         }
     }
 
-    tc_epilogue<BN, NSPLIT == 3, NP>(smem, &bar_done, tmem_d, nkb, M, N, m0, n0, bn0, C, ldc, biasp, relu, mask, ldm, accumulate, C_lo, dots);
+    tc_epilogue<BN, NSPLIT == 3, NP>(smem, &bar_done, tmem_d, nkb, M, N, m0, n0, bn0, C, ldc, biasp, relu, mask, ldm, accumulate, dots);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0)
@@ -684,7 +668,7 @@ tc_gemm_kernel(int M, int N, int K, const float *__restrict__ A, long long sam, 
 template <int AMODE, int BMODE, int NSPLIT, int BN, bool ASYNC = false, int NP = 4>
 int launch(dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam, long long sak,
            const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias, int relu,
-           const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2, const float *bias2, float *C_lo,
+           const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2, const float *bias2,
            const TcDots &dots)
 {
     constexpr int PARTS = NSPLIT == 3 ? 2 : 1;
@@ -703,7 +687,7 @@ int launch(dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long 
         configured[dev] = true;
     }
     HRP_CUDA_OK(hrp_launch_pdl(kern, grid, dim3(TC_LAUNCH_THREADS), (size_t)SMEM, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc,
-                               bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots));
+                               bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots));
     return 0;
 }
 
@@ -711,9 +695,9 @@ template <int AMODE, int BMODE, int NP = 4>
 int dispatch(int bn, int nsplit, dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam,
              long long sak, const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias,
              int relu, const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2,
-             const float *bias2, float *C_lo, const TcDots &dots)
+             const float *bias2, const TcDots &dots)
 {
-#define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots
+#define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots
     if constexpr (NP == 4)   // (never with the fused epilogue, the only user of NP = 8)
         if (bn == 32 && nsplit == 3) return launch<AMODE, BMODE, 3, 32>(HRP_TC_ARGS);
     if (bn <= 64)
@@ -727,9 +711,9 @@ template <int NP = 4>
 int dispatch_async(int bn, int nsplit, dim3 grid, cudaStream_t s, int M, int N, int K, const float *A, long long sam,
                    long long sak, const float *B, long long sbn, long long sbk, float *C, int ldc, const float *bias,
                    int relu, const float *mask, int ldm, int accumulate, int k_chunk, int nseg, const float *B2,
-                   const float *bias2, float *C_lo, const TcDots &dots)
+                   const float *bias2, const TcDots &dots)
 {
-#define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots
+#define HRP_TC_ARGS grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots
     if (bn == 64)
         return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 64, true, NP>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 64, true, NP>(HRP_TC_ARGS);
     return nsplit == 3 ? launch<ST_K4, ST_K2, 3, 128, true, NP>(HRP_TC_ARGS) : launch<ST_K4, ST_K2, 1, 128, true, NP>(HRP_TC_ARGS);
@@ -755,7 +739,7 @@ int hrp_tc_gemm_bn(int M, int N, int splits, int nseg, int narrow)
 int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sak, const float *B, long long sbn,
                 long long sbk, float *C, int ldc, const float *bias, int relu, const float *mask, int ldm,
                 int accumulate, int splits, int nsplit, cudaStream_t s, int nseg, const float *B2, const float *bias2,
-                float *C_lo, const TcDots *dots_in, int narrow)
+                const TcDots *dots_in, int narrow)
 {
     const TcDots dots = dots_in ? *dots_in : TcDots{nullptr, nullptr, 0, 0, nullptr, 0};
     int k_chunk = K;
@@ -778,7 +762,7 @@ int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sa
     if (narrow && bn32 && bn == 64 && nsplit == 3 && N % 32 == 0 && N >= 64 && mt * ((N + 63) / 64) * splits <= 148 && !dots.out)
         bn = 32;
     dim3 grid((N + bn - 1) / bn, mt, splits);
-    if (dots.out && (splits != 1 || dots.H % bn != 0 || N % bn != 0 || ldc % 4 != 0 || !aligned(C, 16) || mask || C_lo ||
+    if (dots.out && (splits != 1 || dots.H % bn != 0 || N % bn != 0 || ldc % 4 != 0 || !aligned(C, 16) || mask ||
                      dots.A < 1 || dots.A > 8)) {
         hrp_set_error("hrp_tc_gemm: the fused row-dot epilogue needs whole, aligned tiles that do not straddle H, and 1..8 "
                       "head rows");
@@ -789,16 +773,16 @@ int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sa
     const bool a_k4 = akc && K % 4 == 0 && sam % 4 == 0 && aligned(A, 16);
     const bool b_k2 = bkc && K % 2 == 0 && sbn % 2 == 0 && aligned(B, 8) && (nseg == 0 || aligned(B2, 8));
     const bool b_k4 = bkc && K % 4 == 0 && sbn % 4 == 0 && aligned(B, 16) && (nseg == 0 || aligned(B2, 16));
-#define HRP_TC_GO(am, bm) dispatch<am, bm>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots)
+#define HRP_TC_GO(am, bm) dispatch<am, bm>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots)
     int rc;
     if (dots.out && dots.A > 4) {
         // a categorical head of more than four logits: eight partial sums per row.  Only the operand layouts of the act
         // path are instantiated (K-contiguous activations and weights), chosen by the rule below; the alignment of
         // critic.0 in the flat buffer follows n (offset = n mod 4 floats past a 16-byte boundary)
-#define HRP_TC_GO8(am, bm) dispatch<am, bm, 8>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots)
+#define HRP_TC_GO8(am, bm) dispatch<am, bm, 8>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots)
         if (a_k4 && b_k2 && nsplit == 1)
             rc = dispatch_async<8>(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate,
-                                   k_chunk, nseg, B2, bias2, C_lo, dots);
+                                   k_chunk, nseg, B2, bias2, dots);
         else if (a_k4 && b_k4) rc = HRP_TC_GO8(ST_K4, ST_K4);
         else if (a_k4 && b_k2) rc = HRP_TC_GO8(ST_K4, ST_K2);
         else if (akc && bkc) rc = HRP_TC_GO8(ST_K1, ST_K1);
@@ -811,7 +795,7 @@ int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sa
     }
     // cp.async staging pays off for the single-pass mode only (measured: 3xTF32 hidden forward 12.6 us register-staged
     // vs 14.5 us cp.async -- the lo tiles need a second pass through shared memory; TF32 H=512 19.6 -> 16.6 us)
-    if (a_k4 && b_k2 && nsplit == 1) rc = dispatch_async(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, C_lo, dots);
+    if (a_k4 && b_k2 && nsplit == 1) rc = dispatch_async(bn, nsplit, grid, s, M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, mask, ldm, accumulate, k_chunk, nseg, B2, bias2, dots);
     else if (a_k4 && b_k4) rc = HRP_TC_GO(ST_K4, ST_K4);
     else if (a_k4 && b_k2) rc = HRP_TC_GO(ST_K4, ST_K2);
     else if (a_k4 && sbn == 1) rc = HRP_TC_GO(ST_K4, ST_MN1);

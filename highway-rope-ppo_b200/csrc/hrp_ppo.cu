@@ -261,7 +261,7 @@ heads_wgrad_partial_kernel(const float *__restrict__ dmean, const float *__restr
 __global__ void gather_batch_kernel(const float *__restrict__ states, const float *__restrict__ pre_tanh,
                                     const float *__restrict__ olp, const float *__restrict__ adv,
                                     const float *__restrict__ ret, const long long *__restrict__ idx, long long B, int S,
-                                    int A, float *__restrict__ x, float *__restrict__ x_lo, float *__restrict__ z,
+                                    int A, float *__restrict__ x, float *__restrict__ z,
                                     float *__restrict__ o_olp, float *__restrict__ o_adv, float *__restrict__ o_ret)
 {
     hrp_pdl_release();   // the first GEMM of the step sets itself up meanwhile (it waits before it reads x)
@@ -271,38 +271,11 @@ __global__ void gather_batch_kernel(const float *__restrict__ states, const floa
     long long b = i / W;
     int c = (int)(i - b * W);
     long long src = idx[b];
-    if (c < S) {
-        const float v = states[(size_t)src * S + c];
-        x[b * S + c] = v;
-        x_lo[b * S + c] = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);   // the TMA GEMM's pre-split operand
-    }
+    if (c < S) x[b * S + c] = states[(size_t)src * S + c];
     else if (c < S + A) z[b * A + (c - S)] = pre_tanh[(size_t)src * A + (c - S)];
     else if (c == S + A) o_olp[b] = olp[src];
     else if (c == S + A + 1) o_adv[b] = adv[src];
     else o_ret[b] = ret[src];
-}
-
-// the weight operands of the TMA GEMMs (hrp_gemm_tma.cu): 16-byte aligned copies of shared.0 / shared.2 / the row-stacked
-// [actor_mean.0 ; critic.0] (the flat parameter buffer holds them at 8-byte aligned offsets, which a tensor map cannot
-// address), their 3xTF32 "lo" parts x - trunc_tf32(x), and the stacked bias [ba1 | bc1].  One launch per parameter
-// change (every optimizer step; once per rollout).
-__global__ void __launch_bounds__(256)
-prepare_weights_kernel(const float *__restrict__ params, Layout L, float *__restrict__ w1, float *__restrict__ w1_lo,
-                       float *__restrict__ w2, float *__restrict__ w2_lo, float *__restrict__ wac,
-                       float *__restrict__ wac_lo, float *__restrict__ bac)
-{
-    const long long n1 = (long long)L.H * L.S, n2 = (long long)L.H * L.H;
-    const long long total = n1 + 3 * n2 + 2 * L.H;
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total) return;
-    float v, *dst, *dlo = nullptr;
-    if (i < n1) { v = params[L.w1 + i]; dst = w1 + i; dlo = w1_lo + i; }
-    else if (i < n1 + n2) { long long j = i - n1; v = params[L.w2 + j]; dst = w2 + j; dlo = w2_lo + j; }
-    else if (i < n1 + 2 * n2) { long long j = i - n1 - n2; v = params[L.wa1 + j]; dst = wac + j; dlo = wac_lo + j; }
-    else if (i < n1 + 3 * n2) { long long j = i - n1 - 2 * n2; v = params[L.wc1 + j]; dst = wac + n2 + j; dlo = wac_lo + n2 + j; }
-    else { long long j = i - n1 - 3 * n2; v = j < L.H ? params[L.ba1 + j] : params[L.bc1 + j - L.H]; dst = bac + j; }
-    *dst = v;
-    if (dlo) *dlo = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -480,8 +453,8 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
                            const float *__restrict__ old_lp, const float *__restrict__ adv,
                            const float *__restrict__ ret, long long B, int A, float eps_clip, float value_coef,
                            float entropy_coef, float scale, float *__restrict__ dmean, float *__restrict__ dvalue,
-                           float *__restrict__ da1, float *__restrict__ dc1, float *__restrict__ d_lo /* nullable */,
-                           float *__restrict__ dlog_std, float *__restrict__ metrics, float *__restrict__ part,
+                           float *__restrict__ da1, float *__restrict__ dc1, float *__restrict__ dlog_std,
+                           float *__restrict__ metrics, float *__restrict__ part,
                            unsigned *__restrict__ counter)
 {
     __shared__ float out_s[HLB_ROWS][5], dmean_s[HLB_ROWS][4], dvalue_s[HLB_ROWS];
@@ -599,10 +572,6 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
             const float ga = ma[r] > 0.f ? sacc : 0.f, gc = mc[r] > 0.f ? dvalue_s[r] * wck : 0.f;
             da1[o] = ga;
             dc1[o] = gc;
-            if (d_lo) {   // the TMA GEMMs' pre-split operand: x - trunc_tf32(x), same [B, 2H] layout
-                d_lo[o] = ga - __uint_as_float(__float_as_uint(ga) & 0xFFFFE000u);
-                d_lo[o + (dc1 - da1)] = gc - __uint_as_float(__float_as_uint(gc) & 0xFFFFE000u);
-            }
         }
     }
     __syncthreads();
@@ -855,8 +824,8 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
                                const float *__restrict__ adv, const float *__restrict__ ret, long long B, int n,
                                float eps_clip, float value_coef, float entropy_coef, float scale,
                                float *__restrict__ dlogit, float *__restrict__ dvalue, float *__restrict__ da1,
-                               float *__restrict__ dc1, float *__restrict__ d_lo /* nullable */,
-                               float *__restrict__ metrics, float *__restrict__ part, unsigned *__restrict__ counter)
+                               float *__restrict__ dc1, float *__restrict__ metrics, float *__restrict__ part,
+                               unsigned *__restrict__ counter)
 {
     __shared__ float out_s[HLB_ROWS][CAT_MAX + 1], dl_s[HLB_ROWS][CAT_MAX], dvalue_s[HLB_ROWS];
     __shared__ float red[8][8];
@@ -980,10 +949,6 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
             const float ga = ma[r] > 0.f ? sacc : 0.f, gc = mc[r] > 0.f ? dvalue_s[r] * wck : 0.f;
             da1[o] = ga;
             dc1[o] = gc;
-            if (d_lo) {   // the TMA GEMMs' pre-split operand: x - trunc_tf32(x), same [B, 2H] layout
-                d_lo[o] = ga - __uint_as_float(__float_as_uint(ga) & 0xFFFFE000u);
-                d_lo[o + (dc1 - da1)] = gc - __uint_as_float(__float_as_uint(gc) & 0xFFFFE000u);
-            }
         }
     }
     __syncthreads();
@@ -1164,12 +1129,6 @@ struct hrp_ppo {
     float *wt_ac, *wt_2;                     // transposed weights: [H, 2H] (actor_mean.0 | critic.0) and [H, H] (shared.2)
     float *part_w[3];                        // split-K partials of the three weight-gradient GEMMs
     float *part_b[3];                        // column-sum partials of the three bias gradients (<= 64 chunks)
-    // TMA GEMM path (hrp_gemm_tma.cu): "lo" twins of every GEMM operand and the prepared weight copies
-    float *x_lo, *h1_lo, *h2_lo, *ac_lo, *d12_lo, *dh2_lo, *dh1_lo;
-    float *w1p, *w1p_lo, *w2p, *w2p_lo, *wacp, *wacp_lo, *bacp;
-    bool tma_capable;                        // shapes / alignments a tensor map accepts
-    bool hold_prepared;                      // the prepared copies match `prepared_for` and may be reused
-    const float *prepared_for;
     float *part_h;                           // head-gradient partials (<= 64 chunks)
     float *loss_part;                        // heads_loss_backward_kernel partial sums [CTAs][8]
     unsigned *loss_counter;
@@ -1184,16 +1143,8 @@ struct hrp_ppo {
 int hrp_tc_gemm(int M, int N, int K, const float *A, long long sam, long long sak, const float *B, long long sbn,
                 long long sbk, float *C, int ldc, const float *bias, int relu, const float *mask, int ldm,
                 int accumulate, int splits, int nsplit, cudaStream_t s, int nseg = 0, const float *B2 = nullptr,
-                const float *bias2 = nullptr, float *C_lo = nullptr, const TcDots *dots = nullptr, int narrow = 0);
+                const float *bias2 = nullptr, const TcDots *dots = nullptr, int narrow = 0);
 int hrp_tc_gemm_bn(int M, int N, int splits, int nseg, int narrow = 0);
-
-// TMA-fed 3xTF32 path on pre-split operands (hrp_gemm_tma.cu)
-int hrp_tma_gemm(int M, int N, int K, const float *A, const float *A_lo, long long sam, long long sak, const float *B,
-                 const float *B_lo, long long sbn, long long sbk, float *C, float *C_lo, int ldc, const float *bias, int relu,
-                 const float *mask, int ldm, int splits, int bn_hint, cudaStream_t s);
-int hrp_split_lo(const float *x, float *lo, long long n, cudaStream_t s);
-bool hrp_tma_gemm_ok(int M, int N, int K, const float *A, long long sam, long long sak, const float *A_lo, const float *B,
-                     long long sbn, long long sbk, const float *B_lo);
 
 // math mode of the hidden-layer GEMMs: 0 = fp32 SIMT, 1 = TF32 tcgen05, 3 = 3xTF32 tcgen05 (default)
 static int g_math_mode = 3;
@@ -1204,8 +1155,7 @@ static int gemm(bool AT, bool BT, int M, int N, int K, const float *A, int lda, 
 {
     if (g_math_mode != 0 && N >= 32 && M >= 32)
         return hrp_tc_gemm(M, N, K, A, AT ? 1 : lda, AT ? lda : 1, B, BT ? ldb : 1, BT ? 1 : ldb, C, ldc, bias, relu,
-                           mask, ldm, accumulate, splits, g_math_mode == 1 ? 1 : 3, s, 0, nullptr, nullptr, nullptr, nullptr,
-                           narrow);
+                           mask, ldm, accumulate, splits, g_math_mode == 1 ? 1 : 3, s, 0, nullptr, nullptr, nullptr, narrow);
     int k_chunk = K;
     if (splits > 1) {
         k_chunk = ((K + splits - 1) / splits + GK - 1) / GK * GK;
@@ -1250,60 +1200,6 @@ static int colsum(ReducePlan &plan, float *part, const float *G, int ldg, long l
     return 0;
 }
 
-// The TMA-fed GEMM path (hrp_gemm_tma.cu) is OPT-IN (HRP_TMA=1).  Measured on B200 (B = 4096, H = 256,
-// profiles/r02_gemm_bench.txt, r02_timeline_*.txt): alone, its kernel beats the register-staged one on every hidden
-// shape (9.2 against 13.4 us for 4096 x 256 x 256, 12.9 against 18.2 us for K = 512, 9 us against 24 us for the
-// batch-contracting weight gradients), but one CTA owns an SM (192 KB of operand stages): the next kernel of a
-// dependent-launch chain cannot set itself up beside it and the side-stream GEMMs cannot share its SMs, and the whole
-// optimizer step comes out at 136 us against 131 us, the policy forward at 40 against 37 us.  The default therefore
-// stays the register-staged kernel (96 KB, two CTAs per SM).
-static bool use_tma(const hrp_ppo *h)
-{
-    const char *e = getenv("HRP_TMA");
-    return g_math_mode == 3 && h->tma_capable && e && e[0] == '1';
-}
-
-// aligned weight copies + lo parts + stacked bias for the TMA GEMMs; skipped while the caller holds them valid
-static int prepare_weights(hrp_ppo *h, const float *params, cudaStream_t s)
-{
-    if (h->hold_prepared && h->prepared_for == params) return 0;
-    const Layout &L = h->L;
-    const long long total = (long long)L.H * L.S + 3ll * L.H * L.H + 2 * L.H;
-    prepare_weights_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(params, L, h->w1p, h->w1p_lo, h->w2p, h->w2p_lo,
-                                                                          h->wacp, h->wacp_lo, h->bacp);
-    HRP_CUDA_OK(cudaGetLastError());
-    h->prepared_for = params;
-    return 0;
-}
-
-// trunk + hidden head layers on the TMA path: x (and x_lo) -> h1, h2, ac = [a1 | c1], each with its lo twin
-static int forward_tma(hrp_ppo *h, const float *params, const float *x, const float *x_lo, long long B, cudaStream_t s)
-{
-    const Layout &L = h->L;
-    const int H = L.H, S = L.S, Bi = (int)B;
-    // Which kernel serves which layer is a measured choice (tools/gemm_bench.py, tools/trace_update.py, B = 4096):
-    // the short-K first layer and the 2H-wide [actor | critic] layer are faster register-staged (6.0 / 14 us in the
-    // step against 9.3 / 18 us TMA-fed: two CTAs per SM, and no lo twin to write for [a1 | c1], which feeds the heads),
-    // the H x H trunk layer is faster TMA-fed (8.4 against 10.1 us).  HRP_TMA_ALL=1 sends all three through TMA.
-    static const bool tma_all = getenv("HRP_TMA_ALL") != nullptr;
-    (void)x_lo;
-    if (tma_all) {
-        if (hrp_tma_gemm(Bi, H, S, x, x_lo, S, 1, h->w1p, h->w1p_lo, S, 1, h->h1, h->h1_lo, H, params + L.b1, 1, nullptr, 0, 1, 0, s) < 0) return -2;
-    } else {
-        if (hrp_tc_gemm(Bi, H, S, x, S, 1, params + L.w1, S, 1, h->h1, H, params + L.b1, 1, nullptr, 0, 0, 1, 3, s, 0, nullptr, nullptr, h->h1_lo) < 0) return -2;
-    }
-    if (hrp_tma_gemm(Bi, H, H, h->h1, h->h1_lo, H, 1, h->w2p, h->w2p_lo, H, 1, h->h2, h->h2_lo, H, params + L.b2, 1, nullptr, 0, 1, 0, s) < 0) return -2;
-    // [a1 | c1] feeds the heads, not another GEMM: no lo twin
-    if (tma_all) {
-        if (hrp_tma_gemm(Bi, 2 * H, H, h->h2, h->h2_lo, H, 1, h->wacp, h->wacp_lo, H, 1, h->ac, nullptr, 2 * H, h->bacp, 1, nullptr, 0, 1, 0, s) < 0) return -2;
-    } else {
-        if (hrp_tc_gemm(Bi, 2 * H, H, h->h2, H, 1, params + L.wa1, H, 1, h->ac, 2 * H, params + L.ba1, 1, nullptr, 0, 0, 1, 3, s, H,
-                        params + L.wc1, params + L.bc1) < 0)
-            return -2;
-    }
-    return 0;
-}
-
 // shared trunk and the two hidden head layers; the latter are one GEMM over the row-stacked weights
 // [actor_mean.0 ; critic.0] into h->ac = [a1 | c1]
 static int forward_impl(hrp_ppo *h, const float *params, const float *x, long long B, float *mean, float *value,
@@ -1311,18 +1207,6 @@ static int forward_impl(hrp_ppo *h, const float *params, const float *x, long lo
 {
     const Layout &L = h->L;
     int H = L.H, S = L.S, A = L.A, Bi = (int)B;
-    if (use_tma(h) && Bi >= 32) {
-        // external states: their lo part is formed here (inside the update it comes from the gather kernel)
-        if (int rc = prepare_weights(h, params, s)) return rc;
-        if (getenv("HRP_TMA_ALL"))
-            if (int rc = hrp_split_lo(x, h->x_lo, B * S, s)) return rc;
-        if (int rc = forward_tma(h, params, x, h->x_lo, B, s)) return rc;
-        if (!mean) return 0;
-        heads_kernel<<<(unsigned)((B + 7) / 8), 256, 0, s>>>(h->ac, h->ac + H, params + L.wa2, params + L.ba2, params + L.wc2,
-                                                            params + L.bc2, 2 * H, B, H, A, mean, value);
-        HRP_CUDA_OK(cudaGetLastError());
-        return 0;
-    }
     if (gemm(false, true, Bi, H, S, x, S, params + L.w1, S, h->h1, H, params + L.b1, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
     if (gemm(false, true, Bi, H, H, h->h1, H, params + L.w2, H, h->h2, H, params + L.b2, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
     if (g_math_mode != 0 && H % 64 == 0 && Bi >= 32) {
@@ -1516,13 +1400,13 @@ static int act_impl(hrp_ppo *h, const float *params, const float *states, const 
         static const bool fuse_on = !(getenv("HRP_FUSE_HEADS") && getenv("HRP_FUSE_HEADS")[0] == '0');
         const int H = L.H, Bi = (int)batch;
         const int bn = hrp_tc_gemm_bn(Bi, 2 * H, 1, H, 1);
-        if (fuse_on && g_math_mode != 0 && !(use_tma(h) && Bi >= 32) && H % 64 == 0 && Bi >= 32 && H % bn == 0) {
+        if (fuse_on && g_math_mode != 0 && H % 64 == 0 && Bi >= 32 && H % bn == 0) {
             if (gemm(false, true, Bi, H, L.S, states, L.S, params + L.w1, L.S, h->h1, H, params + L.b1, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
             if (gemm(false, true, Bi, H, H, h->h1, H, params + L.w2, H, h->h2, H, params + L.b2, 1, nullptr, 0, 0, 1, s, 1) < 0) return -2;
             // partial sums in the (idle) backward scratch d12: [2 H / bn tiles][B][4 or 8] <= [B][2 H] floats
             const TcDots dots{params + L.wa2, params + L.wc2, H, L.A, h->d12, 1};
             if (hrp_tc_gemm(Bi, 2 * H, H, h->h2, H, 1, params + L.wa1, H, 1, h->ac, 2 * H, params + L.ba1, 1, nullptr, 0, 0, 1,
-                            g_math_mode == 1 ? 1 : 3, s, H, params + L.wc1, params + L.bc1, nullptr, &dots, 1) < 0)
+                            g_math_mode == 1 ? 1 : 3, s, H, params + L.wc1, params + L.bc1, &dots, 1) < 0)
                 return -2;
             if (h->cat) {
                 auto kern = L.A <= 4 ? heads_finish_cat_kernel<4> : heads_finish_cat_kernel<8>;
@@ -1572,19 +1456,6 @@ int hrp_gemm_strided(int32_t M, int32_t N, int32_t K, const float *A, int64_t sa
 {
     if (!A || !B || !C || M < 1 || N < 1 || K < 1 || ldc < N) { hrp_set_error("hrp_gemm_strided: bad arguments"); return -1; }
     if (mode != 1 && mode != 3) { hrp_set_error("hrp_gemm_strided: mode must be 1 (TF32) or 3 (3xTF32)"); return -1; }
-    if (mode == 3 && !getenv("HRP_NO_TMA") && hrp_tma_gemm_ok(M, N, K, A, sam, sak, A, B, sbn, sbk, B)) {   // (tests, tools)
-        // the TMA path wants the operands pre-split: form the lo parts in temporaries on the caller's stream
-        cudaStream_t s = (cudaStream_t)stream;
-        const size_t na = sak == 1 ? (size_t)M * sam : (size_t)K * sak, nb = sbk == 1 ? (size_t)N * sbn : (size_t)K * sbk;
-        float *lo = nullptr;
-        HRP_CUDA_OK(cudaMallocAsync(&lo, (na + nb + 64) * sizeof(float), s));
-        float *a_lo = lo, *b_lo = lo + (na + 31) / 32 * 32;
-        int rc = hrp_split_lo(A, a_lo, (long long)na, s);
-        if (!rc) rc = hrp_split_lo(B, b_lo, (long long)nb, s);
-        if (!rc) rc = hrp_tma_gemm(M, N, K, A, a_lo, sam, sak, B, b_lo, sbn, sbk, C, nullptr, ldc, bias, relu, nullptr, 0, 1, 0, s);
-        HRP_CUDA_OK(cudaFreeAsync(lo, s));
-        return rc < 0 ? rc : 0;
-    }
     int rc = hrp_tc_gemm(M, N, K, A, sam, sak, B, sbn, sbk, C, ldc, bias, relu, nullptr, 0, 0, 1, mode,
                          (cudaStream_t)stream);
     return rc < 0 ? rc : 0;
@@ -1654,10 +1525,7 @@ static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
     auto pad = [](size_t n) { return (n + 31) / 32 * 32; };
     const size_t sizes[] = {B * S, B * A, B, B, B, B * H, B * H, 2 * B * H, B * A, B * A, B, B, 2 * B * H, B * H, B * H,
                             2 * H * H, H * H, cap * 2 * H * H, cap * H * H, cap * H * S, 64 * 2 * H, 64 * H, 64 * H,
-                            64 * ((A + 1) * H + A + 1), ((B + HLB_ROWS - 1) / HLB_ROWS) * 8, 32,
-                            // lo twins (x, h1, h2, ac, d12, dh2, dh1) and prepared weights (w1, w2, wac: copy + lo; bac)
-                            B * S, B * H, B * H, 2 * B * H, 2 * B * H, B * H, B * H,
-                            H * S, H * S, H * H, H * H, 2 * H * H, 2 * H * H, 2 * H};
+                            64 * ((A + 1) * H + A + 1), ((B + HLB_ROWS - 1) / HLB_ROWS) * 8, 32};
     size_t n = 0;
     for (size_t q : sizes) n += pad(q);
     cudaError_t ce = cudaMalloc(&h->ws, n * sizeof(float));
@@ -1674,13 +1542,6 @@ static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
     for (int q = 0; q < 3; ++q) h->part_b[q] = take();
     h->part_h = take(); h->loss_part = take();
     h->loss_counter = (unsigned *)take();
-    h->x_lo = take(); h->h1_lo = take(); h->h2_lo = take(); h->ac_lo = take(); h->d12_lo = take(); h->dh2_lo = take();
-    h->dh1_lo = take();
-    h->w1p = take(); h->w1p_lo = take(); h->w2p = take(); h->w2p_lo = take(); h->wacp = take(); h->wacp_lo = take();
-    h->bacp = take();
-    // a tensor map needs 16-byte aligned row pitches; tiles of 32 / 64 columns
-    h->tma_capable = hidden_dim % 32 == 0 && state_dim % 4 == 0;
-    h->hold_prepared = false; h->prepared_for = nullptr;
     ce = cudaMemset(h->loss_counter, 0, 32 * sizeof(float));
     for (int q = 0; q < 2 && ce == cudaSuccess; ++q) ce = cudaStreamCreateWithFlags(&h->side[q], cudaStreamNonBlocking);
     for (int q = 0; q < 8 && ce == cudaSuccess; ++q) ce = cudaEventCreateWithFlags(&h->ev[q], cudaEventDisableTiming);
@@ -1697,14 +1558,6 @@ int hrp_ppo_destroy(hrp_ppo *h)
     for (int q = 0; q < 2; ++q) if (h->side[q]) cudaStreamDestroy(h->side[q]);
     for (int q = 0; q < 8; ++q) if (h->ev[q]) cudaEventDestroy(h->ev[q]);
     delete h;
-    return 0;
-}
-
-int hrp_ppo_hold_weights(hrp_ppo *h, int32_t hold)
-{
-    if (!h) { hrp_set_error("hrp_ppo_hold_weights: null handle"); return -1; }
-    h->hold_prepared = hold != 0;
-    if (!hold) h->prepared_for = nullptr;
     return 0;
 }
 
@@ -1824,95 +1677,7 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         return ce != cudaSuccess ? ce : cudaStreamWaitEvent(to, h->ev[e], 0);
     };
     const int Az = h->cat ? 1 : A;   // floats per row of pre_tanh: the sampled id of a categorical policy
-    // the categorical head's loss kernel (the Gaussian one is launched in place below)
-    auto heads_loss_cat = [&](const float *z_, const float *olp_, const float *ad_, const float *rt_, float *d_lo) {
-        return hrp_launch_pdl(heads_loss_backward_cat_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
-                              (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
-                              params + L.wc2, params + L.bc2, z_, olp_, ad_, rt_, B, A, eps_clip, value_coef, entropy_coef,
-                              loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, d_lo, metrics, h->loss_part,
-                              h->loss_counter);
-    };
     auto heads_wgrad = h->cat && A > 4 ? heads_wgrad_partial_kernel<8> : heads_wgrad_partial_kernel<4>;
-    h->hold_prepared = false;   // the caller is about to change the parameters (optimizer step)
-    if (use_tma(h) && Bi >= 32) {
-        // ---- TMA path: every GEMM operand has a "lo" twin written by its producer; the weight-gradient GEMMs read
-        // the batch-major activations as MN-major operands and the input-gradient GEMMs read W[out, in] as the
-        // MN-major B operand (no transposed copies).
-        HRP_CUDA_OK(after(0, s, s1));
-        if (int rc = prepare_weights(h, params, s1)) return rc;          // side 1: needs the parameters only
-        HRP_CUDA_OK(cudaEventRecord(h->ev[3], s1));
-        const float *x_lo = h->x_lo;
-        if (idx) {
-            const long long *ix = (const long long *)idx;
-            long long tot = B * (S + Az + 3);
-            gather_batch_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix,
-                                                                             B, S, Az, h->x, h->x_lo, h->z, h->olp, h->adv,
-                                                                             h->ret);
-            HRP_CUDA_OK(cudaGetLastError());
-            x = h->x; z = h->z; olp = h->olp; ad = h->adv; rt = h->ret;
-        } else {
-            if (int rc = hrp_split_lo(x, h->x_lo, B * S, s)) return rc;
-        }
-        HRP_CUDA_OK(cudaStreamWaitEvent(s, h->ev[3], 0));
-        if (int rc = forward_tma(h, params, x, x_lo, B, s)) return rc;
-        if (h->cat) HRP_CUDA_OK(heads_loss_cat(z, olp, ad, rt, h->d12_lo));
-        else HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
-                                   (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
-                                   params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip,
-                                   value_coef, entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, h->d12_lo,
-                                   grad + L.log_std, metrics, h->loss_part, h->loss_counter));
-        ReducePlan plan;
-        plan.nseg = 0; plan.blocks = 0;
-        // split-K over the batch: 512 rows (16 K-blocks) per CTA.  The three weight-gradient GEMMs of H = 256 are then
-        // 64 + 64 + 16 CTAs, one wave of the 148 SMs together (a TMA GEMM CTA owns its SM: 192 KB of shared memory)
-        int splits = (int)((B + 511) / 512);
-        if (const char *e = getenv("HRP_WGRAD_ROWS")) splits = (int)((B + atoi(e) - 1) / atoi(e));
-        if (splits > h->splits_cap) splits = h->splits_cap;
-        if (splits < 1) splits = 1;
-        // dW[N_out, K_in] = dY^T X over the batch: A(m, k) = dY[k, m], B(n, k) = X[k, n], both MN-major
-        auto wgrad_tma = [&](float *part, int Nout, int Kin, const float *dY, const float *dY_lo, int lddy, const float *X,
-                             const float *X_lo, int ldx, float *dW, int n1, float *dW2, cudaStream_t st) -> int {
-            int used = hrp_tma_gemm(Nout, Kin, Bi, dY, dY_lo, 1, lddy, X, X_lo, 1, ldx, part, nullptr, Kin, nullptr, 0, nullptr,
-                                    0, splits, 0, st);
-            if (used < 0) return used;
-            plan_add(plan, part, (long long)Nout * Kin, used, dW, (long long)n1 * Kin, dW2);
-            return 0;
-        };
-        // side 0 -- heads
-        HRP_CUDA_OK(after(1, s, s0));
-        {
-            int chunks = (int)((B + 63) / 64);
-            if (chunks > 64) chunks = 64;
-            int rows_per = (int)((B + chunks - 1) / chunks);
-            dim3 grid((H + 31) / 32, chunks);
-            heads_wgrad<<<grid, 256, 0, s0>>>(h->dmean, h->dvalue, h->ac, h->ac + H, H2, B, H, A, rows_per, h->part_h);
-            HRP_CUDA_OK(cudaGetLastError());
-            plan_add(plan, h->part_h, (long long)A * H + A + H + 1, chunks, grad + L.wa2, (long long)A * H + A, grad + L.wc2);
-        }
-        // side 1: [dWa1 ; dWc1] as one GEMM, [dba1 | dbc1] as one column sum
-        HRP_CUDA_OK(after(2, s, s1));
-        if (wgrad_tma(h->part_w[0], H2, H, h->d12, h->d12_lo, H2, h->h2, h->h2_lo, H, grad + L.wa1, H, grad + L.wc1, s1)) return -2;
-        if (colsum(plan, h->part_b[0], h->d12, H2, B, H2, grad + L.ba1, H, grad + L.bc1, s1)) return -2;
-        // main: d(h2) = [d(a1) | d(c1)] [Wa1 ; Wc1] (.) (h2 > 0): B(n, k) = wac[k, n]
-        if (hrp_tma_gemm(Bi, H, H2, h->d12, h->d12_lo, H2, 1, h->wacp, h->wacp_lo, 1, H, h->dh2, h->dh2_lo, H, nullptr, 0, h->h2, H,
-                         1, 0, s) < 0)
-            return -2;
-        HRP_CUDA_OK(after(4, s, s0));   // side 0 (behind the heads): dW2, db2 -- side 1 is busy with [dWa1 ; dWc1]
-        if (wgrad_tma(h->part_w[1], H, H, h->dh2, h->dh2_lo, H, h->h1, h->h1_lo, H, grad + L.w2, H, nullptr, s0)) return -2;
-        if (colsum(plan, h->part_b[1], h->dh2, H, B, H, grad + L.b2, H, nullptr, s0)) return -2;
-        // main: d(h1) = d(h2) W2 (.) (h1 > 0); dW1; side 0: db1
-        if (hrp_tma_gemm(Bi, H, H, h->dh2, h->dh2_lo, H, 1, h->w2p, h->w2p_lo, 1, H, h->dh1, h->dh1_lo, H, nullptr, 0, h->h1, H, 1,
-                         0, s) < 0)
-            return -2;
-        HRP_CUDA_OK(after(5, s, s0));
-        if (colsum(plan, h->part_b[2], h->dh1, H, B, H, grad + L.b1, H, nullptr, s0)) return -2;
-        if (wgrad_tma(h->part_w[2], H, S, h->dh1, h->dh1_lo, H, x, x_lo, S, grad + L.w1, H, nullptr, s)) return -2;
-        HRP_CUDA_OK(after(6, s0, s));
-        HRP_CUDA_OK(after(7, s1, s));
-        final_reduce_kernel<<<plan.blocks, 256, 0, s>>>(plan);
-        HRP_CUDA_OK(cudaGetLastError());
-        return 0;
-    }
     // side stream 1: transposed weight copies for the input-gradient GEMMs (needs the parameters only)
     HRP_CUDA_OK(after(0, s, s1));
     {
@@ -1925,17 +1690,21 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
         const long long *ix = (const long long *)idx;
         long long tot = B * (S + Az + 3);
         gather_batch_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix, B,
-                                                                         S, Az, h->x, h->x_lo, h->z, h->olp, h->adv, h->ret);
+                                                                         S, Az, h->x, h->z, h->olp, h->adv, h->ret);
         HRP_CUDA_OK(cudaGetLastError());
         x = h->x; z = h->z; olp = h->olp; ad = h->adv; rt = h->ret;
     }
     if (int rc = forward_impl(h, params, x, B, nullptr, nullptr, s)) return rc;   // trunk + hidden head layers
-    if (h->cat) HRP_CUDA_OK(heads_loss_cat(z, olp, ad, rt, (float *)nullptr));
+    if (h->cat) HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_cat_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256),
+                                           0, s, (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2,
+                                           params + L.ba2, params + L.wc2, params + L.bc2, z, olp, ad, rt, B, A, eps_clip,
+                                           value_coef, entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H,
+                                           metrics, h->loss_part, h->loss_counter));
     else HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
                                (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
                                params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip, value_coef,
-                               entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, (float *)nullptr,
-                               grad + L.log_std, metrics, h->loss_part, h->loss_counter));
+                               entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, grad + L.log_std, metrics,
+                               h->loss_part, h->loss_counter));
     const float *a1 = h->ac, *c1 = h->ac + H;
     ReducePlan plan;
     plan.nseg = 0; plan.blocks = 0;

@@ -108,11 +108,6 @@ class ActorCritic:
         # exploration noise is keyed by (seed, global row, draw), so shards draw different noise and a sharded
         # rollout reproduces the single-process one
         self.row_base = 0
-        # the native weight copies of the tensor-core path are kept across forward / act calls while the parameters
-        # are unchanged: torch's version counter sees every in-place torch write to the flat buffer (load_state_dict,
-        # copy_ through a view), `native_updates` counts the optimizer steps the library applied through raw pointers
-        self.native_updates = 0
-        self._held_key = None
 
     def _ensure_workspace(self, batch: int) -> None:
         if batch <= self.max_batch:
@@ -174,17 +169,6 @@ class ActorCritic:
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
 
-    def _sync_weight_copies(self) -> None:
-        """Before a forward / act call: let the library reuse its weight copies if nothing wrote the parameters."""
-        key = (self.flat._version, self.native_updates, self._h.value, self.workspace_generation)
-        if key != self._held_key:
-            self._lib.hrp_ppo_hold_weights(self._h, 0)   # refresh on this call ...
-            self._held_key = key
-            self._hold_next = True
-        elif getattr(self, "_hold_next", False):
-            self._lib.hrp_ppo_hold_weights(self._h, 1)   # ... and keep from the next one on
-            self._hold_next = False
-
     def _as_states(self, x) -> torch.Tensor:
         if torch.is_tensor(x) and x.dtype == torch.float32 and x.device == self.device and x.is_contiguous():
             return x
@@ -204,7 +188,6 @@ class ActorCritic:
         self._ensure_workspace(B)
         mean = torch.empty((B, self.action_dim), dtype=torch.float32, device=self.device)
         value = torch.empty((B, 1), dtype=torch.float32, device=self.device)
-        self._sync_weight_copies()
         _lib.check(self._lib.hrp_ppo_forward(self._h, self.flat.data_ptr(), xb.data_ptr(), B, mean.data_ptr(),
                                              value.data_ptr(), self._stream()), "hrp_ppo_forward")
         std = None if self.discrete else self.log_std.exp()
@@ -217,15 +200,11 @@ class ActorCritic:
     # -- batched get_action: everything stays on the device -------------------------------------
     def act(self, states: torch.Tensor, noise: Optional[torch.Tensor] = None, deterministic: bool = False,
             out: Optional[Dict[str, torch.Tensor]] = None, lane: int = 0,
-            stream: Optional[int] = None, draw_counter: Optional[torch.Tensor] = None,
-            reuse_weight_copies: bool = False) -> Dict[str, torch.Tensor]:
+            stream: Optional[int] = None, draw_counter: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         """``get_action`` for [B, S] states -> dict(action, pre_tanh [B, A]; log_prob, value [B]).  ``stream``: raw
         ``cudaStream_t`` to enqueue on instead of torch's current stream (the multiplexer's stream ring).
         ``draw_counter``: int64 CUDA tensor [2] = (draw, 0) that replaces the host-side draw counter of the sampling
-        path, so that the call can be captured in a CUDA graph and replayed (``new_draw_counter``); such a capture
-        always contains the weight preparation, i.e. a replay sees the current parameters -- unless
-        ``reuse_weight_copies`` says that an earlier call of the SAME capture already prepared them (the second and
-        later steps of a captured rollout).
+        path, so that the call can be captured in a CUDA graph and replayed (``new_draw_counter``).
 
         ``lane`` > 0 selects a separate native workspace (same parameters) so that calls on different CUDA streams
         may overlap: the two env groups of the pipelined host-buffer loop (bench.py e2e) act concurrently.
@@ -241,11 +220,6 @@ class ActorCritic:
         self._ensure_workspace(B)
         if out is None:
             out = self._new_act_out(B)
-        if draw_counter is not None:
-            self._lib.hrp_ppo_hold_weights(self._h, 1 if reuse_weight_copies else 0)
-            self._held_key = None
-        else:
-            self._sync_weight_copies()
         if stream is None:
             stream = self._stream()
         if not deterministic and noise is None and draw_counter is not None:
@@ -322,7 +296,7 @@ class ActorCritic:
         return torch.tensor([self._draw, 0], dtype=torch.int64, device=self.device)
 
     def _act_lane(self, states, B, out, lane, deterministic, noise, draw_counter=None):
-        """act() on an additional workspace (its GEMM scratch, weight copies and hold state are its own)."""
+        """act() on an additional workspace (its GEMM scratch is its own)."""
         if deterministic or noise is not None:
             raise ValueError("workspace lanes serve the sampling rollout path only")
         lanes = self.__dict__.setdefault("_lanes", {})
@@ -338,7 +312,6 @@ class ActorCritic:
         if out is None:
             out = self._new_act_out(B)
         if draw_counter is not None:
-            self._lib.hrp_ppo_hold_weights(h[0], 0)
             _lib.check(self._lib.hrp_ppo_act_sample_ctr(h[0], self.flat.data_ptr(), states.data_ptr(), self._noise_seed,
                                                         draw_counter.data_ptr(), int(self.row_base), B,
                                                         out["action"].data_ptr(), out["pre_tanh"].data_ptr(),
@@ -599,10 +572,10 @@ class PPOAgent:
 
     def act(self, states: torch.Tensor, deterministic: bool = False, noise: Optional[torch.Tensor] = None,
             out: Optional[Dict[str, torch.Tensor]] = None, lane: int = 0, stream: Optional[int] = None,
-            draw_counter: Optional[torch.Tensor] = None, reuse_weight_copies: bool = False) -> Dict[str, torch.Tensor]:
+            draw_counter: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
         self.launches += 1
         return self.actor_critic.act(states, noise=noise, deterministic=deterministic, out=out, lane=lane, stream=stream,
-                                     draw_counter=draw_counter, reuse_weight_copies=reuse_weight_copies)
+                                     draw_counter=draw_counter)
 
     # -- distributed helpers (ppo/distributed.py) ---------------------------------------------------
     @staticmethod
@@ -672,7 +645,6 @@ class PPOAgent:
     # -- one optimizer step on minibatch ``idx`` (device int64) ----------------------------------
     def _minibatch_step(self, flat: Dict[str, torch.Tensor], idx: Optional[torch.Tensor], B: int, world: int) -> None:
         ac, opt, s = self.actor_critic, self.optimizer, self.actor_critic._stream()
-        ac.native_updates += 1   # the parameters change through raw pointers: the held weight copies are stale
         if world > 1 and self._comm is not None:
             self.grad = self._grad_parity[self._lib.hrp_comm_parity(self._comm)]   # the buffer of this step's parity
         _lib.check(self._lib.hrp_ppo_loss_grad(
@@ -779,7 +751,6 @@ class PPOAgent:
                     _lib.check(self._lib.hrp_comm_note_replay(self._comm), "hrp_comm_note_replay")
                     self.grad = self._grad_parity[parity]
                 g.replay()
-                ac.native_updates += 1
                 self.launches += 2
             st["warm"] = True
 

@@ -254,7 +254,7 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
             if counter is None:
                 agent.act(states[t], noise=None if noise is None else noise[t], out=out)
             else:
-                agent.act(states[t], out=out, draw_counter=counter, reuse_weight_copies=t > 0)
+                agent.act(states[t], out=out, draw_counter=counter)
             vec_env.step(r["action"][t], out=states[t + 1].view(E, vec_env.N, vec_env.F_out), reward_out=r["reward"][t],
                          terminated_out=r["terminated"][t], truncated_out=r["truncated"][t])
         torch.bitwise_or(r["terminated"], r["truncated"], out=r["done"])
@@ -288,7 +288,6 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     cache["graph"].replay()
     ac._draw += T
     cache["expected"] = ac._draw
-    ac._held_key = None
     agent.launches += T
     vec_env.launches += T
     return r

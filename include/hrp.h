@@ -241,11 +241,6 @@ int hrp_ppo_create_ex(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
                       int32_t device, uint32_t flags, hrp_ppo **out);
 int hrp_ppo_destroy(hrp_ppo *h);
 
-/* The tensor-core path multiplies 16-byte aligned copies of the weight matrices (plus their 3xTF32 "lo" parts), which
- * every forward / act call refreshes from params_dev first.  A caller that knows the parameters have not changed since
- * its previous call may say so: hold = 1 keeps the copies for the following calls with the same params_dev, until
- * hrp_ppo_hold_weights(h, 0) or the next hrp_ppo_loss_grad (a rollout of T policy steps refreshes them once). */
-int hrp_ppo_hold_weights(hrp_ppo *h, int32_t hold);
 /* ActorCritic.forward (agent.py:46-54): states[B,S] -> mean[B,A], value[B] */
 int hrp_ppo_forward(hrp_ppo *h, const float *params_dev, const float *states_dev, int64_t batch,
                     float *mean_dev, float *value_dev, void *stream);

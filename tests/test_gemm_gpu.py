@@ -30,10 +30,10 @@ CASES = [  # (M, N, K, a_k_contig, b_k_contig)
     (512, 256, 4096, False, False),  # [dWa1 ; dWc1]
     (64, 256, 60, True, True),       # the reference's minibatch sizes (main.py:53): one partial M tile
     (32, 128, 128, True, False),
-    (200, 96, 72, True, True),       # ragged M / N / K with 16-byte aligned pitches (tensor-map path)
+    (200, 96, 72, True, True),       # ragged M / N / K with 16-byte aligned pitches
     (72, 200, 136, False, False),
     (136, 72, 200, False, True),
-    (100, 70, 45, True, True),       # ragged edges everywhere, unaligned pitches (register-staged fallback)
+    (100, 70, 45, True, True),       # ragged edges everywhere, unaligned pitches
     (129, 257, 33, False, True),
     (32, 32, 8, True, True),
 ]

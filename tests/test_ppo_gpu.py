@@ -162,8 +162,7 @@ def test_full_update_matches_reference(name):
     assert len(agent.memory) == 0
 
 
-def test_loss_grad_large_batch_matches_oracle():
-    """BASELINE-size minibatch (4096 x S=60, H=256): gradient vs the torch fp32 oracle (split-K wgrad path)."""
+def _check_large_batch_loss_grad(gather):
     S, A, H, B = 60, 2, 256, 4096
     torch.manual_seed(1)
     agent = _agent(S, A, H, B)
@@ -178,11 +177,21 @@ def test_loss_grad_large_batch_matches_oracle():
     r = ppo_ref.loss_and_grad(flat, x, z, old, adv, ret, S, A, H)
     dev = {"states": x.cuda(), "pre_tanh": z.cuda(), "log_prob": old.cuda(), "adv": adv.cuda(), "ret": ret.cuda()}
     agent._metrics.zero_()
-    agent._minibatch_step(dev, None, B, 1)
+    agent._minibatch_step(dev, torch.arange(B, device="cuda:0") if gather else None, B, 1)
     m = agent._metrics.cpu().numpy()
     assert abs(m[0] - r["loss"]) < 5e-5 and abs(m[4] - r["clip_fraction"]) < 1e-3
     want = r["grad"].numpy()
     np.testing.assert_allclose(agent.grad.cpu().numpy(), want, atol=2e-4 * np.abs(want).max() + 1e-6)
+
+
+def test_loss_grad_large_batch_matches_oracle():
+    """BASELINE-size minibatch (4096 x S=60, H=256): gradient vs the torch fp32 oracle (split-K wgrad path)."""
+    _check_large_batch_loss_grad(gather=False)
+
+
+def test_loss_grad_large_batch_through_gather_matches_oracle():
+    """The same minibatch taken from the rollout by the gather kernel (idx = arange(B)), same tolerances."""
+    _check_large_batch_loss_grad(gather=True)
 
 
 def test_checkpoint_roundtrip_and_reference_key_names(tmp_path):
@@ -458,49 +467,6 @@ def test_full_update_at_hidden_512_matches_reference():
     err = float(np.abs(motion[::257] - g["motion_samples"]).max())
     print("H=512 update: max parameter motion", moved, "max error of the sampled entries", err)
     assert err <= 5e-4 * moved   # measured 3.3e-5 of the motion after these 16 optimizer steps
-
-
-def test_tma_gemm_path_matches_the_reference_too(monkeypatch):
-    """HRP_TMA=1 routes the trunk, input-gradient and weight-gradient GEMMs through the TMA-fed kernel on pre-split
-    operands (csrc/hrp_gemm_tma.cu): same fixture, same tolerances as the default path, and the two paths agree."""
-    g = golden("ppo_step_s60_h256_b64.npz")
-    S, A, H, B, _ = (int(v) for v in g["dims"])
-    cu = lambda k: torch.from_numpy(g[k]).cuda()
-    flat = {"states": cu("states"), "pre_tanh": cu("pre_tanh"), "log_prob": cu("old_logp"), "adv": cu("adv"), "ret": cu("ret")}
-    grads = {}
-    for tma in ("0", "1"):
-        monkeypatch.setenv("HRP_TMA", tma)
-        agent = _agent(S, A, H, B)
-        _load_flat(agent, g["params0"])
-        mean, std, value = agent.actor_critic.forward(cu("states"))
-        np.testing.assert_allclose(mean.cpu().numpy(), g["mean"], atol=2e-5)
-        np.testing.assert_allclose(value.cpu().numpy(), g["value"], atol=2e-5)
-        agent._metrics.zero_()
-        agent._minibatch_step(flat, None, B, 1)
-        m = agent._metrics.cpu().numpy()
-        assert abs(m[0] - float(g["loss"])) < 2e-5
-        grads[tma] = agent.grad.cpu().numpy()
-        np.testing.assert_allclose(grads[tma], g["grads"], atol=1e-4 * np.abs(g["grads"]).max() + 2e-6)
-    np.testing.assert_allclose(grads["1"], grads["0"], atol=2e-5 * np.abs(g["grads"]).max() + 1e-7)
-    # BASELINE-size minibatch through the TMA path against the torch fp32 oracle (MN-major weight-gradient GEMMs)
-    monkeypatch.setenv("HRP_TMA", "1")
-    S, A, H, B = 60, 2, 256, 4096
-    torch.manual_seed(1)
-    agent = _agent(S, A, H, B)
-    gen = torch.Generator().manual_seed(2)
-    x = torch.randn(B, S, generator=gen) * 0.5
-    flat0 = agent.actor_critic.flat.cpu()
-    mean, log_std, _ = ppo_ref.forward(flat0, x, S, A, H)
-    z = mean + torch.randn(B, A, generator=gen)
-    logp, _, _ = ppo_ref.evaluate(flat0, x, z, S, A, H)
-    old = logp + 0.2 * torch.randn(B, generator=gen)
-    adv, ret = torch.randn(B, generator=gen), torch.randn(B, generator=gen)
-    r = ppo_ref.loss_and_grad(flat0, x, z, old, adv, ret, S, A, H)
-    dev = {"states": x.cuda(), "pre_tanh": z.cuda(), "log_prob": old.cuda(), "adv": adv.cuda(), "ret": ret.cuda()}
-    agent._metrics.zero_()
-    agent._minibatch_step(dev, torch.arange(B, device="cuda:0"), B, 1)
-    want = r["grad"].numpy()
-    np.testing.assert_allclose(agent.grad.cpu().numpy(), want, atol=2e-4 * np.abs(want).max() + 1e-6)
 
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
