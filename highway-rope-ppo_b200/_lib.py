@@ -82,6 +82,7 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_env_num_vehicles": (C.c_int, [_vp]),
     "hrp_env_reset": (C.c_int, [_vp, _u64, _vp, _vp, _vp]),
     "hrp_env_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "hrp_env_step_final": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hrp_env_observe": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "hrp_env_step_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "hrp_env_reset_host": (C.c_int, [_vp, _u64, _vp]),
@@ -110,6 +111,7 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_ppo_act_multi": (C.c_int, [_vp, _i32, _vp]),
     "hrp_ppo_act_sample_ctr": (C.c_int, [_vp, _vp, _vp, _u64, _vp, _u64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "hrp_gae": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _vp, _vp, _vp]),
+    "hrp_gae_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _vp, _vp, _vp]),
     "hrp_adv_stats": (C.c_int, [_vp, _i64, _vp, _vp]),
     "hrp_adv_normalize": (C.c_int, [_vp, _i64, _vp, _vp]),
     "hrp_ppo_loss_grad": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp,

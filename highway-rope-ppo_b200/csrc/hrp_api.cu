@@ -296,6 +296,22 @@ int hrp_env_step(hrp_env *h, const float *actions_dev, float *obs_dev, float *re
                            row_vehicle_dev, (cudaStream_t)stream);
 }
 
+int hrp_env_step_final(hrp_env *h, const float *actions_dev, float *obs_dev, float *reward_dev,
+                       uint8_t *terminated_dev, uint8_t *truncated_dev, float *final_obs_dev, const int32_t *perm_dev,
+                       int32_t *row_vehicle_dev, void *stream)
+{
+    if (final_obs_dev && final_obs_dev == obs_dev) {
+        hrp_set_error("hrp_env_step_final: final_obs_dev must not be obs_dev (a respawned env writes both)");
+        return -1;
+    }
+    if (!h || !actions_dev || !obs_dev || !reward_dev || !terminated_dev || !truncated_dev) {
+        hrp_set_error("hrp_env_step_final: null argument");
+        return -1;
+    }
+    return hrp_launch_step(h->P, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
+                           row_vehicle_dev, (cudaStream_t)stream, final_obs_dev);
+}
+
 int hrp_env_observe(hrp_env *h, float *obs_dev, const int32_t *perm_dev, int32_t *row_vehicle_dev,
                     void *stream)
 {

@@ -870,11 +870,13 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
 }
 
 // ---------------------------------------------------------------------------------------
-template <typename R, int WARPS>
+// FINAL: the instantiation with the final-observation output (hrp_env_step_final).  A compile-time switch, so that the
+// default kernels carry none of its code: the step kernel is sensitive to instruction-cache pressure (DESIGN.md §3.1).
+template <typename R, int WARPS, bool FINAL = false>
 __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restrict__ actions, float *__restrict__ obs,
                                           float *__restrict__ reward, uint8_t *__restrict__ term,
                                           uint8_t *__restrict__ trunc, const int32_t *__restrict__ perm,
-                                          int32_t *__restrict__ row_vehicle)
+                                          int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs = nullptr)
 {
     __shared__ WarpS<R> smem[WARPS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -963,18 +965,42 @@ __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restri
     }
     done = __shfl_sync(HRP_FULL, done, 0);
     uint32_t draw = P.obs_draw[e];
-    if (done && P.autoreset) {
-        uint32_t ep = P.episode[e] + 1;
-        spawn_env(P, S, u, e, lane, ep, xref);
-        if (lane == 0) { P.episode[e] = ep; tnow = 0.0; }
-    } else {
+    if constexpr (FINAL) {
+        // Pass 0, finished envs only: the observation of the terminal state into final_obs, before a respawn overwrites
+        // it -- the same publish of the headings and the same shuffle draw as the observation of pass 1, so it is bit
+        // for bit what an autoreset = 0 handle returns (in shuffled mode both observations of the step use one row
+        // permutation; row_vehicle describes `obs` only).  Pass 1 is the default path below.  A loop rather than a
+        // second call: with one call site each, observe_env and spawn_env are compiled as in the default kernel, so
+        // both observations round exactly as the default kernel's does.
+#pragma unroll 1
+        for (int pass = done ? 0 : 1; pass < 2; ++pass) {
+            if (pass == 1 && done && P.autoreset) {
+                uint32_t ep = P.episode[e] + 1;
+                spawn_env(P, S, u, e, lane, ep, xref);
+                if (lane == 0) { P.episode[e] = ep; tnow = 0.0; }
+            } else {
 #pragma unroll
-        for (int q = 0; q < 2; ++q)
-            if (lane + 32 * q < P.V) S.h[lane + 32 * q] = u[q].h;
-        __syncwarp();
+                for (int q = 0; q < 2; ++q)
+                    if (lane + 32 * q < P.V) S.h[lane + 32 * q] = u[q].h;
+                __syncwarp();
+            }
+            if (pass == 1 && lane == 0) { P.time[e] = tnow; P.obs_draw[e] = draw + 1; }
+            observe_env(P, S, e, lane, pass ? obs : final_obs, perm, pass ? row_vehicle : nullptr, draw);
+        }
+    } else {
+        if (done && P.autoreset) {
+            uint32_t ep = P.episode[e] + 1;
+            spawn_env(P, S, u, e, lane, ep, xref);
+            if (lane == 0) { P.episode[e] = ep; tnow = 0.0; }
+        } else {
+#pragma unroll
+            for (int q = 0; q < 2; ++q)
+                if (lane + 32 * q < P.V) S.h[lane + 32 * q] = u[q].h;
+            __syncwarp();
+        }
+        if (lane == 0) { P.time[e] = tnow; P.obs_draw[e] = draw + 1; }
+        observe_env(P, S, e, lane, obs, perm, row_vehicle, draw);
     }
-    if (lane == 0) { P.time[e] = tnow; P.obs_draw[e] = draw + 1; }
-    observe_env(P, S, e, lane, obs, perm, row_vehicle, draw);
     store_env(P, u, e, lane);
 }
 
@@ -992,6 +1018,22 @@ hrp_step_kernel_f64(const EnvDev P, const float *__restrict__ actions, float *__
                     const int32_t *__restrict__ perm, int32_t *__restrict__ row_vehicle)
 {
     step_body<double, HRP_WARPS_PER_CTA_F64>(P, actions, obs, reward, term, trunc, perm, row_vehicle);
+}
+// the same two with the final-observation output: final_obs[E, N, F_out] of the envs whose episode ended on this step
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA, HRP_STEP_CTAS_PER_SM)
+hrp_step_kernel_final(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                      float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                      const int32_t *__restrict__ perm, int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs)
+{
+    step_body<float, HRP_WARPS_PER_CTA, true>(P, actions, obs, reward, term, trunc, perm, row_vehicle, final_obs);
+}
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA_F64)
+hrp_step_kernel_f64_final(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                          float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                          const int32_t *__restrict__ perm, int32_t *__restrict__ row_vehicle,
+                          float *__restrict__ final_obs)
+{
+    step_body<double, HRP_WARPS_PER_CTA_F64, true>(P, actions, obs, reward, term, trunc, perm, row_vehicle, final_obs);
 }
 
 template <typename R, int WARPS>
@@ -1051,15 +1093,25 @@ hrp_embed_kernel(int kind, int edim, int use_euclid, int ego_idx, float max_dist
 }  // namespace
 
 int hrp_launch_step(const EnvDev &P, const float *actions, float *obs, float *reward, uint8_t *term,
-                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s)
+                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s, float *final_obs)
 {
     if (P.real64) {
         int grid = (P.E + HRP_WARPS_PER_CTA_F64 - 1) / HRP_WARPS_PER_CTA_F64;
+        if (final_obs) {
+            HRP_CUDA_OK(hrp_launch_pdl(hrp_step_kernel_f64_final, dim3(grid), dim3(32 * HRP_WARPS_PER_CTA_F64), 0, s, P,
+                                       actions, obs, reward, term, trunc, perm, row_vehicle, final_obs));
+            return 0;
+        }
         HRP_CUDA_OK(hrp_launch_pdl(hrp_step_kernel_f64, dim3(grid), dim3(32 * HRP_WARPS_PER_CTA_F64), 0, s, P, actions, obs,
                                    reward, term, trunc, perm, row_vehicle));
         return 0;
     }
     int grid = (P.E + HRP_WARPS_PER_CTA - 1) / HRP_WARPS_PER_CTA;
+    if (final_obs) {
+        HRP_CUDA_OK(hrp_launch_pdl(hrp_step_kernel_final, dim3(grid), dim3(32 * HRP_WARPS_PER_CTA), 0, s, P, actions, obs,
+                                   reward, term, trunc, perm, row_vehicle, final_obs));
+        return 0;
+    }
     HRP_CUDA_OK(hrp_launch_pdl(hrp_step_kernel, dim3(grid), dim3(32 * HRP_WARPS_PER_CTA), 0, s, P, actions, obs, reward, term,
                                trunc, perm, row_vehicle));
     return 0;

@@ -114,9 +114,10 @@ struct TcDots {
     int skip_store;    // do not write the activation itself
 };
 
-// launchers implemented in hrp_env.cu
+// launchers implemented in hrp_env.cu.  final_obs non-null: the final-observation instantiation of the step kernel.
 int hrp_launch_step(const EnvDev &P, const float *actions, float *obs, float *reward, uint8_t *term,
-                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s);
+                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
+                    float *final_obs = nullptr);
 int hrp_launch_observe(const EnvDev &P, float *obs, const int32_t *perm, int32_t *row_vehicle,
                        cudaStream_t s);
 int hrp_launch_reset(const EnvDev &P, const uint8_t *mask, float *obs, cudaStream_t s);

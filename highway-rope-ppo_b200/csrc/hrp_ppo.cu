@@ -1015,6 +1015,36 @@ __global__ void gae_kernel(const float *__restrict__ reward, const float *__rest
     }
 }
 
+// gae_kernel with time-limit bootstrapping (hrp_gae_ex): a truncated step that did not also terminate is bootstrapped
+// with V(s_final) instead of 0.  The bootstrap is a select, so final_value rows of other steps are never read into the
+// arithmetic (they may hold anything).  Without a truncated step (or final_value == nullptr) every operation is the
+// one gae_kernel performs on done = terminated | truncated, so the result is bit-identical.
+__global__ void gae_ex_kernel(const float *__restrict__ reward, const float *__restrict__ value,
+                              const uint8_t *__restrict__ terminated, const uint8_t *__restrict__ truncated,
+                              const float *__restrict__ final_value, const float *__restrict__ last_value, long long T,
+                              long long E, double gamma, double lam, float *__restrict__ adv, float *__restrict__ ret)
+{
+    long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= E) return;
+    double next_v = last_value ? (double)last_value[e] : 0.0;
+    float last_adv = 0.f;
+    for (long long t = T - 1; t >= 0; --t) {
+        size_t o = (size_t)t * E + e;
+        const bool term = terminated[o] != 0, tr = truncated[o] != 0;
+        const bool boot = final_value && tr && !term;   // a crash on the last step is not bootstrapped
+        double nd = 1.0 - (double)(term || tr);
+        double v = (double)value[o];
+        double bv = boot ? (double)final_value[o] : next_v;
+        double bm = boot ? 1.0 : nd;
+        double delta = (double)reward[o] + gamma * bv * bm - v;
+        float a = (float)(delta + gamma * lam * nd * (double)last_adv);
+        adv[o] = a;
+        ret[o] = a + value[o];
+        last_adv = a;
+        next_v = v;
+    }
+}
+
 // sum, sum of squares, count of the local advantages (fp64), deterministic two-stage
 __global__ void __launch_bounds__(256)
 adv_stats_kernel(const float *__restrict__ adv, long long n, double *__restrict__ part)
@@ -1630,6 +1660,22 @@ int hrp_gae(const float *reward, const float *value, const uint8_t *done, const 
     if (!reward || !value || !done || !adv || !ret || T < 1 || E < 1) { hrp_set_error("hrp_gae: bad arguments"); return -1; }
     gae_kernel<<<(unsigned)((E + 127) / 128), 128, 0, (cudaStream_t)stream>>>(reward, value, done, last_value, T, E,
                                                                             gamma, lam, adv, ret);
+    HRP_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int hrp_gae_ex(const float *reward, const float *value, const uint8_t *terminated, const uint8_t *truncated,
+               const float *final_value, const float *last_value, int64_t T, int64_t E, double gamma, double lam,
+               float *adv, float *ret, void *stream)
+{
+    const char *missing = !reward ? "reward_dev" : !value ? "value_dev" : !terminated ? "terminated_dev"
+                        : !truncated ? "truncated_dev" : !adv ? "adv_dev" : !ret ? "ret_dev" : nullptr;
+    if (missing) { hrp_set_error("hrp_gae_ex: %s is null", missing); return -1; }
+    if (T < 1) { hrp_set_error("hrp_gae_ex: T = %lld < 1", (long long)T); return -1; }
+    if (E < 1) { hrp_set_error("hrp_gae_ex: E = %lld < 1", (long long)E); return -1; }
+    gae_ex_kernel<<<(unsigned)((E + 127) / 128), 128, 0, (cudaStream_t)stream>>>(reward, value, terminated, truncated,
+                                                                               final_value, last_value, T, E, gamma, lam,
+                                                                               adv, ret);
     HRP_CUDA_OK(cudaGetLastError());
     return 0;
 }

@@ -217,13 +217,17 @@ class HighwayVecEnv:
     def step(self, actions: torch.Tensor, perm: Optional[torch.Tensor] = None,
              row_vehicle: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
              reward_out: Optional[torch.Tensor] = None, terminated_out: Optional[torch.Tensor] = None,
-             truncated_out: Optional[torch.Tensor] = None):
+             truncated_out: Optional[torch.Tensor] = None, final_obs_out: Optional[torch.Tensor] = None):
         """One policy step of every env.  ``actions``: float32 [E, 2] on the device.
 
         Returns (obs [E,N,F_out], reward [E], terminated [E] uint8, truncated [E] uint8); the
         tensors are the handle's own output buffers unless ``out`` (observation) / ``reward_out`` /
         ``terminated_out`` / ``truncated_out`` name the caller's (contiguous, e.g. the slot of a rollout buffer: the
         kernel then writes the rollout directly, no copy kernels between the step and the next policy forward).
+
+        ``final_obs_out`` (contiguous float32 CUDA tensor of E x N x F_out, not ``out``): every env whose episode ended
+        on this step writes the observation of its terminal state there, before the respawn (``hrp_env_step_final``);
+        the other rows are left as they are.
         """
         if actions.device != self.device or actions.dtype != torch.float32 or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.float32).contiguous()
@@ -237,9 +241,19 @@ class HighwayVecEnv:
         rew = self.reward if reward_out is None else reward_out
         term = self.terminated if terminated_out is None else terminated_out
         trunc = self.truncated if truncated_out is None else truncated_out
-        _lib.check(self._lib.hrp_env_step(self._h, actions.data_ptr(), obs.data_ptr(), rew.data_ptr(),
-                                          term.data_ptr(), trunc.data_ptr(), _lib.ptr(perm),
-                                          _lib.ptr(row_vehicle), self._stream()), "hrp_env_step")
+        if final_obs_out is None:
+            _lib.check(self._lib.hrp_env_step(self._h, actions.data_ptr(), obs.data_ptr(), rew.data_ptr(),
+                                              term.data_ptr(), trunc.data_ptr(), _lib.ptr(perm),
+                                              _lib.ptr(row_vehicle), self._stream()), "hrp_env_step")
+        else:
+            if (not final_obs_out.is_cuda or final_obs_out.dtype != torch.float32 or not final_obs_out.is_contiguous()
+                    or final_obs_out.numel() != obs.numel()):
+                raise ValueError(f"final_obs_out must be a contiguous float32 CUDA tensor of {self.num_envs} x "
+                                 f"{self.N} x {self.F_out}")
+            _lib.check(self._lib.hrp_env_step_final(self._h, actions.data_ptr(), obs.data_ptr(), rew.data_ptr(),
+                                                    term.data_ptr(), trunc.data_ptr(), final_obs_out.data_ptr(),
+                                                    _lib.ptr(perm), _lib.ptr(row_vehicle), self._stream()),
+                       "hrp_env_step_final")
         self.launches += 1
         return obs, rew, term, trunc
 

@@ -99,6 +99,7 @@ class ActorCritic:
             self._views[name] = view
             off += n
         self._h = C.c_void_p()
+        self._head_scratch: Optional[torch.Tensor] = None   # policy-head output of critic_into
         self.max_batch = 0
         self.workspace_generation = 0   # bumped whenever the native workspace is re-created (CUDA-graph cache key)
         self._ensure_workspace(max_batch)
@@ -178,7 +179,8 @@ class ActorCritic:
         return x.contiguous()
 
     # -- ActorCritic.forward (agent.py:46-54) --------------------------------------------------
-    def forward(self, x):
+    def forward(self, x, *, out=None):
+        """``out`` = (mean [B, A], value [B]): preallocated outputs (contiguous float32), e.g. for a captured launch."""
         x = self._as_states(x)
         single = x.dim() == 1
         xb = x.view(1, -1) if single else x.reshape(-1, x.shape[-1])
@@ -186,8 +188,14 @@ class ActorCritic:
         if xb.shape[1] != self.state_dim:
             raise ValueError(f"expected states of width {self.state_dim}, got {xb.shape[1]}")
         self._ensure_workspace(B)
-        mean = torch.empty((B, self.action_dim), dtype=torch.float32, device=self.device)
-        value = torch.empty((B, 1), dtype=torch.float32, device=self.device)
+        if out is None:
+            mean = torch.empty((B, self.action_dim), dtype=torch.float32, device=self.device)
+            value = torch.empty((B, 1), dtype=torch.float32, device=self.device)
+        else:
+            mean, value = out
+            if mean.numel() != B * self.action_dim or value.numel() != B:
+                raise ValueError(f"out must hold [{B}, {self.action_dim}] means and [{B}] values")
+            value = value.view(B, 1)
         _lib.check(self._lib.hrp_ppo_forward(self._h, self.flat.data_ptr(), xb.data_ptr(), B, mean.data_ptr(),
                                              value.data_ptr(), self._stream()), "hrp_ppo_forward")
         std = None if self.discrete else self.log_std.exp()
@@ -196,6 +204,16 @@ class ActorCritic:
         return mean, std, value
 
     __call__ = forward
+
+    def critic_into(self, states: torch.Tensor, value_out: torch.Tensor) -> torch.Tensor:
+        """V(states) of [B, S] device states into ``value_out`` [B], with no allocation per call (capturable in a CUDA
+        graph; the policy head's output goes to a scratch buffer of this instance)."""
+        B = states.shape[0]
+        self._ensure_workspace(B)
+        if self._head_scratch is None or self._head_scratch.shape[0] < self.max_batch:
+            self._head_scratch = torch.empty((self.max_batch, self.action_dim), dtype=torch.float32, device=self.device)
+        self.forward(states, out=(self._head_scratch[:B], value_out))
+        return value_out
 
     # -- batched get_action: everything stays on the device -------------------------------------
     def act(self, states: torch.Tensor, noise: Optional[torch.Tensor] = None, deterministic: bool = False,
@@ -394,6 +412,7 @@ class PPOMemory:
         self.dones: List[bool] = []
         self.values: List[float] = []
         self.rollout = None
+        self.bootstrap_truncated = False   # the device rollout was collected with final_states / final_value
 
     def __len__(self):
         if self.rollout is not None:
@@ -402,10 +421,15 @@ class PPOMemory:
 
     # -- device-resident [T, E] rollout -----------------------------------------------------------
     def begin_rollout(self, T: int, E: int, state_dim: int, action_dim: int,
-                      pre_dim: Optional[int] = None) -> Dict[str, torch.Tensor]:
+                      pre_dim: Optional[int] = None, bootstrap_truncated: bool = False) -> Dict[str, torch.Tensor]:
         """Allocate (or reuse) time-major buffers: states [T+1,E,S] (slot T holds the bootstrap
         observation), action [T,E,A], pre_tanh [T,E,pre_dim] (default A), log_prob/value/reward [T,E],
-        done [T,E] uint8."""
+        done [T,E] uint8.
+
+        ``bootstrap_truncated``: also final_states [T,E,S] (the observation each finished episode ended in) and
+        final_value [T,E] (the critic's value of it), zero-filled when allocated, and ``update`` bootstraps truncated
+        steps with final_value (``hrp_gae_ex``).  A rollout begun without the flag gets the reference's semantics
+        (truncation masks the bootstrap), whatever the reused buffers hold."""
         pre_dim = action_dim if pre_dim is None else pre_dim
         r = self.rollout
         if (r is None or r["reward"].shape != (T, E) or r["states"].shape[2] != state_dim
@@ -421,7 +445,12 @@ class PPOMemory:
                  # what the step kernel writes; `done` = terminated | truncated, formed once per rollout
                  "terminated": torch.empty((T, E), dtype=torch.uint8, device=d),
                  "truncated": torch.empty((T, E), dtype=torch.uint8, device=d)}
+        if bootstrap_truncated and "final_states" not in r:
+            d = self.device
+            r["final_states"] = torch.zeros((T, E, state_dim), dtype=torch.float32, device=d)
+            r["final_value"] = torch.zeros((T, E), dtype=torch.float32, device=d)
         self.rollout = r
+        self.bootstrap_truncated = bool(bootstrap_truncated)
         return r
 
     def _from_lists(self) -> Dict[str, torch.Tensor]:
@@ -464,8 +493,14 @@ class PPOMemory:
                 r["log_prob"].reshape(-1))
 
 
-def gae(reward: torch.Tensor, value: torch.Tensor, done: torch.Tensor, last_value, gamma: float, lam: float):
-    """``PPOMemory.compute_advantages`` over time-major [T, E] tensors (reverse scan kernel)."""
+def gae(reward: torch.Tensor, value: torch.Tensor, done: Optional[torch.Tensor], last_value, gamma: float, lam: float,
+        *, terminated: Optional[torch.Tensor] = None, truncated: Optional[torch.Tensor] = None,
+        final_value: Optional[torch.Tensor] = None):
+    """``PPOMemory.compute_advantages`` over time-major [T, E] tensors (reverse scan kernel).
+
+    With ``terminated`` and ``truncated`` (``done`` is then ignored) a truncated step that did not terminate is
+    bootstrapped with ``final_value`` [T, E], V of the observation the episode ended in (``hrp_gae_ex``); rows of other
+    steps are not read.  ``final_value=None``: the same as ``done = terminated | truncated``."""
     lib = _lib.load()
     T, E = reward.shape
     dev = reward.device
@@ -474,6 +509,22 @@ def gae(reward: torch.Tensor, value: torch.Tensor, done: torch.Tensor, last_valu
     last_value = last_value.to(device=dev, dtype=torch.float32).reshape(E).contiguous()
     adv = torch.empty((T, E), dtype=torch.float32, device=dev)
     ret = torch.empty((T, E), dtype=torch.float32, device=dev)
+    if terminated is not None or truncated is not None:
+        if terminated is None or truncated is None:
+            raise ValueError("gae: terminated and truncated go together")
+        terminated = terminated.to(torch.uint8).contiguous()
+        truncated = truncated.to(torch.uint8).contiguous()
+        if final_value is not None:
+            final_value = final_value.to(device=dev, dtype=torch.float32).contiguous()
+            if final_value.numel() != T * E:
+                raise ValueError(f"final_value must hold [{T}, {E}] values")
+        _lib.check(lib.hrp_gae_ex(reward.contiguous().data_ptr(), value.contiguous().data_ptr(), terminated.data_ptr(),
+                                  truncated.data_ptr(), _lib.ptr(final_value), last_value.data_ptr(), T, E,
+                                  float(gamma), float(lam), adv.data_ptr(), ret.data_ptr(),
+                                  torch.cuda.current_stream(dev).cuda_stream), "hrp_gae_ex")
+        return adv, ret
+    if final_value is not None:
+        raise ValueError("gae: final_value needs terminated and truncated")
     done = done.to(torch.uint8).contiguous()
     _lib.check(lib.hrp_gae(reward.contiguous().data_ptr(), value.contiguous().data_ptr(), done.data_ptr(),
                            last_value.data_ptr(), T, E, float(gamma), float(lam), adv.data_ptr(), ret.data_ptr(),
@@ -769,7 +820,11 @@ class PPOAgent:
         S = ac.state_dim
         world = self._world()
         stream = ac._stream()
-        adv, ret = gae(r["reward"], r["value"], r["done"], last_value, self.gamma, self.lam)
+        if mem.rollout is not None and mem.bootstrap_truncated:   # collect_rollout(bootstrap_truncated=True)
+            adv, ret = gae(r["reward"], r["value"], None, last_value, self.gamma, self.lam, terminated=r["terminated"],
+                           truncated=r["truncated"], final_value=r["final_value"])
+        else:
+            adv, ret = gae(r["reward"], r["value"], r["done"], last_value, self.gamma, self.lam)
         # advantage normalisation over the whole (global) buffer, unbiased std (agent.py:204)
         adv_n = adv.clone()
         _lib.check(self._lib.hrp_adv_stats(adv_n.data_ptr(), n, self._stats.data_ptr(), stream), "hrp_adv_stats")

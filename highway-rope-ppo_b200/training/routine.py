@@ -211,7 +211,8 @@ def _act_widths(vec_env, agent):
 
 
 def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
-                    noise: Optional[torch.Tensor] = None, use_graph: Optional[bool] = None) -> Dict[str, torch.Tensor]:
+                    noise: Optional[torch.Tensor] = None, use_graph: Optional[bool] = None,
+                    bootstrap_truncated: bool = False) -> Dict[str, torch.Tensor]:
     """T lock-step policy steps of every env into ``agent.memory``'s device rollout.
 
     The env kernel writes each observation straight into the rollout's next state slot, reward and flags into their
@@ -226,6 +227,12 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
 
     A discrete agent on a ``DiscreteMetaAction`` env writes action [T, E, 2] = (id, 0), which the env step reads as it
     is, and pre_tanh [T, E, 1] = id.
+
+    ``bootstrap_truncated=True`` handles time limits the standard way instead (not the reference's, which treats a
+    truncation as a termination): the step also writes the observation each finished episode ended in into
+    ``final_states[t]`` (``hrp_env_step_final``), the critic computes ``final_value[t]`` from it with the parameters
+    that produced ``value[t]``, and ``agent.update`` bootstraps every truncated step with it.  Two more launches per
+    step (the critic pass runs over all E rows; only the truncated ones are read), inside the captured graph.
     """
     A, Z = _act_widths(vec_env, agent)
     E, S = vec_env.num_envs, vec_env.N * vec_env.F_out
@@ -236,11 +243,12 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
         # (a single env acts through the matrix-vector kernel, which keeps its draw counter on the host)
         use_graph = noise is None and E > 1 and getattr(agent, "use_cuda_graphs", True)
     cache = getattr(agent, "_rollout_graph", None)
+    boot = bool(bootstrap_truncated)
     key = (getattr(vec_env, "uid", id(vec_env)), getattr(vec_env, "param_version", 0), T, E, S, A, Z,
-           ac.workspace_generation, ac.row_base)
+           ac.workspace_generation, ac.row_base, boot)
     if use_graph and cache is not None and cache["key"] == key and agent.memory.rollout is None:
         agent.memory.rollout = cache["r"]     # the buffers the captured launches write (PPOAgent.update dropped them)
-    r = agent.memory.begin_rollout(T, E, S, A, Z)
+    r = agent.memory.begin_rollout(T, E, S, A, Z, bootstrap_truncated=boot)
     states = r["states"]
     if obs is None:
         vec_env.observe(out=states[0].view(E, vec_env.N, vec_env.F_out))
@@ -256,7 +264,11 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
             else:
                 agent.act(states[t], out=out, draw_counter=counter)
             vec_env.step(r["action"][t], out=states[t + 1].view(E, vec_env.N, vec_env.F_out), reward_out=r["reward"][t],
-                         terminated_out=r["terminated"][t], truncated_out=r["truncated"][t])
+                         terminated_out=r["terminated"][t], truncated_out=r["truncated"][t],
+                         final_obs_out=r["final_states"][t] if boot else None)
+            if boot:
+                ac.critic_into(r["final_states"][t], r["final_value"][t])
+                agent.launches += 1
         torch.bitwise_or(r["terminated"], r["truncated"], out=r["done"])
 
     if not use_graph or noise is not None:
@@ -288,30 +300,32 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     cache["graph"].replay()
     ac._draw += T
     cache["expected"] = ac._draw
-    agent.launches += T
+    agent.launches += 2 * T if boot else T
     vec_env.launches += T
     return r
 
 
-def rollout_and_update(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None):
+def rollout_and_update(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None, bootstrap_truncated: bool = False):
     """One PPO iteration: T x E samples collected, then ``agent.update`` bootstrapped from V(s_T).
+    ``bootstrap_truncated``: see ``collect_rollout``.
     Returns (update metrics, the observation the next rollout starts from)."""
-    r = collect_rollout(vec_env, agent, T, obs)
+    r = collect_rollout(vec_env, agent, T, obs, bootstrap_truncated=bootstrap_truncated)
     last_obs = r["states"][T].clone()
     _, _, last_v = agent.actor_critic.forward(last_obs)
     return agent.update(last_value=last_v.view(-1)), last_obs
 
 
-def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, logger=None):
+def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, logger=None,
+                     bootstrap_truncated: bool = False):
     """``iterations`` PPO iterations on E lock-step envs; returns the list of update metrics with
-    mean step reward and samples/s added."""
+    mean step reward and samples/s added.  ``bootstrap_truncated``: see ``collect_rollout``."""
     logger = logger or logging.getLogger(__name__)
     _act_widths(vec_env, agent)
     obs = vec_env.reset(seed=seed)
     history = []
     for it in range(iterations):
         t0 = time.time()
-        metrics, obs = rollout_and_update(vec_env, agent, T, obs=obs)
+        metrics, obs = rollout_and_update(vec_env, agent, T, obs=obs, bootstrap_truncated=bootstrap_truncated)
         torch.cuda.synchronize(vec_env.device)
         dt = time.time() - t0
         metrics["samples_per_s"] = T * vec_env.num_envs / dt

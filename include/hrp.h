@@ -129,6 +129,21 @@ int hrp_env_step(hrp_env *env, const float *actions_dev, float *obs_dev, float *
                  uint8_t *terminated_dev, uint8_t *truncated_dev, const int32_t *perm_dev,
                  int32_t *row_vehicle_dev, void *stream);
 
+/* hrp_env_step that also returns the observation each finished episode ended in -- what a vectorised env with autoreset
+ * hands back as the final observation, so that a time-limit truncation can be bootstrapped with V(s_final).
+ * final_obs_dev (nullable) [E,N,F_out]: an env whose episode ended on this step (terminated or truncated) writes the
+ * observation of its terminal state there, BEFORE the respawn overwrites that state, with the normalisation, clipping,
+ * row order and embedding of obs_dev.  It uses the step's own shuffle draw and advances no counter: it is bit for bit
+ * the observation an autoreset = 0 handle returns from the same state and actions, and the new episode's first
+ * observation in obs_dev is unchanged.  In shuffled mode both observations therefore share one row permutation; an
+ * injected perm_dev applies to both.  row_vehicle_dev describes obs_dev only.  Rows of envs that did not finish, and of
+ * envs the step mask skips, are not written.  With autoreset = 0, final_obs[e] == obs[e] for every finished env.
+ * final_obs_dev NULL launches exactly what hrp_env_step launches; final_obs_dev == obs_dev is an error.  The default
+ * kernels carry none of this code: it is a separate instantiation of the step kernel (fp32 and HRP_ENV_REAL64). */
+int hrp_env_step_final(hrp_env *env, const float *actions_dev, float *obs_dev, float *reward_dev,
+                       uint8_t *terminated_dev, uint8_t *truncated_dev, float *final_obs_dev,
+                       const int32_t *perm_dev, int32_t *row_vehicle_dev, void *stream);
+
 /* observation_type.observe() + wrapper.observation() of the current state */
 int hrp_env_observe(hrp_env *env, float *obs_dev, const int32_t *perm_dev, int32_t *row_vehicle_dev,
                     void *stream);
@@ -282,6 +297,17 @@ int hrp_ppo_act_multi(const hrp_act_item *items, int32_t count, void *stream);
 int hrp_gae(const float *reward_dev, const float *value_dev, const uint8_t *done_dev,
             const float *last_value_dev, int64_t T, int64_t E, double gamma, double lam,
             float *adv_dev, float *ret_dev, void *stream);
+/* GAE with time-limit bootstrapping (the standard treatment of truncation; the reference treats it as termination,
+ * which hrp_gae keeps).  terminated_dev / truncated_dev [T,E] uint8 as the step wrote them, final_value_dev (nullable)
+ * [T,E] = V(final observation) of the step.  Per (t, e), fp64 arithmetic, float32 store of every A_t:
+ *   term = terminated; trunc = truncated && !terminated (a crash on the last step is not bootstrapped); done = term|trunc
+ *   boot = trunc ? final_value : (done ? 0 : V_{t+1});  delta = r + gamma boot - V_t;  A = delta + gamma lam (1-done) A_{t+1}
+ * boot is a select: final_value rows of steps that were not truncated are never read into the arithmetic and may hold
+ * anything, NaN included.  final_value_dev NULL, or no truncated step: bit-identical to hrp_gae with
+ * done = terminated | truncated.  Bad arguments return -1 with a message naming the field, before any launch. */
+int hrp_gae_ex(const float *reward_dev, const float *value_dev, const uint8_t *terminated_dev,
+               const uint8_t *truncated_dev, const float *final_value_dev, const float *last_value_dev, int64_t T,
+               int64_t E, double gamma, double lam, float *adv_dev, float *ret_dev, void *stream);
 /* advantage normalisation (agent.py:204): (a-mean)/(std_unbiased+1e-8), in place.
  * hrp_adv_stats writes (sum, sum of squares, n) of the local shard to stats_dev[0..2] (fp64;
  * stats_dev must hold 3 + 512 doubles, the tail is scratch); a sharded run all-reduces those

@@ -6,7 +6,10 @@ pair, on the same per-rank minibatches.  Run with one rank per GPU:
 World size 2: the two-term sums are commutative, so the parameters must agree BIT FOR BIT after every step.  More
 ranks: NCCL's reduction order differs from rank order, so the summed GRADIENT of the first step is compared (1e-5 of
 its max-abs; Adam turns last-bit differences of near-zero gradients into +-lr parameter moves, which makes the
-parameters themselves a poor yardstick).  Every rank must hold identical parameters at the end in any case."""
+parameters themselves a poor yardstick).  Every rank must hold identical parameters at the end in any case.
+
+``--bootstrap-truncated``: the graph-replayed updates run on rollouts collected with time-limit bootstrapping
+(final_value of truncated steps, hrp_gae_ex); GAE is per env, so the sharded update needs no other exchange."""
 import os
 import sys
 import time
@@ -22,6 +25,7 @@ torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
 dist.init_process_group("nccl", device_id=dev)
 S, A, H, B, steps = 60, 2, 256, 4096, 24
+BOOT = "--bootstrap-truncated" in sys.argv
 
 
 def make(p2p: bool) -> PPOAgent:
@@ -82,7 +86,7 @@ ok = ranks_equal and moved > 1e-4 and grad_err < 1e-5 and (same if world == 2 el
 def rollout(agent, seed):
     T, E = 6, 2048
     gg = torch.Generator(device=dev).manual_seed(seed)
-    r = agent.memory.begin_rollout(T, E, S, A)
+    r = agent.memory.begin_rollout(T, E, S, A, bootstrap_truncated=BOOT)
     r["states"].copy_(torch.randn(T + 1, E, S, generator=gg, device=dev) * 0.5)
     r["pre_tanh"].copy_(torch.randn(T, E, A, generator=gg, device=dev))
     r["action"].copy_(torch.tanh(r["pre_tanh"]))
@@ -90,6 +94,11 @@ def rollout(agent, seed):
     r["value"].copy_(torch.randn(T, E, generator=gg, device=dev))
     r["reward"].copy_(torch.rand(T, E, generator=gg, device=dev))
     r["done"].copy_((torch.rand(T, E, generator=gg, device=dev) < 0.05).to(torch.uint8))
+    if BOOT:
+        r["terminated"].copy_(r["done"])
+        r["truncated"].copy_((torch.rand(T, E, generator=gg, device=dev) < 0.1).to(torch.uint8))
+        r["final_value"].copy_(torch.randn(T, E, generator=gg, device=dev))
+        r["done"].copy_(r["terminated"] | r["truncated"])
 
 
 torch.manual_seed(1)
@@ -105,7 +114,8 @@ gathered = [torch.empty_like(flat) for _ in range(world)]
 dist.all_gather(gathered, flat)
 upd_equal = all(torch.equal(gathered[0], x) for x in gathered)
 if rank == 0:
-    print(f"world {world}: two graph-replayed updates (18 optimizer steps, both parities): identical on every rank: {upd_equal}; "
+    print(f"world {world}: two graph-replayed updates (18 optimizer steps, both parities"
+          f"{', bootstrapped truncation' if BOOT else ''}): identical on every rank: {upd_equal}; "
           f"exchange: {'peer-memory kernel' if upd._comm is not None else 'nccl'}; graphs captured: {len(upd._graph_state['graphs'])}")
 ok = ok and upd_equal
 upd.close()
