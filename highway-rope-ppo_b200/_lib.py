@@ -22,6 +22,7 @@ HRP_MAX_EMBED = 64
 FEATURE_CODES = {"presence": 0, "x": 1, "y": 2, "vx": 3, "vy": 4, "heading": 5, "cos_h": 6, "sin_h": 7}
 EMBED_NONE, EMBED_ROPE, EMBED_DIST, EMBED_RANK = 0, 1, 2, 3
 PPO_CATEGORICAL = 1   # HRP_PPO_CATEGORICAL
+EPISODE_STATS_LEN = 6 + 6 * 512   # HRP_EPISODE_STATS_LEN: doubles of hrp_episode_stats' stats_dev
 
 
 class HrpError(RuntimeError):
@@ -114,6 +115,7 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_gae_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _vp, _vp, _vp]),
     "hrp_adv_stats": (C.c_int, [_vp, _i64, _vp, _vp]),
     "hrp_adv_normalize": (C.c_int, [_vp, _i64, _vp, _vp]),
+    "hrp_episode_stats": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "hrp_ppo_loss_grad": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp,
                                     _vp, _vp]),
     "hrp_clip_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),

@@ -20,6 +20,9 @@ from typing import Any, Dict, Optional
 import numpy as np
 import torch
 
+from ..ppo import distributed
+from .episodes import episode_stats, new_stats, policy_steps, summarize
+
 ARTIFACTS_DIR = os.path.join("artifacts", "highway-ppo")
 
 
@@ -315,20 +318,180 @@ def rollout_and_update(vec_env, agent, T: int, obs: Optional[torch.Tensor] = Non
     return agent.update(last_value=last_v.view(-1)), last_obs
 
 
+def evaluate_vectorized(eval_env, agent, exp_seed: int = 0, use_graph: Optional[bool] = None) -> Dict[str, Any]:
+    """One deterministic episode per env of ``eval_env``, all at once: the batched counterpart of ``evaluate``.
+
+    Env e plays the reference's evaluation episode with seed ``exp_seed + 1000 + env_id_base + e`` (per-env seeds and a
+    full reset: bit for bit the episode ``evaluate(env, agent, K, exp_seed)`` starts on a single-env handle), so shards
+    with consecutive ``env_id_base`` play the episode set of one process.  Gaussian agents act with tanh(mean),
+    categorical ones with the argmax.  Each of the ``policy_steps`` steps after which highway-v0 truncates is an act, a
+    step masked by the envs still running and one ``hrp_episode_stats`` launch that freezes the envs whose episode
+    ended, so per-episode returns and lengths stay on the device and the host synchronises once.  The whole evaluation
+    is captured as one CUDA graph by the second call and replayed by later calls with the same env, agent workspace
+    and seeds (the first call runs launch by launch; ``use_graph=False`` always does).
+
+    ``eval_env`` becomes an evaluation handle: this installs its per-env seeds and step mask.  In shuffled row order
+    the shuffle draws continue from one evaluation to the next, as they do on a single-env handle.
+
+    Returns mean / std (population) / min / max of the returns, length_mean, terminated_fraction, episodes, and the
+    per-episode ``returns`` (float64) and ``lengths`` (int32) as numpy arrays.  Under ``torch.distributed`` the six
+    sums are all-reduced, so episodes, mean, std, length_mean and terminated_fraction are global; min, max and the
+    arrays are this rank's."""
+    _act_widths(eval_env, agent)
+    ac = agent.actor_critic
+    K, S, dev = eval_env.num_envs, eval_env.N * eval_env.F_out, eval_env.device
+    steps = policy_steps(eval_env.config["duration"], eval_env.config["policy_frequency"])
+    buf = getattr(eval_env, "_eval_buffers", None)
+    if buf is None or buf["exp_seed"] != int(exp_seed):
+        base = int(exp_seed) + 1000 + int(eval_env.env_id_base)
+        buf = {"exp_seed": int(exp_seed),
+               "seeds": torch.arange(base, base + K, dtype=torch.int64, device=dev),
+               "active": torch.zeros(K, dtype=torch.uint8, device=dev),
+               "ret": torch.zeros(K, dtype=torch.float64, device=dev),
+               "len": torch.zeros(K, dtype=torch.int32, device=dev),
+               "stats": new_stats(dev),
+               "obs": torch.empty((2, K, eval_env.N, eval_env.F_out), dtype=torch.float32, device=dev),
+               "reward": torch.empty(K, dtype=torch.float32, device=dev),
+               "terminated": torch.empty(K, dtype=torch.uint8, device=dev),
+               "truncated": torch.empty(K, dtype=torch.uint8, device=dev)}
+        eval_env.set_env_seeds(buf["seeds"])
+        eval_env.set_step_mask(buf["active"])
+        eval_env._eval_buffers = buf
+    # policy outputs per (action, pre_tanh) width, kept as long as the buffers: captured launches write them
+    widths = ("act",) + tuple(ac.act_widths())
+    if widths not in buf:
+        buf[widths] = ac._new_act_out(K)
+    act = buf[widths]
+
+    def run():
+        buf["active"].fill_(1)
+        buf["ret"].zero_()
+        buf["len"].zero_()
+        buf["stats"].zero_()
+        eval_env.reset(out=buf["obs"][0])   # every env: the mask steers steps only
+        for t in range(steps):
+            agent.act(buf["obs"][t % 2].view(K, S), deterministic=True, out=act)
+            eval_env.step(act["action"], out=buf["obs"][(t + 1) % 2], reward_out=buf["reward"],
+                          terminated_out=buf["terminated"], truncated_out=buf["truncated"])
+            episode_stats(buf["reward"], buf["terminated"], buf["truncated"], buf["ret"], buf["len"], buf["stats"],
+                          active=buf["active"])
+
+    if use_graph is None:
+        # (a single env acts through the matrix-vector kernel, which allocates its output row)
+        use_graph = K > 1 and getattr(agent, "use_cuda_graphs", True)
+    ac._ensure_workspace(K)
+    key = (eval_env.uid, eval_env.param_version, ac.workspace_generation, id(buf), K, steps)
+    cache = getattr(agent, "_eval_graph", None)
+    if not use_graph or cache is None or cache["key"] != key:
+        run()                           # the first evaluation of a configuration runs eagerly ...
+        if use_graph:
+            agent._eval_graph = {"key": key, "graph": None}
+    else:
+        if cache["graph"] is None:      # ... the second one is captured
+            graph = torch.cuda.CUDAGraph()
+            cur = torch.cuda.current_stream(dev)
+            side = torch.cuda.Stream(dev)
+            side.wait_stream(cur)
+            with torch.cuda.stream(side):
+                graph.capture_begin()
+                try:
+                    run()
+                finally:
+                    graph.capture_end()
+            cur.wait_stream(side)
+            cache["graph"] = graph
+        cache["graph"].replay()
+        agent.launches += steps
+        eval_env.launches += 1 + steps
+    sums = buf["stats"][:6]
+    if distributed.world_size() > 1:
+        distributed.allreduce_sum_(sums)
+    host = torch.cat([sums, buf["ret"], buf["len"].double()]).cpu().numpy()   # the evaluation's one synchronisation
+    returns, lengths = host[6:6 + K].copy(), host[6 + K:].astype(np.int32)
+    s = summarize(host[:6])
+    if s["episodes"] != K * distributed.world_size():
+        raise RuntimeError(f"evaluate_vectorized: {s['episodes']} episodes finished within {steps} steps, expected "
+                           f"{K * distributed.world_size()}")
+    return {"mean": s["return_mean"], "std": s["return_std"], "min": float(returns.min()), "max": float(returns.max()),
+            "length_mean": s["length_mean"], "terminated_fraction": s["terminated_fraction"],
+            "episodes": s["episodes"], "returns": returns, "lengths": lengths}
+
+
+def eval_env_for(vec_env, num_envs: int):
+    """An evaluation handle of ``num_envs`` envs with ``vec_env``'s resolved config and its ``EmbedSpec`` (the same table
+    object: a RankPE evaluation sees the training table, not a new draw), no autoreset.  Its ``env_id_base`` is the
+    shard index of ``vec_env`` times ``num_envs``, so that W shards evaluate the episodes one process of W x
+    ``num_envs`` envs would."""
+    from ..envs.highway_vec import HighwayVecEnv
+
+    shard = int(vec_env.env_id_base) // int(vec_env.num_envs)
+    return HighwayVecEnv(vec_env.config, num_envs, device=vec_env.device, embed=vec_env.embed, autoreset=False,
+                         env_id_base=shard * int(num_envs), real64=vec_env.real64)
+
+
 def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, logger=None,
-                     bootstrap_truncated: bool = False):
-    """``iterations`` PPO iterations on E lock-step envs; returns the list of update metrics with
-    mean step reward and samples/s added.  ``bootstrap_truncated``: see ``collect_rollout``."""
+                     bootstrap_truncated: bool = False, eval_episodes: int = 0, eval_interval: int = 10,
+                     best_checkpoint: Optional[str] = None):
+    """``iterations`` PPO iterations on E lock-step envs; returns the list of update metrics with samples/s and the
+    training episodes added.  ``bootstrap_truncated``: see ``collect_rollout``.
+
+    Training episodes: after each rollout one ``hrp_episode_stats`` launch over its rewards and flags, with per-env
+    return / length carries zeroed by the reset here, so an episode spanning two rollouts counts once, in the
+    iteration it ends in.  ``episodes``, ``episode_return_mean``, ``episode_return_std`` (population),
+    ``episode_length_mean`` and ``terminated_fraction`` are those of the episodes that ended during the iteration (NaN
+    when none did); under ``torch.distributed`` the six sums are all-reduced, so every rank reports global figures.
+
+    ``eval_episodes`` > 0: before iterations 0, ``eval_interval``, 2 ``eval_interval``, ... the policy is evaluated on
+    that many deterministic episodes per rank (``evaluate_vectorized`` on a handle of its own, ``eval_env_for``; seeds
+    ``seed + 1000 + global env id``, the reference's evaluation seeds with ``seed`` as the experiment seed), recorded
+    as ``eval_return_mean`` / ``eval_return_std`` / ``eval_length_mean`` / ``eval_terminated_fraction`` in that
+    iteration's metrics.  ``best_checkpoint``: path that ``agent.save`` (rank 0) writes whenever the evaluation mean
+    beats the best so far."""
     logger = logger or logging.getLogger(__name__)
     _act_widths(vec_env, agent)
+    if eval_episodes and eval_interval < 1:
+        raise ValueError(f"eval_interval must be >= 1, got {eval_interval}")
     obs = vec_env.reset(seed=seed)
+    E, dev = vec_env.num_envs, vec_env.device
+    carry_ret = torch.zeros(E, dtype=torch.float64, device=dev)
+    carry_len = torch.zeros(E, dtype=torch.int32, device=dev)
+    stats = new_stats(dev)
+    eval_env = eval_env_for(vec_env, eval_episodes) if eval_episodes else None
+    best = -float("inf")
     history = []
-    for it in range(iterations):
-        t0 = time.time()
-        metrics, obs = rollout_and_update(vec_env, agent, T, obs=obs, bootstrap_truncated=bootstrap_truncated)
-        torch.cuda.synchronize(vec_env.device)
-        dt = time.time() - t0
-        metrics["samples_per_s"] = T * vec_env.num_envs / dt
-        history.append(metrics)
-        logger.info("iter=%d loss=%.4f samples/s=%.0f", it, metrics["loss"], metrics["samples_per_s"])
+    try:
+        for it in range(iterations):
+            ev = None
+            if eval_env is not None and it % eval_interval == 0:
+                ev = evaluate_vectorized(eval_env, agent, exp_seed=seed)
+                if ev["mean"] > best:
+                    best = ev["mean"]
+                    if best_checkpoint is not None and distributed.rank() == 0:
+                        agent.save(best_checkpoint)
+            t0 = time.time()
+            r = collect_rollout(vec_env, agent, T, obs, bootstrap_truncated=bootstrap_truncated)
+            stats[:6].zero_()
+            episode_stats(r["reward"], r["terminated"], r["truncated"], carry_ret, carry_len, stats)
+            obs = r["states"][T].clone()
+            _, _, last_v = agent.actor_critic.forward(obs)
+            metrics = agent.update(last_value=last_v.view(-1))
+            if distributed.world_size() > 1:
+                distributed.allreduce_sum_(stats[:6])
+            torch.cuda.synchronize(dev)
+            dt = time.time() - t0
+            metrics["samples_per_s"] = T * E / dt
+            s = summarize(stats[:6].tolist())
+            metrics.update(episodes=s["episodes"], episode_return_mean=s["return_mean"],
+                           episode_return_std=s["return_std"], episode_length_mean=s["length_mean"],
+                           terminated_fraction=s["terminated_fraction"])
+            if ev is not None:
+                metrics.update(eval_return_mean=ev["mean"], eval_return_std=ev["std"],
+                               eval_length_mean=ev["length_mean"], eval_terminated_fraction=ev["terminated_fraction"])
+            history.append(metrics)
+            logger.info("iter=%d loss=%.4f samples/s=%.0f episodes=%d return=%.3f%s", it, metrics["loss"],
+                        metrics["samples_per_s"], s["episodes"], s["return_mean"],
+                        "" if ev is None else f" eval_return={ev['mean']:.3f}")
+    finally:
+        if eval_env is not None:
+            eval_env.close()
     return history

@@ -314,6 +314,26 @@ int hrp_gae_ex(const float *reward_dev, const float *value_dev, const uint8_t *t
  * three numbers before hrp_adv_normalize consumes them. */
 int hrp_adv_stats(const float *adv_dev, int64_t n, double *stats_dev, void *stream);
 int hrp_adv_normalize(float *adv_dev, int64_t n, const double *stats_dev, void *stream);
+/* episode returns and lengths (the reference's ep_reward / evaluate bookkeeping, training/routine.py:14-29,143) over the
+ * time-major [T,E] reward / terminated / truncated buffers the step wrote, forward scan, one thread per env.
+ * return_dev[E] (fp64) and length_dev[E] (int32) carry each env's running episode across calls, so an episode may span
+ * two rollouts; the caller zeroes them when it resets the envs.  For each step t, in order, of an env that takes part:
+ * ret += (double)reward[t,e] (a sequential fp64 sum, bit-exact against Python's ep_reward += reward) and len += 1; if
+ * terminated | truncated, the episode is counted.  A step both terminated and truncated counts as terminated (the rule
+ * of hrp_gae_ex).
+ *   active_dev NULL (training): after an episode is counted ret and len restart at 0 (the env has autoreset).
+ *   active_dev[E] uint8 (evaluation): only envs with active[e] != 0 take part; when an env's first episode ends,
+ *     active[e] = 0 and ret / len keep that episode.  The same buffer serves as the handle's step mask
+ *     (hrp_env_set_step_mask), so a finished env stops stepping and its return stays on the device.
+ * stats_dev is accumulated into (+=), fp64: [0] episodes finished, [1] sum of returns, [2] sum of squared returns,
+ * [3] sum of lengths, [4] episodes that ended by termination, [5] episodes that ended by truncation only.  It must hold
+ * 6 + 6 * 512 doubles: the tail is scratch for per-CTA partials, which are added in a fixed order, so equal inputs give
+ * the same bits on every run; a sharded run all-reduces the six sums.  Bad arguments (a null pointer other than
+ * active_dev, T < 1, E < 1) return -1 with a message naming the field, before any launch. */
+#define HRP_EPISODE_STATS_LEN (6 + 6 * 512)
+int hrp_episode_stats(const float *reward_dev, const uint8_t *terminated_dev, const uint8_t *truncated_dev, int64_t T,
+                      int64_t E, uint8_t *active_dev, double *return_dev, int32_t *length_dev, double *stats_dev,
+                      void *stream);
 /* one minibatch of PPOAgent.update (agent.py:218-245 + backward): evaluate, clipped surrogate,
  * value MSE, entropy; writes d(loss)/d(params) into grad_dev[P] (overwritten) and
  * metrics_dev[8] += (loss, policy_loss, value_loss, entropy, clip_fraction, approx_kl, 1, 0).
