@@ -19,7 +19,11 @@ HRP_MAX_FEATURES = 8
 HRP_MAX_LANES = 8
 HRP_MAX_EMBED = 64
 
-FEATURE_CODES = {"presence": 0, "x": 1, "y": 2, "vx": 3, "vy": 4, "heading": 5, "cos_h": 6, "sin_h": 7}
+HRP_MAX_GRID_VALUES = HRP_MAX_OBS_ROWS * HRP_MAX_FEATURES   # F * W * H of an OccupancyGrid observation
+
+# "on_road" (HRP_F_ON_ROAD) is the OccupancyGrid road layer: valid in a grid only
+FEATURE_CODES = {"presence": 0, "x": 1, "y": 2, "vx": 3, "vy": 4, "heading": 5, "cos_h": 6, "sin_h": 7, "on_road": 8}
+OBS_KINEMATICS, OBS_OCCUPANCY_GRID = 0, 1   # HRP_OBS_*
 EMBED_NONE, EMBED_ROPE, EMBED_DIST, EMBED_RANK = 0, 1, 2, 3
 PPO_CATEGORICAL = 1   # HRP_PPO_CATEGORICAL
 EPISODE_STATS_LEN = 6 + 6 * 512   # HRP_EPISODE_STATS_LEN: doubles of hrp_episode_stats' stats_dev
@@ -47,6 +51,8 @@ class HrpCfg(C.Structure):
         ("embed_kind", C.c_int32), ("embed_dim", C.c_int32), ("embed_use_euclidean", C.c_int32),
         ("embed_max_dist", C.c_double),
         ("autoreset", C.c_int32), ("embed_ego_idx", C.c_int32),
+        ("obs_type", C.c_int32), ("grid_align", C.c_int32),
+        ("grid_lo", C.c_double * 2), ("grid_hi", C.c_double * 2), ("grid_step", C.c_double * 2),
     ]
 
 
@@ -80,6 +86,7 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_env_create_ex": (C.c_int, [C.POINTER(HrpCfg), _vp, _i64, _i32, _u64, _i32, C.c_uint32, C.POINTER(_vp)]),
     "hrp_env_destroy": (C.c_int, [_vp]),
     "hrp_env_obs_dim": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32)]),
+    "hrp_env_grid_shape": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32)]),
     "hrp_env_num_vehicles": (C.c_int, [_vp]),
     "hrp_env_reset": (C.c_int, [_vp, _u64, _vp, _vp, _vp]),
     "hrp_env_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -28,6 +28,7 @@ void hrp_set_error(const char *fmt, ...)
 struct hrp_env {
     hrp_cfg cfg;
     EnvDev P;
+    GridDev G;
     int device;
     void *arena;  // one allocation behind every state array
     size_t arena_bytes;
@@ -90,7 +91,7 @@ __global__ void __launch_bounds__(256) fetch_host_kernel(const uint4 *__restrict
 extern "C" {
 
 const char *hrp_last_error(void) { return g_err; }
-int hrp_version(void) { return 1; }
+int hrp_version(void) { return 2; }   // 2: OccupancyGrid fields of hrp_cfg, hrp_env_grid_shape
 int hrp_device_count(void)
 {
     int n = 0;
@@ -109,6 +110,56 @@ int hrp_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out
     return 0;
 }
 
+// W (axis 0) or H (axis 1) of an OccupancyGrid config: floor((hi - lo) / step) in fp64, 0 when it is not a count >= 1
+static int grid_extent(const hrp_cfg *c, int axis)
+{
+    const double n = floor((c->grid_hi[axis] - c->grid_lo[axis]) / c->grid_step[axis]);
+    return (c->grid_step[axis] > 0.0 && n >= 1.0 && n <= HRP_MAX_GRID_VALUES) ? (int)n : 0;
+}
+
+static int validate_grid(const hrp_cfg *c)
+{
+    if (c->obs_nfeat < 1 || c->obs_nfeat > HRP_MAX_FEATURES) {
+        hrp_set_error("feature count %d outside [1, %d]", c->obs_nfeat, HRP_MAX_FEATURES);
+        return -1;
+    }
+    for (int f = 0; f < c->obs_nfeat; ++f)
+        if (c->obs_feat[f] < HRP_F_PRESENCE || c->obs_feat[f] > HRP_F_ON_ROAD) {
+            hrp_set_error("unsupported feature code %d", c->obs_feat[f]);
+            return -1;
+        }
+    for (int a = 0; a < 2; ++a) {
+        if (!(c->grid_step[a] > 0.0) || !isfinite(c->grid_step[a]) || !isfinite(c->grid_lo[a]) || !isfinite(c->grid_hi[a])) {
+            hrp_set_error("grid_step[%d] = %g must be > 0 and grid_size[%d] = [%g, %g] finite", a, c->grid_step[a], a,
+                          c->grid_lo[a], c->grid_hi[a]);
+            return -1;
+        }
+        if (!grid_extent(c, a)) {
+            hrp_set_error("grid_size[%d] = [%g, %g] with grid_step %g holds no cell", a, c->grid_lo[a], c->grid_hi[a],
+                          c->grid_step[a]);
+            return -1;
+        }
+    }
+    const int W = grid_extent(c, 0), H = grid_extent(c, 1);
+    if ((long long)c->obs_nfeat * W * H > HRP_MAX_GRID_VALUES) {
+        hrp_set_error("grid features x W x H = %d x %d x %d exceeds %d", c->obs_nfeat, W, H, HRP_MAX_GRID_VALUES);
+        return -1;
+    }
+    if (c->embed_kind != HRP_EMBED_NONE) {
+        hrp_set_error("embed_kind %d: an OccupancyGrid observation takes no embedding", c->embed_kind);
+        return -1;
+    }
+    if (c->policy_frequency < 1 || c->simulation_frequency < c->policy_frequency) {
+        hrp_set_error("bad simulation/policy frequency %d/%d", c->simulation_frequency, c->policy_frequency);
+        return -1;
+    }
+    if (c->ego_mode != 0 && c->ego_mode != 1) {
+        hrp_set_error("ego_mode %d not in {0,1}", c->ego_mode);
+        return -1;
+    }
+    return 0;
+}
+
 static int validate_cfg(const hrp_cfg *c, int64_t table_len)
 {
     if (c->vehicles_count < 0 || c->vehicles_count + 1 > HRP_MAX_VEHICLES) {
@@ -119,6 +170,11 @@ static int validate_cfg(const hrp_cfg *c, int64_t table_len)
         hrp_set_error("lanes_count %d outside [1, %d]", c->lanes_count, HRP_MAX_LANES);
         return -1;
     }
+    if (c->obs_type != HRP_OBS_KINEMATICS && c->obs_type != HRP_OBS_OCCUPANCY_GRID) {
+        hrp_set_error("obs_type %d not in {0 (Kinematics), 1 (OccupancyGrid)}", c->obs_type);
+        return -1;
+    }
+    if (c->obs_type == HRP_OBS_OCCUPANCY_GRID) return validate_grid(c);
     if (c->obs_vehicles < 1 || c->obs_vehicles > HRP_MAX_OBS_ROWS) {
         hrp_set_error("observation vehicles_count %d outside [1, %d]", c->obs_vehicles, HRP_MAX_OBS_ROWS);
         return -1;
@@ -215,6 +271,23 @@ int hrp_env_create_ex(const hrp_cfg *cfg, const float *embed_table_host, int64_t
     P.gap_factor = exp(-5.0 / 40.0 * cfg->lanes_count);
     P.initial_lane = cfg->initial_lane_id;
     P.env_id_base = env_id_base; P.seed = 0;
+    GridDev &G = h->G;
+    G.obs_type = cfg->obs_type;
+    G.gx = G.gy = -1;
+    if (cfg->obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        // the observation is [F][W][H]: rows F and columns W*H for every N * F_out consumer
+        G.gw = grid_extent(cfg, 0); G.gh = grid_extent(cfg, 1);
+        G.galign = cfg->grid_align ? 1 : 0;
+        for (int a = 0; a < 2; ++a) { G.glo[a] = cfg->grid_lo[a]; G.gstep[a] = cfg->grid_step[a]; }
+        for (int f = cfg->obs_nfeat - 1; f >= 0; --f) {
+            if (!cfg->obs_has_range[f]) continue;
+            if (cfg->obs_feat[f] == HRP_F_X) G.gx = f;
+            if (cfg->obs_feat[f] == HRP_F_Y) G.gy = f;
+        }
+        P.N = cfg->obs_nfeat; P.Fout = G.gw * G.gh;
+        P.normalize = 1; P.absolute = 0; P.sorted = 1; P.see_behind = 0;
+        P.embed_kind = HRP_EMBED_NONE; P.embed_dim = 0; P.ego_idx = 0;
+    }
 
     size_t n = (size_t)num_envs * HRP_VS, ne = (size_t)num_envs;
     const size_t rsz = P.real64 ? sizeof(double) : sizeof(float);
@@ -245,7 +318,7 @@ int hrp_env_create_ex(const hrp_cfg *cfg, const float *embed_table_host, int64_t
     }
     P.table = h->table_dev;
     // spawn episode 0 with seed 0 so that a handle is always in a valid state
-    if (int rc = hrp_launch_reset(P, nullptr, nullptr, 0)) { return rc; }
+    if (int rc = hrp_launch_reset(P, G, nullptr, nullptr, 0)) { return rc; }
     HRP_CUDA_OK(cudaDeviceSynchronize());
     *out = h;
     return 0;
@@ -275,13 +348,22 @@ int hrp_env_obs_dim(const hrp_env *h, int32_t *rows, int32_t *cols)
     if (cols) *cols = h->P.Fout;
     return 0;
 }
+int hrp_env_grid_shape(const hrp_env *h, int32_t *features, int32_t *width, int32_t *height)
+{
+    if (!h) { hrp_set_error("null handle"); return -1; }
+    if (h->G.obs_type != HRP_OBS_OCCUPANCY_GRID) { hrp_set_error("hrp_env_grid_shape: not an OccupancyGrid handle"); return -1; }
+    if (features) *features = h->P.F;
+    if (width) *width = h->G.gw;
+    if (height) *height = h->G.gh;
+    return 0;
+}
 int hrp_env_num_vehicles(const hrp_env *h) { return h ? h->P.V : -1; }
 
 int hrp_env_reset(hrp_env *h, uint64_t seed, const uint8_t *mask_dev, float *obs_dev, void *stream)
 {
     if (!h) { hrp_set_error("null handle"); return -1; }
     h->P.seed = seed;
-    return hrp_launch_reset(h->P, mask_dev, obs_dev, (cudaStream_t)stream);
+    return hrp_launch_reset(h->P, h->G, mask_dev, obs_dev, (cudaStream_t)stream);
 }
 
 int hrp_env_step(hrp_env *h, const float *actions_dev, float *obs_dev, float *reward_dev,
@@ -292,7 +374,11 @@ int hrp_env_step(hrp_env *h, const float *actions_dev, float *obs_dev, float *re
         hrp_set_error("hrp_env_step: null argument");
         return -1;
     }
-    return hrp_launch_step(h->P, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
+    if (perm_dev && h->G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        hrp_set_error("hrp_env_step: perm_dev must be NULL for an OccupancyGrid handle (a grid has no row order)");
+        return -1;
+    }
+    return hrp_launch_step(h->P, h->G, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
                            row_vehicle_dev, (cudaStream_t)stream);
 }
 
@@ -308,7 +394,11 @@ int hrp_env_step_final(hrp_env *h, const float *actions_dev, float *obs_dev, flo
         hrp_set_error("hrp_env_step_final: null argument");
         return -1;
     }
-    return hrp_launch_step(h->P, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
+    if (perm_dev && h->G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        hrp_set_error("hrp_env_step_final: perm_dev must be NULL for an OccupancyGrid handle (a grid has no row order)");
+        return -1;
+    }
+    return hrp_launch_step(h->P, h->G, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
                            row_vehicle_dev, (cudaStream_t)stream, final_obs_dev);
 }
 
@@ -316,7 +406,11 @@ int hrp_env_observe(hrp_env *h, float *obs_dev, const int32_t *perm_dev, int32_t
                     void *stream)
 {
     if (!h || !obs_dev) { hrp_set_error("hrp_env_observe: null argument"); return -1; }
-    return hrp_launch_observe(h->P, obs_dev, perm_dev, row_vehicle_dev, (cudaStream_t)stream);
+    if (perm_dev && h->G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        hrp_set_error("hrp_env_observe: perm_dev must be NULL for an OccupancyGrid handle (a grid has no row order)");
+        return -1;
+    }
+    return hrp_launch_observe(h->P, h->G, obs_dev, perm_dev, row_vehicle_dev, (cudaStream_t)stream);
 }
 
 static int ensure_host_path(hrp_env *h)
@@ -391,14 +485,14 @@ static int step_host_impl(hrp_env *h, const float *actions, float *obs_host, flo
             cudaHostGetDevicePointer((void **)&r_dev, reward_host, 0) == cudaSuccess &&
             cudaHostGetDevicePointer((void **)&te_dev, terminated_host, 0) == cudaSuccess &&
             cudaHostGetDevicePointer((void **)&tr_dev, truncated_host, 0) == cudaSuccess) {
-            if (int rc = hrp_launch_step(h->P, d_act, o_dev, r_dev, te_dev, tr_dev, nullptr, nullptr, s)) return rc;
+            if (int rc = hrp_launch_step(h->P, h->G, d_act, o_dev, r_dev, te_dev, tr_dev, nullptr, nullptr, s)) return rc;
             if (!sync) return 0;
             HRP_CUDA_OK(cudaStreamSynchronize(s));
             return 0;
         }
         cudaGetLastError();   // not mapped: fall through to the copies
     }
-    if (int rc = hrp_launch_step(h->P, d_act, h->d_obs, h->d_reward, h->d_term, h->d_trunc, nullptr, nullptr, s))
+    if (int rc = hrp_launch_step(h->P, h->G, d_act, h->d_obs, h->d_reward, h->d_term, h->d_trunc, nullptr, nullptr, s))
         return rc;
     HRP_CUDA_OK(cudaMemcpyAsync(pin_o ? obs_host : h->h_obs, h->d_obs, no * sizeof(float), cudaMemcpyDeviceToHost, s));
     HRP_CUDA_OK(cudaMemcpyAsync(pin_r ? reward_host : h->h_reward, h->d_reward, E * sizeof(float), cudaMemcpyDeviceToHost, s));
@@ -442,7 +536,7 @@ int hrp_env_reset_host(hrp_env *h, uint64_t seed, float *obs_host)
     size_t no = (size_t)h->P.E * h->P.N * h->P.Fout;
     h->P.seed = seed;
     const bool pin_o = is_pinned(obs_host);
-    if (int rc = hrp_launch_reset(h->P, nullptr, h->d_obs, h->host_stream)) return rc;
+    if (int rc = hrp_launch_reset(h->P, h->G, nullptr, h->d_obs, h->host_stream)) return rc;
     HRP_CUDA_OK(cudaMemcpyAsync(pin_o ? obs_host : h->h_obs, h->d_obs, no * sizeof(float), cudaMemcpyDeviceToHost,
                                 h->host_stream));
     HRP_CUDA_OK(cudaStreamSynchronize(h->host_stream));

@@ -635,6 +635,111 @@ __device__ void observe_env(const EnvDev &P, WarpS<R> &S, int e, int lane, float
 }
 
 // ---------------------------------------------------------------------------------------
+// OccupancyGridObservation.observe (absolute=False, as_image=False; DESIGN.md §3.1), warp-cooperative.  fp64 in both
+// instantiations, every operation an explicit round-to-nearest intrinsic: a cell index is a floor, and the fp64
+// validation kernel must decide it bit for bit as the sequential fp64 restatement (tests/grid_oracle.py) does, with
+// no contraction into FMAs.  Compiled into the grid kernels only (the OBS template parameter below).
+__device__ __forceinline__ double grid_lmap(double v, double lo, double hi)     // utils.lmap(v, [lo, hi], [-1, 1])
+{
+    return __dadd_rn(-1.0, __ddiv_rn(__dmul_rn(__dsub_rn(v, lo), 2.0), __dsub_rn(hi, lo)));
+}
+__device__ __forceinline__ double grid_unlmap(double v, double lo, double hi)   // utils.lmap(v, [-1, 1], [lo, hi])
+{
+    return __dadd_rn(lo, __ddiv_rn(__dmul_rn(__dadd_rn(v, 1.0), __dsub_rn(hi, lo)), 2.0));
+}
+// pos_to_index of an ego-relative position: cell id ix * H + iy, or -1 outside [0, W) x [0, H)
+__device__ __forceinline__ int grid_cell(const GridDev &G, double px, double py, double c, double s)
+{
+    if (G.galign) {   // [[c, s], [-s, c]] @ p
+        const double rx = __dadd_rn(__dmul_rn(c, px), __dmul_rn(s, py));
+        const double ry = __dadd_rn(__dmul_rn(-s, px), __dmul_rn(c, py));
+        px = rx; py = ry;
+    }
+    const double fx = floor(__ddiv_rn(__dsub_rn(px, G.glo[0]), G.gstep[0]));
+    const double fy = floor(__ddiv_rn(__dsub_rn(py, G.glo[1]), G.gstep[1]));
+    return (fx >= 0.0 && fx < (double)G.gw && fy >= 0.0 && fy < (double)G.gh) ? (int)fx * G.gh + (int)fy : -1;
+}
+// Vehicle.to_dict(ego)[code]: x, y, vx, vy relative to the ego, the rest absolute
+template <typename R> __device__ __forceinline__ double grid_feature(const WarpS<R> &S, int code, int k)
+{
+    switch (code) {
+    case HRP_F_PRESENCE: return 1.0;
+    case HRP_F_X: return __dsub_rn(S.x[k], S.x[0]);
+    case HRP_F_Y: return __dsub_rn((double)S.y[k], (double)S.y[0]);
+    case HRP_F_VX: return __dsub_rn(__dmul_rn((double)S.rec[k].v, (double)S.rec[k].ch), __dmul_rn((double)S.rec[0].v, (double)S.rec[0].ch));
+    case HRP_F_VY: return __dsub_rn(__dmul_rn((double)S.rec[k].v, (double)S.rec[k].sh), __dmul_rn((double)S.rec[0].v, (double)S.rec[0].sh));
+    case HRP_F_HEADING: return (double)S.h[k];
+    case HRP_F_COS_H: return (double)S.rec[k].ch;
+    case HRP_F_SIN_H: return (double)S.rec[k].sh;
+    }
+    return 0.0;
+}
+template <typename R>
+__device__ void observe_grid(const EnvDev &P, const GridDev &G, WarpS<R> &S, int e, int lane, float *__restrict__ obs,
+                             int32_t *__restrict__ cell_vehicle)
+{
+    const int V = P.V, F = P.F, C = G.gw * G.gh;
+    for (int i = lane; i < F * C; i += 32) S.obs[i] = 0.f;   // an empty cell is NaN upstream, and nan_to_num makes it 0
+    const double ex = S.x[0], ey = (double)S.y[0];
+    const double c = (double)S.rec[0].ch, s = (double)S.rec[0].sh;
+    // every vehicle, the ego included: its cell into the shuffle-key scratch (the grid draws no permutation)
+    int cell[2];
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        const int k = lane + 32 * q;
+        cell[q] = -1;
+        if (k < V) {
+            double px = __dsub_rn(S.x[k], ex), py = __dsub_rn((double)S.y[k], ey);
+            if (G.gx >= 0) px = grid_unlmap(grid_lmap(px, P.lo[G.gx], P.hi[G.gx]), P.lo[G.gx], P.hi[G.gx]);
+            if (G.gy >= 0) py = grid_unlmap(grid_lmap(py, P.lo[G.gy], P.hi[G.gy]), P.lo[G.gy], P.hi[G.gy]);
+            cell[q] = grid_cell(G, px, py, c, s);
+            S.skey[k] = (uint32_t)cell[q];
+        }
+    }
+    __syncwarp();
+    // upstream writes the vehicles in reverse list order, so the lowest index owns a shared cell
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        const int k = lane + 32 * q;
+        bool own = cell[q] >= 0;
+        for (int j = 0; j < k && own; ++j) own = S.skey[j] != (uint32_t)cell[q];
+        if (!own) continue;
+        for (int f = 0; f < F; ++f) {
+            const int code = P.feat[f];
+            if (code == HRP_F_ON_ROAD) continue;
+            double v = grid_feature(S, code, k);
+            if (P.has_range[f]) v = grid_lmap(v, P.lo[f], P.hi[f]);
+            if (P.clip) v = fmin(fmax(v, -1.0), 1.0);
+            S.obs[f * C + cell[q]] = (float)v;
+        }
+    }
+    // fill_road_layer_by_lanes: waypoints ex - 100 + i * min(grid_step), i < ceil(200 / step), clipped to the road,
+    // at (w, 4 L) on every lane, spread over the warp
+    for (int f = 0; f < F; ++f) {
+        if (P.feat[f] != HRP_F_ON_ROAD) continue;
+        const double step = fmin(G.gstep[0], G.gstep[1]);
+        const double start = __dsub_rn(ex, 100.0);
+        const int n = (int)ceil(__ddiv_rn(__dsub_rn(__dadd_rn(ex, 100.0), start), step));
+        for (int i = lane; i < P.lanes * n; i += 32) {
+            const int L = i / n, w = i - L * n;
+            const double wx = fmin(fmax(__dadd_rn(start, __dmul_rn((double)w, step)), 0.0), 10000.0);
+            const int cc = grid_cell(G, __dsub_rn(wx, ex), __dsub_rn(4.0 * L, ey), c, s);
+            if (cc >= 0) S.obs[f * C + cc] = 1.f;
+        }
+    }
+    __syncwarp();
+    float *out = obs + (size_t)e * F * C;
+    for (int i = lane; i < F * C; i += 32) out[i] = S.obs[i];
+    if (cell_vehicle)
+        for (int i = lane; i < C; i += 32) {
+            int who = -1;
+            for (int j = 0; j < V && who < 0; ++j) who = S.skey[j] == (uint32_t)i ? j : -1;
+            cell_vehicle[(size_t)e * C + i] = who;
+        }
+    __syncwarp();
+}
+
+// ---------------------------------------------------------------------------------------
 // One simulation frame: Road.act() then Road.step(dt) (SURVEY A.11)
 template <typename R>
 __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int lane, double xref)
@@ -872,11 +977,14 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
 // ---------------------------------------------------------------------------------------
 // FINAL: the instantiation with the final-observation output (hrp_env_step_final).  A compile-time switch, so that the
 // default kernels carry none of its code: the step kernel is sensitive to instruction-cache pressure (DESIGN.md §3.1).
-template <typename R, int WARPS, bool FINAL = false>
+// OBS: the observation epilogue, HRP_OBS_KINEMATICS or HRP_OBS_OCCUPANCY_GRID -- compile-time for the same reason, and
+// with one call site of observe_env / observe_grid per instantiation.
+template <typename R, int WARPS, bool FINAL = false, int OBS = HRP_OBS_KINEMATICS>
 __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restrict__ actions, float *__restrict__ obs,
                                           float *__restrict__ reward, uint8_t *__restrict__ term,
                                           uint8_t *__restrict__ trunc, const int32_t *__restrict__ perm,
-                                          int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs = nullptr)
+                                          int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs = nullptr,
+                                          const GridDev &G = GridDev{})
 {
     __shared__ WarpS<R> smem[WARPS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -985,7 +1093,10 @@ __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restri
                 __syncwarp();
             }
             if (pass == 1 && lane == 0) { P.time[e] = tnow; P.obs_draw[e] = draw + 1; }
-            observe_env(P, S, e, lane, pass ? obs : final_obs, perm, pass ? row_vehicle : nullptr, draw);
+            if constexpr (OBS == HRP_OBS_OCCUPANCY_GRID)
+                observe_grid(P, G, S, e, lane, pass ? obs : final_obs, pass ? row_vehicle : nullptr);
+            else
+                observe_env(P, S, e, lane, pass ? obs : final_obs, perm, pass ? row_vehicle : nullptr, draw);
         }
     } else {
         if (done && P.autoreset) {
@@ -999,7 +1110,10 @@ __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restri
             __syncwarp();
         }
         if (lane == 0) { P.time[e] = tnow; P.obs_draw[e] = draw + 1; }
-        observe_env(P, S, e, lane, obs, perm, row_vehicle, draw);
+        if constexpr (OBS == HRP_OBS_OCCUPANCY_GRID)
+            observe_grid(P, G, S, e, lane, obs, row_vehicle);
+        else
+            observe_env(P, S, e, lane, obs, perm, row_vehicle, draw);
     }
     store_env(P, u, e, lane);
 }
@@ -1034,6 +1148,25 @@ hrp_step_kernel_f64_final(const EnvDev P, const float *__restrict__ actions, flo
                           float *__restrict__ final_obs)
 {
     step_body<double, HRP_WARPS_PER_CTA_F64, true>(P, actions, obs, reward, term, trunc, perm, row_vehicle, final_obs);
+}
+// the OccupancyGrid instantiations of the four: obs[E, F, W, H], row_vehicle[E, W * H] (the vehicle of each cell)
+template <bool FINAL>
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA, HRP_STEP_CTAS_PER_SM)
+hrp_step_kernel_grid(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                     float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                     int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs, const GridDev G)
+{
+    step_body<float, HRP_WARPS_PER_CTA, FINAL, HRP_OBS_OCCUPANCY_GRID>(P, actions, obs, reward, term, trunc, nullptr,
+                                                                        row_vehicle, final_obs, G);
+}
+template <bool FINAL>
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA_F64)
+hrp_step_kernel_f64_grid(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                         float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                         int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs, const GridDev G)
+{
+    step_body<double, HRP_WARPS_PER_CTA_F64, FINAL, HRP_OBS_OCCUPANCY_GRID>(P, actions, obs, reward, term, trunc,
+                                                                             nullptr, row_vehicle, final_obs, G);
 }
 
 template <typename R, int WARPS>
@@ -1073,6 +1206,41 @@ hrp_reset_kernel(const EnvDev P, const uint8_t *__restrict__ mask, float *__rest
     store_env(P, u, e, lane);
 }
 
+// the two above with the OccupancyGrid observation (the shuffle counter advances as for Kinematics)
+template <typename R, int WARPS>
+__global__ void __launch_bounds__(32 * WARPS)
+hrp_observe_kernel_grid(const EnvDev P, const GridDev G, float *__restrict__ obs, int32_t *__restrict__ cell_vehicle)
+{
+    __shared__ WarpS<R> smem[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int e = blockIdx.x * WARPS + warp;
+    if (e >= P.E) return;
+    WarpS<R> &S = smem[warp];
+    Veh<R> u[2];
+    double xref;
+    load_env(P, S, u, e, lane, xref);
+    observe_grid(P, G, S, e, lane, obs, cell_vehicle);
+    if (lane == 0) P.obs_draw[e] += 1;
+}
+
+template <typename R, int WARPS>
+__global__ void __launch_bounds__(32 * WARPS)
+hrp_reset_kernel_grid(const EnvDev P, const GridDev G, const uint8_t *__restrict__ mask, float *__restrict__ obs)
+{
+    __shared__ WarpS<R> smem[WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int e = blockIdx.x * WARPS + warp;
+    if (e >= P.E) return;
+    if (mask && !mask[e]) return;
+    WarpS<R> &S = smem[warp];
+    Veh<R> u[2];
+    double xref;
+    spawn_env(P, S, u, e, lane, 0u, xref);
+    if (lane == 0) { P.episode[e] = 0; P.time[e] = 0.0; P.obs_draw[e] += 1; }
+    if (obs) observe_grid(P, G, S, e, lane, obs, nullptr);
+    store_env(P, u, e, lane);
+}
+
 // standalone wrapper.observation() over caller-provided [B, N, F] observations
 __global__ void __launch_bounds__(128)
 hrp_embed_kernel(int kind, int edim, int use_euclid, int ego_idx, float max_dist,
@@ -1092,9 +1260,20 @@ hrp_embed_kernel(int kind, int edim, int use_euclid, int ego_idx, float max_dist
 
 }  // namespace
 
-int hrp_launch_step(const EnvDev &P, const float *actions, float *obs, float *reward, uint8_t *term,
+int hrp_launch_step(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward, uint8_t *term,
                     uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s, float *final_obs)
 {
+    if (G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        const int warps = P.real64 ? HRP_WARPS_PER_CTA_F64 : HRP_WARPS_PER_CTA;
+        const dim3 grid((P.E + warps - 1) / warps), block(32 * warps);
+        if (P.real64)
+            HRP_CUDA_OK(hrp_launch_pdl(final_obs ? hrp_step_kernel_f64_grid<true> : hrp_step_kernel_f64_grid<false>, grid,
+                                       block, 0, s, P, actions, obs, reward, term, trunc, row_vehicle, final_obs, G));
+        else
+            HRP_CUDA_OK(hrp_launch_pdl(final_obs ? hrp_step_kernel_grid<true> : hrp_step_kernel_grid<false>, grid, block,
+                                       0, s, P, actions, obs, reward, term, trunc, row_vehicle, final_obs, G));
+        return 0;
+    }
     if (P.real64) {
         int grid = (P.E + HRP_WARPS_PER_CTA_F64 - 1) / HRP_WARPS_PER_CTA_F64;
         if (final_obs) {
@@ -1116,10 +1295,17 @@ int hrp_launch_step(const EnvDev &P, const float *actions, float *obs, float *re
                                trunc, perm, row_vehicle));
     return 0;
 }
-int hrp_launch_observe(const EnvDev &P, float *obs, const int32_t *perm, int32_t *row_vehicle,
+int hrp_launch_observe(const EnvDev &P, const GridDev &G, float *obs, const int32_t *perm, int32_t *row_vehicle,
                        cudaStream_t s)
 {
-    if (P.real64) {
+    if (G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        const int warps = P.real64 ? HRP_WARPS_PER_CTA_F64 : HRP_WARPS_PER_CTA;
+        const int grid = (P.E + warps - 1) / warps;
+        if (P.real64)
+            hrp_observe_kernel_grid<double, HRP_WARPS_PER_CTA_F64><<<grid, 32 * warps, 0, s>>>(P, G, obs, row_vehicle);
+        else
+            hrp_observe_kernel_grid<float, HRP_WARPS_PER_CTA><<<grid, 32 * warps, 0, s>>>(P, G, obs, row_vehicle);
+    } else if (P.real64) {
         int grid = (P.E + HRP_WARPS_PER_CTA_F64 - 1) / HRP_WARPS_PER_CTA_F64;
         hrp_observe_kernel<double, HRP_WARPS_PER_CTA_F64><<<grid, 32 * HRP_WARPS_PER_CTA_F64, 0, s>>>(P, obs, perm, row_vehicle);
     } else {
@@ -1129,9 +1315,16 @@ int hrp_launch_observe(const EnvDev &P, float *obs, const int32_t *perm, int32_t
     HRP_CUDA_OK(cudaGetLastError());
     return 0;
 }
-int hrp_launch_reset(const EnvDev &P, const uint8_t *mask, float *obs, cudaStream_t s)
+int hrp_launch_reset(const EnvDev &P, const GridDev &G, const uint8_t *mask, float *obs, cudaStream_t s)
 {
-    if (P.real64) {
+    if (G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
+        const int warps = P.real64 ? HRP_WARPS_PER_CTA_F64 : HRP_WARPS_PER_CTA;
+        const int grid = (P.E + warps - 1) / warps;
+        if (P.real64)
+            hrp_reset_kernel_grid<double, HRP_WARPS_PER_CTA_F64><<<grid, 32 * warps, 0, s>>>(P, G, mask, obs);
+        else
+            hrp_reset_kernel_grid<float, HRP_WARPS_PER_CTA><<<grid, 32 * warps, 0, s>>>(P, G, mask, obs);
+    } else if (P.real64) {
         int grid = (P.E + HRP_WARPS_PER_CTA_F64 - 1) / HRP_WARPS_PER_CTA_F64;
         hrp_reset_kernel<double, HRP_WARPS_PER_CTA_F64><<<grid, 32 * HRP_WARPS_PER_CTA_F64, 0, s>>>(P, mask, obs);
     } else {

@@ -53,6 +53,15 @@ struct EnvDev {
 };
 #define HRP_TRACE_FIELDS 7
 
+// The OccupancyGrid observation's parameters: a second by-value argument of the grid kernels only, so that the default
+// kernels keep their parameter block (and with it their code) exactly.  gx / gy: the feature slot whose range
+// normalises the x / y position (inverse-mapped before the cell index, as upstream does), -1 for none.
+struct GridDev {
+    int obs_type;   // HRP_OBS_*: which kernels the launchers pick
+    int gw, gh, galign, gx, gy;
+    double glo[2], gstep[2];
+};
+
 // Philox4x32-10 (Salmon et al. SC'11), the counter-based generator behind spawn and shuffle.
 __host__ __device__ __forceinline__ void hrp_philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                     uint32_t k0, uint32_t k1, uint32_t out[4])
@@ -115,12 +124,12 @@ struct TcDots {
 };
 
 // launchers implemented in hrp_env.cu.  final_obs non-null: the final-observation instantiation of the step kernel.
-int hrp_launch_step(const EnvDev &P, const float *actions, float *obs, float *reward, uint8_t *term,
+int hrp_launch_step(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward, uint8_t *term,
                     uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
                     float *final_obs = nullptr);
-int hrp_launch_observe(const EnvDev &P, float *obs, const int32_t *perm, int32_t *row_vehicle,
+int hrp_launch_observe(const EnvDev &P, const GridDev &G, float *obs, const int32_t *perm, int32_t *row_vehicle,
                        cudaStream_t s);
-int hrp_launch_reset(const EnvDev &P, const uint8_t *mask, float *obs, cudaStream_t s);
+int hrp_launch_reset(const EnvDev &P, const GridDev &G, const uint8_t *mask, float *obs, cudaStream_t s);
 int hrp_launch_embed(int kind, int embed_dim, int use_euclid, int ego_idx, float max_dist,
                      const float *table, const float *obs, float *out, long long batch, int rows,
                      int cols, const float *dist_override, cudaStream_t s);

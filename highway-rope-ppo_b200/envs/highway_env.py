@@ -33,13 +33,13 @@ class HighwayEnv:
     def _make(self, embed: Optional[EmbedSpec]) -> None:
         self.vec = HighwayVecEnv(self._user_config, 1, device=self._device, embed=embed, autoreset=False)
         self.config = self.vec.config
-        N, F = self.vec.N, self.vec.F_out
-        self.observation_space = Box(-np.inf, np.inf, (N, F), np.float32)
+        shape = self.vec.obs_shape   # (N, F_out), or (F, W, H) for an OccupancyGrid
+        self.observation_space = Box(-np.inf, np.inf, shape, np.float32)
         if self.vec.cfg.ego_mode == 0:
             self.action_space = Box(-1.0, 1.0, (2,), np.float32)
         else:
             self.action_space = Discrete(5)
-        self._obs = np.zeros((1, N, F), dtype=np.float32)
+        self._obs = np.zeros((1,) + shape, dtype=np.float32)
         self._reward = np.zeros(1, dtype=np.float32)
         self._term = np.zeros(1, dtype=np.uint8)
         self._trunc = np.zeros(1, dtype=np.uint8)

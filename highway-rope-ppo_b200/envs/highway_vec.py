@@ -36,6 +36,13 @@ OBS_DEFAULTS: Dict[str, Any] = {
     "features_range": None, "absolute": False, "order": "sorted", "normalize": True, "clip": True,
     "see_behind": False, "observe_intentions": False, "include_obstacles": True,
 }
+# OccupancyGridObservation's defaults (highway-env 1.10.1): features_range None means +-2 Vehicle.MAX_SPEED on vx / vy
+GRID_DEFAULTS: Dict[str, Any] = {
+    "type": "OccupancyGrid", "features": ["presence", "vx", "vy", "on_road"],
+    "grid_size": [[-27.5, 27.5], [-27.5, 27.5]], "grid_step": [5, 5], "features_range": None,
+    "absolute": False, "align_to_vehicle_axes": False, "clip": True, "as_image": False,
+}
+GRID_FEATURES_RANGE: Dict[str, Any] = {"vx": [-80.0, 80.0], "vy": [-80.0, 80.0]}
 
 
 class EmbedSpec:
@@ -59,8 +66,11 @@ def resolve_config(cfg: Dict[str, Any]) -> Dict[str, Any]:
     observation kwargs completed with KinematicObservation's defaults."""
     full = dict(ENV_DEFAULTS)
     full.update(cfg)
-    obs = dict(OBS_DEFAULTS)
-    obs.update(full.get("observation") or {})
+    user_obs = full.get("observation") or {}
+    # the observation class follows its type: OccupancyGrid takes its own defaults (the keys a Kinematics base config
+    # leaves behind, vehicles_count, order, normalize ..., are ignored by it as upstream's **kwargs are)
+    obs = dict(GRID_DEFAULTS if user_obs.get("type") == "OccupancyGrid" else OBS_DEFAULTS)
+    obs.update(user_obs)
     full["observation"] = obs
     full.setdefault("action", {"type": "DiscreteMetaAction"})
     return full
@@ -68,18 +78,19 @@ def resolve_config(cfg: Dict[str, Any]) -> Dict[str, Any]:
 
 def build_cfg(cfg: Dict[str, Any], embed: Optional[EmbedSpec] = None, autoreset: bool = True) -> HrpCfg:
     """highway-env style config dict -> ``hrp_cfg``.  Raises ``ValueError`` for what the kernels
-    do not implement (only Kinematics observations, IDM traffic, one controlled vehicle)."""
+    do not implement (Kinematics and OccupancyGrid observations, IDM traffic, one controlled vehicle)."""
     full = resolve_config(cfg)
     obs, act = full["observation"], full["action"]
-    if obs.get("type", "Kinematics") != "Kinematics":
-        raise ValueError(f"observation type {obs.get('type')!r} is not implemented (Kinematics only)")
+    if obs.get("type", "Kinematics") not in ("Kinematics", "OccupancyGrid"):
+        raise ValueError(f"observation type {obs.get('type')!r} is not implemented (Kinematics and OccupancyGrid only)")
     if act.get("type") not in ("ContinuousAction", "DiscreteMetaAction"):
         raise ValueError(f"action type {act.get('type')!r} is not implemented")
     if act.get("type") == "ContinuousAction" and not (act.get("longitudinal", True) and act.get("lateral", True)):
         raise ValueError("ContinuousAction needs longitudinal=True and lateral=True (reference config)")
     if int(full.get("controlled_vehicles", 1)) != 1:
         raise ValueError("exactly one controlled vehicle per env is supported")
-    if obs.get("order", "sorted") not in ("sorted", "shuffled"):
+    grid = obs["type"] == "OccupancyGrid"
+    if not grid and obs.get("order", "sorted") not in ("sorted", "shuffled"):
         raise ValueError(f"observation order {obs.get('order')!r} must be 'sorted' or 'shuffled'")
     c = HrpCfg()
     c.lanes_count = int(full["lanes_count"])
@@ -97,9 +108,17 @@ def build_cfg(cfg: Dict[str, Any], embed: Optional[EmbedSpec] = None, autoreset:
     c.right_lane_reward = float(full["right_lane_reward"])
     c.high_speed_reward = float(full["high_speed_reward"])
     c.reward_speed_lo, c.reward_speed_hi = (float(v) for v in full["reward_speed_range"])
+    c.autoreset = int(bool(autoreset))
+    if grid:
+        if embed is not None and embed.kind != EMBED_NONE:
+            raise ValueError("an OccupancyGrid observation takes no embedding")
+        _grid_cfg(c, obs)
+        return c
     feats = list(obs["features"])
     if len(feats) > _lib.HRP_MAX_FEATURES:
         raise ValueError(f"at most {_lib.HRP_MAX_FEATURES} features are supported")
+    if "on_road" in feats:
+        raise ValueError("feature 'on_road' is an OccupancyGrid layer; a Kinematics observation has no such column")
     c.obs_vehicles = int(obs["vehicles_count"])
     c.obs_nfeat = len(feats)
     width = 4.0 * c.lanes_count
@@ -122,8 +141,47 @@ def build_cfg(cfg: Dict[str, Any], embed: Optional[EmbedSpec] = None, autoreset:
     c.embed_use_euclidean = int(e.use_euclidean)
     c.embed_max_dist = e.max_dist
     c.embed_ego_idx = e.ego_idx
-    c.autoreset = int(bool(autoreset))
     return c
+
+
+def grid_shape(obs: Dict[str, Any]):
+    """(W, H) of an OccupancyGrid config: ``floor((size[a][1] - size[a][0]) / step[a])`` in fp64."""
+    size, step = obs["grid_size"], obs["grid_step"]
+    return tuple(int(math.floor((float(size[a][1]) - float(size[a][0])) / float(step[a]))) for a in range(2))
+
+
+def _grid_cfg(c: HrpCfg, obs: Dict[str, Any]) -> None:
+    """The OccupancyGrid fields of ``hrp_cfg`` (``obs`` resolved); ``ValueError`` for what the kernel does not do."""
+    if obs.get("absolute"):
+        raise ValueError("OccupancyGrid absolute=True is not implemented (upstream raises NotImplementedError)")
+    if obs.get("as_image"):
+        raise ValueError("OccupancyGrid as_image=True is not implemented")
+    feats = list(obs["features"])
+    if not 1 <= len(feats) <= _lib.HRP_MAX_FEATURES:
+        raise ValueError(f"an OccupancyGrid takes 1 to {_lib.HRP_MAX_FEATURES} features, got {len(feats)}")
+    size, step = obs["grid_size"], obs["grid_step"]
+    if len(size) != 2 or any(len(r) != 2 for r in size) or len(step) != 2:
+        raise ValueError(f"grid_size must be [[x0, x1], [y0, y1]] and grid_step [sx, sy]; got {size}, {step}")
+    if not all(float(s) > 0 and math.isfinite(float(s)) for s in step):
+        raise ValueError(f"grid_step must be positive, got {step}")
+    W, H = grid_shape(obs)
+    if W < 1 or H < 1 or len(feats) * W * H > _lib.HRP_MAX_GRID_VALUES:
+        raise ValueError(f"grid of {len(feats)} x {W} x {H} outside 1 <= W, H and F x W x H <= {_lib.HRP_MAX_GRID_VALUES}")
+    ranges = obs.get("features_range") or GRID_FEATURES_RANGE   # a user dict replaces the default entirely
+    c.obs_type = _lib.OBS_OCCUPANCY_GRID
+    c.obs_nfeat = len(feats)
+    for i, name in enumerate(feats):
+        if name not in FEATURE_CODES:
+            raise ValueError(f"feature {name!r} is not implemented; known: {sorted(FEATURE_CODES)}")
+        c.obs_feat[i] = FEATURE_CODES[name]
+        if name in ranges and name != "on_road":
+            c.obs_has_range[i] = 1
+            c.obs_lo[i], c.obs_hi[i] = float(ranges[name][0]), float(ranges[name][1])
+    c.obs_clip = int(bool(obs["clip"]))
+    c.grid_align = int(bool(obs["align_to_vehicle_axes"]))
+    for a in range(2):
+        c.grid_lo[a], c.grid_hi[a] = float(size[a][0]), float(size[a][1])
+        c.grid_step[a] = float(step[a])
 
 
 class HighwayVecEnv:
@@ -164,10 +222,17 @@ class HighwayVecEnv:
         self.V = int(lib.hrp_env_num_vehicles(h))
         rows, cols = C.c_int32(), C.c_int32()
         _lib.check(lib.hrp_env_obs_dim(h, C.byref(rows), C.byref(cols)), "hrp_env_obs_dim")
+        # rows x cols: N x F_out for Kinematics, F x (W * H) for a grid, so that every N * F_out consumer sizes both
         self.N, self.F_out = int(rows.value), int(cols.value)
         self.F = int(self.cfg.obs_nfeat)
+        self.grid = self.cfg.obs_type == _lib.OBS_OCCUPANCY_GRID
+        self._obs_shape = (self.N, self.F_out)
+        if self.grid:
+            f, w, hh = C.c_int32(), C.c_int32(), C.c_int32()
+            _lib.check(lib.hrp_env_grid_shape(h, C.byref(f), C.byref(w), C.byref(hh)), "hrp_env_grid_shape")
+            self._obs_shape = (int(f.value), int(w.value), int(hh.value))
         E = self.num_envs
-        self.obs = torch.zeros((E, self.N, self.F_out), dtype=torch.float32, device=self.device)
+        self.obs = torch.zeros((E,) + self._obs_shape, dtype=torch.float32, device=self.device)
         self.reward = torch.zeros(E, dtype=torch.float32, device=self.device)
         self.terminated = torch.zeros(E, dtype=torch.uint8, device=self.device)
         self.truncated = torch.zeros(E, dtype=torch.uint8, device=self.device)
@@ -195,7 +260,8 @@ class HighwayVecEnv:
 
     @property
     def obs_shape(self):
-        return (self.N, self.F_out)
+        """(N, F_out) for Kinematics, (F, W, H) for an OccupancyGrid."""
+        return self._obs_shape
 
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -220,7 +286,7 @@ class HighwayVecEnv:
              truncated_out: Optional[torch.Tensor] = None, final_obs_out: Optional[torch.Tensor] = None):
         """One policy step of every env.  ``actions``: float32 [E, 2] on the device.
 
-        Returns (obs [E,N,F_out], reward [E], terminated [E] uint8, truncated [E] uint8); the
+        Returns (obs [E,N,F_out] -- [E,F,W,H] for a grid --, reward [E], terminated [E] uint8, truncated [E] uint8); the
         tensors are the handle's own output buffers unless ``out`` (observation) / ``reward_out`` /
         ``terminated_out`` / ``truncated_out`` name the caller's (contiguous, e.g. the slot of a rollout buffer: the
         kernel then writes the rollout directly, no copy kernels between the step and the next policy forward).
@@ -235,6 +301,8 @@ class HighwayVecEnv:
             raise ValueError(f"actions must hold {self.num_envs} x 2 floats, got shape {tuple(actions.shape)}")
         obs = self.obs if out is None else out
         if perm is not None:
+            if self.grid:
+                raise ValueError("perm: an OccupancyGrid observation has no row order")
             perm = perm.to(device=self.device, dtype=torch.int32).contiguous()
             if perm.numel() != self.num_envs * (self.N - 1):
                 raise ValueError("perm must be [E, N-1]")

@@ -62,7 +62,7 @@ class _Group:
         self.seeds_host, self.seeds = pin(R, dtype=torch.int64), torch.zeros(R, dtype=torch.int64, device=d)
         self.mask_host, self.mask = pin(R, dtype=torch.uint8), torch.zeros(R, dtype=torch.uint8, device=d)
         self.reset_mask = torch.zeros(R, dtype=torch.uint8, device=d)
-        self.obs_host = pin(R, env.N, env.F_out)
+        self.obs_host = pin(R, *env.obs_shape)   # (N, F_out), or (F, W, H) for an OccupancyGrid: what the single env returns
         A = 2
         # per experiment: action | pre_tanh | log_prob | value, written by its policy kernels, read back in one copy
         self.res, self.res_host = torch.zeros((R, 2 * A + 2), device=d), pin(R, 2 * A + 2)

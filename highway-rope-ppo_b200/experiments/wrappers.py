@@ -18,6 +18,7 @@ from .rank_embed import RankEmbedWrapper
 from .rope_embed import RotaryEmbedWrapper, rope_inv_freq
 
 _SHUFFLED = (Condition.SHUFFLED, Condition.SHUFFLED_RANKPE, Condition.SHUFFLED_DISTPE, Condition.SHUFFLED_ROPE)
+_EMBEDDED = (Condition.SHUFFLED_RANKPE, Condition.SHUFFLED_DISTPE, Condition.SHUFFLED_ROPE)
 
 
 def _merge(dst: Dict[str, Any], src: Dict[str, Any]) -> None:
@@ -35,6 +36,10 @@ def _resolve(exp_condition: Condition, base_cfg: Dict[str, Any], d_embed: Option
     cfg = copy.deepcopy(base_cfg)
     _merge(cfg, env_overrides)
     obs_cfg = cfg.setdefault("observation", {})
+    # an OccupancyGrid has no rows to order or to embed: SORTED / SHUFFLED select it unchanged (its `order` is ignored),
+    # the embedding conditions are refused before any device work
+    if obs_cfg.get("type") == "OccupancyGrid" and exp_condition in _EMBEDDED:
+        raise ValueError(f"condition {exp_condition.name} embeds observation rows; an OccupancyGrid observation has none")
     # setdefault: a base config that already names an order keeps it (SURVEY.md F3 -- with the stock
     # HIGHWAY_CONFIG, which says "sorted", the SHUFFLED_* conditions are NOT shuffled unless
     # env_overrides={"observation": {"order": "shuffled"}} is passed)

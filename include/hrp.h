@@ -35,9 +35,13 @@ extern "C" {
 #define HRP_MAX_EMBED 64
 #define HRP_MAX_EMBED_COLS 1024 /* F of hrp_embed_apply on caller-provided observations */
 
+#define HRP_MAX_GRID_VALUES (HRP_MAX_OBS_ROWS * HRP_MAX_FEATURES) /* F*W*H of an OccupancyGrid observation */
+
 /* Kinematics feature codes (highway-env Vehicle.to_dict keys used by
- * config/base_config.py:9,11-19) */
-enum { HRP_F_PRESENCE = 0, HRP_F_X, HRP_F_Y, HRP_F_VX, HRP_F_VY, HRP_F_HEADING, HRP_F_COS_H, HRP_F_SIN_H };
+ * config/base_config.py:9,11-19); HRP_F_ON_ROAD is the OccupancyGrid road layer and is valid in a grid only */
+enum { HRP_F_PRESENCE = 0, HRP_F_X, HRP_F_Y, HRP_F_VX, HRP_F_VY, HRP_F_HEADING, HRP_F_COS_H, HRP_F_SIN_H, HRP_F_ON_ROAD };
+/* observation types */
+enum { HRP_OBS_KINEMATICS = 0, HRP_OBS_OCCUPANCY_GRID = 1 };
 /* observation embedding fused behind the Kinematics observation */
 enum { HRP_EMBED_NONE = 0, HRP_EMBED_ROPE = 1, HRP_EMBED_DIST = 2, HRP_EMBED_RANK = 3 };
 
@@ -79,6 +83,16 @@ typedef struct hrp_cfg {
     /* vec-env behaviour */
     int32_t autoreset;             /* respawn inside the step that ended the episode */
     int32_t embed_ego_idx;         /* ego_idx of the embed wrappers (row the distance refers to) */
+    /* OccupancyGridObservation (absolute=False, as_image=False).  obs_type 0 (all of this zero) is Kinematics.  A grid
+     * uses obs_nfeat / obs_feat (HRP_F_ON_ROAD allowed), obs_has_range / obs_lo / obs_hi as features_range and obs_clip
+     * as clip; obs_vehicles, obs_normalize, obs_absolute, obs_sorted and obs_see_behind are ignored, and embed_kind
+     * must be HRP_EMBED_NONE.  W = floor((grid_hi[0] - grid_lo[0]) / grid_step[0]), H likewise (fp64), 1 <= W, H and
+     * F*W*H <= HRP_MAX_GRID_VALUES.  The observation is float32 [F][W][H]; DESIGN.md §3.1 states its semantics. */
+    int32_t obs_type;              /* HRP_OBS_* */
+    int32_t grid_align;            /* align_to_vehicle_axes */
+    double  grid_lo[2];            /* grid_size[0][0], grid_size[1][0] */
+    double  grid_hi[2];            /* grid_size[0][1], grid_size[1][1] */
+    double  grid_step[2];
 } hrp_cfg;
 
 /* Host-side SoA view of the simulator state, [num_envs * V] per vehicle field
@@ -114,7 +128,10 @@ int hrp_env_create(const hrp_cfg *cfg, const float *embed_table_host, int64_t em
 int hrp_env_create_ex(const hrp_cfg *cfg, const float *embed_table_host, int64_t embed_table_len,
                       int32_t num_envs, uint64_t env_id_base, int32_t device, uint32_t flags, hrp_env **out);
 int hrp_env_destroy(hrp_env *env);
+/* observation extent per env: rows = N and cols = F_out for Kinematics, rows = F and cols = W*H for a grid */
 int hrp_env_obs_dim(const hrp_env *env, int32_t *rows, int32_t *cols);
+/* F, W, H of an OccupancyGrid handle; -1 for a Kinematics handle */
+int hrp_env_grid_shape(const hrp_env *env, int32_t *features, int32_t *width, int32_t *height);
 int hrp_env_num_vehicles(const hrp_env *env);
 
 /* env.reset(seed=...) (training/routine.py:18,127): counter-based spawn of every env whose
@@ -124,7 +141,9 @@ int hrp_env_reset(hrp_env *env, uint64_t seed, const uint8_t *mask_dev, float *o
 /* env.step(action) (training/routine.py:24,134): 15 fused sub-steps + observation + embedding.
  * actions_dev[E,2] float32 (ContinuousAction) or [E,2] with the meta-action id in column 0.
  * perm_dev (nullable) [E,N-1] int32 injects the row shuffle; row_vehicle_dev (nullable)
- * [E,N] int32 receives the vehicle index shown in each row (-1 padding). */
+ * [E,N] int32 receives the vehicle index shown in each row (-1 padding).
+ * OccupancyGrid handle: obs_dev is [E,F,W,H]; perm_dev must be NULL (-1 otherwise); row_vehicle_dev is [E,W*H] and
+ * receives the vehicle whose values fill each cell, -1 for a cell no vehicle is in. */
 int hrp_env_step(hrp_env *env, const float *actions_dev, float *obs_dev, float *reward_dev,
                  uint8_t *terminated_dev, uint8_t *truncated_dev, const int32_t *perm_dev,
                  int32_t *row_vehicle_dev, void *stream);
