@@ -53,6 +53,7 @@ class HrpCfg(C.Structure):
         ("autoreset", C.c_int32), ("embed_ego_idx", C.c_int32),
         ("obs_type", C.c_int32), ("grid_align", C.c_int32),
         ("grid_lo", C.c_double * 2), ("grid_hi", C.c_double * 2), ("grid_step", C.c_double * 2),
+        ("ego_collisions_only", C.c_int32),
     ]
 
 

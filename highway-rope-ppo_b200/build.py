@@ -14,7 +14,7 @@ ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_DIR = os.path.join(PKG_DIR, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libhrp_b200.so")
-SOURCES = ["hrp_env.cu", "hrp_api.cu", "hrp_ppo.cu", "hrp_mlp_tc.cu", "hrp_comm.cu", "hrp_episodes.cu"]
+SOURCES = ["hrp_env.cu", "hrp_env_fast.cu", "hrp_api.cu", "hrp_ppo.cu", "hrp_mlp_tc.cu", "hrp_comm.cu", "hrp_episodes.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC",
@@ -24,7 +24,9 @@ NVCC_FLAGS = [
 # approximations that lose their error bound at the 2 pi angles RoPE / DistPE reach.  The epilogue's float32 operation
 # order is kept by explicit __f*_rn intrinsics (exact whatever these flags say); the fp64 validation instantiation is
 # not affected by them.  The PPO files stay IEEE.
+# hrp_env_fast.cu is hrp_env.cu built with the highway-fast-v0 collision pass, so it takes the same flags.
 EXTRA_FLAGS = {"hrp_env.cu": ["-ftz=true", "-prec-div=false", "-prec-sqrt=false"]}
+EXTRA_FLAGS["hrp_env_fast.cu"] = EXTRA_FLAGS["hrp_env.cu"]
 
 
 def _sources():

@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(256) fetch_host_kernel(const uint4 *__restrict
 extern "C" {
 
 const char *hrp_last_error(void) { return g_err; }
-int hrp_version(void) { return 2; }   // 2: OccupancyGrid fields of hrp_cfg, hrp_env_grid_shape
+int hrp_version(void) { return 3; }   // 2: OccupancyGrid fields of hrp_cfg, hrp_env_grid_shape; 3: ego_collisions_only
 int hrp_device_count(void)
 {
     int n = 0;
@@ -162,6 +162,10 @@ static int validate_grid(const hrp_cfg *c)
 
 static int validate_cfg(const hrp_cfg *c, int64_t table_len)
 {
+    if (c->ego_collisions_only != 0 && c->ego_collisions_only != 1) {
+        hrp_set_error("ego_collisions_only %d not in {0 (highway-v0), 1 (highway-fast-v0)}", c->ego_collisions_only);
+        return -1;
+    }
     if (c->vehicles_count < 0 || c->vehicles_count + 1 > HRP_MAX_VEHICLES) {
         hrp_set_error("vehicles_count %d outside [0, %d]", c->vehicles_count, HRP_MAX_VEHICLES - 1);
         return -1;
@@ -378,8 +382,8 @@ int hrp_env_step(hrp_env *h, const float *actions_dev, float *obs_dev, float *re
         hrp_set_error("hrp_env_step: perm_dev must be NULL for an OccupancyGrid handle (a grid has no row order)");
         return -1;
     }
-    return hrp_launch_step(h->P, h->G, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
-                           row_vehicle_dev, (cudaStream_t)stream);
+    return hrp_launch_step(h->P, h->G, h->cfg.ego_collisions_only != 0, actions_dev, obs_dev, reward_dev, terminated_dev,
+                           truncated_dev, perm_dev, row_vehicle_dev, (cudaStream_t)stream);
 }
 
 int hrp_env_step_final(hrp_env *h, const float *actions_dev, float *obs_dev, float *reward_dev,
@@ -398,8 +402,8 @@ int hrp_env_step_final(hrp_env *h, const float *actions_dev, float *obs_dev, flo
         hrp_set_error("hrp_env_step_final: perm_dev must be NULL for an OccupancyGrid handle (a grid has no row order)");
         return -1;
     }
-    return hrp_launch_step(h->P, h->G, actions_dev, obs_dev, reward_dev, terminated_dev, truncated_dev, perm_dev,
-                           row_vehicle_dev, (cudaStream_t)stream, final_obs_dev);
+    return hrp_launch_step(h->P, h->G, h->cfg.ego_collisions_only != 0, actions_dev, obs_dev, reward_dev, terminated_dev,
+                           truncated_dev, perm_dev, row_vehicle_dev, (cudaStream_t)stream, final_obs_dev);
 }
 
 int hrp_env_observe(hrp_env *h, float *obs_dev, const int32_t *perm_dev, int32_t *row_vehicle_dev,
@@ -485,14 +489,17 @@ static int step_host_impl(hrp_env *h, const float *actions, float *obs_host, flo
             cudaHostGetDevicePointer((void **)&r_dev, reward_host, 0) == cudaSuccess &&
             cudaHostGetDevicePointer((void **)&te_dev, terminated_host, 0) == cudaSuccess &&
             cudaHostGetDevicePointer((void **)&tr_dev, truncated_host, 0) == cudaSuccess) {
-            if (int rc = hrp_launch_step(h->P, h->G, d_act, o_dev, r_dev, te_dev, tr_dev, nullptr, nullptr, s)) return rc;
+            if (int rc = hrp_launch_step(h->P, h->G, h->cfg.ego_collisions_only != 0, d_act, o_dev, r_dev, te_dev, tr_dev,
+                                         nullptr, nullptr, s))
+                return rc;
             if (!sync) return 0;
             HRP_CUDA_OK(cudaStreamSynchronize(s));
             return 0;
         }
         cudaGetLastError();   // not mapped: fall through to the copies
     }
-    if (int rc = hrp_launch_step(h->P, h->G, d_act, h->d_obs, h->d_reward, h->d_term, h->d_trunc, nullptr, nullptr, s))
+    if (int rc = hrp_launch_step(h->P, h->G, h->cfg.ego_collisions_only != 0, d_act, h->d_obs, h->d_reward, h->d_term,
+                                 h->d_trunc, nullptr, nullptr, s))
         return rc;
     HRP_CUDA_OK(cudaMemcpyAsync(pin_o ? obs_host : h->h_obs, h->d_obs, no * sizeof(float), cudaMemcpyDeviceToHost, s));
     HRP_CUDA_OK(cudaMemcpyAsync(pin_r ? reward_host : h->h_reward, h->d_reward, E * sizeof(float), cudaMemcpyDeviceToHost, s));

@@ -740,8 +740,9 @@ __device__ void observe_grid(const EnvDev &P, const GridDev &G, WarpS<R> &S, int
 }
 
 // ---------------------------------------------------------------------------------------
-// One simulation frame: Road.act() then Road.step(dt) (SURVEY A.11)
-template <typename R>
+// One simulation frame: Road.act() then Road.step(dt) (SURVEY A.11).  EGO_ONLY: highway-fast-v0's collision rule
+// (hrp_cfg.ego_collisions_only; DESIGN.md Appendix C): only the pairs (0, k) are tested.
+template <typename R, bool EGO_ONLY = false>
 __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int lane, double xref)
 {
     const int V = P.V;
@@ -911,50 +912,79 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
     __syncwarp();
     rank_repair(S, V, lane);
 
-    // ---- collisions: pairs within the pre-check radius are neighbours in rank order
-    int a[2];
-    R xa[2];
-#pragma unroll
-    for (int q = 0; q < 2; ++q) {
-        a[q] = lane + 32 * q < V ? (int)S.order[lane + 32 * q] : -1;
-        xa[q] = S.rec[max(a[q], 0)].xr;
-    }
-    for (int off = 1; off < V; ++off) {
-        int b[2];
-        bool cand[2];
+    if constexpr (EGO_ONLY) {
+        // ---- collisions of highway-fast-v0: lane l tests pairs (0, l) and (0, l + 32) in one pass.  The ego's
+        // partners can sit any number of ranks away (two uncontrolled vehicles between them are not tested against
+        // each other), so this is a window on |x_k - x_0|, not the rank-neighbour sweep below.
+        const R x0 = S.rec[0].xr;
 #pragma unroll
         for (int q = 0; q < 2; ++q) {
-            int s2 = lane + 32 * q + off;
-            cand[q] = a[q] >= 0 && s2 < V;
-            b[q] = 0;
-            if (cand[q]) {
-                b[q] = S.order[s2];
-                cand[q] = S.rec[b[q]].xr - xa[q] <= window;  // >= sqrt(29) + max speed * dt
-            }
-        }
-        if (!__any_sync(HRP_FULL, cand[0] || cand[1])) break;
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            int ev = 0, ei = 0, ej = 0;
+            const int k = lane + 32 * q;
+            int ev = 0;
             R tx = R(0), ty = R(0);
-            if (cand[q]) {
-                ei = min(a[q], b[q]); ej = max(a[q], b[q]);
-                ev = collide_pair(S, ei, ej, dt, tx, ty);
-            }
+            if (k >= 1 && k < V && fabs(S.rec[k].xr - x0) <= window) ev = collide_pair(S, 0, k, dt, tx, ty);
             unsigned evm = __ballot_sync(HRP_FULL, ev != 0);
-            while (evm) {  // rare: serialise so that the last pair in (i, j) order wins the impact
+            while (evm) {  // rare: serialise in k order, so that the ego keeps the impact of its last pair
                 int src = __ffs(evm) - 1;
                 evm &= evm - 1;
                 int bv = __shfl_sync(HRP_FULL, ev, src);
-                int bi = __shfl_sync(HRP_FULL, ei, src), bj = __shfl_sync(HRP_FULL, ej, src);
                 R btx = __shfl_sync(HRP_FULL, tx, src), bty = __shfl_sync(HRP_FULL, ty, src);
                 if (lane == 0) {
+                    const int bk = src + 32 * q;
                     if (bv & 2) {
-                        int ki = 64 + bj, kj = bi;  // pairs (i, *) come after every pair (*, i)
-                        if (ki > S.impkey[bi]) { S.impkey[bi] = ki; S.impx[bi] = R(0.5) * btx; S.impy[bi] = R(0.5) * bty; }
-                        if (kj > S.impkey[bj]) { S.impkey[bj] = kj; S.impx[bj] = R(-0.5) * btx; S.impy[bj] = R(-0.5) * bty; }
+                        S.impkey[0] = 64 + bk; S.impx[0] = R(0.5) * btx; S.impy[0] = R(0.5) * bty;
+                        S.impkey[bk] = 0; S.impx[bk] = R(-0.5) * btx; S.impy[bk] = R(-0.5) * bty;
                     }
-                    if (bv & 1) { S.crash[bi] = 1; S.crash[bj] = 1; }
+                    if (bv & 1) { S.crash[0] = 1; S.crash[bk] = 1; }
+                }
+            }
+        }
+    } else {
+        // ---- collisions: pairs within the pre-check radius are neighbours in rank order
+        int a[2];
+        R xa[2];
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            a[q] = lane + 32 * q < V ? (int)S.order[lane + 32 * q] : -1;
+            xa[q] = S.rec[max(a[q], 0)].xr;
+        }
+        for (int off = 1; off < V; ++off) {
+            int b[2];
+            bool cand[2];
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                int s2 = lane + 32 * q + off;
+                cand[q] = a[q] >= 0 && s2 < V;
+                b[q] = 0;
+                if (cand[q]) {
+                    b[q] = S.order[s2];
+                    cand[q] = S.rec[b[q]].xr - xa[q] <= window;  // >= sqrt(29) + max speed * dt
+                }
+            }
+            if (!__any_sync(HRP_FULL, cand[0] || cand[1])) break;
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                int ev = 0, ei = 0, ej = 0;
+                R tx = R(0), ty = R(0);
+                if (cand[q]) {
+                    ei = min(a[q], b[q]); ej = max(a[q], b[q]);
+                    ev = collide_pair(S, ei, ej, dt, tx, ty);
+                }
+                unsigned evm = __ballot_sync(HRP_FULL, ev != 0);
+                while (evm) {  // rare: serialise so that the last pair in (i, j) order wins the impact
+                    int src = __ffs(evm) - 1;
+                    evm &= evm - 1;
+                    int bv = __shfl_sync(HRP_FULL, ev, src);
+                    int bi = __shfl_sync(HRP_FULL, ei, src), bj = __shfl_sync(HRP_FULL, ej, src);
+                    R btx = __shfl_sync(HRP_FULL, tx, src), bty = __shfl_sync(HRP_FULL, ty, src);
+                    if (lane == 0) {
+                        if (bv & 2) {
+                            int ki = 64 + bj, kj = bi;  // pairs (i, *) come after every pair (*, i)
+                            if (ki > S.impkey[bi]) { S.impkey[bi] = ki; S.impx[bi] = R(0.5) * btx; S.impy[bi] = R(0.5) * bty; }
+                            if (kj > S.impkey[bj]) { S.impkey[bj] = kj; S.impx[bj] = R(-0.5) * btx; S.impy[bj] = R(-0.5) * bty; }
+                        }
+                        if (bv & 1) { S.crash[bi] = 1; S.crash[bj] = 1; }
+                    }
                 }
             }
         }
@@ -979,7 +1009,8 @@ __device__ void simulate_frame(const EnvDev &P, WarpS<R> &S, Veh<R> (&u)[2], int
 // default kernels carry none of its code: the step kernel is sensitive to instruction-cache pressure (DESIGN.md §3.1).
 // OBS: the observation epilogue, HRP_OBS_KINEMATICS or HRP_OBS_OCCUPANCY_GRID -- compile-time for the same reason, and
 // with one call site of observe_env / observe_grid per instantiation.
-template <typename R, int WARPS, bool FINAL = false, int OBS = HRP_OBS_KINEMATICS>
+// EGO_ONLY: highway-fast-v0's ego-only collision pass (simulate_frame) -- compile-time for the same reason.
+template <typename R, int WARPS, bool FINAL = false, int OBS = HRP_OBS_KINEMATICS, bool EGO_ONLY = false>
 __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restrict__ actions, float *__restrict__ obs,
                                           float *__restrict__ reward, uint8_t *__restrict__ term,
                                           uint8_t *__restrict__ trunc, const int32_t *__restrict__ perm,
@@ -1032,7 +1063,7 @@ __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restri
     __syncwarp();
 
     for (int frame = 0; frame < P.frames; ++frame) {
-        simulate_frame(P, S, u, lane, xref);
+        simulate_frame<R, EGO_ONLY>(P, S, u, lane, xref);
         if (P.trace) {   // validation aid: the intra-step trajectory, for the frame-by-frame parity check
             double *t = P.trace + (((size_t)e * P.frames + frame) * HRP_VS) * HRP_TRACE_FIELDS;
 #pragma unroll
@@ -1118,6 +1149,12 @@ __device__ __forceinline__ void step_body(const EnvDev &P, const float *__restri
     store_env(P, u, e, lane);
 }
 
+// The kernels and launchers below are built twice.  This file on its own is the default translation unit: every
+// highway-v0 kernel.  hrp_env_fast.cu includes it with HRP_ENV_FAST_TU defined and gets the highway-fast-v0 step
+// kernels instead.  A separate translation unit because the compiler's inlining choices for the shared device
+// functions depend on how many kernels call them: kept apart, the default kernels compile exactly as they would without
+// the fast ones.
+#ifndef HRP_ENV_FAST_TU
 __global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA, HRP_STEP_CTAS_PER_SM)
 hrp_step_kernel(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
                 float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
@@ -1258,11 +1295,40 @@ hrp_embed_kernel(int kind, int edim, int use_euclid, int ego_idx, float max_dist
                 out + (size_t)b * N * Fout, dist_override ? dist_override + (size_t)b * N : nullptr);
 }
 
+#else
+// highway-fast-v0 (hrp_cfg.ego_collisions_only = 1): the eight step kernels of the default translation unit with the
+// ego-only collision pass, fp32 / fp64 x with and without final_obs x Kinematics / OccupancyGrid.  One parameter list for all of them (perm is
+// NULL for a grid, G unused by Kinematics), so that the launcher picks one from a table.
+template <bool FINAL, int OBS>
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA, HRP_STEP_CTAS_PER_SM)
+hrp_step_kernel_ego(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                    float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                    const int32_t *__restrict__ perm, int32_t *__restrict__ row_vehicle, float *__restrict__ final_obs,
+                    const GridDev G)
+{
+    step_body<float, HRP_WARPS_PER_CTA, FINAL, OBS, true>(P, actions, obs, reward, term, trunc, perm, row_vehicle,
+                                                          final_obs, G);
+}
+template <bool FINAL, int OBS>
+__global__ void __launch_bounds__(32 * HRP_WARPS_PER_CTA_F64)
+hrp_step_kernel_f64_ego(const EnvDev P, const float *__restrict__ actions, float *__restrict__ obs,
+                        float *__restrict__ reward, uint8_t *__restrict__ term, uint8_t *__restrict__ trunc,
+                        const int32_t *__restrict__ perm, int32_t *__restrict__ row_vehicle,
+                        float *__restrict__ final_obs, const GridDev G)
+{
+    step_body<double, HRP_WARPS_PER_CTA_F64, FINAL, OBS, true>(P, actions, obs, reward, term, trunc, perm, row_vehicle,
+                                                               final_obs, G);
+}
+#endif
 }  // namespace
 
-int hrp_launch_step(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward, uint8_t *term,
-                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s, float *final_obs)
+#ifndef HRP_ENV_FAST_TU
+int hrp_launch_step(const EnvDev &P, const GridDev &G, bool ego_only, const float *actions, float *obs, float *reward,
+                    uint8_t *term, uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
+                    float *final_obs)
 {
+    if (ego_only)
+        return hrp_launch_step_ego(P, G, actions, obs, reward, term, trunc, perm, row_vehicle, s, final_obs);
     if (G.obs_type == HRP_OBS_OCCUPANCY_GRID) {
         const int warps = P.real64 ? HRP_WARPS_PER_CTA_F64 : HRP_WARPS_PER_CTA;
         const dim3 grid((P.E + warps - 1) / warps), block(32 * warps);
@@ -1345,3 +1411,23 @@ int hrp_launch_embed(int kind, int embed_dim, int use_euclid, int ego_idx, float
     HRP_CUDA_OK(cudaGetLastError());
     return 0;
 }
+#else
+int hrp_launch_step_ego(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward,
+                        uint8_t *term, uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
+                        float *final_obs)
+{
+    typedef void (*StepKernel)(const EnvDev, const float *, float *, float *, uint8_t *, uint8_t *, const int32_t *,
+                               int32_t *, float *, const GridDev);
+    static const StepKernel kernels[2][2][2] = {   // [real64][final_obs][grid]
+        {{hrp_step_kernel_ego<false, HRP_OBS_KINEMATICS>, hrp_step_kernel_ego<false, HRP_OBS_OCCUPANCY_GRID>},
+         {hrp_step_kernel_ego<true, HRP_OBS_KINEMATICS>, hrp_step_kernel_ego<true, HRP_OBS_OCCUPANCY_GRID>}},
+        {{hrp_step_kernel_f64_ego<false, HRP_OBS_KINEMATICS>, hrp_step_kernel_f64_ego<false, HRP_OBS_OCCUPANCY_GRID>},
+         {hrp_step_kernel_f64_ego<true, HRP_OBS_KINEMATICS>, hrp_step_kernel_f64_ego<true, HRP_OBS_OCCUPANCY_GRID>}}};
+    const bool grid = G.obs_type == HRP_OBS_OCCUPANCY_GRID;
+    const int warps = P.real64 ? HRP_WARPS_PER_CTA_F64 : HRP_WARPS_PER_CTA;
+    HRP_CUDA_OK(hrp_launch_pdl(kernels[P.real64 ? 1 : 0][final_obs ? 1 : 0][grid ? 1 : 0],
+                               dim3((P.E + warps - 1) / warps), dim3(32 * warps), 0, s, P, actions, obs, reward,
+                               term, trunc, grid ? nullptr : perm, row_vehicle, final_obs, G));
+    return 0;
+}
+#endif

@@ -124,9 +124,15 @@ struct TcDots {
 };
 
 // launchers implemented in hrp_env.cu.  final_obs non-null: the final-observation instantiation of the step kernel.
-int hrp_launch_step(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward, uint8_t *term,
-                    uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
+// ego_only: the highway-fast-v0 instantiations (hrp_cfg.ego_collisions_only), whose collision pass tests the ego's
+// pairs only.
+int hrp_launch_step(const EnvDev &P, const GridDev &G, bool ego_only, const float *actions, float *obs, float *reward,
+                    uint8_t *term, uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
                     float *final_obs = nullptr);
+// the highway-fast-v0 step kernels (hrp_env_fast.cu), which hrp_launch_step forwards to
+int hrp_launch_step_ego(const EnvDev &P, const GridDev &G, const float *actions, float *obs, float *reward,
+                        uint8_t *term, uint8_t *trunc, const int32_t *perm, int32_t *row_vehicle, cudaStream_t s,
+                        float *final_obs);
 int hrp_launch_observe(const EnvDev &P, const GridDev &G, float *obs, const int32_t *perm, int32_t *row_vehicle,
                        cudaStream_t s);
 int hrp_launch_reset(const EnvDev &P, const GridDev &G, const uint8_t *mask, float *obs, cudaStream_t s);

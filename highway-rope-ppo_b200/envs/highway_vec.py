@@ -1,4 +1,4 @@
-"""E lock-step highway-v0 episodes on one GPU, behind ``libhrp_b200.so``.
+"""E lock-step highway-v0 (or highway-fast-v0) episodes on one GPU, behind ``libhrp_b200.so``.
 
 This is the batched counterpart of what the reference obtains from
 ``gym.make("highway-v0", config=cfg)`` (``experiments/wrappers.py:80``) plus the observation
@@ -31,6 +31,12 @@ ENV_DEFAULTS: Dict[str, Any] = {
     "simulation_frequency": 15, "policy_frequency": 1,
     "other_vehicles_type": "highway_env.vehicle.behavior.IDMVehicle",
 }
+# HighwayEnvFast.default_config(): HighwayEnv's updated with these (highway-env 1.10.1).  The variant also switches off
+# collision checks between uncontrolled vehicles (hrp_cfg.ego_collisions_only; DESIGN.md Appendix C).
+FAST_ENV_DEFAULTS: Dict[str, Any] = dict(ENV_DEFAULTS, simulation_frequency=5, lanes_count=3, vehicles_count=20,
+                                         duration=30, ego_spacing=1.5)
+# the config key "gym_id" (this package's key: upstream ignores unknown keys) selects the env id
+ENV_IDS: Dict[str, Dict[str, Any]] = {"highway-v0": ENV_DEFAULTS, "highway-fast-v0": FAST_ENV_DEFAULTS}
 OBS_DEFAULTS: Dict[str, Any] = {
     "type": "Kinematics", "vehicles_count": 5, "features": ["presence", "x", "y", "vx", "vy"],
     "features_range": None, "absolute": False, "order": "sorted", "normalize": True, "clip": True,
@@ -62,10 +68,15 @@ class EmbedSpec:
 
 
 def resolve_config(cfg: Dict[str, Any]) -> Dict[str, Any]:
-    """``HighwayEnv.default_config()`` shallow-updated by ``cfg`` (highway-env's ``configure``),
-    observation kwargs completed with KinematicObservation's defaults."""
-    full = dict(ENV_DEFAULTS)
+    """The ``default_config()`` of ``cfg["gym_id"]`` (``"highway-v0"`` when absent, or ``"highway-fast-v0"``)
+    shallow-updated by ``cfg`` (highway-env's ``configure``), observation kwargs completed with KinematicObservation's
+    defaults.  The resolved dict keeps ``gym_id``.  Another id is a ``ValueError``."""
+    gym_id = cfg.get("gym_id", "highway-v0")
+    if gym_id not in ENV_IDS:
+        raise ValueError(f"gym_id {gym_id!r} is not implemented; accepted ids: {', '.join(map(repr, ENV_IDS))}")
+    full = dict(ENV_IDS[gym_id])
     full.update(cfg)
+    full["gym_id"] = gym_id
     user_obs = full.get("observation") or {}
     # the observation class follows its type: OccupancyGrid takes its own defaults (the keys a Kinematics base config
     # leaves behind, vehicles_count, order, normalize ..., are ignored by it as upstream's **kwargs are)
@@ -109,6 +120,7 @@ def build_cfg(cfg: Dict[str, Any], embed: Optional[EmbedSpec] = None, autoreset:
     c.high_speed_reward = float(full["high_speed_reward"])
     c.reward_speed_lo, c.reward_speed_hi = (float(v) for v in full["reward_speed_range"])
     c.autoreset = int(bool(autoreset))
+    c.ego_collisions_only = int(full["gym_id"] == "highway-fast-v0")
     if grid:
         if embed is not None and embed.kind != EMBED_NONE:
             raise ValueError("an OccupancyGrid observation takes no embedding")
@@ -185,7 +197,7 @@ def _grid_cfg(c: HrpCfg, obs: Dict[str, Any]) -> None:
 
 
 class HighwayVecEnv:
-    """``num_envs`` highway-v0 episodes stepped in lock-step on ``device``.
+    """``num_envs`` highway-v0 episodes (highway-fast-v0 with ``cfg["gym_id"]``) stepped in lock-step on ``device``.
 
     ``env_id_base`` is the global id of this shard's first env: spawn and shuffle draws are a
     function of (seed, global env id, episode), so a run sharded over G GPUs sees the same
@@ -197,6 +209,10 @@ class HighwayVecEnv:
     def __init__(self, cfg: Dict[str, Any], num_envs: int, device: Any = "cuda", embed: Optional[EmbedSpec] = None,
                  autoreset: bool = True, env_id_base: int = 0, seed: int = 0, real64: bool = False):
         # real64: the fp64 VALIDATION instantiation of the kernels (HRP_ENV_REAL64; parity tests only, slow)
+        # the configuration is checked first: an unknown gym_id or observation is a ValueError before any device work
+        self.config = resolve_config(cfg)
+        self.embed = embed or EmbedSpec()
+        self.cfg = build_cfg(cfg, self.embed, autoreset)
         lib = _lib.load()
         _lib.require_device()
         self.device = torch.device(device)
@@ -204,9 +220,6 @@ class HighwayVecEnv:
             raise _lib.HrpError("HighwayVecEnv needs a CUDA device: there is no CPU path")
         self.dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         self.device = torch.device("cuda", self.dev_index)
-        self.config = resolve_config(cfg)
-        self.embed = embed or EmbedSpec()
-        self.cfg = build_cfg(cfg, self.embed, autoreset)
         self.num_envs = int(num_envs)
         self.seed = int(seed)
         table = self.embed.table

@@ -2,7 +2,7 @@
 
     python -m highway_rope_ppo_b200.main --get-total-experiments
     python -m highway_rope_ppo_b200.main --run-single-experiment <name or unique prefix>
-    python -m highway_rope_ppo_b200.main --array-task-id 3 --slurm-num-tasks 68 [--n-jobs 16]
+    python -m highway_rope_ppo_b200.main --array-task-id 3 --slurm-num-tasks 68 [--n-jobs 16] [--gym-id highway-fast-v0]
     torchrun --nproc-per-node 8 -m highway_rope_ppo_b200.main --n-jobs 32        # the whole grid, 8 GPUs x 32 runs at a time
 
 The experiment grid, names, selection rules and the end-of-run summary are the reference's
@@ -33,6 +33,8 @@ def parse(argv: Optional[List[str]] = None) -> argparse.Namespace:
     p.add_argument("--get-total-experiments", action="store_true", help="Print total number of experiments and exit")
     p.add_argument("--artifacts-dir", type=str, default=None)
     p.add_argument("--max-episodes", type=int, default=None, help="override Experiment.max_episodes (smoke runs)")
+    p.add_argument("--gym-id", type=str, default=None, choices=("highway-v0", "highway-fast-v0"),
+                   help="env id of every experiment (the config key gym_id; default: the base config's, highway-v0)")
     return p.parse_args(argv)
 
 
@@ -64,7 +66,8 @@ def main(argv: Optional[List[str]] = None) -> int:
     log.info(f"rank {rank}/{world}: launching {len(mine)} of {len(selected)} experiments, {jobs} at a time")
     from .config.base_config import HIGHWAY_CONFIG
 
-    results = run_experiments(mine, HIGHWAY_CONFIG, artifacts_dir=args.artifacts_dir, multiplex=jobs)
+    base = HIGHWAY_CONFIG if args.gym_id is None else dict(HIGHWAY_CONFIG, gym_id=args.gym_id)
+    results = run_experiments(mine, base, artifacts_dir=args.artifacts_dir, multiplex=jobs)
     succ = sum(1 for r in results if r.get("status") == "COMPLETED")
     log.info(f"Summary: {succ} succeeded, {len(results) - succ} failed.")
     for cond, (score, name) in summarize(results).items():

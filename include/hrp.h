@@ -45,7 +45,7 @@ enum { HRP_OBS_KINEMATICS = 0, HRP_OBS_OCCUPANCY_GRID = 1 };
 /* observation embedding fused behind the Kinematics observation */
 enum { HRP_EMBED_NONE = 0, HRP_EMBED_ROPE = 1, HRP_EMBED_DIST = 2, HRP_EMBED_RANK = 3 };
 
-/* highway-v0 config (config/base_config.py:5-39 over HighwayEnv.default_config) */
+/* highway-v0 / highway-fast-v0 config (config/base_config.py:5-39 over HighwayEnv.default_config) */
 typedef struct hrp_cfg {
     int32_t lanes_count;
     int32_t vehicles_count;        /* other vehicles; V = vehicles_count + 1 */
@@ -93,6 +93,10 @@ typedef struct hrp_cfg {
     double  grid_lo[2];            /* grid_size[0][0], grid_size[1][0] */
     double  grid_hi[2];            /* grid_size[0][1], grid_size[1][1] */
     double  grid_step[2];
+    /* the env id's collision rule: 0 is highway-v0 (every pair of vehicles is tested), 1 is highway-fast-v0
+     * (HighwayEnvFast: the uncontrolled vehicles do not check collisions, so only the ego's pairs (0, k) are tested;
+     * DESIGN.md Appendix C).  Any other value is an error (-1). */
+    int32_t ego_collisions_only;
 } hrp_cfg;
 
 /* Host-side SoA view of the simulator state, [num_envs * V] per vehicle field
