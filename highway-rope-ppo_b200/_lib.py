@@ -126,7 +126,10 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_episode_stats": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "hrp_ppo_loss_grad": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp,
                                     _vp, _vp]),
+    "hrp_ppo_loss_grad_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp,
+                                       _f32, _vp, _vp, _vp]),
     "hrp_clip_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),
+    "hrp_clip_adam_step_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp]),
     "hrp_comm_create": (C.c_int, [_i32, _i32, _i64, _i32, C.POINTER(_vp), _vp]),
     "hrp_comm_connect": (C.c_int, [_vp, _vp]),
     "hrp_comm_grad": (_vp, [_vp]),
@@ -134,6 +137,7 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_comm_parity": (C.c_int, [_vp]),
     "hrp_comm_note_replay": (C.c_int, [_vp]),
     "hrp_clip_adam_step_p2p": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),
+    "hrp_clip_adam_step_p2p_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp]),
     "hrp_comm_status": (C.c_int, [_vp]),
     "hrp_comm_destroy": (C.c_int, [_vp]),
 }

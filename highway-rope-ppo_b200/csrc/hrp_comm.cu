@@ -80,11 +80,13 @@ __device__ __forceinline__ void wait_words(const unsigned *mine, int world, int 
     __syncthreads();
 }
 
+// LR_DEV: the learning rate is *lr_dev, as in hrp_ppo.cu's clip_adam_kernel
+template <bool LR_DEV>
 __global__ void __launch_bounds__(P2P_THREADS)
 clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long long npad, unsigned *__restrict__ epoch_dev,
                      float *__restrict__ p, float *__restrict__ m, float *__restrict__ v, int32_t *__restrict__ step,
                      long long n, double lr, double beta1, double beta2, double eps, float max_norm,
-                     float *__restrict__ part, unsigned *__restrict__ arrive)
+                     float *__restrict__ part, unsigned *__restrict__ arrive, const double *__restrict__ lr_dev)
 {
     namespace cg = cooperative_groups;
     cg::grid_group grid = cg::this_grid();
@@ -161,7 +163,7 @@ clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long lo
             float c = max_norm / (total_norm + 1e-6f);
             s_coef = max_norm > 0.f ? fminf(c, 1.f) : 1.f;
             double bc1 = 1.0 - pow(beta1, (double)k), bc2 = 1.0 - pow(beta2, (double)k);
-            s_step_size = (float)(lr / bc1);
+            s_step_size = (float)((LR_DEV ? *lr_dev : lr) / bc1);
             s_bc2_sqrt = (float)sqrt(bc2);
         }
     }
@@ -240,20 +242,20 @@ float *hrp_comm_grad(hrp_comm *c) { return c ? c->local + (size_t)(c->issued & 1
 float *hrp_comm_grad_parity(hrp_comm *c, int32_t parity) { return c ? c->local + (size_t)(parity & 1) * c->npad : nullptr; }
 int hrp_comm_parity(hrp_comm *c) { return c ? (int)(c->issued & 1) : -1; }
 
-int hrp_clip_adam_step_p2p(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
-                           double beta1, double beta2, double eps, float max_grad_norm, float *scratch, void *stream)
+}  // extern "C"
+
+template <bool LR_DEV>
+static int clip_adam_p2p_launch(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
+                                const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                                float *scratch, void *stream)
 {
-    if (!c || !c->connected || !params || !exp_avg || !exp_avg_sq || !step || !scratch) {
-        hrp_set_error("hrp_clip_adam_step_p2p: bad arguments (hrp_comm_connect first)");
-        return -1;
-    }
     static int max_ctas_dev[HRP_MAX_DEVICES] = {0};
     if (c->device < 0 || c->device >= HRP_MAX_DEVICES) { hrp_set_error("device index %d not supported", c->device); return -1; }
     int &max_ctas = max_ctas_dev[c->device];
     if (max_ctas == 0) {
         int sms = 0, per_sm = 0;
         HRP_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
-        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_p2p_kernel, P2P_THREADS, 0));
+        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_p2p_kernel<LR_DEV>, P2P_THREADS, 0));
         max_ctas = sms * per_sm < P2P_MAX_CTAS ? sms * per_sm : P2P_MAX_CTAS;
         if (max_ctas < 1) { hrp_set_error("hrp_clip_adam_step_p2p: kernel does not fit the device"); return -2; }
     }
@@ -265,11 +267,39 @@ int hrp_clip_adam_step_p2p(hrp_comm *c, float *params, float *exp_avg, float *ex
     int world = c->world, rank = c->rank, parity = (int)(c->issued & 1);
     unsigned *epoch = c->epoch, *arrive = c->epoch + 2;
     void *args[] = {&T, &world, &rank, &parity, &npad, &epoch, &params, &exp_avg, &exp_avg_sq, &step, &n, &lr, &beta1, &beta2,
-                    &eps, &max_grad_norm, &scratch, &arrive};
-    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_p2p_kernel, dim3(ctas), dim3(P2P_THREADS), args, 0,
+                    &eps, &max_grad_norm, &scratch, &arrive, &lr_dev};
+    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_p2p_kernel<LR_DEV>, dim3(ctas), dim3(P2P_THREADS), args, 0,
                                             (cudaStream_t)stream));
     c->issued += 1;
     return 0;
+}
+
+extern "C" {
+
+int hrp_clip_adam_step_p2p(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
+                           double beta1, double beta2, double eps, float max_grad_norm, float *scratch, void *stream)
+{
+    if (!c || !c->connected || !params || !exp_avg || !exp_avg_sq || !step || !scratch) {
+        hrp_set_error("hrp_clip_adam_step_p2p: bad arguments (hrp_comm_connect first)");
+        return -1;
+    }
+    return clip_adam_p2p_launch<false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps, max_grad_norm,
+                                       scratch, stream);
+}
+
+int hrp_clip_adam_step_p2p_ex(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
+                              const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                              float *scratch, void *stream)
+{
+    const char *bad = !c ? "comm" : !c->connected ? "comm (hrp_comm_connect first)" : !params ? "params_dev"
+                    : !exp_avg ? "exp_avg_dev" : !exp_avg_sq ? "exp_avg_sq_dev" : !step ? "step_dev"
+                    : !scratch ? "scratch_dev" : nullptr;
+    if (bad) { hrp_set_error("hrp_clip_adam_step_p2p_ex: bad argument %s", bad); return -1; }
+    if (!lr_dev)
+        return clip_adam_p2p_launch<false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps,
+                                           max_grad_norm, scratch, stream);
+    return clip_adam_p2p_launch<true>(c, params, exp_avg, exp_avg_sq, step, lr, lr_dev, beta1, beta2, eps, max_grad_norm,
+                                      scratch, stream);
 }
 
 /* a captured graph replays the parity it was captured with: the host says which step it is about to replay */

@@ -15,6 +15,8 @@
 // log_std, A = n logits in actor_mean.2.
 #include <cooperative_groups.h>
 #include <math.h>
+
+#include <cmath>
 #include <stdlib.h>
 
 #include "hrp_internal.cuh"
@@ -257,15 +259,19 @@ heads_wgrad_partial_kernel(const float *__restrict__ dmean, const float *__restr
         }
     }
 }
-// gather the minibatch out of the rollout in one launch: states, pre_tanh, old log-prob, advantage, return
+// gather the minibatch out of the rollout in one launch: states, pre_tanh, old log-prob, advantage, return, and with
+// VOLD the rollout's value (the clipped value loss).  The VOLD arguments come last, so the default instantiation keeps
+// the parameter block it had before them.
+template <bool VOLD>
 __global__ void gather_batch_kernel(const float *__restrict__ states, const float *__restrict__ pre_tanh,
                                     const float *__restrict__ olp, const float *__restrict__ adv,
                                     const float *__restrict__ ret, const long long *__restrict__ idx, long long B, int S,
                                     int A, float *__restrict__ x, float *__restrict__ z,
-                                    float *__restrict__ o_olp, float *__restrict__ o_adv, float *__restrict__ o_ret)
+                                    float *__restrict__ o_olp, float *__restrict__ o_adv, float *__restrict__ o_ret,
+                                    const float *__restrict__ vold, float *__restrict__ o_vold)
 {
     hrp_pdl_release();   // the first GEMM of the step sets itself up meanwhile (it waits before it reads x)
-    const int W = S + A + 3;
+    const int W = S + A + (VOLD ? 4 : 3);
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= B * W) return;
     long long b = i / W;
@@ -275,7 +281,22 @@ __global__ void gather_batch_kernel(const float *__restrict__ states, const floa
     else if (c < S + A) z[b * A + (c - S)] = pre_tanh[(size_t)src * A + (c - S)];
     else if (c == S + A) o_olp[b] = olp[src];
     else if (c == S + A + 1) o_adv[b] = adv[src];
-    else o_ret[b] = ret[src];
+    else if (!VOLD || c == S + A + 2) o_ret[b] = ret[src];
+    else o_vold[b] = vold[src];
+}
+
+// The clipped value loss (VCLIP of the loss kernels): with v the new value, vo the rollout's, R the return and c the
+// clip, the per-sample term is max((v - R)^2, (vo + clamp(v - vo, -c, c) - R)^2).  Returns the term and writes
+// d(term)/d(v) / 2 to *half_grad with torch autograd's rules: maximum splits the gradient half and half on a tie, clamp
+// passes it where -c <= v - vo <= c.
+__device__ __forceinline__ float clipped_value_term(float v, float vo, float R, float c, float *half_grad)
+{
+    const float d1 = v - R, dvo = v - vo;
+    const float d2 = (vo + fminf(fmaxf(dvo, -c), c)) - R;
+    const float l1 = d1 * d1, l2 = d2 * d2;
+    const float g2 = dvo >= -c && dvo <= c ? d2 : 0.f;
+    *half_grad = l1 > l2 ? d1 : (l2 > l1 ? g2 : 0.5f * d1 + 0.5f * g2);
+    return fmaxf(l1, l2);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -445,6 +466,7 @@ heads_act_kernel(const float *__restrict__ a1, const float *__restrict__ c1, con
 // Every CTA leaves 8 partial sums in part[blockIdx.x][8]; the CTA that finishes last adds them in block order
 // (deterministic) and writes d(log_std) and the metrics.  `counter` returns to zero.
 constexpr int HLB_ROWS = 16;
+template <bool VCLIP>
 __global__ void __launch_bounds__(256)
 heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict__ c1, int ld, int H,
                            const float *__restrict__ wa2, const float *__restrict__ ba2,
@@ -455,7 +477,7 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
                            float entropy_coef, float scale, float *__restrict__ dmean, float *__restrict__ dvalue,
                            float *__restrict__ da1, float *__restrict__ dc1, float *__restrict__ dlog_std,
                            float *__restrict__ metrics, float *__restrict__ part,
-                           unsigned *__restrict__ counter)
+                           unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip)
 {
     __shared__ float out_s[HLB_ROWS][5], dmean_s[HLB_ROWS][4], dvalue_s[HLB_ROWS];
     __shared__ float red[8][8];
@@ -525,12 +547,13 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
             dmean_s[r][a] = dm;
             vals[4 + a] = dlp * dls[a];
         }
-        float dv = out_s[r][A] - ret[b];
+        float dv = out_s[r][A] - ret[b], vterm = dv * dv;
+        if (VCLIP) vterm = clipped_value_term(out_s[r][A], old_value[b], ret[b], value_clip, &dv);
         float dvv = value_coef * 2.f * dv * scale;
         dvalue[b] = dvv;
         dvalue_s[r] = dvv;
         vals[0] = -fminf(surr1, surr2);
-        vals[1] = dv * dv;
+        vals[1] = vterm;
         vals[2] = fabsf(ratio - 1.f) > eps_clip ? 1.f : 0.f;
         vals[3] = (ratio - 1.f) - lr;
     }
@@ -816,6 +839,7 @@ heads_finish_cat_kernel(const float *__restrict__ part, int tiles_a, int tiles, 
 //   d(logit_j) = scale [-g ratio (delta_{id,j} - p_j) + c_ent p_j (log p_j + H)]   (g = d min(surr1, surr2) / d ratio)
 // and d(value).  Phase 2: d(a1) | d(c1) under the ReLU masks.  Partial sums per CTA: policy loss, value error, clip
 // count, approx-KL, entropy; the last CTA adds them in block order and writes the metrics.  No log_std gradient.
+template <bool VCLIP>
 __global__ void __launch_bounds__(256)
 heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__restrict__ c1, int ld, int H,
                                const float *__restrict__ wa2, const float *__restrict__ ba2,
@@ -825,7 +849,7 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
                                float eps_clip, float value_coef, float entropy_coef, float scale,
                                float *__restrict__ dlogit, float *__restrict__ dvalue, float *__restrict__ da1,
                                float *__restrict__ dc1, float *__restrict__ metrics, float *__restrict__ part,
-                               unsigned *__restrict__ counter)
+                               unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip)
 {
     __shared__ float out_s[HLB_ROWS][CAT_MAX + 1], dl_s[HLB_ROWS][CAT_MAX], dvalue_s[HLB_ROWS];
     __shared__ float red[8][8];
@@ -902,12 +926,13 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
             dl_s[r][j] = j < n ? dl : 0.f;
             if (j < n) dlogit[b * n + j] = dl;
         }
-        float dv = out_s[r][CAT_MAX] - ret[b];
+        float dv = out_s[r][CAT_MAX] - ret[b], vterm = dv * dv;
+        if (VCLIP) vterm = clipped_value_term(out_s[r][CAT_MAX], old_value[b], ret[b], value_clip, &dv);
         float dvv = value_coef * 2.f * dv * scale;
         dvalue[b] = dvv;
         dvalue_s[r] = dvv;
         vals[0] = -fminf(surr1, surr2);
-        vals[1] = dv * dv;
+        vals[1] = vterm;
         vals[2] = fabsf(ratio - 1.f) > eps_clip ? 1.f : 0.f;
         vals[3] = (ratio - 1.f) - lr;
         vals[4] = ent;
@@ -1087,12 +1112,15 @@ __global__ void adv_normalize_kernel(float *__restrict__ adv, long long n, const
 // clip_grad_norm_ + Adam.step (agent.py:249-252) in ONE cooperative launch: every CTA leaves the sum of squares of
 // its slice of the gradient in part[blockIdx.x], the grid synchronises, every CTA adds the partials in the same
 // fixed order (so the clip coefficient is identical everywhere and from run to run), then updates its slice and
-// CTA 0 advances the step counter.  ADAM_MAX_CTAS partials fit the caller's 128-float scratch buffer.
+// CTA 0 advances the step counter.  ADAM_MAX_CTAS partials fit the caller's 128-float scratch buffer.  LR_DEV: the
+// learning rate is *lr_dev, read when the step size is formed (a captured launch follows a schedule the host writes
+// there); the argument comes last, so the default instantiation keeps its parameter block.
 constexpr int ADAM_MAX_CTAS = 120, ADAM_THREADS = 512;
+template <bool LR_DEV>
 __global__ void __launch_bounds__(ADAM_THREADS)
 clip_adam_kernel(float *__restrict__ p, const float *__restrict__ g, float *__restrict__ m,
                  float *__restrict__ v, int32_t *__restrict__ step, long long n, double lr, double beta1,
-                 double beta2, double eps, float max_norm, float *__restrict__ part)
+                 double beta2, double eps, float max_norm, float *__restrict__ part, const double *__restrict__ lr_dev)
 {
     __shared__ float red[ADAM_THREADS / 32];
     __shared__ float s_coef, s_step_size, s_bc2_sqrt;
@@ -1123,7 +1151,7 @@ clip_adam_kernel(float *__restrict__ p, const float *__restrict__ g, float *__re
             float c = max_norm / (total_norm + 1e-6f);
             s_coef = max_norm > 0.f ? fminf(c, 1.f) : 1.f;
             double bc1 = 1.0 - pow(beta1, (double)k), bc2 = 1.0 - pow(beta2, (double)k);
-            s_step_size = (float)(lr / bc1);
+            s_step_size = (float)((LR_DEV ? *lr_dev : lr) / bc1);
             s_bc2_sqrt = (float)sqrt(bc2);
             if (blockIdx.x == 0) step[0] = k;
         }
@@ -1151,6 +1179,7 @@ struct hrp_ppo {
     int device;
     float *ws;  // one arena
     float *x, *z, *olp, *adv, *ret;          // gathered minibatch
+    float *vold;                             // gathered rollout values (clipped value loss)
     float *h1, *h2;                          // trunk activations [B,H]
     float *ac;                               // actor | critic hidden activations, one [B, 2H] matrix
     float *mean, *value, *dmean, *dvalue;    // heads and their gradients (mean / dmean: logits when categorical)
@@ -1555,7 +1584,7 @@ static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
     auto pad = [](size_t n) { return (n + 31) / 32 * 32; };
     const size_t sizes[] = {B * S, B * A, B, B, B, B * H, B * H, 2 * B * H, B * A, B * A, B, B, 2 * B * H, B * H, B * H,
                             2 * H * H, H * H, cap * 2 * H * H, cap * H * H, cap * H * S, 64 * 2 * H, 64 * H, 64 * H,
-                            64 * ((A + 1) * H + A + 1), ((B + HLB_ROWS - 1) / HLB_ROWS) * 8, 32};
+                            64 * ((A + 1) * H + A + 1), ((B + HLB_ROWS - 1) / HLB_ROWS) * 8, 32, B};
     size_t n = 0;
     for (size_t q : sizes) n += pad(q);
     cudaError_t ce = cudaMalloc(&h->ws, n * sizeof(float));
@@ -1572,6 +1601,7 @@ static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
     for (int q = 0; q < 3; ++q) h->part_b[q] = take();
     h->part_h = take(); h->loss_part = take();
     h->loss_counter = (unsigned *)take();
+    h->vold = take();
     ce = cudaMemset(h->loss_counter, 0, 32 * sizeof(float));
     for (int q = 0; q < 2 && ce == cudaSuccess; ++q) ce = cudaStreamCreateWithFlags(&h->side[q], cudaStreamNonBlocking);
     for (int q = 0; q < 8 && ce == cudaSuccess; ++q) ce = cudaEventCreateWithFlags(&h->ev[q], cudaEventDisableTiming);
@@ -1701,10 +1731,13 @@ int hrp_adv_normalize(float *adv, int64_t n, const double *stats, void *stream)
     return 0;
 }
 
-int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
-                      const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx, int64_t batch,
-                      float eps_clip, float value_coef, float entropy_coef, float loss_scale, float *grad,
-                      float *metrics, void *stream)
+}  // extern "C"
+
+// hrp_ppo_loss_grad, and with old_value non-NULL the clipped value loss of hrp_ppo_loss_grad_ex (the VCLIP kernels)
+static int loss_grad_impl(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
+                          const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx,
+                          int64_t batch, float eps_clip, float value_coef, float entropy_coef, float loss_scale,
+                          const float *old_value, float value_clip, float *grad, float *metrics, void *stream)
 {
     if (!h || !params || !states || !pre_tanh || !old_log_prob || !adv || !ret || !grad) {
         hrp_set_error("hrp_ppo_loss_grad: null argument");
@@ -1715,7 +1748,8 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
     const Layout &L = h->L;
     const int H = L.H, S = L.S, A = L.A, Bi = (int)batch, H2 = 2 * H;
     const long long B = batch;
-    const float *x = states, *z = pre_tanh, *olp = old_log_prob, *ad = adv, *rt = ret;
+    const float *x = states, *z = pre_tanh, *olp = old_log_prob, *ad = adv, *rt = ret, *vo = old_value;
+    const bool vclip = old_value != nullptr;
     // `from` has produced something `to` consumes (also valid while the caller's stream is being captured: the side
     // streams join the capture and are joined back before this function returns)
     auto after = [&](int e, cudaStream_t from, cudaStream_t to) -> cudaError_t {
@@ -1734,23 +1768,27 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
     }
     if (idx) {
         const long long *ix = (const long long *)idx;
-        long long tot = B * (S + Az + 3);
-        gather_batch_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix, B,
-                                                                         S, Az, h->x, h->z, h->olp, h->adv, h->ret);
+        long long tot = B * (S + Az + (vclip ? 4 : 3));
+        auto gather = vclip ? gather_batch_kernel<true> : gather_batch_kernel<false>;
+        gather<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(states, pre_tanh, old_log_prob, adv, ret, ix, B, S, Az, h->x,
+                                                              h->z, h->olp, h->adv, h->ret, old_value, h->vold);
         HRP_CUDA_OK(cudaGetLastError());
         x = h->x; z = h->z; olp = h->olp; ad = h->adv; rt = h->ret;
+        if (vclip) vo = h->vold;
     }
     if (int rc = forward_impl(h, params, x, B, nullptr, nullptr, s)) return rc;   // trunk + hidden head layers
-    if (h->cat) HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_cat_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256),
+    if (h->cat) HRP_CUDA_OK(hrp_launch_pdl(vclip ? heads_loss_backward_cat_kernel<true> : heads_loss_backward_cat_kernel<false>,
+                                           dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256),
                                            0, s, (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2,
                                            params + L.ba2, params + L.wc2, params + L.bc2, z, olp, ad, rt, B, A, eps_clip,
                                            value_coef, entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H,
-                                           metrics, h->loss_part, h->loss_counter));
-    else HRP_CUDA_OK(hrp_launch_pdl(heads_loss_backward_kernel, dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
+                                           metrics, h->loss_part, h->loss_counter, vo, value_clip));
+    else HRP_CUDA_OK(hrp_launch_pdl(vclip ? heads_loss_backward_kernel<true> : heads_loss_backward_kernel<false>,
+                               dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
                                (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
                                params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip, value_coef,
                                entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, grad + L.log_std, metrics,
-                               h->loss_part, h->loss_counter));
+                               h->loss_part, h->loss_counter, vo, value_clip));
     const float *a1 = h->ac, *c1 = h->ac + H;
     ReducePlan plan;
     plan.nseg = 0; plan.blocks = 0;
@@ -1792,14 +1830,11 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, cons
     return 0;
 }
 
-int hrp_clip_adam_step(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
-                       double lr, double beta1, double beta2, double eps, float max_grad_norm, float *scratch,
-                       void *stream)
+template <bool LR_DEV>
+static int clip_adam_launch(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
+                            double lr, const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                            float *scratch, void *stream)
 {
-    if (!params || !grad || !exp_avg || !exp_avg_sq || !step || !scratch || n < 1) {
-        hrp_set_error("hrp_clip_adam_step: bad arguments");
-        return -1;
-    }
     cudaStream_t s = (cudaStream_t)stream;
     // per device: a process may drive several GPUs (ExperimentRunner with a device pool)
     static int max_ctas_dev[HRP_MAX_DEVICES] = {0};
@@ -1810,16 +1845,68 @@ int hrp_clip_adam_step(float *params, const float *grad, float *exp_avg, float *
     if (max_ctas == 0) {
         int sms = 0, per_sm = 0;
         HRP_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_kernel, ADAM_THREADS, 0));
+        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_kernel<LR_DEV>, ADAM_THREADS, 0));
         max_ctas = sms * per_sm < ADAM_MAX_CTAS ? sms * per_sm : ADAM_MAX_CTAS;
         if (max_ctas < 1) { hrp_set_error("hrp_clip_adam_step: kernel does not fit the device"); return -2; }
     }
     int ctas = (int)((n + ADAM_THREADS - 1) / ADAM_THREADS);
     if (ctas > max_ctas) ctas = max_ctas;
     long long n_ = n;
-    void *args[] = {&params, &grad, &exp_avg, &exp_avg_sq, &step, &n_, &lr, &beta1, &beta2, &eps, &max_grad_norm, &scratch};
-    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_kernel, dim3(ctas), dim3(ADAM_THREADS), args, 0, s));
+    void *args[] = {&params, &grad, &exp_avg, &exp_avg_sq, &step, &n_, &lr, &beta1, &beta2, &eps, &max_grad_norm, &scratch,
+                    &lr_dev};
+    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_kernel<LR_DEV>, dim3(ctas), dim3(ADAM_THREADS), args, 0, s));
     return 0;
+}
+
+extern "C" {
+
+int hrp_ppo_loss_grad(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
+                      const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx, int64_t batch,
+                      float eps_clip, float value_coef, float entropy_coef, float loss_scale, float *grad,
+                      float *metrics, void *stream)
+{
+    return loss_grad_impl(h, params, states, pre_tanh, old_log_prob, adv, ret, idx, batch, eps_clip, value_coef,
+                          entropy_coef, loss_scale, nullptr, 0.f, grad, metrics, stream);
+}
+
+int hrp_ppo_loss_grad_ex(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
+                         const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx,
+                         int64_t batch, float eps_clip, float value_coef, float entropy_coef, float loss_scale,
+                         const float *old_value, float value_clip, float *grad, float *metrics, void *stream)
+{
+    // checked first: the other arguments are then validated exactly as hrp_ppo_loss_grad validates them
+    if (old_value && !(std::isfinite(value_clip) && value_clip > 0.f)) {
+        hrp_set_error("hrp_ppo_loss_grad_ex: value_clip must be finite and > 0 with old_value_dev, got %g", (double)value_clip);
+        return -1;
+    }
+    return loss_grad_impl(h, params, states, pre_tanh, old_log_prob, adv, ret, idx, batch, eps_clip, value_coef,
+                          entropy_coef, loss_scale, old_value, value_clip, grad, metrics, stream);
+}
+
+int hrp_clip_adam_step(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
+                       double lr, double beta1, double beta2, double eps, float max_grad_norm, float *scratch,
+                       void *stream)
+{
+    if (!params || !grad || !exp_avg || !exp_avg_sq || !step || !scratch || n < 1) {
+        hrp_set_error("hrp_clip_adam_step: bad arguments");
+        return -1;
+    }
+    return clip_adam_launch<false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
+                                   max_grad_norm, scratch, stream);
+}
+
+int hrp_clip_adam_step_ex(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
+                          double lr, const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                          float *scratch, void *stream)
+{
+    const char *bad = !params ? "params_dev" : !grad ? "grad_dev" : !exp_avg ? "exp_avg_dev" : !exp_avg_sq ? "exp_avg_sq_dev"
+                    : !step ? "step_dev" : !scratch ? "scratch_dev" : n < 1 ? "n" : nullptr;
+    if (bad) { hrp_set_error("hrp_clip_adam_step_ex: bad argument %s", bad); return -1; }
+    if (!lr_dev)
+        return clip_adam_launch<false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
+                                       max_grad_norm, scratch, stream);
+    return clip_adam_launch<true>(params, grad, exp_avg, exp_avg_sq, step, n, lr, lr_dev, beta1, beta2, eps,
+                                  max_grad_norm, scratch, stream);
 }
 
 }  // extern "C"

@@ -21,6 +21,7 @@ format as the reference; the arithmetic runs in ``libhrp_b200.so``:
 """
 from __future__ import annotations
 
+import math
 import os
 
 import ctypes as C
@@ -533,10 +534,14 @@ def gae(reward: torch.Tensor, value: torch.Tensor, done: Optional[torch.Tensor],
 
 
 class _AdamState:
-    """``optim.Adam(params, lr)`` as flat moment buffers + a device step counter."""
+    """``optim.Adam(params, lr)`` as flat moment buffers + a device step counter.
+
+    ``lr_dev``: None (the learning rate is a launch argument, baked into captured graphs), or a float64 [1] device
+    tensor that the Adam kernels read when they run (``PPOAgent.set_lr``); assigning ``lr`` then also writes it."""
 
     def __init__(self, ac: ActorCritic, lr: float):
         self.ac = ac
+        self.lr_dev: Optional[torch.Tensor] = None
         self.lr, self.betas, self.eps = float(lr), (0.9, 0.999), 1e-8
         d = ac.device
         self.exp_avg = torch.zeros(ac.num_params, dtype=torch.float32, device=d)
@@ -547,6 +552,16 @@ class _AdamState:
                               "amsgrad": False, "maximize": False, "foreach": None, "capturable": False,
                               "differentiable": False, "fused": None, "decoupled_weight_decay": False,
                               "params": list(range(len(ac.shapes)))}]
+
+    @property
+    def lr(self) -> float:
+        return self._lr
+
+    @lr.setter
+    def lr(self, value: float) -> None:
+        self._lr = float(value)
+        if self.lr_dev is not None:
+            self.lr_dev.fill_(self._lr)   # stream-ordered before the next update's launches or graph replays
 
     def state_dict(self) -> Dict[str, Any]:
         """Same structure as ``torch.optim.Adam.state_dict()`` over ``ActorCritic.parameters()``."""
@@ -587,7 +602,14 @@ class PPOAgent:
     def __init__(self, state_dim: int, action_dim: int, lr: float = 1e-4, gamma: float = 0.99, lam: float = 0.95,
                  eps_clip: float = 0.2, value_coef: float = 0.5, entropy_coef: float = 0.005,
                  max_grad_norm: float = 0.5, epochs: int = 6, batch_size: int = 64, hidden_dim: int = 128,
-                 logger: Optional[logging.Logger] = None, device: Any = "cuda", *, discrete: bool = False):
+                 logger: Optional[logging.Logger] = None, device: Any = "cuda", *, discrete: bool = False,
+                 clip_value: Optional[float] = None):
+        """``clip_value`` = c (keyword-only, off by default): the clipped value loss, max((v - R)^2, (v_old +
+        clamp(v - v_old, -c, c) - R)^2) per sample with v_old the value the rollout stored (``hrp_ppo_loss_grad_ex``),
+        weighted like the reference's value MSE; the ``value_loss`` and ``loss`` metrics report it."""
+        if clip_value is not None and not (math.isfinite(float(clip_value)) and float(clip_value) > 0):
+            raise ValueError(f"clip_value must be a finite number > 0 or None, got {clip_value!r}")
+        self.clip_value = None if clip_value is None else float(clip_value)
         self._lib = _lib.load()
         self.device = _cuda_device(device)
         self.discrete = bool(discrete)
@@ -615,6 +637,16 @@ class PPOAgent:
         self.use_p2p = os.environ.get("HRP_P2P", "1") != "0" and distributed.backend() == "nccl"
         self._comm = None
         self._comm_keep = None
+
+    def set_lr(self, lr: float) -> None:
+        """Set the learning rate of the following optimizer steps.  The first call moves it into device memory
+        (``optimizer.lr_dev``, read by ``hrp_clip_adam_step_ex`` / ``hrp_clip_adam_step_p2p_ex`` when they run), so that
+        a schedule calling this every update keeps replaying the captured minibatch graphs instead of capturing new
+        ones.  Every call writes the value on the current stream, outside any graph."""
+        opt = self.optimizer
+        if opt.lr_dev is None:
+            opt.lr_dev = torch.empty(1, dtype=torch.float64, device=self.device)
+        opt.lr = lr
 
     # -- acting ----------------------------------------------------------------------------------
     def select_action(self, state, deterministic: bool = False):
@@ -698,25 +730,39 @@ class PPOAgent:
         ac, opt, s = self.actor_critic, self.optimizer, self.actor_critic._stream()
         if world > 1 and self._comm is not None:
             self.grad = self._grad_parity[self._lib.hrp_comm_parity(self._comm)]   # the buffer of this step's parity
-        _lib.check(self._lib.hrp_ppo_loss_grad(
-            ac._h, ac.flat.data_ptr(), flat["states"].data_ptr(), flat["pre_tanh"].data_ptr(),
-            flat["log_prob"].data_ptr(), flat["adv"].data_ptr(), flat["ret"].data_ptr(), _lib.ptr(idx), B,
-            float(self.eps_clip), float(self.value_coef), float(self.entropy_coef), distributed.loss_scale(B, world),
-            self.grad.data_ptr(), self._metrics.data_ptr(), s), "hrp_ppo_loss_grad")
+        loss_args = (ac._h, ac.flat.data_ptr(), flat["states"].data_ptr(), flat["pre_tanh"].data_ptr(),
+                     flat["log_prob"].data_ptr(), flat["adv"].data_ptr(), flat["ret"].data_ptr(), _lib.ptr(idx), B,
+                     float(self.eps_clip), float(self.value_coef), float(self.entropy_coef),
+                     distributed.loss_scale(B, world))
+        if self.clip_value is None:
+            _lib.check(self._lib.hrp_ppo_loss_grad(*loss_args, self.grad.data_ptr(), self._metrics.data_ptr(), s),
+                       "hrp_ppo_loss_grad")
+        else:
+            _lib.check(self._lib.hrp_ppo_loss_grad_ex(*loss_args, flat["value"].data_ptr(), self.clip_value,
+                                                      self.grad.data_ptr(), self._metrics.data_ptr(), s),
+                       "hrp_ppo_loss_grad_ex")
+        lr_dev = opt.lr_dev
         if world > 1 and self._comm is not None:
             # all_reduce + clip + Adam as one kernel over peer memory
-            _lib.check(self._lib.hrp_clip_adam_step_p2p(
-                self._comm, ac.flat.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
-                opt.step_dev.data_ptr(), opt.lr, opt.betas[0], opt.betas[1], opt.eps, float(self.max_grad_norm),
-                opt.scratch.data_ptr(), s), "hrp_clip_adam_step_p2p")
+            args = (self._comm, ac.flat.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
+                    opt.step_dev.data_ptr(), opt.lr)
+            tail = (opt.betas[0], opt.betas[1], opt.eps, float(self.max_grad_norm), opt.scratch.data_ptr(), s)
+            if lr_dev is None:
+                _lib.check(self._lib.hrp_clip_adam_step_p2p(*args, *tail), "hrp_clip_adam_step_p2p")
+            else:
+                _lib.check(self._lib.hrp_clip_adam_step_p2p_ex(*args, lr_dev.data_ptr(), *tail),
+                           "hrp_clip_adam_step_p2p_ex")
             self.launches += 2
             return
         if world > 1:
             self._allreduce(self.grad)
-        _lib.check(self._lib.hrp_clip_adam_step(
-            ac.flat.data_ptr(), self.grad.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
-            opt.step_dev.data_ptr(), ac.num_params, opt.lr, opt.betas[0], opt.betas[1], opt.eps,
-            float(self.max_grad_norm), opt.scratch.data_ptr(), s), "hrp_clip_adam_step")
+        args = (ac.flat.data_ptr(), self.grad.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
+                opt.step_dev.data_ptr(), ac.num_params, opt.lr)
+        tail = (opt.betas[0], opt.betas[1], opt.eps, float(self.max_grad_norm), opt.scratch.data_ptr(), s)
+        if lr_dev is None:
+            _lib.check(self._lib.hrp_clip_adam_step(*args, *tail), "hrp_clip_adam_step")
+        else:
+            _lib.check(self._lib.hrp_clip_adam_step_ex(*args, lr_dev.data_ptr(), *tail), "hrp_clip_adam_step_ex")
         self.launches += 2
 
     def release_graphs(self) -> None:
@@ -760,9 +806,12 @@ class PPOAgent:
         persistent buffers so that the captured pointers stay valid.  The first epoch of a new configuration runs
         eagerly (it also warms every kernel variant before anything is captured)."""
         ac = self.actor_critic
-        # the workspace generation, not its address: a re-created workspace may reuse the freed one's address
+        # the workspace generation, not its address: a re-created workspace may reuse the freed one's address.  A
+        # learning rate in device memory (set_lr) is read by the captured steps, so its value is not part of the key.
+        opt = self.optimizer
         key = (n, bs, world, ac.workspace_generation, float(self.eps_clip), float(self.value_coef), float(self.entropy_coef),
-               float(self.max_grad_norm), self.optimizer.lr, self.optimizer.betas, self.optimizer.eps)
+               float(self.max_grad_norm), opt.lr if opt.lr_dev is None else "lr_dev", opt.betas, opt.eps,
+               self.clip_value)
         st = self._graph_state
         if st is None or st["key"] != key:
             d = self.device
@@ -836,6 +885,8 @@ class PPOAgent:
         flat = {"states": r["states"].reshape(-1, S)[:n].contiguous(),
                 "pre_tanh": r["pre_tanh"].reshape(n, ac.act_widths()[1]),
                 "log_prob": r["log_prob"].reshape(n), "adv": adv_n.view(n), "ret": ret.view(n)}
+        if self.clip_value is not None:   # the rollout's values, the v_old of the clipped value loss
+            flat["value"] = r["value"].reshape(n)
         # one permutation per update, reused by every epoch (agent.py:140-147,205)
         perm = np.arange(n, dtype=np.int64)
         np.random.shuffle(perm)

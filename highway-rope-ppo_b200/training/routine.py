@@ -429,9 +429,15 @@ def eval_env_for(vec_env, num_envs: int):
                          env_id_base=shard * int(num_envs), real64=vec_env.real64)
 
 
+def linear_lr(lr0: float, it: int, iterations: int) -> float:
+    """CleanRL's linear annealing (``anneal_lr``): the learning rate of iteration ``it`` (0-based) of ``iterations``,
+    lr0 * (1 - it / iterations), from lr0 at the first iteration down to lr0 / iterations at the last."""
+    return float(lr0) * (1.0 - it / iterations)
+
+
 def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, logger=None,
                      bootstrap_truncated: bool = False, eval_episodes: int = 0, eval_interval: int = 10,
-                     best_checkpoint: Optional[str] = None):
+                     best_checkpoint: Optional[str] = None, anneal_lr: bool = False):
     """``iterations`` PPO iterations on E lock-step envs; returns the list of update metrics with samples/s and the
     training episodes added.  ``bootstrap_truncated``: see ``collect_rollout``.
 
@@ -446,7 +452,11 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
     ``seed + 1000 + global env id``, the reference's evaluation seeds with ``seed`` as the experiment seed), recorded
     as ``eval_return_mean`` / ``eval_return_std`` / ``eval_length_mean`` / ``eval_terminated_fraction`` in that
     iteration's metrics.  ``best_checkpoint``: path that ``agent.save`` (rank 0) writes whenever the evaluation mean
-    beats the best so far."""
+    beats the best so far.
+
+    ``anneal_lr``: iteration ``it`` runs with ``linear_lr(lr0, it, iterations)``, lr0 being the agent's learning rate at
+    entry, set through ``agent.set_lr`` (the learning rate lives in device memory, so the captured minibatch graphs are
+    replayed, not captured again).  Every iteration's metrics hold the ``lr`` its update ran with."""
     logger = logger or logging.getLogger(__name__)
     _act_widths(vec_env, agent)
     if eval_episodes and eval_interval < 1:
@@ -459,8 +469,11 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
     eval_env = eval_env_for(vec_env, eval_episodes) if eval_episodes else None
     best = -float("inf")
     history = []
+    lr0 = agent.optimizer.lr
     try:
         for it in range(iterations):
+            if anneal_lr:
+                agent.set_lr(linear_lr(lr0, it, iterations))
             ev = None
             if eval_env is not None and it % eval_interval == 0:
                 ev = evaluate_vectorized(eval_env, agent, exp_seed=seed)
@@ -480,6 +493,7 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
             torch.cuda.synchronize(dev)
             dt = time.time() - t0
             metrics["samples_per_s"] = T * E / dt
+            metrics["lr"] = agent.optimizer.lr
             s = summarize(stats[:6].tolist())
             metrics.update(episodes=s["episodes"], episode_return_mean=s["return_mean"],
                            episode_return_std=s["return_std"], episode_length_mean=s["length_mean"],

@@ -367,6 +367,20 @@ int hrp_ppo_loss_grad(hrp_ppo *h, const float *params_dev, const float *states_d
                       const float *ret_dev, const int64_t *idx_dev, int64_t batch, float eps_clip,
                       float value_coef, float entropy_coef, float loss_scale, float *grad_dev,
                       float *metrics_dev, void *stream);
+/* hrp_ppo_loss_grad with the clipped value loss (PPO's clip_range_vf).  old_value_dev NULL: exactly hrp_ppo_loss_grad
+ * (value_clip is not read).  old_value_dev non-NULL: [rollout rows] float32, the value the rollout stored for each sample,
+ * gathered through idx_dev like the other per-sample inputs (read as [B] when idx_dev is NULL); value_clip = c must be
+ * finite and > 0.  With v the new value, vo the old one and R the return, the value term of every sample becomes
+ *   max((v - R)^2, (vo + clamp(v - vo, -c, c) - R)^2)
+ * weighted as before (value_coef * the minibatch mean), and metrics_dev[2] accumulates it.  Its gradient follows torch
+ * autograd on that expression: maximum splits it half and half on a tie, clamp passes it where -c <= v - vo <= c.
+ * Gaussian and categorical handles; capturable and launched with programmatic dependent launch like hrp_ppo_loss_grad.
+ * Bad arguments return -1 with a message naming the field, before any launch. */
+int hrp_ppo_loss_grad_ex(hrp_ppo *h, const float *params_dev, const float *states_dev,
+                         const float *pre_tanh_dev, const float *old_log_prob_dev, const float *adv_dev,
+                         const float *ret_dev, const int64_t *idx_dev, int64_t batch, float eps_clip,
+                         float value_coef, float entropy_coef, float loss_scale, const float *old_value_dev,
+                         float value_clip, float *grad_dev, float *metrics_dev, void *stream);
 /* clip_grad_norm_ + Adam.step (agent.py:247-252) fused over the flat buffers: ONE cooperative launch (per-CTA
  * sums of squares, grid synchronisation, clip coefficient, Adam).  step_dev[1] int32 is incremented on device
  * (bias correction).  The launch is capturable in a CUDA graph. */
@@ -374,6 +388,14 @@ int hrp_clip_adam_step(float *params_dev, const float *grad_dev, float *exp_avg_
                        float *exp_avg_sq_dev, int32_t *step_dev, int64_t n, double lr, double beta1,
                        double beta2, double eps, float max_grad_norm, float *scratch_dev /* >=128 floats */,
                        void *stream);
+/* hrp_clip_adam_step with the learning rate in device memory, so that a captured step follows a schedule.  lr_dev NULL:
+ * exactly what hrp_clip_adam_step launches.  lr_dev non-NULL: one double, read by the kernel when it runs, in place of lr
+ * (which is then not read) and in the same arithmetic, so *lr_dev == lr gives the same bits.  The caller writes it in
+ * stream order before the launch, or before the replay of a graph that holds the launch.  Bad arguments return -1 with
+ * a message naming the field, before any launch. */
+int hrp_clip_adam_step_ex(float *params_dev, const float *grad_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
+                          int32_t *step_dev, int64_t n, double lr, const double *lr_dev, double beta1, double beta2,
+                          double eps, float max_grad_norm, float *scratch_dev /* >=128 floats */, void *stream);
 
 /* ---- the gradient exchange of the sharded PPO update, fused with clip + Adam (csrc/hrp_comm.cu) --------------
  * One process per GPU on one box.  hrp_comm_create allocates this rank's peer-visible buffers and returns their
@@ -397,6 +419,11 @@ int hrp_comm_note_replay(hrp_comm *comm);     /* a captured step is about to be 
 int hrp_clip_adam_step_p2p(hrp_comm *comm, float *params_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
                            int32_t *step_dev, double lr, double beta1, double beta2, double eps,
                            float max_grad_norm, float *scratch_dev /* >=128 floats */, void *stream);
+/* hrp_clip_adam_step_p2p with the learning rate in device memory: lr_dev as in hrp_clip_adam_step_ex (NULL: exactly
+ * hrp_clip_adam_step_p2p).  Bad arguments return -1 with a message naming the field, before any launch. */
+int hrp_clip_adam_step_p2p_ex(hrp_comm *comm, float *params_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
+                              int32_t *step_dev, double lr, const double *lr_dev, double beta1, double beta2, double eps,
+                              float max_grad_norm, float *scratch_dev /* >=128 floats */, void *stream);
 /* synchronous: 0, or -4 when some cross-GPU wait timed out (a peer never arrived; ~15 s bound per wait) */
 int hrp_comm_status(hrp_comm *comm);
 int hrp_comm_destroy(hrp_comm *comm);

@@ -9,7 +9,11 @@ its max-abs; Adam turns last-bit differences of near-zero gradients into +-lr pa
 parameters themselves a poor yardstick).  Every rank must hold identical parameters at the end in any case.
 
 ``--bootstrap-truncated``: the graph-replayed updates run on rollouts collected with time-limit bootstrapping
-(final_value of truncated steps, hrp_gae_ex); GAE is per env, so the sharded update needs no other exchange."""
+(final_value of truncated steps, hrp_gae_ex); GAE is per env, so the sharded update needs no other exchange.
+
+``--ppo-options``: three more graph-replayed updates each with the peer-memory exchange and with the NCCL all-reduce,
+with the clipped value loss (clip_value) and a linearly annealed learning rate in device memory (set_lr before every
+update): the ranks must agree bit for bit, and the minibatch graphs must be captured once."""
 import os
 import sys
 import time
@@ -26,6 +30,7 @@ dev = torch.device("cuda", local)
 dist.init_process_group("nccl", device_id=dev)
 S, A, H, B, steps = 60, 2, 256, 4096, 24
 BOOT = "--bootstrap-truncated" in sys.argv
+OPTS = "--ppo-options" in sys.argv
 
 
 def make(p2p: bool) -> PPOAgent:
@@ -119,6 +124,32 @@ if rank == 0:
           f"exchange: {'peer-memory kernel' if upd._comm is not None else 'nccl'}; graphs captured: {len(upd._graph_state['graphs'])}")
 ok = ok and upd_equal
 upd.close()
+if OPTS:
+    from highway_rope_ppo_b200.training.routine import linear_lr
+
+    for use_p2p in (True, False):
+        torch.manual_seed(2)
+        agent = PPOAgent(S, A, lr=3e-4, hidden_dim=H, batch_size=B, epochs=3, device=dev, clip_value=0.2)
+        agent.use_p2p = use_p2p
+        states = []
+        for u in range(3):
+            rollout(agent, 2000 + 10 * u + rank)
+            agent.set_lr(linear_lr(3e-4, u, 3))
+            np.random.seed(7 + u)
+            agent.update(last_value=0.0)
+            st = agent._graph_state
+            states.append((id(st), sorted(id(x) for x in st["graphs"].values())))
+        flat = agent.actor_critic.flat
+        gathered = [torch.empty_like(flat) for _ in range(world)]
+        dist.all_gather(gathered, flat)
+        eq = all(torch.equal(gathered[0], x) for x in gathered)
+        once = states[0] == states[1] == states[2]
+        if rank == 0:
+            print(f"world {world}: anneal_lr + clip_value, three graph-replayed updates, exchange "
+                  f"{'peer-memory kernel' if agent._comm is not None else 'nccl'}: identical on every rank: {eq}; "
+                  f"graphs captured once: {once}")
+        ok = ok and eq and once
+        agent.close()
 p2p.close()
 dist.barrier()
 sys.stdout.flush()
