@@ -27,6 +27,18 @@ OBS_KINEMATICS, OBS_OCCUPANCY_GRID = 0, 1   # HRP_OBS_*
 EMBED_NONE, EMBED_ROPE, EMBED_DIST, EMBED_RANK = 0, 1, 2, 3
 PPO_CATEGORICAL = 1   # HRP_PPO_CATEGORICAL
 EPISODE_STATS_LEN = 6 + 6 * 512   # HRP_EPISODE_STATS_LEN: doubles of hrp_episode_stats' stats_dev
+VECNORM_MAX_S = 4608                # HRP_VECNORM_MAX_S: 64 rows x (8 features + 64 embedding columns)
+VECNORM_MAX_E = 1 << 24             # HRP_VECNORM_MAX_E
+
+
+def vecnorm_moments_len(C: int) -> int:
+    """HRP_VECNORM_MOMENTS_LEN: doubles of one rank's batch moments over C columns."""
+    return 1 + 2 * C
+
+
+def vecnorm_scratch_len(C: int) -> int:
+    """HRP_VECNORM_SCRATCH_LEN: doubles of the scratch of hrp_vecnorm_moments / hrp_vecnorm_merge."""
+    return 256 + 256 * C
 
 
 class HrpError(RuntimeError):
@@ -138,6 +150,9 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_comm_note_replay": (C.c_int, [_vp]),
     "hrp_clip_adam_step_p2p": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),
     "hrp_clip_adam_step_p2p_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp]),
+    "hrp_vecnorm_moments": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _f64, _vp, _vp, _vp]),
+    "hrp_vecnorm_merge": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "hrp_vecnorm_apply": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _vp]),
     "hrp_comm_status": (C.c_int, [_vp]),
     "hrp_comm_destroy": (C.c_int, [_vp]),
 }

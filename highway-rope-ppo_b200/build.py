@@ -14,7 +14,8 @@ ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_DIR = os.path.join(PKG_DIR, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libhrp_b200.so")
-SOURCES = ["hrp_env.cu", "hrp_env_fast.cu", "hrp_api.cu", "hrp_ppo.cu", "hrp_mlp_tc.cu", "hrp_comm.cu", "hrp_episodes.cu"]
+SOURCES = ["hrp_env.cu", "hrp_env_fast.cu", "hrp_api.cu", "hrp_ppo.cu", "hrp_mlp_tc.cu", "hrp_comm.cu", "hrp_episodes.cu",
+           "hrp_norm.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC",

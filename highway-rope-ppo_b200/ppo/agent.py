@@ -422,7 +422,8 @@ class PPOMemory:
 
     # -- device-resident [T, E] rollout -----------------------------------------------------------
     def begin_rollout(self, T: int, E: int, state_dim: int, action_dim: int,
-                      pre_dim: Optional[int] = None, bootstrap_truncated: bool = False) -> Dict[str, torch.Tensor]:
+                      pre_dim: Optional[int] = None, bootstrap_truncated: bool = False,
+                      reward_raw: bool = False) -> Dict[str, torch.Tensor]:
         """Allocate (or reuse) time-major buffers: states [T+1,E,S] (slot T holds the bootstrap
         observation), action [T,E,A], pre_tanh [T,E,pre_dim] (default A), log_prob/value/reward [T,E],
         done [T,E] uint8.
@@ -430,7 +431,9 @@ class PPOMemory:
         ``bootstrap_truncated``: also final_states [T,E,S] (the observation each finished episode ended in) and
         final_value [T,E] (the critic's value of it), zero-filled when allocated, and ``update`` bootstraps truncated
         steps with final_value (``hrp_gae_ex``).  A rollout begun without the flag gets the reference's semantics
-        (truncation masks the bootstrap), whatever the reused buffers hold."""
+        (truncation masks the bootstrap), whatever the reused buffers hold.
+
+        ``reward_raw``: also reward_raw [T,E], the env's rewards before a ``VecNormalize`` scaled them into reward."""
         pre_dim = action_dim if pre_dim is None else pre_dim
         r = self.rollout
         if (r is None or r["reward"].shape != (T, E) or r["states"].shape[2] != state_dim
@@ -450,6 +453,8 @@ class PPOMemory:
             d = self.device
             r["final_states"] = torch.zeros((T, E, state_dim), dtype=torch.float32, device=d)
             r["final_value"] = torch.zeros((T, E), dtype=torch.float32, device=d)
+        if reward_raw and "reward_raw" not in r:
+            r["reward_raw"] = torch.empty((T, E), dtype=torch.float32, device=self.device)
         self.rollout = r
         self.bootstrap_truncated = bool(bootstrap_truncated)
         return r

@@ -236,6 +236,10 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     ``final_states[t]`` (``hrp_env_step_final``), the critic computes ``final_value[t]`` from it with the parameters
     that produced ``value[t]``, and ``agent.update`` bootstraps every truncated step with it.  Two more launches per
     step (the critic pass runs over all E rows; only the truncated ones are read), inside the captured graph.
+
+    On a ``VecNormalize`` (envs/vec_normalize.py) the states are the normalized observations and the statistics are
+    updated inside the captured graph.  With ``norm_reward`` the rollout also holds ``reward_raw`` [T, E], the env's
+    rewards, while ``reward`` holds the normalized ones that GAE and the update read.
     """
     A, Z = _act_widths(vec_env, agent)
     E, S = vec_env.num_envs, vec_env.N * vec_env.F_out
@@ -251,7 +255,8 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
            ac.workspace_generation, ac.row_base, boot)
     if use_graph and cache is not None and cache["key"] == key and agent.memory.rollout is None:
         agent.memory.rollout = cache["r"]     # the buffers the captured launches write (PPOAgent.update dropped them)
-    r = agent.memory.begin_rollout(T, E, S, A, Z, bootstrap_truncated=boot)
+    raw = bool(getattr(vec_env, "norm_reward", False))
+    r = agent.memory.begin_rollout(T, E, S, A, Z, bootstrap_truncated=boot, reward_raw=raw)
     states = r["states"]
     if obs is None:
         vec_env.observe(out=states[0].view(E, vec_env.N, vec_env.F_out))
@@ -266,9 +271,10 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
                 agent.act(states[t], noise=None if noise is None else noise[t], out=out)
             else:
                 agent.act(states[t], out=out, draw_counter=counter)
+            extra = {"raw_reward_out": r["reward_raw"][t]} if raw else {}
             vec_env.step(r["action"][t], out=states[t + 1].view(E, vec_env.N, vec_env.F_out), reward_out=r["reward"][t],
                          terminated_out=r["terminated"][t], truncated_out=r["truncated"][t],
-                         final_obs_out=r["final_states"][t] if boot else None)
+                         final_obs_out=r["final_states"][t] if boot else None, **extra)
             if boot:
                 ac.critic_into(r["final_states"][t], r["final_value"][t])
                 agent.launches += 1
@@ -304,7 +310,7 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     ac._draw += T
     cache["expected"] = ac._draw
     agent.launches += 2 * T if boot else T
-    vec_env.launches += T
+    vec_env.launches += T * getattr(vec_env, "step_launches", 1)
     return r
 
 
@@ -402,7 +408,7 @@ def evaluate_vectorized(eval_env, agent, exp_seed: int = 0, use_graph: Optional[
             cache["graph"] = graph
         cache["graph"].replay()
         agent.launches += steps
-        eval_env.launches += 1 + steps
+        eval_env.launches += getattr(eval_env, "reset_launches", 1) + steps * getattr(eval_env, "step_launches", 1)
     sums = buf["stats"][:6]
     if distributed.world_size() > 1:
         distributed.allreduce_sum_(sums)
@@ -421,12 +427,22 @@ def eval_env_for(vec_env, num_envs: int):
     """An evaluation handle of ``num_envs`` envs with ``vec_env``'s resolved config and its ``EmbedSpec`` (the same table
     object: a RankPE evaluation sees the training table, not a new draw), no autoreset.  Its ``env_id_base`` is the
     shard index of ``vec_env`` times ``num_envs``, so that W shards evaluate the episodes one process of W x
-    ``num_envs`` envs would."""
+    ``num_envs`` envs would.
+
+    On a ``VecNormalize`` the handle is wrapped in ``VecNormalize(handle, training=False, norm_reward=False)`` that
+    reads the training wrapper's statistics tensors: evaluation sees the current statistics, frozen, and raw rewards."""
     from ..envs.highway_vec import HighwayVecEnv
+    from ..envs.vec_normalize import VecNormalize
 
     shard = int(vec_env.env_id_base) // int(vec_env.num_envs)
-    return HighwayVecEnv(vec_env.config, num_envs, device=vec_env.device, embed=vec_env.embed, autoreset=False,
-                         env_id_base=shard * int(num_envs), real64=vec_env.real64)
+    env = HighwayVecEnv(vec_env.config, num_envs, device=vec_env.device, embed=vec_env.embed, autoreset=False,
+                        env_id_base=shard * int(num_envs), real64=vec_env.real64)
+    if not isinstance(vec_env, VecNormalize):
+        return env
+    w = VecNormalize(env, training=False, norm_obs=vec_env.norm_obs, norm_reward=False, clip_obs=vec_env.clip_obs,
+                     clip_reward=vec_env.clip_reward, gamma=vec_env.gamma, epsilon=vec_env.epsilon)
+    w.share_statistics(vec_env)
+    return w
 
 
 def linear_lr(lr0: float, it: int, iterations: int) -> float:
@@ -452,7 +468,8 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
     ``seed + 1000 + global env id``, the reference's evaluation seeds with ``seed`` as the experiment seed), recorded
     as ``eval_return_mean`` / ``eval_return_std`` / ``eval_length_mean`` / ``eval_terminated_fraction`` in that
     iteration's metrics.  ``best_checkpoint``: path that ``agent.save`` (rank 0) writes whenever the evaluation mean
-    beats the best so far.
+    beats the best so far; on a ``VecNormalize`` its statistics go to ``best_checkpoint + ".vecnormalize"`` beside it
+    (``VecNormalize.save``), and the episode figures are those of the raw rewards.
 
     ``anneal_lr``: iteration ``it`` runs with ``linear_lr(lr0, it, iterations)``, lr0 being the agent's learning rate at
     entry, set through ``agent.set_lr`` (the learning rate lives in device memory, so the captured minibatch graphs are
@@ -481,10 +498,13 @@ def train_vectorized(vec_env, agent, iterations: int, T: int, seed: int = 0, log
                     best = ev["mean"]
                     if best_checkpoint is not None and distributed.rank() == 0:
                         agent.save(best_checkpoint)
+                        if hasattr(vec_env, "obs_rms"):
+                            vec_env.save(best_checkpoint + ".vecnormalize")
             t0 = time.time()
             r = collect_rollout(vec_env, agent, T, obs, bootstrap_truncated=bootstrap_truncated)
             stats[:6].zero_()
-            episode_stats(r["reward"], r["terminated"], r["truncated"], carry_ret, carry_len, stats)
+            episode_stats(r["reward_raw"] if getattr(vec_env, "norm_reward", False) else r["reward"], r["terminated"],
+                          r["truncated"], carry_ret, carry_len, stats)
             obs = r["states"][T].clone()
             _, _, last_v = agent.actor_critic.forward(obs)
             metrics = agent.update(last_value=last_v.view(-1))

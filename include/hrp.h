@@ -428,6 +428,44 @@ int hrp_clip_adam_step_p2p_ex(hrp_comm *comm, float *params_dev, float *exp_avg_
 int hrp_comm_status(hrp_comm *comm);
 int hrp_comm_destroy(hrp_comm *comm);
 
+/* ---- running observation / reward normalization (SB3 VecNormalize; csrc/hrp_norm.cu) ------------------------------
+ * Running statistics are fp64: obs_rms_dev = [mean S][var S][count], ret_rms_dev = [mean, var, count].  A training step
+ * is three launches on one stream: hrp_vecnorm_moments -> hrp_vecnorm_merge -> hrp_vecnorm_apply.  Every reduction
+ * runs in a fixed order, so equal inputs give the same bits.
+ *
+ * hrp_vecnorm_moments: batch moments of the C = S (+1 with reward_dev) columns of obs_dev [E][S] (NULL with S = 0).
+ * With reward_dev non-NULL, column S is the return carry, updated in place first:
+ * returns_dev[e] = returns_dev[e] * gamma + reward_dev[e] (fp64, no FMA).  The result goes to moments_dev:
+ * [n][mean C][M2 C] (HRP_VECNORM_MOMENTS_LEN(C) doubles, M2 = sum of squared deviations).  A sharded caller gathers
+ * these blocks of every rank, rank-major, and passes them to hrp_vecnorm_merge.  scratch_dev holds
+ * HRP_VECNORM_SCRATCH_LEN(C) doubles, zero-filled before its first use; every call leaves it reusable, for any C.
+ *
+ * hrp_vecnorm_merge: combines the R moment blocks of moments_dev [R][HRP_VECNORM_MOMENTS_LEN(S + has_ret)] in rank
+ * order (Chan et al.) and merges them into the running statistics as RunningMeanStd.update does; counts grow by the
+ * summed n.  obs_rms_dev is NULL with S = 0, ret_rms_dev with has_ret = 0.  scratch_dev: as above.
+ *
+ * hrp_vecnorm_apply: obs_dev (in place) and, where terminated_dev[e] | truncated_dev[e], row e of final_obs_dev become
+ * clip((x - mean) / sqrt(var + epsilon), +-clip_obs), computed in fp64 and rounded once.  reward_out_dev[e] =
+ * clip(reward_dev[e] / sqrt(ret var + epsilon), +-clip_reward).  returns_dev[e] = 0 where the env is done.  Every
+ * pointer but the flags is nullable by part: obs_dev with obs_rms_dev (S = 0 when absent), final_obs_dev needs the
+ * flags, reward_dev with reward_out_dev and ret_rms_dev.
+ *
+ * Bad arguments (E outside [1, 2^24], S outside [0, 4608], no column at all, non-finite or non-positive clips,
+ * epsilon < 0, gamma outside [0, 1], R < 1, a required NULL) return -1 with a message naming the field, before any
+ * launch. */
+#define HRP_VECNORM_MAX_S 4608
+#define HRP_VECNORM_MAX_E (1 << 24)
+#define HRP_VECNORM_MOMENTS_LEN(C) (1 + 2 * (C))
+#define HRP_VECNORM_SCRATCH_LEN(C) (256 + 256 * (C))
+int hrp_vecnorm_moments(const float *obs_dev, int64_t E, int32_t S, const float *reward_dev, double *returns_dev,
+                        double gamma, double *moments_dev, double *scratch_dev, void *stream);
+int hrp_vecnorm_merge(const double *moments_dev, int32_t R, int32_t S, int32_t has_ret, double *obs_rms_dev,
+                      double *ret_rms_dev, double *scratch_dev, void *stream);
+int hrp_vecnorm_apply(float *obs_dev, float *final_obs_dev, const uint8_t *terminated_dev,
+                      const uint8_t *truncated_dev, int64_t E, int32_t S, const float *reward_dev, float *reward_out_dev,
+                      double *returns_dev, const double *obs_rms_dev, const double *ret_rms_dev, double clip_obs,
+                      double clip_reward, double epsilon, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

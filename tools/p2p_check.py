@@ -13,7 +13,12 @@ parameters themselves a poor yardstick).  Every rank must hold identical paramet
 
 ``--ppo-options``: three more graph-replayed updates each with the peer-memory exchange and with the NCCL all-reduce,
 with the clipped value loss (clip_value) and a linearly annealed learning rate in device memory (set_lr before every
-update): the ranks must agree bit for bit, and the minibatch graphs must be captured once."""
+update): the ranks must agree bit for bit, and the minibatch graphs must be captured once.
+
+``--vecnormalize`` (only this check): envs sharded over the ranks behind ``VecNormalize``.  After three rollouts (the
+second captured with the moments all-gather inside the graph, the third replayed) every rank must hold bit-identical
+running statistics; after a reset and one step with fixed actions the sharded statistics must match the numpy
+restatement (tests/vecnormalize_oracle.py) over all envs of all ranks, within 1e-12 relative."""
 import os
 import sys
 import time
@@ -29,6 +34,74 @@ torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
 dist.init_process_group("nccl", device_id=dev)
 S, A, H, B, steps = 60, 2, 256, 4096, 24
+
+
+def _finish(ok):
+    dist.barrier()
+    sys.stdout.flush()
+    # communicator teardown after NCCL work captured in graphs: give it 20 s (see the end of this file)
+    import threading
+
+    threading.Timer(20.0, lambda: (print("destroy_process_group did not return within 20 s", flush=True),
+                                   os._exit(0 if ok else 1))).start()
+    dist.destroy_process_group()
+    os._exit(0 if ok else 1)
+
+
+if "--vecnormalize" in sys.argv:
+    import numpy as np
+
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
+    from vecnormalize_oracle import VecNormOracle  # noqa: E402
+
+    from highway_rope_ppo_b200.config.base_config import HIGHWAY_CONFIG  # noqa: E402
+    from highway_rope_ppo_b200.envs.highway_vec import HighwayVecEnv  # noqa: E402
+    from highway_rope_ppo_b200.envs.vec_normalize import VecNormalize  # noqa: E402
+    from highway_rope_ppo_b200.training.routine import collect_rollout  # noqa: E402
+
+    E, T, seed = 1024, 8, 3
+    cfg = dict(HIGHWAY_CONFIG, duration=5)
+
+    def gathered(t):
+        out = [torch.empty_like(t) for _ in range(world)]
+        dist.all_gather(out, t.contiguous())
+        return out
+
+    w = VecNormalize(HighwayVecEnv(cfg, E, device=dev, env_id_base=rank * E, seed=seed))
+    torch.manual_seed(0)
+    agent = PPOAgent(w.N * w.F_out, A, lr=3e-4, hidden_dim=64, batch_size=512, epochs=1, device=dev)
+    obs = w.reset(seed=seed).clone()
+    for _ in range(3):
+        r = collect_rollout(w, agent, T, obs, bootstrap_truncated=True)
+        obs = r["states"][T].clone()
+    captured = agent._rollout_graph["graph"] is not None
+    bufs = [gathered(x) for x in (w.obs_rms.buf, w.ret_rms.buf, w.returns)]
+    same = all(torch.equal(b[0], x) for b in bufs[:2] for x in b)
+    # reset + one step with fixed actions against the restatement over all ranks' envs
+    plain = HighwayVecEnv(cfg, E, device=dev, env_id_base=rank * E, seed=seed + 1)
+    w2 = VecNormalize(HighwayVecEnv(cfg, E, device=dev, env_id_base=rank * E, seed=seed + 1))
+    raw0 = plain.reset(seed=seed + 1).clone()   # reset and step return the handle's own buffers: keep the reset's
+    w2.reset(seed=seed + 1)
+    a = torch.linspace(-1, 1, 2 * E * world, device=dev).view(world * E, 2)[rank * E:(rank + 1) * E].contiguous()
+    po, pr, pte, ptr = (x.clone() for x in plain.step(a))
+    w2.step(a)
+    allv = [torch.cat(gathered(x)).cpu().numpy() for x in (raw0, po, pr, pte, ptr)]
+    o = VecNormOracle(world * E, plain.obs_shape)
+    o.reset(allv[0])
+    o.step(allv[1], allv[2], allv[3], allv[4])
+    mean, var = w2.obs_rms.mean.cpu().numpy(), w2.obs_rms.var.cpu().numpy()
+    match = (np.allclose(mean, o.obs_rms.mean, rtol=1e-12, atol=1e-15) and np.allclose(var, o.obs_rms.var, rtol=1e-12, atol=1e-15)
+             and abs(float(w2.obs_rms.count) - o.obs_rms.count) <= 1e-12 * o.obs_rms.count
+             and abs(float(w2.ret_rms.mean) - o.ret_rms.mean) <= 1e-12 * abs(o.ret_rms.mean) + 1e-15
+             and abs(float(w2.ret_rms.var) - o.ret_rms.var) <= 1e-12 * abs(o.ret_rms.var) + 1e-15
+             and abs(float(w2.ret_rms.count) - o.ret_rms.count) <= 1e-12 * o.ret_rms.count
+             and np.array_equal(torch.cat(gathered(w2.returns)).cpu().numpy(), o.returns))
+    match = bool(all(gathered(torch.tensor([int(match)], device=dev))[i].item() for i in range(world)))
+    if rank == 0:
+        print(f"world {world}: vecnormalize: ranks bit-identical: {same}; rollout graph captured: {captured}; "
+              f"reset + one step matches one process: {match}", flush=True)
+    agent.close()
+    _finish(same and match and captured)
 BOOT = "--bootstrap-truncated" in sys.argv
 OPTS = "--ppo-options" in sys.argv
 
