@@ -142,6 +142,13 @@ SIGNATURES: Dict[str, Any] = {
                                        _f32, _vp, _vp, _vp]),
     "hrp_clip_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),
     "hrp_clip_adam_step_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp]),
+    "hrp_ppo_loss_grad_kl": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp,
+                                       _f32, _vp, _vp, _vp, _vp, _vp]),
+    "hrp_clip_adam_step_kl": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp, _vp,
+                                        _f64, _vp]),
+    "hrp_graph_if_create": (C.c_int, [_vp, _vp, _vp, C.POINTER(_vp)]),
+    "hrp_graph_if_launch": (C.c_int, [_vp, _vp]),
+    "hrp_graph_if_destroy": (C.c_int, [_vp]),
     "hrp_comm_create": (C.c_int, [_i32, _i32, _i64, _i32, C.POINTER(_vp), _vp]),
     "hrp_comm_connect": (C.c_int, [_vp, _vp]),
     "hrp_comm_grad": (_vp, [_vp]),
@@ -150,6 +157,8 @@ SIGNATURES: Dict[str, Any] = {
     "hrp_comm_note_replay": (C.c_int, [_vp]),
     "hrp_clip_adam_step_p2p": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _f64, _f32, _vp, _vp]),
     "hrp_clip_adam_step_p2p_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp]),
+    "hrp_clip_adam_step_p2p_kl": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _f64, _vp, _f64, _f64, _f64, _f32, _vp, _vp, _f64,
+                                            _vp]),
     "hrp_vecnorm_moments": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _f64, _vp, _vp, _vp]),
     "hrp_vecnorm_merge": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     "hrp_vecnorm_apply": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _f64, _f64, _f64, _vp]),

@@ -80,13 +80,19 @@ __device__ __forceinline__ void wait_words(const unsigned *mine, int world, int 
     __syncthreads();
 }
 
-// LR_DEV: the learning rate is *lr_dev, as in hrp_ppo.cu's clip_adam_kernel
-template <bool LR_DEV>
+// LR_DEV: the learning rate is *lr_dev, as in hrp_ppo.cu's clip_adam_kernel.  KL (target_kl early stopping): the
+// exchange covers n = P + 1 floats, the last being every rank's approx-KL share, so the summed KL arrives with the
+// gradient (the same bits on every rank); clip and Adam cover the first P.  The step is not taken when *stop is already
+// set or the summed KL exceeds kl_limit, and in the second case the kernel raises *stop: both are read before the grid
+// barrier, the word is written after it.  The exchange itself (flags, epoch) runs either way, so a rank never waits for
+// a peer that skipped it.
+template <bool LR_DEV, bool KL>
 __global__ void __launch_bounds__(P2P_THREADS)
 clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long long npad, unsigned *__restrict__ epoch_dev,
                      float *__restrict__ p, float *__restrict__ m, float *__restrict__ v, int32_t *__restrict__ step,
                      long long n, double lr, double beta1, double beta2, double eps, float max_norm,
-                     float *__restrict__ part, unsigned *__restrict__ arrive, const double *__restrict__ lr_dev)
+                     float *__restrict__ part, unsigned *__restrict__ arrive, const double *__restrict__ lr_dev,
+                     unsigned *__restrict__ stop, double kl_limit)
 {
     namespace cg = cooperative_groups;
     cg::grid_group grid = cg::this_grid();
@@ -96,6 +102,7 @@ clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long lo
     // read before anything of this step is written (CTA 0 advances them at the very end, after the grid barrier)
     const unsigned epoch = *epoch_dev + 1u;
     const int k = step[0] + 1;
+    const bool stopped = KL && *stop != 0u;
     unsigned *flags_of[HRP_MAX_RANKS];
 #pragma unroll
     for (int q = 0; q < HRP_MAX_RANKS; ++q) flags_of[q] = q < world ? (unsigned *)(T.base[q] + 4 * npad) : nullptr;
@@ -137,8 +144,10 @@ clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long lo
     // 4. the complete sum is local once every slice has arrived
     wait_words(mine, world, 1, epoch, epoch_dev + 1);
     const float *gsum = T.base[rank] + (size_t)(2 + parity) * npad;
+    const long long np = KL ? n - 1 : n;   // floats of the parameters
+    const bool skip = KL && (stopped || (double)__ldcg(gsum + np) > kl_limit);
     float s = 0.f;
-    for (long long i = i0; i < n; i += stride) {
+    for (long long i = i0; i < np; i += stride) {
         const float g = __ldcg(gsum + i);
         s = fmaf(g, g, s);
     }
@@ -170,7 +179,7 @@ clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long lo
     __syncthreads();
     const float w1 = (float)(1.0 - beta1), b2 = (float)beta2, w2 = (float)(1.0 - beta2), ep = (float)eps;
     const float coef = s_coef, step_size = s_step_size, bc2_sqrt = s_bc2_sqrt;
-    for (long long i = i0; i < n; i += stride) {
+    for (long long i = i0; i < (skip ? 0 : np); i += stride) {
         float gi = __ldcg(gsum + i) * coef;
         float mi = m[i] + w1 * (gi - m[i]);
         float vi = v[i] * b2 + w2 * gi * gi;
@@ -179,7 +188,11 @@ clip_adam_p2p_kernel(const PeerTable T, int world, int rank, int parity, long lo
         p[i] = p[i] - step_size * (mi / denom);
     }
     // every CTA read step[0] / *epoch_dev before the grid barrier above
-    if (blockIdx.x == 0 && threadIdx.x == 0) { step[0] = k; *epoch_dev = epoch; }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        if (!skip) step[0] = k;
+        else if (!stopped) *stop = 1u;
+        *epoch_dev = epoch;
+    }
 }
 
 inline size_t comm_floats(long long n) { return (size_t)(4 * ((n + 31) / 32 * 32) + 64); }
@@ -244,10 +257,10 @@ int hrp_comm_parity(hrp_comm *c) { return c ? (int)(c->issued & 1) : -1; }
 
 }  // extern "C"
 
-template <bool LR_DEV>
+template <bool LR_DEV, bool KL>
 static int clip_adam_p2p_launch(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
                                 const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
-                                float *scratch, void *stream)
+                                float *scratch, void *stream, unsigned *stop = nullptr, double kl_limit = 0.0)
 {
     static int max_ctas_dev[HRP_MAX_DEVICES] = {0};
     if (c->device < 0 || c->device >= HRP_MAX_DEVICES) { hrp_set_error("device index %d not supported", c->device); return -1; }
@@ -255,7 +268,7 @@ static int clip_adam_p2p_launch(hrp_comm *c, float *params, float *exp_avg, floa
     if (max_ctas == 0) {
         int sms = 0, per_sm = 0;
         HRP_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
-        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_p2p_kernel<LR_DEV>, P2P_THREADS, 0));
+        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_p2p_kernel<LR_DEV, KL>, P2P_THREADS, 0));
         max_ctas = sms * per_sm < P2P_MAX_CTAS ? sms * per_sm : P2P_MAX_CTAS;
         if (max_ctas < 1) { hrp_set_error("hrp_clip_adam_step_p2p: kernel does not fit the device"); return -2; }
     }
@@ -267,8 +280,8 @@ static int clip_adam_p2p_launch(hrp_comm *c, float *params, float *exp_avg, floa
     int world = c->world, rank = c->rank, parity = (int)(c->issued & 1);
     unsigned *epoch = c->epoch, *arrive = c->epoch + 2;
     void *args[] = {&T, &world, &rank, &parity, &npad, &epoch, &params, &exp_avg, &exp_avg_sq, &step, &n, &lr, &beta1, &beta2,
-                    &eps, &max_grad_norm, &scratch, &arrive, &lr_dev};
-    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_p2p_kernel<LR_DEV>, dim3(ctas), dim3(P2P_THREADS), args, 0,
+                    &eps, &max_grad_norm, &scratch, &arrive, &lr_dev, &stop, &kl_limit};
+    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_p2p_kernel<LR_DEV, KL>, dim3(ctas), dim3(P2P_THREADS), args, 0,
                                             (cudaStream_t)stream));
     c->issued += 1;
     return 0;
@@ -283,8 +296,8 @@ int hrp_clip_adam_step_p2p(hrp_comm *c, float *params, float *exp_avg, float *ex
         hrp_set_error("hrp_clip_adam_step_p2p: bad arguments (hrp_comm_connect first)");
         return -1;
     }
-    return clip_adam_p2p_launch<false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps, max_grad_norm,
-                                       scratch, stream);
+    return clip_adam_p2p_launch<false, false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps, max_grad_norm,
+                                              scratch, stream);
 }
 
 int hrp_clip_adam_step_p2p_ex(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
@@ -296,10 +309,30 @@ int hrp_clip_adam_step_p2p_ex(hrp_comm *c, float *params, float *exp_avg, float 
                     : !scratch ? "scratch_dev" : nullptr;
     if (bad) { hrp_set_error("hrp_clip_adam_step_p2p_ex: bad argument %s", bad); return -1; }
     if (!lr_dev)
-        return clip_adam_p2p_launch<false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps,
-                                           max_grad_norm, scratch, stream);
-    return clip_adam_p2p_launch<true>(c, params, exp_avg, exp_avg_sq, step, lr, lr_dev, beta1, beta2, eps, max_grad_norm,
-                                      scratch, stream);
+        return clip_adam_p2p_launch<false, false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps,
+                                                  max_grad_norm, scratch, stream);
+    return clip_adam_p2p_launch<true, false>(c, params, exp_avg, exp_avg_sq, step, lr, lr_dev, beta1, beta2, eps, max_grad_norm,
+                                             scratch, stream);
+}
+
+int hrp_clip_adam_step_p2p_kl(hrp_comm *c, float *params, float *exp_avg, float *exp_avg_sq, int32_t *step, double lr,
+                              const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                              float *scratch, uint32_t *stop, double kl_limit, void *stream)
+{
+    const char *bad = !c ? "comm" : !c->connected ? "comm (hrp_comm_connect first)" : !params ? "params_dev"
+                    : !exp_avg ? "exp_avg_dev" : !exp_avg_sq ? "exp_avg_sq_dev" : !step ? "step_dev"
+                    : !scratch ? "scratch_dev" : stop && c->n < 2 ? "comm (created with n_floats = P + 1 >= 2)"
+                    : stop && !(isfinite(kl_limit) && kl_limit > 0.0) ? "kl_limit" : nullptr;
+    if (bad) { hrp_set_error("hrp_clip_adam_step_p2p_kl: bad argument %s", bad); return -1; }
+    if (!stop)
+        return lr_dev ? clip_adam_p2p_launch<true, false>(c, params, exp_avg, exp_avg_sq, step, lr, lr_dev, beta1, beta2,
+                                                          eps, max_grad_norm, scratch, stream)
+                      : clip_adam_p2p_launch<false, false>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2,
+                                                           eps, max_grad_norm, scratch, stream);
+    return lr_dev ? clip_adam_p2p_launch<true, true>(c, params, exp_avg, exp_avg_sq, step, lr, lr_dev, beta1, beta2, eps,
+                                                     max_grad_norm, scratch, stream, stop, kl_limit)
+                  : clip_adam_p2p_launch<false, true>(c, params, exp_avg, exp_avg_sq, step, lr, nullptr, beta1, beta2, eps,
+                                                      max_grad_norm, scratch, stream, stop, kl_limit);
 }
 
 /* a captured graph replays the parity it was captured with: the host says which step it is about to replay */

@@ -465,8 +465,12 @@ heads_act_kernel(const float *__restrict__ a1, const float *__restrict__ c1, con
 // memory.  Phase 2: the CTA writes d(a1) | d(c1) = (dmean Wa2 | dvalue Wc2) under the ReLU masks for its rows.
 // Every CTA leaves 8 partial sums in part[blockIdx.x][8]; the CTA that finishes last adds them in block order
 // (deterministic) and writes d(log_std) and the metrics.  `counter` returns to zero.
+// KL (target_kl early stopping): the last CTA also writes this shard's approx-KL share, the value it adds to
+// metrics[5], to *kl_out, and adds to the metrics only while *stop == 0 (a stopped update's later minibatches do not
+// count).  The gradient is the same either way.  The arguments come last, so the default instantiation keeps its
+// parameter block.
 constexpr int HLB_ROWS = 16;
-template <bool VCLIP>
+template <bool VCLIP, bool KL>
 __global__ void __launch_bounds__(256)
 heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict__ c1, int ld, int H,
                            const float *__restrict__ wa2, const float *__restrict__ ba2,
@@ -477,7 +481,8 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
                            float entropy_coef, float scale, float *__restrict__ dmean, float *__restrict__ dvalue,
                            float *__restrict__ da1, float *__restrict__ dc1, float *__restrict__ dlog_std,
                            float *__restrict__ metrics, float *__restrict__ part,
-                           unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip)
+                           unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip,
+                           float *__restrict__ kl_out, const unsigned *__restrict__ stop)
 {
     __shared__ float out_s[HLB_ROWS][5], dmean_s[HLB_ROWS][4], dvalue_s[HLB_ROWS];
     __shared__ float red[8][8];
@@ -634,7 +639,8 @@ heads_loss_backward_kernel(const float *__restrict__ a1, const float *__restrict
         float frac = (float)B * scale;  // share of the global minibatch held by this shard
         float loss = pol + value_coef * val - entropy_coef * ent * frac;
         for (int a = 0; a < A; ++a) dlog_std[a] = tot[4 + a] - entropy_coef * frac;
-        if (metrics) {
+        if (KL) *kl_out = tot[3] * scale;
+        if (metrics && (!KL || *stop == 0u)) {
             metrics[0] += loss; metrics[1] += pol; metrics[2] += val; metrics[3] += ent * frac;
             metrics[4] += tot[2] * scale; metrics[5] += tot[3] * scale; metrics[6] += frac;
         }
@@ -839,7 +845,8 @@ heads_finish_cat_kernel(const float *__restrict__ part, int tiles_a, int tiles, 
 //   d(logit_j) = scale [-g ratio (delta_{id,j} - p_j) + c_ent p_j (log p_j + H)]   (g = d min(surr1, surr2) / d ratio)
 // and d(value).  Phase 2: d(a1) | d(c1) under the ReLU masks.  Partial sums per CTA: policy loss, value error, clip
 // count, approx-KL, entropy; the last CTA adds them in block order and writes the metrics.  No log_std gradient.
-template <bool VCLIP>
+// KL: as in heads_loss_backward_kernel.
+template <bool VCLIP, bool KL>
 __global__ void __launch_bounds__(256)
 heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__restrict__ c1, int ld, int H,
                                const float *__restrict__ wa2, const float *__restrict__ ba2,
@@ -849,7 +856,8 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
                                float eps_clip, float value_coef, float entropy_coef, float scale,
                                float *__restrict__ dlogit, float *__restrict__ dvalue, float *__restrict__ da1,
                                float *__restrict__ dc1, float *__restrict__ metrics, float *__restrict__ part,
-                               unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip)
+                               unsigned *__restrict__ counter, const float *__restrict__ old_value, float value_clip,
+                               float *__restrict__ kl_out, const unsigned *__restrict__ stop)
 {
     __shared__ float out_s[HLB_ROWS][CAT_MAX + 1], dl_s[HLB_ROWS][CAT_MAX], dvalue_s[HLB_ROWS];
     __shared__ float red[8][8];
@@ -1010,7 +1018,8 @@ heads_loss_backward_cat_kernel(const float *__restrict__ a1, const float *__rest
         float pol = tot[0] * scale, val = tot[1] * scale, ent = tot[4] * scale;   // ent: this shard's share of the mean
         float frac = (float)B * scale;
         float loss = pol + value_coef * val - entropy_coef * ent;
-        if (metrics) {
+        if (KL) *kl_out = tot[3] * scale;
+        if (metrics && (!KL || *stop == 0u)) {
             metrics[0] += loss; metrics[1] += pol; metrics[2] += val; metrics[3] += ent;
             metrics[4] += tot[2] * scale; metrics[5] += tot[3] * scale; metrics[6] += frac;
         }
@@ -1115,19 +1124,26 @@ __global__ void adv_normalize_kernel(float *__restrict__ adv, long long n, const
 // CTA 0 advances the step counter.  ADAM_MAX_CTAS partials fit the caller's 128-float scratch buffer.  LR_DEV: the
 // learning rate is *lr_dev, read when the step size is formed (a captured launch follows a schedule the host writes
 // there); the argument comes last, so the default instantiation keeps its parameter block.
+// KL (target_kl early stopping): the step is not taken when *stop is already set or when the minibatch's approx-KL *kl
+// exceeds kl_limit (strictly, compared in double); in the second case the kernel raises *stop.  Every CTA reads both
+// before the grid barrier and the word is written after it, so all CTAs take the same decision; a step not taken changes
+// no parameter, moment or step counter.
 constexpr int ADAM_MAX_CTAS = 120, ADAM_THREADS = 512;
-template <bool LR_DEV>
+template <bool LR_DEV, bool KL>
 __global__ void __launch_bounds__(ADAM_THREADS)
 clip_adam_kernel(float *__restrict__ p, const float *__restrict__ g, float *__restrict__ m,
                  float *__restrict__ v, int32_t *__restrict__ step, long long n, double lr, double beta1,
-                 double beta2, double eps, float max_norm, float *__restrict__ part, const double *__restrict__ lr_dev)
+                 double beta2, double eps, float max_norm, float *__restrict__ part, const double *__restrict__ lr_dev,
+                 const float *__restrict__ kl, unsigned *__restrict__ stop, double kl_limit)
 {
     __shared__ float red[ADAM_THREADS / 32];
     __shared__ float s_coef, s_step_size, s_bc2_sqrt;
+    const bool skip = KL && (*stop != 0u || (double)*kl > kl_limit);
     const long long stride = (long long)gridDim.x * blockDim.x;
     const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     float s = 0.f;
-    for (long long i = i0; i < n; i += stride) s = fmaf(g[i], g[i], s);
+    if (!skip)
+        for (long long i = i0; i < n; i += stride) s = fmaf(g[i], g[i], s);
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(HRP_FULL, s, d);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
@@ -1139,6 +1155,10 @@ clip_adam_kernel(float *__restrict__ p, const float *__restrict__ g, float *__re
     }
     const int k = step[0] + 1;   // read before the barrier, advanced after it
     cooperative_groups::this_grid().sync();
+    if (KL && skip) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) *stop = 1u;
+        return;
+    }
     if (threadIdx.x < 32) {
         // partials in index order, four per lane, then a fixed shuffle tree
         float t = 0.f;
@@ -1737,7 +1757,8 @@ int hrp_adv_normalize(float *adv, int64_t n, const double *stats, void *stream)
 static int loss_grad_impl(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
                           const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx,
                           int64_t batch, float eps_clip, float value_coef, float entropy_coef, float loss_scale,
-                          const float *old_value, float value_clip, float *grad, float *metrics, void *stream)
+                          const float *old_value, float value_clip, float *grad, float *metrics, void *stream,
+                          float *kl_out = nullptr, const unsigned *stop = nullptr)
 {
     if (!h || !params || !states || !pre_tanh || !old_log_prob || !adv || !ret || !grad) {
         hrp_set_error("hrp_ppo_loss_grad: null argument");
@@ -1777,18 +1798,23 @@ static int loss_grad_impl(hrp_ppo *h, const float *params, const float *states, 
         if (vclip) vo = h->vold;
     }
     if (int rc = forward_impl(h, params, x, B, nullptr, nullptr, s)) return rc;   // trunk + hidden head layers
-    if (h->cat) HRP_CUDA_OK(hrp_launch_pdl(vclip ? heads_loss_backward_cat_kernel<true> : heads_loss_backward_cat_kernel<false>,
+    const bool kl = kl_out != nullptr;
+    auto loss_cat = vclip ? (kl ? heads_loss_backward_cat_kernel<true, true> : heads_loss_backward_cat_kernel<true, false>)
+                          : (kl ? heads_loss_backward_cat_kernel<false, true> : heads_loss_backward_cat_kernel<false, false>);
+    auto loss_gauss = vclip ? (kl ? heads_loss_backward_kernel<true, true> : heads_loss_backward_kernel<true, false>)
+                            : (kl ? heads_loss_backward_kernel<false, true> : heads_loss_backward_kernel<false, false>);
+    if (h->cat) HRP_CUDA_OK(hrp_launch_pdl(loss_cat,
                                            dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256),
                                            0, s, (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2,
                                            params + L.ba2, params + L.wc2, params + L.bc2, z, olp, ad, rt, B, A, eps_clip,
                                            value_coef, entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H,
-                                           metrics, h->loss_part, h->loss_counter, vo, value_clip));
-    else HRP_CUDA_OK(hrp_launch_pdl(vclip ? heads_loss_backward_kernel<true> : heads_loss_backward_kernel<false>,
+                                           metrics, h->loss_part, h->loss_counter, vo, value_clip, kl_out, stop));
+    else HRP_CUDA_OK(hrp_launch_pdl(loss_gauss,
                                dim3((unsigned)((B + HLB_ROWS - 1) / HLB_ROWS)), dim3(256), 0, s,
                                (const float *)h->ac, (const float *)(h->ac + H), H2, H, params + L.wa2, params + L.ba2,
                                params + L.wc2, params + L.bc2, params + L.log_std, z, olp, ad, rt, B, A, eps_clip, value_coef,
                                entropy_coef, loss_scale, h->dmean, h->dvalue, h->d12, h->d12 + H, grad + L.log_std, metrics,
-                               h->loss_part, h->loss_counter, vo, value_clip));
+                               h->loss_part, h->loss_counter, vo, value_clip, kl_out, stop));
     const float *a1 = h->ac, *c1 = h->ac + H;
     ReducePlan plan;
     plan.nseg = 0; plan.blocks = 0;
@@ -1830,10 +1856,11 @@ static int loss_grad_impl(hrp_ppo *h, const float *params, const float *states, 
     return 0;
 }
 
-template <bool LR_DEV>
+template <bool LR_DEV, bool KL>
 static int clip_adam_launch(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
                             double lr, const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
-                            float *scratch, void *stream)
+                            float *scratch, void *stream, const float *kl = nullptr, unsigned *stop = nullptr,
+                            double kl_limit = 0.0)
 {
     cudaStream_t s = (cudaStream_t)stream;
     // per device: a process may drive several GPUs (ExperimentRunner with a device pool)
@@ -1845,7 +1872,7 @@ static int clip_adam_launch(float *params, const float *grad, float *exp_avg, fl
     if (max_ctas == 0) {
         int sms = 0, per_sm = 0;
         HRP_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_kernel<LR_DEV>, ADAM_THREADS, 0));
+        HRP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, clip_adam_kernel<LR_DEV, KL>, ADAM_THREADS, 0));
         max_ctas = sms * per_sm < ADAM_MAX_CTAS ? sms * per_sm : ADAM_MAX_CTAS;
         if (max_ctas < 1) { hrp_set_error("hrp_clip_adam_step: kernel does not fit the device"); return -2; }
     }
@@ -1853,8 +1880,8 @@ static int clip_adam_launch(float *params, const float *grad, float *exp_avg, fl
     if (ctas > max_ctas) ctas = max_ctas;
     long long n_ = n;
     void *args[] = {&params, &grad, &exp_avg, &exp_avg_sq, &step, &n_, &lr, &beta1, &beta2, &eps, &max_grad_norm, &scratch,
-                    &lr_dev};
-    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_kernel<LR_DEV>, dim3(ctas), dim3(ADAM_THREADS), args, 0, s));
+                    &lr_dev, &kl, &stop, &kl_limit};
+    HRP_CUDA_OK(cudaLaunchCooperativeKernel((const void *)clip_adam_kernel<LR_DEV, KL>, dim3(ctas), dim3(ADAM_THREADS), args, 0, s));
     return 0;
 }
 
@@ -1891,8 +1918,8 @@ int hrp_clip_adam_step(float *params, const float *grad, float *exp_avg, float *
         hrp_set_error("hrp_clip_adam_step: bad arguments");
         return -1;
     }
-    return clip_adam_launch<false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
-                                   max_grad_norm, scratch, stream);
+    return clip_adam_launch<false, false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
+                                          max_grad_norm, scratch, stream);
 }
 
 int hrp_clip_adam_step_ex(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
@@ -1903,10 +1930,49 @@ int hrp_clip_adam_step_ex(float *params, const float *grad, float *exp_avg, floa
                     : !step ? "step_dev" : !scratch ? "scratch_dev" : n < 1 ? "n" : nullptr;
     if (bad) { hrp_set_error("hrp_clip_adam_step_ex: bad argument %s", bad); return -1; }
     if (!lr_dev)
-        return clip_adam_launch<false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
-                                       max_grad_norm, scratch, stream);
-    return clip_adam_launch<true>(params, grad, exp_avg, exp_avg_sq, step, n, lr, lr_dev, beta1, beta2, eps,
-                                  max_grad_norm, scratch, stream);
+        return clip_adam_launch<false, false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2, eps,
+                                              max_grad_norm, scratch, stream);
+    return clip_adam_launch<true, false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, lr_dev, beta1, beta2, eps,
+                                         max_grad_norm, scratch, stream);
+}
+
+int hrp_ppo_loss_grad_kl(hrp_ppo *h, const float *params, const float *states, const float *pre_tanh,
+                         const float *old_log_prob, const float *adv, const float *ret, const int64_t *idx,
+                         int64_t batch, float eps_clip, float value_coef, float entropy_coef, float loss_scale,
+                         const float *old_value, float value_clip, float *kl_out, const uint32_t *stop, float *grad,
+                         float *metrics, void *stream)
+{
+    if ((kl_out == nullptr) != (stop == nullptr)) {
+        hrp_set_error("hrp_ppo_loss_grad_kl: bad argument %s (kl_out_dev and stop_dev go together)",
+                      kl_out ? "stop_dev" : "kl_out_dev");
+        return -1;
+    }
+    if (old_value && !(std::isfinite(value_clip) && value_clip > 0.f)) {
+        hrp_set_error("hrp_ppo_loss_grad_kl: value_clip must be finite and > 0 with old_value_dev, got %g", (double)value_clip);
+        return -1;
+    }
+    return loss_grad_impl(h, params, states, pre_tanh, old_log_prob, adv, ret, idx, batch, eps_clip, value_coef,
+                          entropy_coef, loss_scale, old_value, value_clip, grad, metrics, stream, kl_out, stop);
+}
+
+int hrp_clip_adam_step_kl(float *params, const float *grad, float *exp_avg, float *exp_avg_sq, int32_t *step, int64_t n,
+                          double lr, const double *lr_dev, double beta1, double beta2, double eps, float max_grad_norm,
+                          float *scratch, const float *kl, uint32_t *stop, double kl_limit, void *stream)
+{
+    const char *bad = !params ? "params_dev" : !grad ? "grad_dev" : !exp_avg ? "exp_avg_dev" : !exp_avg_sq ? "exp_avg_sq_dev"
+                    : !step ? "step_dev" : !scratch ? "scratch_dev" : n < 1 ? "n"
+                    : (kl == nullptr) != (stop == nullptr) ? (kl ? "stop_dev" : "kl_dev")
+                    : kl && !(std::isfinite(kl_limit) && kl_limit > 0.0) ? "kl_limit" : nullptr;
+    if (bad) { hrp_set_error("hrp_clip_adam_step_kl: bad argument %s", bad); return -1; }
+    if (!kl)
+        return lr_dev ? clip_adam_launch<true, false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, lr_dev, beta1, beta2,
+                                                      eps, max_grad_norm, scratch, stream)
+                      : clip_adam_launch<false, false>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1,
+                                                       beta2, eps, max_grad_norm, scratch, stream);
+    return lr_dev ? clip_adam_launch<true, true>(params, grad, exp_avg, exp_avg_sq, step, n, lr, lr_dev, beta1, beta2, eps,
+                                                 max_grad_norm, scratch, stream, kl, stop, kl_limit)
+                  : clip_adam_launch<false, true>(params, grad, exp_avg, exp_avg_sq, step, n, lr, nullptr, beta1, beta2,
+                                                  eps, max_grad_norm, scratch, stream, kl, stop, kl_limit);
 }
 
 }  // extern "C"

@@ -603,18 +603,52 @@ class _AdamState:
             self.eps = float(groups[0].get("eps", self.eps))
 
 
+class _GatedGraph:
+    """A captured minibatch graph behind the target_kl gate: ``[gate] -> IF (stop word == 0) { graph }``, instantiated
+    by ``hrp_graph_if_create`` from the graph's ``cudaGraph_t``.  ``state`` is the agent's [stop word, openings]."""
+
+    def __init__(self, lib, graph: "torch.cuda.CUDAGraph", state: torch.Tensor):
+        self._lib, self.graph = lib, graph
+        self.handle = C.c_void_p()
+        _lib.check(lib.hrp_graph_if_create(C.c_void_p(graph.raw_cuda_graph()), state.data_ptr(), state.data_ptr() + 4,
+                                           C.byref(self.handle)), "hrp_graph_if_create")
+
+    def __del__(self):  # pragma: no cover
+        try:
+            if self.handle:
+                self._lib.hrp_graph_if_destroy(self.handle)   # an exec still in flight is freed when it completes
+                self.handle = None
+        except Exception:
+            pass
+
+
 class PPOAgent:
     def __init__(self, state_dim: int, action_dim: int, lr: float = 1e-4, gamma: float = 0.99, lam: float = 0.95,
                  eps_clip: float = 0.2, value_coef: float = 0.5, entropy_coef: float = 0.005,
                  max_grad_norm: float = 0.5, epochs: int = 6, batch_size: int = 64, hidden_dim: int = 128,
                  logger: Optional[logging.Logger] = None, device: Any = "cuda", *, discrete: bool = False,
-                 clip_value: Optional[float] = None):
+                 clip_value: Optional[float] = None, target_kl: Optional[float] = None):
         """``clip_value`` = c (keyword-only, off by default): the clipped value loss, max((v - R)^2, (v_old +
         clamp(v - v_old, -c, c) - R)^2) per sample with v_old the value the rollout stored (``hrp_ppo_loss_grad_ex``),
-        weighted like the reference's value MSE; the ``value_loss`` and ``loss`` metrics report it."""
+        weighted like the reference's value MSE; the ``value_loss`` and ``loss`` metrics report it.
+
+        ``target_kl`` (keyword-only, off by default): SB3's early stopping.  When a minibatch's approx-KL exceeds
+        1.5 * target_kl its optimizer step is not taken, nor any later one of the update; its loss terms still enter the
+        metrics, those of the minibatches after it do not.  Decided on the device (a stop word the loss and Adam kernels
+        read, ``hrp_ppo_loss_grad_kl`` / ``hrp_clip_adam_step_kl``), and the replayed minibatch graphs sit behind a
+        conditional node that skips a stopped update's remaining steps (``hrp_graph_if_create``).  ``update`` then also
+        returns ``optimizer_steps`` and ``stopped_early``."""
         if clip_value is not None and not (math.isfinite(float(clip_value)) and float(clip_value) > 0):
             raise ValueError(f"clip_value must be a finite number > 0 or None, got {clip_value!r}")
         self.clip_value = None if clip_value is None else float(clip_value)
+        if target_kl is not None:
+            try:
+                ok = not isinstance(target_kl, bool) and math.isfinite(float(target_kl)) and float(target_kl) > 0
+            except (TypeError, ValueError):
+                ok = False
+            if not ok:
+                raise ValueError(f"target_kl must be a finite number > 0 or None, got {target_kl!r}")
+        self.target_kl = None if target_kl is None else float(target_kl)
         self._lib = _lib.load()
         self.device = _cuda_device(device)
         self.discrete = bool(discrete)
@@ -627,7 +661,13 @@ class PPOAgent:
         self.logger = logger or logging.getLogger(__name__)
         self.memory = PPOMemory(batch_size=batch_size, device=self.device)
         P = self.actor_critic.num_params
-        self.grad = torch.zeros(P, dtype=torch.float32, device=self.device)
+        # target_kl: one more float after the gradient holds the minibatch's approx-KL share, so that every gradient
+        # exchange sums it with the gradient; [stop word, gate openings] (uint32 on the device); step_dev at update_begin
+        self._grad_len = P + (1 if self.target_kl is not None else 0)
+        self.grad = torch.zeros(self._grad_len, dtype=torch.float32, device=self.device)
+        if self.target_kl is not None:
+            self._kl_state = torch.zeros(2, dtype=torch.int32, device=self.device)
+            self._step0 = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._metrics = torch.zeros(8, dtype=torch.float32, device=self.device)
         self._stats = torch.zeros(3 + 512, dtype=torch.float64, device=self.device)
         self.launches = 0  # hrp_* calls enqueued by this agent (each is >= 1 kernel of this library)
@@ -684,7 +724,7 @@ class PPOAgent:
             return False
         import torch.distributed as dist
 
-        lib, P = self._lib, self.actor_critic.num_params
+        lib, P = self._lib, self._grad_len
         handle = (C.c_ubyte * 64)()
         comm = C.c_void_p()
         rc = lib.hrp_comm_create(world, distributed.rank(), P, self.device.index, C.byref(comm), handle)
@@ -726,7 +766,7 @@ class PPOAgent:
         self.release_graphs()
         if self._comm is not None:
             torch.cuda.synchronize(self.device)
-            self.grad = torch.zeros(self.actor_critic.num_params, dtype=torch.float32, device=self.device)
+            self.grad = torch.zeros(self._grad_len, dtype=torch.float32, device=self.device)
             self._lib.hrp_comm_destroy(self._comm)
             self._comm, self._comm_keep, self._grad_parity = None, None, None
 
@@ -739,7 +779,15 @@ class PPOAgent:
                      flat["log_prob"].data_ptr(), flat["adv"].data_ptr(), flat["ret"].data_ptr(), _lib.ptr(idx), B,
                      float(self.eps_clip), float(self.value_coef), float(self.entropy_coef),
                      distributed.loss_scale(B, world))
-        if self.clip_value is None:
+        kl = self.target_kl is not None
+        if kl:
+            kl_ptr, stop_ptr = self.grad.data_ptr() + 4 * ac.num_params, self._kl_state.data_ptr()
+            kl_limit = 1.5 * self.target_kl
+            _lib.check(self._lib.hrp_ppo_loss_grad_kl(*loss_args, _lib.ptr(flat.get("value")),
+                                                      0.0 if self.clip_value is None else self.clip_value, kl_ptr,
+                                                      stop_ptr, self.grad.data_ptr(), self._metrics.data_ptr(), s),
+                       "hrp_ppo_loss_grad_kl")
+        elif self.clip_value is None:
             _lib.check(self._lib.hrp_ppo_loss_grad(*loss_args, self.grad.data_ptr(), self._metrics.data_ptr(), s),
                        "hrp_ppo_loss_grad")
         else:
@@ -752,7 +800,10 @@ class PPOAgent:
             args = (self._comm, ac.flat.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
                     opt.step_dev.data_ptr(), opt.lr)
             tail = (opt.betas[0], opt.betas[1], opt.eps, float(self.max_grad_norm), opt.scratch.data_ptr(), s)
-            if lr_dev is None:
+            if kl:
+                _lib.check(self._lib.hrp_clip_adam_step_p2p_kl(*args, _lib.ptr(lr_dev), *tail[:-1], stop_ptr, kl_limit,
+                                                               s), "hrp_clip_adam_step_p2p_kl")
+            elif lr_dev is None:
                 _lib.check(self._lib.hrp_clip_adam_step_p2p(*args, *tail), "hrp_clip_adam_step_p2p")
             else:
                 _lib.check(self._lib.hrp_clip_adam_step_p2p_ex(*args, lr_dev.data_ptr(), *tail),
@@ -764,7 +815,10 @@ class PPOAgent:
         args = (ac.flat.data_ptr(), self.grad.data_ptr(), opt.exp_avg.data_ptr(), opt.exp_avg_sq.data_ptr(),
                 opt.step_dev.data_ptr(), ac.num_params, opt.lr)
         tail = (opt.betas[0], opt.betas[1], opt.eps, float(self.max_grad_norm), opt.scratch.data_ptr(), s)
-        if lr_dev is None:
+        if kl:
+            _lib.check(self._lib.hrp_clip_adam_step_kl(*args, _lib.ptr(lr_dev), *tail[:-1], kl_ptr, stop_ptr, kl_limit, s),
+                       "hrp_clip_adam_step_kl")
+        elif lr_dev is None:
             _lib.check(self._lib.hrp_clip_adam_step(*args, *tail), "hrp_clip_adam_step")
         else:
             _lib.check(self._lib.hrp_clip_adam_step_ex(*args, lr_dev.data_ptr(), *tail), "hrp_clip_adam_step_ex")
@@ -777,8 +831,8 @@ class PPOAgent:
             self._graph_state = None
 
     # -- the epochs x minibatches loop as CUDA graphs --------------------------------------------------
-    def _capture(self, fn, world: int) -> "torch.cuda.CUDAGraph":
-        g = torch.cuda.CUDAGraph()
+    def _capture(self, fn, world: int, keep_graph: bool = False) -> "torch.cuda.CUDAGraph":
+        g = torch.cuda.CUDAGraph(keep_graph=keep_graph)
         if world > 1:   # collectives inside: torch's context (full synchronisation, allocator quiesced) as before
             with torch.cuda.graph(g):
                 fn()
@@ -816,7 +870,7 @@ class PPOAgent:
         opt = self.optimizer
         key = (n, bs, world, ac.workspace_generation, float(self.eps_clip), float(self.value_coef), float(self.entropy_coef),
                float(self.max_grad_norm), opt.lr if opt.lr_dev is None else "lr_dev", opt.betas, opt.eps,
-               self.clip_value)
+               self.clip_value, self.target_kl)
         st = self._graph_state
         if st is None or st["key"] != key:
             d = self.device
@@ -833,6 +887,10 @@ class PPOAgent:
         # in, nothing between the replays.  Many (a sweep run at batch 32: 64 and more): one graph per distinct size,
         # fed through the index buffer, because capturing dominates there.
         shared = len(starts) > 32
+        # target_kl: each replayed step runs behind a gate on the stop word (hrp_graph_if_create), so a stopped update's
+        # remaining steps are skipped, not merely neutralised.  Not with the NCCL all-reduce captured inside: every
+        # rank runs those bodies, whose kernels the stop word gates.
+        gated = self.target_kl is not None and (world == 1 or self._comm is not None)
         for epoch in range(self.epochs):
             for i, start in enumerate(starts):
                 B = min(bs, n - start)
@@ -850,12 +908,17 @@ class PPOAgent:
                 g = st["graphs"].get(gkey)
                 if g is None:
                     # (capturing advances the parity)
-                    g = self._capture(lambda: self._minibatch_step(st["buf"], idx, B, world), world)
+                    g = self._capture(lambda: self._minibatch_step(st["buf"], idx, B, world), world, keep_graph=gated)
+                    if gated:
+                        g = _GatedGraph(self._lib, g, self._kl_state)
                     st["graphs"][gkey] = g
                 elif world > 1 and self._comm is not None:
                     _lib.check(self._lib.hrp_comm_note_replay(self._comm), "hrp_comm_note_replay")
                     self.grad = self._grad_parity[parity]
-                g.replay()
+                if gated:
+                    _lib.check(self._lib.hrp_graph_if_launch(g.handle, ac._stream()), "hrp_graph_if_launch")
+                else:
+                    g.replay()
                 self.launches += 2
             st["warm"] = True
 
@@ -899,6 +962,9 @@ class PPOAgent:
         bs = int(mem.batch_size)
         ac._ensure_workspace(min(bs, n))
         self._metrics.zero_()
+        if self.target_kl is not None:   # every update starts unstopped; steps taken = step_dev - the snapshot
+            self._kl_state.zero_()
+            self._step0.copy_(self.optimizer.step_dev)
         if world > 1:
             self._ensure_comm(world)
         if self.use_cuda_graphs and (world == 1 or self.graph_collectives):
@@ -927,8 +993,10 @@ class PPOAgent:
             var_y = torch.var(y_true) if n > 1 else torch.zeros((), device=self.device)
             var_r = torch.var(y_true - y_pred) if n > 1 else torch.zeros((), device=self.device)
         tail = torch.stack([var_y.float(), var_r.float()])
+        if self.target_kl is not None:   # optimizer steps taken, stop word
+            tail = torch.cat([tail, (self.optimizer.step_dev - self._step0).float(), self._kl_state[:1].float()])
         if getattr(self, "_metrics_host", None) is None:
-            self._metrics_host = torch.zeros(10, dtype=torch.float32).pin_memory()
+            self._metrics_host = torch.zeros(len(tail) + 8, dtype=torch.float32).pin_memory()
         self._metrics_host.copy_(torch.cat([self._metrics, tail]), non_blocking=True)   # the update's single D2H
         done = torch.cuda.Event()
         done.record()
@@ -945,6 +1013,9 @@ class PPOAgent:
                "value_loss": float(host[2] / count), "entropy": float(host[3] / count),
                "clip_fraction": float(host[4] / count), "approx_kl": float(host[5] / count),
                "explained_variance": explained}
+        if self.target_kl is not None:
+            out["optimizer_steps"] = int(host[10])
+            out["stopped_early"] = bool(host[11] != 0)
         self.logger.info(
             "update_complete loss=%.4f policy_loss=%.4f value_loss=%.4f entropy=%.4f clip_frac=%.3f kl=%.5f "
             "explained_var=%.3f", out["loss"], out["policy_loss"], out["value_loss"], out["entropy"],

@@ -397,6 +397,42 @@ int hrp_clip_adam_step_ex(float *params_dev, const float *grad_dev, float *exp_a
                           int32_t *step_dev, int64_t n, double lr, const double *lr_dev, double beta1, double beta2,
                           double eps, float max_grad_norm, float *scratch_dev /* >=128 floats */, void *stream);
 
+/* ---- target_kl early stopping (SB3's PPO(target_kl=...)) -------------------------------------------------------------
+ * A minibatch's approx-KL mean((ratio - 1) - log ratio) is reduced by the loss kernel; when it exceeds 1.5 target_kl the
+ * optimizer step is not taken and no later step of the update is either.  The decision is taken on the device through a
+ * 32-bit stop word (0 = running), which the caller clears before the update.
+ *
+ * hrp_ppo_loss_grad_kl: hrp_ppo_loss_grad_ex, plus, with kl_out_dev / stop_dev non-NULL (both or neither): the last CTA
+ * writes this shard's approx-KL share (the value it adds to metrics_dev[5]) to *kl_out_dev, and metrics_dev is added to
+ * only while *stop_dev == 0.  The gradient is unchanged.  The caller places kl_out_dev at grad_dev + P, so that a
+ * gradient exchange over P + 1 floats also sums the KL in rank order.  Both NULL: exactly hrp_ppo_loss_grad_ex.
+ * hrp_clip_adam_step_kl: hrp_clip_adam_step_ex over the n = P parameters, plus, with kl_dev / stop_dev non-NULL (both or
+ * neither): a no-op when *stop_dev != 0; otherwise when (double)*kl_dev > kl_limit (finite, > 0) it sets *stop_dev = 1
+ * and takes no step (no parameter, moment or step_dev change).  Both NULL: exactly hrp_clip_adam_step_ex.
+ * Bad arguments return -1 with a message naming the field, before any launch. */
+int hrp_ppo_loss_grad_kl(hrp_ppo *h, const float *params_dev, const float *states_dev,
+                         const float *pre_tanh_dev, const float *old_log_prob_dev, const float *adv_dev,
+                         const float *ret_dev, const int64_t *idx_dev, int64_t batch, float eps_clip,
+                         float value_coef, float entropy_coef, float loss_scale, const float *old_value_dev,
+                         float value_clip, float *kl_out_dev, const uint32_t *stop_dev, float *grad_dev,
+                         float *metrics_dev, void *stream);
+int hrp_clip_adam_step_kl(float *params_dev, const float *grad_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
+                          int32_t *step_dev, int64_t n, double lr, const double *lr_dev, double beta1, double beta2,
+                          double eps, float max_grad_norm, float *scratch_dev /* >=128 floats */, const float *kl_dev,
+                          uint32_t *stop_dev, double kl_limit, void *stream);
+
+/* ---- a captured graph behind a device-side gate (csrc/hrp_graph.cu) ---------------------------------------------------
+ * hrp_graph_if_create builds [gate kernel] -> IF { child graph body_graph } (a conditional node; body_graph is a
+ * cudaGraph_t, which is cloned, e.g. torch.cuda.CUDAGraph(keep_graph=True).raw_cuda_graph()) and instantiates it on the
+ * current device.  Each hrp_graph_if_launch runs the gate, which opens the body iff *stop_dev == 0 and then adds one to
+ * *opened_dev; a closed body costs the gate kernel only.  Bad arguments return -1 with a message naming the field, and so
+ * does a graph CUDA refuses to build or instantiate, with the CUDA error text.  hrp_graph_if_destroy: after the launches
+ * have completed. */
+typedef struct hrp_graph_if hrp_graph_if;
+int hrp_graph_if_create(void *body_graph, const uint32_t *stop_dev, uint32_t *opened_dev, hrp_graph_if **out);
+int hrp_graph_if_launch(hrp_graph_if *wrapped, void *stream);
+int hrp_graph_if_destroy(hrp_graph_if *wrapped);
+
 /* ---- the gradient exchange of the sharded PPO update, fused with clip + Adam (csrc/hrp_comm.cu) --------------
  * One process per GPU on one box.  hrp_comm_create allocates this rank's peer-visible buffers and returns their
  * 64-byte cudaIpc handle; the caller gathers the handles of all ranks (rank-major) and passes them to
@@ -424,6 +460,15 @@ int hrp_clip_adam_step_p2p(hrp_comm *comm, float *params_dev, float *exp_avg_dev
 int hrp_clip_adam_step_p2p_ex(hrp_comm *comm, float *params_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
                               int32_t *step_dev, double lr, const double *lr_dev, double beta1, double beta2, double eps,
                               float max_grad_norm, float *scratch_dev /* >=128 floats */, void *stream);
+/* hrp_clip_adam_step_p2p_ex with target_kl early stopping: with stop_dev non-NULL the comm must have been created with
+ * n_floats = P + 1, the last float of each rank's gradient buffer holding its approx-KL share (hrp_ppo_loss_grad_kl's
+ * kl_out_dev); the exchange sums all P + 1, clip and Adam cover P, and the step is decided on the summed KL as in
+ * hrp_clip_adam_step_kl -- the same bits on every rank, so every rank takes the same decision.  The exchange runs either
+ * way.  stop_dev NULL: exactly hrp_clip_adam_step_p2p_ex. */
+int hrp_clip_adam_step_p2p_kl(hrp_comm *comm, float *params_dev, float *exp_avg_dev, float *exp_avg_sq_dev,
+                              int32_t *step_dev, double lr, const double *lr_dev, double beta1, double beta2, double eps,
+                              float max_grad_norm, float *scratch_dev /* >=128 floats */, uint32_t *stop_dev,
+                              double kl_limit, void *stream);
 /* synchronous: 0, or -4 when some cross-GPU wait timed out (a peer never arrived; ~15 s bound per wait) */
 int hrp_comm_status(hrp_comm *comm);
 int hrp_comm_destroy(hrp_comm *comm);

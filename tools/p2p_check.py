@@ -15,6 +15,13 @@ parameters themselves a poor yardstick).  Every rank must hold identical paramet
 with the clipped value loss (clip_value) and a linearly annealed learning rate in device memory (set_lr before every
 update): the ranks must agree bit for bit, and the minibatch graphs must be captured once.
 
+``--target-kl``: target_kl early stopping with each exchange.  The rollouts hold the policy's own log-probs (so the KL
+grows from ~0 during an update) and the limit is the mean KL of an unstopped update on the same data, so the update
+stops part-way: on the peer-memory path (the KL share summed with the gradient, the steps behind the conditional gate)
+and on the NCCL path (the all-reduce over P + 1 floats, the steps replayed unconditionally), every rank must stop at the
+same step with bit-identical parameters, both paths must stop at the same step, and two updates must capture their
+graphs once.
+
 ``--vecnormalize`` (only this check): envs sharded over the ranks behind ``VecNormalize``.  After three rollouts (the
 second captured with the moments all-gather inside the graph, the third replayed) every rank must hold bit-identical
 running statistics; after a reset and one step with fixed actions the sharded statistics must match the numpy
@@ -104,6 +111,7 @@ if "--vecnormalize" in sys.argv:
     _finish(same and match and captured)
 BOOT = "--bootstrap-truncated" in sys.argv
 OPTS = "--ppo-options" in sys.argv
+TKL = "--target-kl" in sys.argv
 
 
 def make(p2p: bool) -> PPOAgent:
@@ -223,6 +231,58 @@ if OPTS:
                   f"graphs captured once: {once}")
         ok = ok and eq and once
         agent.close()
+if TKL:
+    def own_rollout(agent, seed):
+        T, E = 6, 2048
+        gg = torch.Generator(device=dev).manual_seed(seed)
+        r = agent.memory.begin_rollout(T, E, S, A)
+        r["states"].copy_(torch.randn(T + 1, E, S, generator=gg, device=dev) * 0.5)
+        out = agent.act(r["states"][:T].reshape(T * E, S).contiguous(),
+                        noise=torch.randn(T * E, A, generator=gg, device=dev))
+        r["pre_tanh"].copy_(out["pre_tanh"].view(T, E, A))
+        r["action"].copy_(out["action"].view(T, E, A))
+        r["log_prob"].copy_(out["log_prob"].view(T, E))
+        r["value"].copy_(out["value"].view(T, E))
+        r["reward"].copy_(torch.rand(T, E, generator=gg, device=dev))
+        r["done"].copy_((torch.rand(T, E, generator=gg, device=dev) < 0.05).to(torch.uint8))
+
+    torch.manual_seed(3)
+    twin = PPOAgent(S, A, lr=1e-3, hidden_dim=H, batch_size=B, epochs=3, device=dev)
+    twin.use_p2p = False
+    own_rollout(twin, 3000 + rank)
+    np.random.seed(9)
+    target = twin.update(last_value=0.0)["approx_kl"] / 1.5   # all-reduced: the same on every rank
+    twin.close()
+    steps_by_path = []
+    for use_p2p in (True, False):
+        torch.manual_seed(3)
+        agent = PPOAgent(S, A, lr=1e-3, hidden_dim=H, batch_size=B, epochs=3, device=dev, target_kl=target)
+        agent.use_p2p = use_p2p
+        got, states = [], []
+        for u in range(2):
+            own_rollout(agent, 3000 + 10 * u + rank)
+            np.random.seed(9 + u)
+            m = agent.update(last_value=0.0)
+            got.append((m["optimizer_steps"], m["stopped_early"]))
+            st = agent._graph_state
+            states.append((id(st), sorted(id(x) for x in st["graphs"].values())))
+        flat = agent.actor_critic.flat
+        gathered = [torch.empty_like(flat) for _ in range(world)]
+        dist.all_gather(gathered, flat)
+        eq = all(torch.equal(gathered[0], x) for x in gathered)
+        mine = torch.tensor([s for s, _ in got], device=dev)
+        every = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(every, mine)
+        same_steps = all(torch.equal(every[0], x) for x in every)
+        once = states[0] == states[1]
+        if rank == 0:
+            print(f"world {world}: target_kl {target:.3e}, exchange "
+                  f"{'peer-memory kernel' if agent._comm is not None else 'nccl'}: (steps, stopped) per update {got}; "
+                  f"same steps on every rank: {same_steps}; identical on every rank: {eq}; graphs captured once: {once}")
+        ok = ok and eq and same_steps and once and got[0][1]
+        steps_by_path.append(got)
+        agent.close()
+    ok = ok and steps_by_path[0] == steps_by_path[1]
 p2p.close()
 dist.barrier()
 sys.stdout.flush()
