@@ -26,6 +26,7 @@ FEATURE_CODES = {"presence": 0, "x": 1, "y": 2, "vx": 3, "vy": 4, "heading": 5, 
 OBS_KINEMATICS, OBS_OCCUPANCY_GRID = 0, 1   # HRP_OBS_*
 EMBED_NONE, EMBED_ROPE, EMBED_DIST, EMBED_RANK = 0, 1, 2, 3
 PPO_CATEGORICAL = 1   # HRP_PPO_CATEGORICAL
+ACT_MAX_DIM = 1024    # HRP_ACT_MAX_DIM: widest state_dim / hidden_dim of an hrp_ppo_act_multi item
 EPISODE_STATS_LEN = 6 + 6 * 512   # HRP_EPISODE_STATS_LEN: doubles of hrp_episode_stats' stats_dev
 VECNORM_MAX_S = 4608                # HRP_VECNORM_MAX_S: 64 rows x (8 features + 64 embedding columns)
 VECNORM_MAX_E = 1 << 24             # HRP_VECNORM_MAX_E

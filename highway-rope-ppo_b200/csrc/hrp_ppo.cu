@@ -1312,7 +1312,7 @@ static int forward_impl(hrp_ppo *h, const float *params, const float *x, long lo
 // cluster through distributed shared memory, and the cluster synchronises once per layer.  CTA 0 finishes with the two
 // heads, the tanh-Gaussian sample (the same Philox keying and Box-Muller as heads_act_kernel) and the log-prob.
 // One launch serves up to ACT_ITEMS policies of different widths (multiplexed experiments, experiments/multiplex.py).
-constexpr int ACT_CLUSTER = 4, ACT_THREADS = 512, ACT_ITEMS = 32, ACT_MAX_DIM = 1024;
+constexpr int ACT_CLUSTER = 4, ACT_THREADS = 512, ACT_ITEMS = 32, ACT_MAX_DIM = HRP_ACT_MAX_DIM;
 struct ActBatch { hrp_act_item it[ACT_ITEMS]; };
 
 __device__ __forceinline__ void act_layer(const float *__restrict__ W, const float *__restrict__ bias, const float *in, int K,
@@ -1587,11 +1587,25 @@ static int ppo_create(int32_t state_dim, int32_t action_dim, int32_t hidden_dim,
     if (ndev <= 0) { hrp_set_error("no CUDA device: this library has no CPU path"); return -3; }
     if (device < 0 || device >= ndev) { hrp_set_error("device %d not in [0, %d)", device, ndev); return -1; }
     HRP_CUDA_OK(cudaSetDevice(device));
-    if (cat) {
-        // the categorical act kernel keeps its n + 1 head rows in shared memory
+    {
+        // the unfused act kernels keep the A + 1 head rows in shared memory: above 48 KB the launch needs the opt-in.
+        // The limit is raised to everything the device allows (not to this policy's need), so that creating a
+        // narrower policy later cannot lower it under a wider one's.
         const size_t smem = (size_t)(action_dim + 1) * hidden_dim * sizeof(float);
-        if (smem > 48 * 1024)
-            HRP_CUDA_OK(cudaFuncSetAttribute(heads_act_cat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) {
+            const void *kern = cat ? (const void *)heads_act_cat_kernel : (const void *)heads_act_kernel;
+            int optin = 0;
+            cudaFuncAttributes fa;
+            HRP_CUDA_OK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+            HRP_CUDA_OK(cudaFuncGetAttributes(&fa, kern));
+            const size_t room = (size_t)optin - fa.sharedSizeBytes;
+            if (smem > room) {
+                hrp_set_error("hrp_ppo_create: hidden_dim %d with action_dim %d needs %zu bytes of shared memory for the "
+                              "act heads, above the device's %zu", (int)hidden_dim, (int)action_dim, smem, room);
+                return -1;
+            }
+            HRP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)room));
+        }
     }
     hrp_ppo *h = new hrp_ppo();
     h->L = make_layout(state_dim, action_dim, hidden_dim, cat);

@@ -229,10 +229,11 @@ class ActorCritic:
         may overlap: the two env groups of the pipelined host-buffer loop (bench.py e2e) act concurrently.
 
         Categorical policy: action [B, 2] = (id, 0) -- what the meta-action env step reads --, pre_tanh [B, 1] = id;
-        ``noise`` holds one uniform in (0, 1) per row; B = 1 goes through the batched kernels."""
+        ``noise`` holds one uniform in (0, 1) per row; B = 1 goes through the batched kernels, as it does for a Gaussian
+        policy wider than the single-state kernel takes (``_lib.ACT_MAX_DIM``)."""
         states = self._as_states(states)
         B = states.shape[0]
-        if B == 1 and noise is None and not lane and draw_counter is None and not self.discrete:
+        if B == 1 and noise is None and not lane and draw_counter is None and self._fits_act_item():
             return self._act_one(states, deterministic, out, stream)
         if lane:
             return self._act_lane(states, B, out, lane, deterministic, noise, draw_counter)
@@ -278,9 +279,13 @@ class ActorCritic:
     # -- one state: the matrix-vector kernel (what the reference's single-env loop calls once per env step) -------
     def act_item(self, state: torch.Tensor, out_row: torch.Tensor, deterministic: bool) -> "_lib.HrpActItem":
         """The ``hrp_act_item`` of one ``get_action`` call of this policy (advances the draw counter when sampling):
-        ``hrp_ppo_act_multi`` serves many such items, of different policies, in one launch.  Gaussian policies only."""
+        ``hrp_ppo_act_multi`` serves many such items, of different policies, in one launch.  Gaussian policies with
+        state_dim and hidden_dim <= ``_lib.ACT_MAX_DIM`` only."""
         if self.discrete:
             raise ValueError("hrp_ppo_act_multi serves Gaussian policies only")
+        if not self._fits_act_item():
+            raise ValueError(f"hrp_ppo_act_multi takes state_dim and hidden_dim <= {_lib.ACT_MAX_DIM}, this policy has "
+                             f"state_dim {self.state_dim}, hidden_dim {self.hidden_dim}")
         if not deterministic:
             self._draw += 1
         it = _lib.HrpActItem()
@@ -289,6 +294,9 @@ class ActorCritic:
         it.state_dim, it.action_dim, it.hidden_dim = self.state_dim, self.action_dim, self.hidden_dim
         it.deterministic = int(bool(deterministic))
         return it
+
+    def _fits_act_item(self) -> bool:
+        return not self.discrete and max(self.state_dim, self.hidden_dim) <= _lib.ACT_MAX_DIM
 
     def _act_one(self, states, deterministic, out, stream):
         A = self.action_dim

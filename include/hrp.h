@@ -306,7 +306,10 @@ int hrp_ppo_act_sample_ctr(hrp_ppo *h, const float *params_dev, const float *sta
  * as processes and experiments/multiplex.py batches.  Matrix-vector products in fp32 FMA arithmetic (a cluster of CTAs per
  * policy, weights streamed once); the policies may differ in every dimension.  out_dev[2 * action_dim + 2] receives
  * action = tanh(z), pre_tanh = z, log_prob (0 when deterministic), value.  Sampling: Philox4x32-10 keyed by seed,
- * counter (row, draw), as hrp_ppo_act_sample with row_base + row = `row`.  items is a HOST array. */
+ * counter (row, draw), as hrp_ppo_act_sample with row_base + row = `row`.  items is a HOST array.  state_dim and
+ * hidden_dim must be <= HRP_ACT_MAX_DIM (the activations live in shared memory); wider policies act through the
+ * batched entry points with batch = 1. */
+#define HRP_ACT_MAX_DIM 1024
 typedef struct hrp_act_item {
     const float *params_dev;   /* flat parameter buffer of this policy, ActorCritic.parameters() order */
     const float *state_dev;    /* [state_dim] */
