@@ -1114,7 +1114,8 @@ __global__ void adv_normalize_kernel(float *__restrict__ adv, long long n, const
     if (i >= n) return;
     double cnt = stats[2], mean = stats[0] / cnt;
     double var = (stats[1] - cnt * mean * mean) / (cnt - 1.0);  // torch.std: unbiased
-    float m = (float)mean, sd = (float)sqrt(fmax(var, 0.0));
+    // a cancellation below 0 is clamped; n = 1 gives 0/0 = NaN, as torch.std does (fmax would turn it into 0)
+    float m = (float)mean, sd = (float)sqrt(var < 0.0 ? 0.0 : var);
     adv[i] = (adv[i] - m) / (sd + 1e-8f);
 }
 

@@ -248,7 +248,10 @@ def collect_rollout(vec_env, agent, T: int, obs: Optional[torch.Tensor] = None,
     ac.row_base = int(getattr(vec_env, "env_id_base", 0))
     if use_graph is None:
         # (a single env acts through the matrix-vector kernel, which keeps its draw counter on the host)
-        use_graph = noise is None and E > 1 and getattr(agent, "use_cuda_graphs", True)
+        # (and, with several ranks, only where the agent captures its collectives too, graph_collectives: the
+        # VecNormalize moments all-gather runs inside the rollout, and gloo cannot be captured)
+        use_graph = (noise is None and E > 1 and getattr(agent, "use_cuda_graphs", True)
+                     and (distributed.world_size() == 1 or getattr(agent, "graph_collectives", False)))
     cache = getattr(agent, "_rollout_graph", None)
     boot = bool(bootstrap_truncated)
     key = (getattr(vec_env, "uid", id(vec_env)), getattr(vec_env, "param_version", 0), T, E, S, A, Z,
